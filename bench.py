@@ -4,6 +4,9 @@
     python bench.py --gpus 1 --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus 1 ...            # the reference's CPU path (oracle port) on the host cores
     torchrun --nproc-per-node N ... bench.py --gpus N ...    # one rank per GPU
+    python bench.py ... --dump-outputs DIR                   # also save rank 0's hits of the last timed C2 step as .npy
+
+The inputs are deterministic (camera rays of a fixed scene), so the dumps of two builds can be compared output for output.
 
 Headline workload (BASELINE.json configs[1], "C2"): the 1920x1080 primary-ray closest-hit batch against the bunny BVH
 (4,968 triangles + ground sphere, 9,937 nodes). One step = one pass of the closest-hit path over the batch (2,073,600 rays per
@@ -31,6 +34,7 @@ import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True  # the benchmark leaves the source tree as it found it (no __pycache__ next to the package)
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
@@ -51,7 +55,24 @@ def parse():
     ap.add_argument("--impl", choices=["ours", "reference"], default="ours")
     ap.add_argument("--no-render", action="store_true", help="skip the C1 / C3 / C4 legs")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline legs")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the hits of the last timed C2 step to DIR/hits_{leaf,material,t}.npy (float64)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+def dump_hits(directory, hits):
+    """The closest hits of one pass over the C2 batch, one float64 array per field of the hit record (2,073,600 values each,
+    49.8 MB in all). Leaf and material ids are exact in float64 and a miss has leaf = MISS (4294967295). The hit record's t is
+    +inf on a miss; the dump stores -1 there instead, so that every value is finite (a hit has t >= t_min = 1e-3)."""
+    from rtp_b200 import _abi as A
+
+    os.makedirs(directory, exist_ok=True)
+    miss = hits["leaf"] == A.MISS
+    arrays = {"leaf": hits["leaf"], "material": hits["material"], "t": np.where(miss, -1.0, hits["t"])}
+    for field, values in arrays.items():
+        np.save(os.path.join(directory, f"hits_{field}.npy"), values.astype(np.float64))
 
 
 def dist_env():
@@ -153,8 +174,10 @@ def run_reference(args):
         o.hit_full(rays, threads=cores)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        o.hit_full(rays, threads=cores)
+        hits = o.hit_full(rays, threads=cores)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_hits(args.dump_outputs, hits)
     v = args.steps * N_RAYS / dt / 1e6
     line = {
         "impl": "reference", "metric": "Mrays/s", "value": v, "unit": "Mrays/s", "n_gpus": args.gpus, "steps": args.steps,
@@ -509,6 +532,8 @@ def main():
     ms_max, ms_own = ctx.time_device(c2_step, args.steps, max(args.warmup, 3))
     if sampler:
         sampler.active = False
+    if args.dump_outputs and rank == 0:  # before the legs below overwrite d_hits
+        dump_hits(args.dump_outputs, d_hits.cpu().numpy().view(A.HIT_DTYPE).reshape(-1))
     value = args.steps * N_RAYS * world / (ms_max * 1e-3) / 1e6
     kernel_ms = ms_own / args.steps  # one traversal launch (+ one empty deferred launch) per step, back to back on one stream
     launches_per_step = 2 if scene.info().any_order else 1

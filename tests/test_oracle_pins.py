@@ -77,20 +77,21 @@ def test_asset_invariants():
     assert e.shape == (512, 1024, 4) and (e[..., 3] == 255).all()
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/assets"), reason="reference checkout not present (GPU box)")
-def test_fixture_matches_reference_files_through_both_loaders():
-    for name, mesh in (("bunny", assets.bunny()), ("bunny_flat", assets.bunny_flat())):
-        path = f"/root/reference/assets/{name}.obj"
-        for loader in (oracle.obj_load, api.obj.load):
-            m = loader(path)
-            assert m.vertices.tobytes() == mesh.vertices.tobytes() and (m.indices == mesh.indices).all(), (name, loader)
-    for loader in (oracle.tga_load, api.tga.load):
-        assert loader("/root/reference/assets/earthmap.tga").tobytes() == assets.earthmap().tobytes()
-    # earthmap.tga: 24 bpp, descriptor 0x20 (top origin) → the first stored row lands at j = height-1
-    raw = open("/root/reference/assets/earthmap.tga", "rb").read()
-    assert raw[2] == 2 and raw[16] == 24 and raw[17] == 0x20
-    first_stored = np.frombuffer(raw, dtype=np.uint8, count=3, offset=18)[::-1]
-    assert (assets.earthmap()[511, 0, :3] == first_stored).all()
+def test_fixture_bytes_are_pinned():
+    """data/assets.npz holds the reference's bunny.obj, bunny_flat.obj and earthmap.tga as parsed by the oracle's loaders
+    (tests/golden/make_fixtures.py). The asset files are not part of this repository, so the decoded arrays are pinned by digest:
+    a regenerated or edited fixture shows up here."""
+    import hashlib
+
+    def sha(a):
+        return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+    b, f = assets.bunny(), assets.bunny_flat()
+    assert sha(b.vertices) == "c2e0ae9c2eb0afebc8c06f8fbc28cf60e0ed2a8e9363fbb2dbbb8b627d8019fc"
+    assert sha(b.indices.astype(np.uint32)) == "487804de833654c00a0942bf8414a4f2aef39996fb76a373bf10b23481fd6eb1"
+    assert sha(f.vertices) == "23b3b02298c9475a30973e052edebda96564ad736d09c883392bc2f20a464fcb"
+    assert sha(f.indices.astype(np.uint32)) == "21a7c11a84e8106b716ec70fbde2c056ef4812eea2e62723534ef7efc3a6bf5d"
+    assert sha(assets.earthmap()) == "adbe9f16ab1c382f8fd913f55abc61e356a22766ae82d60a19c9294ff8910831"
 
 
 def test_obj_parser_subset(tmp_path):
