@@ -319,6 +319,10 @@ int rtp_scene_leaf_order(const rtp_scene* scene, uint32_t* leaf_ids_out, size_t 
 /* Host-only half of rtp_scene_create: validates the description, runs `Bvh::new` (bvh.rs:70-91) and
  * reports the leaf ids in depth-first order plus the tree shape, without touching a device. */
 int rtp_bvh_build_order(const rtp_scene_desc* desc, uint32_t* leaf_ids_out, size_t cap, rtp_scene_info* info);
+/* Host-only view of the any-order walk's scene tables: the culled-set box (the union of the boxes of every primitive that is
+ * not big, rounded outward to f32 as the culling tree stores boxes: min xyz, max xyz; +inf / -inf if there is none), the number
+ * of leaves of the order-free culling tree and how many of them are big primitives (0 if there is no such tree). Tests only. */
+int rtp_bvh_culled_set(const rtp_scene_desc* desc, float box_out[6], uint32_t* free_tree_leaves, uint32_t* free_tree_big_leaves);
 
 /* ---------------------------------------------------------------- closest hit ----------- */
 

@@ -192,6 +192,7 @@ PROTOTYPES = {
     "rtp_scene_destroy": (None, [C.c_void_p]),
     "rtp_scene_get_info": (C.c_int, [C.c_void_p, _P(SceneInfo)]),
     "rtp_bvh_build_order": (C.c_int, [_P(SceneDesc), C.c_void_p, C.c_size_t, _P(SceneInfo)]),
+    "rtp_bvh_culled_set": (C.c_int, [_P(SceneDesc), _P(C.c_float), _P(C.c_uint32), _P(C.c_uint32)]),
     "rtp_scene_leaf_order": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t]),
     "rtp_trace_closest": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, _P(Stats)]),
     "rtp_trace_closest_full": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, _P(Stats)]),

@@ -487,6 +487,16 @@ def bvh_build_order(scene: ExampleScene):
     return out[: info.n_leaves], info
 
 
+def bvh_culled_set(scene: ExampleScene):
+    """rtp_bvh_culled_set, host only: (culled-set box as float32 [min xyz, max xyz], leaves of the order-free tree, big ones among them)"""
+    lib = A.load()
+    desc, keep = build_desc(scene)
+    box = (C.c_float * 6)()
+    leaves, big = C.c_uint32(0), C.c_uint32(0)
+    _check(lib, lib.rtp_bvh_culled_set(C.byref(desc), box, C.byref(leaves), C.byref(big)))
+    return np.array(box[:], dtype=np.float32), leaves.value, big.value
+
+
 class PinnedBuffer:
     """Page-locked host array from rtp_host_alloc, exposed as a numpy array."""
 

@@ -372,7 +372,19 @@ __global__ void __launch_bounds__(256) records_kernel(const rtp_hittable* __rest
 struct AnyConsts {
     unsigned long long E, A, C, R, mag;  // bit patterns of non-negative doubles: atomicMax orders them like the values
     unsigned int spheres, _pad;
+    unsigned long long lo[3], hi[3];     // union of the boxes that are not big: ~order_key(min), order_key(max), both by atomicMax
 };
+// a double's bits as an unsigned key that orders like the value (-0 below +0)
+__device__ __forceinline__ unsigned long long order_key(double x) {
+    const unsigned long long u = static_cast<unsigned long long>(__double_as_longlong(x));
+    return (u >> 63) ? ~u : (u | 0x8000000000000000ull);
+}
+static double from_order_key(unsigned long long k) {
+    const unsigned long long u = (k >> 63) ? (k & 0x7FFFFFFFFFFFFFFFull) : ~k;
+    double x;
+    std::memcpy(&x, &u, 8);
+    return x;
+}
 __global__ void __launch_bounds__(256) any_consts_kernel(const DPrim* __restrict__ prims, const rtp_hittable* __restrict__ hs, const double* __restrict__ extent, uint32_t n,
                                                           const uint32_t* __restrict__ big, uint32_t n_big, AnyConsts* __restrict__ out) {
     const uint32_t s = blockIdx.x * blockDim.x + threadIdx.x;
@@ -383,6 +395,7 @@ __global__ void __launch_bounds__(256) any_consts_kernel(const DPrim* __restrict
     atomicMax(&out->mag, static_cast<unsigned long long>(__double_as_longlong(mag)));
     for (uint32_t k = 0; k < n_big; ++k)
         if ((big[k] & 0x7FFFFFFFu) == s) return;
+    for (int k = 0; k < 3; ++k) { atomicMax(&out->lo[k], ~order_key(p.bmin[k])); atomicMax(&out->hi[k], order_key(p.bmax[k])); }
     const bool sphere = hs[p.leaf].kind == RTP_HITTABLE_SPHERE;
     if (sphere) {
         out->spheres = 1u;
@@ -784,6 +797,12 @@ int device_build_scene(const rtp_scene_desc* d, FlatScene* out, bool timing) {
     out->any_C = as_double(hc.C) * (1.0 + 1e-12);
     out->any_R = as_double(hc.R) * (1.0 + 1e-12);
     out->any_spheres = hc.spheres != 0u;
+    {
+        double lo[3], hi[3];
+        for (int k = 0; k < 3; ++k) { lo[k] = from_order_key(~hc.lo[k]); hi[k] = from_order_key(hc.hi[k]); }
+        if (hc.hi[0] == 0ull) lo[0] = 1.0, hi[0] = 0.0;  // every primitive is big: the empty box
+        culled_set_box(lo, hi, out->cull);
+    }
     out->any_ok = out->wide_depth <= 48;
     out->free_depth = 0;
     return RTP_OK;

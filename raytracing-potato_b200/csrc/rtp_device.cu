@@ -1360,7 +1360,8 @@ __global__ void __launch_bounds__(128, OUT == OUT_TAIL ? 4 : kTraceBlocksPerSM) 
 //     of travelling through the tree as window-exempt children: the step carries no big-mask load and no per-child selects,
 //     and the walk starts with the window already closed to the nearest big hit. Testing them first is the same sequential
 //     process (the claim in DESIGN.md 4b does not depend on the order in which leaves are looked at); a big leaf met again in
-//     the tree is skipped (kWideBig);
+//     the rank-ordered tree is skipped (kWideBig), the order-free tree has none. A ray whose window then closes before the
+//     culled-set box (every other leaf) is finished without a walk;
 //   * rays are read with ld.global.nc.L1::no_allocate and results written with st.global.cs: the 80 B/ray stream does not
 //     displace the culling tree from L1.
 // ---------------------------------------------------------------------------------------------
@@ -1632,9 +1633,16 @@ __global__ void __launch_bounds__(128, RTP_ANY_BLOCKS) trace_any_kernel(DSceneVi
                         best = kNoPrim; best_t = tmax;
                         T_win = tmax; T_up = __double2float_ru(tmax);
                         leaf0 = 0u; leaf1 = 0u; sp = sbase;
-                        node = 0u;
                         // the big primitives first, all lanes of the refill together
                         for (uint32_t k = 0; k < sc.n_big; ++k) test_leaf(kWideLeaf | ((sc.big[k] >> 31) << 30) | (sc.big[k] & kWideSlotMask));
+                        // then the culled-set box (every leaf that is not big lies inside it) against the window those tests left, with
+                        // the node test's arithmetic: rejected, the ray is done without a walk (most primary rays of the bunny scenes
+                        // end on the ground sphere in front of the bunny's box)
+                        const float cn = fmaxf(fmaxf(fmaf(sx ? sc.cull[3] : sc.cull[0], ix, clx), fmaf(sy ? sc.cull[4] : sc.cull[1], iy, cly)),
+                                               fmaxf(fmaf(sz ? sc.cull[5] : sc.cull[2], iz, clz), tmin_dn));
+                        const float cf = fminf(fminf(fmaf(sx ? sc.cull[0] : sc.cull[3], ix, chx), fmaf(sy ? sc.cull[1] : sc.cull[4], iy, chy)),
+                                               fminf(fmaf(sz ? sc.cull[2] : sc.cull[5], iz, chz), T_up));
+                        node = cf >= cn ? 0u : kNone;
                     }
                 }
             }
@@ -2175,6 +2183,10 @@ int device_scene_upload(const FlatScene& flat, int device, DeviceScene** out) {
     v.any_Cf = std::nextafter(static_cast<float>(flat.any_C), std::numeric_limits<float>::infinity());
     v.any_Rf = flat.any_spheres ? std::nextafter(static_cast<float>(flat.any_R), std::numeric_limits<float>::infinity()) : -1.0f;
     std::memcpy(v.bg_rgb, flat.background.rgb, sizeof v.bg_rgb);
+    // RTP_ANY_SETUP_CULL=0: a box that every ray enters, so every ray walks (A/B runs of the set-up cull in one process)
+    const char* cv = std::getenv("RTP_ANY_SETUP_CULL");
+    const bool setup_cull = !cv || std::atoi(cv) != 0;
+    for (int k = 0; k < 6; ++k) v.cull[k] = setup_cull ? flat.cull[k] : (k < 3 ? -1.0f : 1.0f) * std::numeric_limits<float>::infinity();
     *out = ds;
     return RTP_OK;
 }
@@ -2697,6 +2709,11 @@ int rtp_scene_digest(const rtp_scene* scene, uint64_t digest_out[4]) {
             hash[i] = h; done[i] = 1;
             levels = std::max(levels, depth_of[i]);
         }
+        if (n_wide) {  // the culled-set box belongs to the culling tree
+            float cull[6];
+            for (int k = 0; k < 6; ++k) cull[k] = ds->view.cull[k] + 0.0f;
+            hash[0] = fnv(hash[0], cull, sizeof cull);
+        }
         digest_out[0] = h0; digest_out[1] = h1; digest_out[2] = n_wide ? hash[0] : 0; digest_out[3] = static_cast<uint64_t>(n_wide) | (static_cast<uint64_t>(levels) << 32);
     } catch (const std::exception& e) {
         return set_error(RTP_ERR_NOMEM, e.what());
@@ -2847,6 +2864,28 @@ int rtp_bvh_build_order(const rtp_scene_desc* desc, uint32_t* leaf_ids_out, size
             info->culling_depth = flat.root_kind == RTP_ROOT_BVH ? flat.wide_depth : 0u;
             info->any_order = flat.any_ok ? 1u : 0u; info->n_big = flat.n_big; info->free_tree_depth = flat.free_depth;
         }
+        return RTP_OK;
+    } catch (const std::exception& e) {
+        return set_error(RTP_ERR_NOMEM, e.what());
+    }
+}
+
+int rtp_bvh_culled_set(const rtp_scene_desc* desc, float box_out[6], uint32_t* free_tree_leaves, uint32_t* free_tree_big_leaves) {
+    if (!box_out || !free_tree_leaves || !free_tree_big_leaves) return set_error(RTP_ERR_INVALID, "null argument");
+    try {
+        FlatScene flat;
+        int rc = flatten_scene(desc, &flat);
+        if (rc != RTP_OK) return rc;
+        std::copy(flat.cull, flat.cull + 6, box_out);
+        uint32_t leaves = 0, big = 0;
+        for (const DWide& w : flat.free_wide)
+            for (int k = 0; k < 4; ++k) {
+                const uint32_t c = w.child[k];
+                if (c == kWideEmpty || !(c & kWideLeaf)) continue;
+                ++leaves;
+                for (uint32_t q = 0; q < flat.n_big; ++q) big += (flat.big[q] & kWideSlotMask) == (c & kWideSlotMask) ? 1u : 0u;
+            }
+        *free_tree_leaves = leaves; *free_tree_big_leaves = big;
         return RTP_OK;
     } catch (const std::exception& e) {
         return set_error(RTP_ERR_NOMEM, e.what());

@@ -207,7 +207,7 @@ struct SeqBuilder {
 // children, in place, until it has four children or only leaves. In-place replacement keeps the children in rank order,
 // so visiting children left to right meets the leaves in the reference's depth-first order.
 // ---------------------------------------------------------------------------------------------
-static void round_out(const double* bmin, const double* bmax, float* lo, float* hi) {
+void round_out(const double* bmin, const double* bmax, float* lo, float* hi) {
     for (int a = 0; a < 3; ++a) {
         const double mag = std::fmax(std::fabs(bmin[a]), std::fabs(bmax[a]));
         const double r = std::ldexp(mag, -21);
@@ -216,6 +216,14 @@ static void round_out(const double* bmin, const double* bmax, float* lo, float* 
         if (static_cast<double>(h) < bmax[a] + r) h = std::nextafterf(h, std::numeric_limits<float>::infinity());
         lo[a] = l; hi[a] = h;
     }
+}
+
+void culled_set_box(const double* lo, const double* hi, float* cull) {
+    if (!(lo[0] <= hi[0])) {
+        for (int a = 0; a < 3; ++a) { cull[a] = std::numeric_limits<float>::infinity(); cull[3 + a] = -std::numeric_limits<float>::infinity(); }
+        return;
+    }
+    round_out(lo, hi, cull, cull + 3);
 }
 
 struct WideBuilder {
@@ -399,14 +407,18 @@ static void prepare_any_order(FlatScene* out) {
         }
     }
     // scene constants of the slack bound (rtp_device.cu any_slack): triangles E, A; spheres C (largest |centre coordinate|, bounded
-    // by the box planes) and R (largest radius) - over the primitives that are not big
+    // by the box planes) and R (largest radius) - over the primitives that are not big; and the union of their boxes, which a ray
+    // must enter within its window to need a walk at all (DSceneView::cull)
     double E = 0.0, A = 0.0, Cs = 0.0, Rs = 0.0;
+    double ulo[3] = {std::numeric_limits<double>::infinity(), std::numeric_limits<double>::infinity(), std::numeric_limits<double>::infinity()};
+    double uhi[3] = {-ulo[0], -ulo[1], -ulo[2]};
     bool spheres = false;
     for (size_t s = 0; s < n; ++s) {
         if (is_big[s]) continue;
         const DPrim& p = out->prims[s];
         double mag = 0.0;
         for (int k = 0; k < 3; ++k) mag = std::fmax(mag, std::fmax(std::fabs(p.bmin[k]), std::fabs(p.bmax[k])));
+        for (int k = 0; k < 3; ++k) { ulo[k] = std::fmin(ulo[k], p.bmin[k]); uhi[k] = std::fmax(uhi[k], p.bmax[k]); }
         if (kind[s] == RTP_HITTABLE_SPHERE) {
             spheres = true;
             Cs = std::fmax(Cs, mag);
@@ -421,17 +433,20 @@ static void prepare_any_order(FlatScene* out) {
     out->any_spheres = spheres;
     out->any_C = Cs * (1.0 + 1e-12);
     out->any_R = Rs * (1.0 + 1e-12);
+    culled_set_box(ulo, uhi, out->cull);
     mark_big(out->wide, is_big);
     out->any_ok = true;
 
     // Free tree. The any-order walk does not need its leaves in the reference's depth-first order (only the re-walk does), so
-    // its lanes may walk a second culling tree built over the MORTON order of the leaf centroids (big primitives first) with
-    // the same SAH-over-a-sequence builder and the same 4-wide collapse; its leaves carry the same slots. Measured: 4-6 %
-    // faster on the bunny (4.06 instead of 4.26 nodes per primary ray, 4 ms of build), no gain on the bunny fields (15.4
-    // instead of 15.6 nodes, 1.5 s of build for 2.5 M leaves) - so only scenes below kFreeTreeLeaves get it by default.
+    // its lanes may walk a second culling tree built over the MORTON order of the leaf centroids with the same SAH-over-a-sequence
+    // builder and the same 4-wide collapse; its leaves carry the same slots. Measured: 4-6 % faster on the bunny (4.06 instead of
+    // 4.26 nodes per primary ray, 4 ms of build), no gain on the bunny fields (15.4 instead of 15.6 nodes, 1.5 s of build for
+    // 2.5 M leaves) - so only scenes below kFreeTreeLeaves get it by default. It holds only the primitives that are not big: those
+    // are tested before the walk starts, and left out the root box no longer spans the ground sphere that every ray enters.
     const char* fv = std::getenv("RTP_FREE_TREE");
     const bool want_free = fv ? std::atoi(fv) != 0 : n < kFreeTreeLeaves;
-    if (!want_free || n < 2) return;
+    const size_t m = n - out->n_big;
+    if (!want_free || n < 2 || m == 0) return;
     double lo[3] = {1e300, 1e300, 1e300}, hi[3] = {-1e300, -1e300, -1e300};
     for (size_t s = 0; s < n; ++s) {
         if (is_big[s]) continue;
@@ -447,7 +462,7 @@ static void prepare_any_order(FlatScene* out) {
     std::vector<std::pair<uint64_t, uint32_t>> keyed(n);
     parallel_chunks(n, [&](size_t a, size_t b) {
         for (size_t s = a; s < b; ++s) {
-            uint64_t key = 0;
+            uint64_t key = 0;  // big primitives sort first and are dropped below
             if (!is_big[s]) {
                 const DPrim& p = out->prims[s];
                 uint64_t q[3];
@@ -462,20 +477,19 @@ static void prepare_any_order(FlatScene* out) {
         }
     });
     std::sort(keyed.begin(), keyed.end());
-    std::vector<BuildItem> seq(n);
-    for (size_t i = 0; i < n; ++i) {
-        const DPrim& p = out->prims[keyed[i].second];
-        seq[i].id = keyed[i].second;
+    std::vector<BuildItem> seq(m);
+    for (size_t i = 0; i < m; ++i) {
+        const DPrim& p = out->prims[keyed[out->n_big + i].second];
+        seq[i].id = keyed[out->n_big + i].second;
         std::memcpy(seq[i].bmin, p.bmin, sizeof p.bmin);
         std::memcpy(seq[i].bmax, p.bmax, sizeof p.bmax);
     }
-    std::vector<DNode> nodes(2 * n - 1);
+    std::vector<DNode> nodes(2 * m - 1);
     SeqBuilder sb{seq, nodes};
-    sb.build(0, n, 0, 1, 4);
+    sb.build(0, m, 0, 1, 4);
     for (DNode& nd : nodes)
         if (nd.prim != kNoPrim) { const uint32_t slot = seq[nd.prim].id; nd.prim = slot; nd.kind = kind[slot]; }
     build_wide(nodes, &out->free_wide, &out->free_boxes, &out->free_depth);
-    mark_big(out->free_wide, is_big);
 }
 
 static bool emit_ok(const rtp_emit& e, uint32_t n_textures) {

@@ -4,6 +4,7 @@
 
 #include <cstddef>
 #include <cstdint>
+#include <limits>
 #include <string>
 #include <vector>
 
@@ -122,6 +123,8 @@ struct DSceneView {  // passed by value to kernels
     double any_A;          // largest |coordinate| of such a triangle
     float any_Ef, any_Af;  // the same, rounded up to f32
     float any_Cf, any_Rf;  // spheres that are not big: largest |centre coordinate| and radius, rounded up; any_Rf < 0: there are none
+    float cull[6];         // culled-set box: the union of the leaf boxes that are not big, rounded out like a DWide child box (min xyz,
+                           // max xyz); a ray whose window closes before it is done after its big-primitive tests. Empty: (+inf, -inf)
 };
 constexpr uint32_t kMaxBig = 8;
 
@@ -167,6 +170,8 @@ struct FlatScene {
     uint32_t big[8] = {0, 0, 0, 0, 0, 0, 0, 0};
     double any_E = 0.0, any_A = 0.0, any_C = 0.0, any_R = 0.0;
     bool any_spheres = false;        // some sphere is not big: the slack bound needs the sphere term
+    float cull[6] = {std::numeric_limits<float>::infinity(), std::numeric_limits<float>::infinity(), std::numeric_limits<float>::infinity(),
+                     -std::numeric_limits<float>::infinity(), -std::numeric_limits<float>::infinity(), -std::numeric_limits<float>::infinity()};  // DSceneView::cull
     double scene_mag = 0.0;    // largest |coordinate| of any node box
     bool boxes_finite = true;  // every box is finite and ordered (min <= max): precondition of the sign-selected slab test, of the
                                // f32 culling walk and of re-shaping the tree; otherwise the reference topology and the literal test are used
@@ -175,6 +180,12 @@ struct FlatScene {
 
 // error plumbing (rtp_host.cpp)
 int set_error(int code, const std::string& msg);
+
+// An exact f64 box as the f32 culling box of a DWide child: rounded outward and inflated by 2^-21 * max(|min|, |max|) per axis
+// (DESIGN.md §4; rtp_host.cpp)
+void round_out(const double* bmin, const double* bmax, float* lo, float* hi);
+// DSceneView::cull of the union [lo, hi] of the leaf boxes that are not big; lo > hi: there are none
+void culled_set_box(const double* lo, const double* hi, float* cull);
 
 // host layer
 // device_build: compute the reference leaf order on the GPU (rtp_build.cu) when the scene is large; host-only callers pass false
