@@ -242,8 +242,8 @@ typedef struct rtp_scene_info {
     uint32_t root_kind;
     uint64_t device_bytes;   /* HBM held by the scene */
     uint32_t culling_depth;  /* levels of the 4-wide culling tree the kernels walk (0 for a List root)            */
-    uint32_t any_order;      /* front-to-back walk: 0 = not used; rtp_scene_get_info: 1 / 2 = kernel build in use;
-                                rtp_bvh_build_order: 1 = the scene is eligible                                     */
+    uint32_t any_order;      /* front-to-back walk: 0 = not used; rtp_scene_get_info: 1 = used, 2 = used on a scene
+                                of >= 262,144 leaves (the same kernel); rtp_bvh_build_order: 1 = the scene is eligible   */
     uint32_t n_big;          /* outsized primitives exempt from distance culling (e.g. a ground sphere), at most 8 */
     uint32_t free_tree_depth;/* levels of the order-free culling tree of the any-order lanes, 0 if there is none  */
 } rtp_scene_info;

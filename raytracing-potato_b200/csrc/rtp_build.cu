@@ -119,22 +119,6 @@ int device_reference_order_dev(const double* d_boxes, uint32_t n, uint32_t* d_or
     return RTP_OK;
 }
 
-int device_reference_order(const double* boxes, uint32_t n, uint32_t* order_out) {
-    double* d_boxes = nullptr;
-    uint32_t* d_order = nullptr;
-    auto cleanup = [&]() { cudaFree(d_boxes); cudaFree(d_order); };
-    if (n == 0) return RTP_OK;
-    if (int rc = ensure_device()) return rc;
-    RTP_CUDA_B(cudaMalloc(reinterpret_cast<void**>(&d_boxes), static_cast<size_t>(n) * 6 * sizeof(double)));
-    RTP_CUDA_B(cudaMalloc(reinterpret_cast<void**>(&d_order), static_cast<size_t>(n) * 4));
-    RTP_CUDA_B(cudaMemcpy(d_boxes, boxes, static_cast<size_t>(n) * 6 * sizeof(double), cudaMemcpyHostToDevice));
-    int rc = device_reference_order_dev(d_boxes, n, d_order);
-    if (rc != RTP_OK) { cleanup(); return rc; }
-    RTP_CUDA_B(cudaMemcpy(order_out, d_order, static_cast<size_t>(n) * 4, cudaMemcpyDeviceToHost));
-    cleanup();
-    return RTP_OK;
-}
-
 }  // namespace rtp
 
 // =================================================================================================================================
@@ -283,7 +267,7 @@ __global__ void __launch_bounds__(256) sah_split_kernel(const Seg* __restrict__ 
     DNode nd;
     const Box6 total = pre[sg.lo + sg.n - 1u];
     for (int a = 0; a < 3; ++a) { nd.bmin[a] = total.lo[a]; nd.bmax[a] = total.hi[a]; }
-    nd.skip = sg.base + 2u * sg.n - 1u; nd.prim = kNoPrim; nd.kind = 0; nd._pad = sg.lo;  // _pad: first slot of the subtree (collapse: big-primitive ranges)
+    nd.skip = sg.base + 2u * sg.n - 1u; nd.prim = kNoPrim; nd.kind = 0; nd._pad = 0;
     nodes[sg.base] = nd;
     uint32_t active = 0;
     const uint32_t child_lo[2] = {sg.lo, sg.lo + k}, child_n[2] = {k, sg.n - k}, child_base[2] = {sg.base + 1u, sg.base + 2u * k};
@@ -292,7 +276,7 @@ __global__ void __launch_bounds__(256) sah_split_kernel(const Seg* __restrict__ 
             DNode lf;
             const Box6 b = ranked[child_lo[c]];
             for (int a = 0; a < 3; ++a) { lf.bmin[a] = b.lo[a]; lf.bmax[a] = b.hi[a]; }
-            lf.skip = child_base[c] + 1u; lf.prim = child_lo[c]; lf.kind = hs[perm[child_lo[c]]].kind; lf._pad = child_lo[c];
+            lf.skip = child_base[c] + 1u; lf.prim = child_lo[c]; lf.kind = hs[perm[child_lo[c]]].kind; lf._pad = 0;
             nodes[child_base[c]] = lf;
         } else {
             ++active;
@@ -483,13 +467,11 @@ __global__ void __launch_bounds__(128) collapse_write_kernel(const DNode* __rest
             float lo[3], hi[3];
             round_out_dev(c.bmin, c.bmax, lo, hi);
             for (int a = 0; a < 3; ++a) { w.plane[a][0][k] = lo[a]; w.plane[a][1][k] = hi[a]; b64[k][a] = c.bmin[a]; b64[k][3 + a] = c.bmax[a]; }
-            // mark_big: the child is, or contains, a big primitive: its slot range [first, first + leaves) holds one of them
-            const uint32_t first = c._pad, leaves = (c.skip - kids[k] + 1u) / 2u;
-            bool has_big = false;
-            for (uint32_t q = 0; q < n_big; ++q) { const uint32_t s = big[q] & 0x7FFFFFFFu; has_big |= s >= first && s < first + leaves; }
-            if (has_big) w.big_mask |= 1u << k;
             if (c.prim != kNoPrim) {
-                w.child[k] = kWideLeaf | (c.kind << 30) | c.prim | (has_big ? kWideBig : 0u);
+                // mark_big: a leaf of one of the big primitives carries kWideBig
+                bool is_big = false;
+                for (uint32_t q = 0; q < n_big; ++q) is_big |= (big[q] & 0x7FFFFFFFu) == c.prim;
+                w.child[k] = kWideLeaf | (c.kind << 30) | c.prim | (is_big ? kWideBig : 0u);
             } else {
                 next[pos] = WideTask{kids[k]};
                 w.child[k] = next_base + pos;

@@ -1048,15 +1048,9 @@ __device__ __noinline__ void trace_deferred(const DSceneView& sc, D3 o, D3 d, Hi
     closest_hit_bvh<false>(sc, o, d, kRayEpsilon, h, lc);
 }
 
-// GEN0: this is segment 0 of a launch whose primary rays were never written to a queue (trace_any_kernel<.., GEN>): the thread
-// regenerates its path's camera ray (same draws, same bits) instead of reading 80 B of ray and state
-#ifndef RTP_SHADE_BLOCKS
-#define RTP_SHADE_BLOCKS 3
-#endif
-template <bool GEN0>
-__global__ void __launch_bounds__(256, RTP_SHADE_BLOCKS) wave_shade_kernel(DSceneView sc, DRender rp, WaveQueues wq, uint32_t bounce, double4* __restrict__ scratch, DCamera cam,
-                                                            size_t n_gen) {
-    const size_t n = GEN0 ? n_gen : static_cast<size_t>(wq.count[bounce]);
+constexpr int kShadeBlocks = 3;  // resident blocks per SM wave_shade_kernel is built for, and its grid
+__global__ void __launch_bounds__(256, kShadeBlocks) wave_shade_kernel(DSceneView sc, DRender rp, WaveQueues wq, uint32_t bounce, double4* __restrict__ scratch) {
+    const size_t n = static_cast<size_t>(wq.count[bounce]);
     const int cur = bounce & 1, nxt = cur ^ 1;
     const unsigned lane = threadIdx.x & 31u;
     const size_t stride = static_cast<size_t>(gridDim.x) * blockDim.x;
@@ -1067,19 +1061,10 @@ __global__ void __launch_bounds__(256, RTP_SHADE_BLOCKS) wave_shade_kernel(DScen
         D3 o = mk(0, 0, 0), d = mk(0, 0, 0);
         uint4 st = make_uint4(0, 0, 0, 0);
         if (q < n) {
-            if (GEN0) {
-                uint32_t gi, gj, gs;
-                path_coords(rp, q, gi, gj, gs);
-                Rng grng;
-                rng_init(grng, rp.seed, gj * rp.width + gi, gs, RTP_RNG_STREAM_PATH);
-                primary_ray(cam, rp, gi, gj, grng, o, d);
-                st = make_uint4(static_cast<uint32_t>(q), grng.k, rp.max_bounce, 0u);
-            } else {
-                const double2* rp2 = reinterpret_cast<const double2*>(wq.rays[cur] + q);
-                const double2 r0 = rp2[0], r1 = rp2[1], r2 = rp2[2];
-                o = mk(r0.x, r0.y, r1.x); d = mk(r1.y, r2.x, r2.y);
-                st = wq.state[cur][q];
-            }
+            const double2* rp2 = reinterpret_cast<const double2*>(wq.rays[cur] + q);
+            const double2 r0 = rp2[0], r1 = rp2[1], r2 = rp2[2];
+            o = mk(r0.x, r0.y, r1.x); d = mk(r1.y, r2.x, r2.y);
+            st = wq.state[cur][q];
             const double2* hp = reinterpret_cast<const double2*>(wq.hits + q);
             const double2 h0 = hp[0], h1 = hp[1];
             uint32_t slotkind = static_cast<uint32_t>(__double2loint(h1.y));
@@ -1151,7 +1136,7 @@ __global__ void __launch_bounds__(256, RTP_SHADE_BLOCKS) wave_shade_kernel(DScen
 // The persistent traversal kernel (state and steps: Walker above). Defined here because its tail mode shades in place.
 // ---------------------------------------------------------------------------------------------
 
-// Tail mode (OUT_TAIL) of the wavefront integrator: when queue `bounce` holds at most `threshold` rays, one launch
+// Tail mode (OUT_TAIL) of the wavefront integrator: when a launch holds at most DeviceScene::tail_threshold paths, one launch
 // carries every surviving path to its end. A lane whose ray is finished shades it in place (shade_vertex) and, if the
 // path scattered, restarts its walker on the scattered ray, so the remaining bounces cost one kernel instead of two
 // launches each, and the culling tree stays warm in L1 across them. Results are the same bits: per path the
@@ -1161,7 +1146,6 @@ struct TailArgs {
     DRender rp;
     double4* scratch;
     uint32_t bounce;
-    uint32_t threshold;
 };
 
 constexpr int kTraceBlocksPerSM = 6;
@@ -1183,7 +1167,7 @@ __global__ void __launch_bounds__(128, OUT == OUT_TAIL ? 4 : kTraceBlocksPerSM) 
         n = static_cast<size_t>(*index.count);
     }
     if (OUT == OUT_TAIL) {
-        if (n == 0 || n > ta.threshold) return;  // the trace/shade pair that follows handles this queue
+        if (n == 0) return;
         rays = ta.q.rays[ta.bounce & 1u];
     }
     uint4 pst = make_uint4(0, 0, 0, 0);  // tail mode: the path state of the lane's ray (WaveQueues::state)
@@ -1347,8 +1331,8 @@ __global__ void __launch_bounds__(128, OUT == OUT_TAIL ? 4 : kTraceBlocksPerSM) 
 }
 
 // ---------------------------------------------------------------------------------------------
-// Pure any-order traversal kernel (DESIGN.md 4b/6). Same walk and the same exactness argument as walker_step_any / any_test
-// above, rebuilt around what the profile of the combined kernel showed (profiles/r01_trace_any_c2.md: 14 % of the executed
+// Pure any-order traversal kernel (DESIGN.md 4b/6). The walk of DESIGN.md 4b (nearest child first, distance culling against a
+// window), built around what the profile of round 1's combined in-order/any-order kernel showed (profiles/r01_trace_any_c2.md: 14 % of the executed
 // instructions were register moves at loop heads, 19 % branch / reconvergence / predicate set-up, 12 % the slab arithmetic):
 //   * one loop with one back edge; lane state is a handful of scalars (node, stack top as a shared-memory ADDRESS, two pending
 //     leaf words), no struct passed by reference through inlined functions with early returns;
@@ -1438,35 +1422,14 @@ __device__ __forceinline__ bool any_slack_of(const DSceneView& sc, D3 o, D3 d, D
     return in_range & (kappa <= 0.25f) & (e_uv <= 0.01f) & (s0f <= 3.0e38f) & (s1f <= 3.0e38f);
 }
 
-#ifndef RTP_ANY_BLOCKS
-#define RTP_ANY_BLOCKS 6  // resident blocks per SM the kernel is built for (register budget 65536 / (128 x blocks))
-#endif
-#ifndef RTP_ANY_STEPS
-#define RTP_ANY_STEPS 2   // walk steps per round of votes
-#endif
-#ifndef RTP_ANY_PREFETCH
-#define RTP_ANY_PREFETCH 2 // L2 prefetch distance of the ray stream, in quarters of (warps of the grid) x (rays per reservation); 0: off
-#endif
-#ifndef RTP_ANY_POPLOOP
-#define RTP_ANY_POPLOOP 2 // stack entries a step may take before it visits a node (1: one per step, as in the first version)
-#endif
-#ifndef RTP_ANY_BRANCHY_PUSH
-#define RTP_ANY_BRANCHY_PUSH 0  // 1: round 2's first version, nested branches around the three pushes
-#endif
-#ifndef RTP_ANY_PICK
-#define RTP_ANY_PICK 1    // 1: a round tests leaves first when more lanes wait for a leaf test than can walk
-#endif
-// GEN (wavefront integrator, segment 0): ray i IS camera path i of the launch (main.rs:70-76: jitter, lens draw, Camera::shoot), made
-// here from (camera, frame parameters) instead of being read from a queue a generate kernel wrote: saves an 80 B/path round trip
-// through HBM and one launch per frame; wave_shade_kernel<GEN0> regenerates the same ray when it shades the vertex.
-struct GenArgs {
-    DCamera cam;
-    DRender rp;
-};
+constexpr int kAnyBlocks = 6;    // resident blocks per SM the kernel is built for (register budget 65536 / (128 x blocks))
+constexpr int kAnySteps = 2;     // walk steps per round of votes
+constexpr int kAnyPrefetch = 2;  // L2 prefetch distance of the ray stream, in quarters of (warps of the grid) x (rays per reservation)
+constexpr int kAnyPopLoop = 2;   // stack entries a step may take before it visits a node (1: one per step, as in the first version)
 
-template <bool COUNT, int OUT, bool GEN>
-__global__ void __launch_bounds__(128, RTP_ANY_BLOCKS) trace_any_kernel(DSceneView sc, const rtp_ray* __restrict__ rays, size_t n, void* __restrict__ out, Counters* counters,
-                                                           WorkQueue* wq, Tuning tune, const unsigned long long* __restrict__ n_dev, DeferList defer, GenArgs gen) {
+template <bool COUNT, int OUT>
+__global__ void __launch_bounds__(128, kAnyBlocks) trace_any_kernel(DSceneView sc, const rtp_ray* __restrict__ rays, size_t n, void* __restrict__ out, Counters* counters,
+                                                       WorkQueue* wq, Tuning tune, const unsigned long long* __restrict__ n_dev, DeferList defer) {
     extern __shared__ __align__(16) uint32_t any_stack[];
     // the launch over the defer list (launch_trace) may be set up while this grid runs: it waits for this grid's completion itself
     asm volatile("griddepcontrol.launch_dependents;");
@@ -1497,7 +1460,7 @@ __global__ void __launch_bounds__(128, RTP_ANY_BLOCKS) trace_any_kernel(DSceneVi
     const int refill_thr = min(tune.refill_min, max(1, lane_cap / 2));
     const float4* __restrict__ tree = reinterpret_cast<const float4*>(sc.any_wide);  // a node = 8 float4: 32-bit indexing (device_scene_upload: < 2^29 nodes)
 
-    // exact test of one leaf in any-order mode (any_test above, on this kernel's scalars)
+    // exact test of one leaf in any-order mode
     auto test_leaf = [&](uint32_t cw) {
         const uint32_t slot = cw & kWideSlotMask, kind = (cw >> 30) & 1u;
         const DPrim* p = sc.prims + slot;
@@ -1579,31 +1542,18 @@ __global__ void __launch_bounds__(128, RTP_ANY_BLOCKS) trace_any_kernel(DSceneVi
                 base = __shfl_sync(0xffffffffu, base, leader);
                 if (base + static_cast<unsigned long long>(cnt) >= n) more = false;
                 const int rank = __popc(free_mask & lt_mask);
-#if RTP_ANY_PREFETCH
-                if (!GEN) {
-                    // the ray stream comes from HBM and the first thing a refill does with a ray is divide by its direction: pull the
-                    // rays some warp will take about one refill from now into L2 (a quarter of the grid's warps x 32 rays up the queue
-                    // per unit of RTP_ANY_PREFETCH). Stateless: the queue is handed out in order, whoever takes them finds them there.
-                    const unsigned long long pf = base + static_cast<unsigned long long>(RTP_ANY_PREFETCH) * (n_warps / 4) * 32ull + static_cast<unsigned>(rank);
-                    if (!busy && rank < cnt && pf < n) asm volatile("prefetch.global.L2 [%0];" ::"l"(rays + pf));
-                }
-#endif
+                // the ray stream comes from HBM and the first thing a refill does with a ray is divide by its direction: pull the
+                // rays some warp will take about one refill from now into L2 (a quarter of the grid's warps x 32 rays up the queue
+                // per unit of kAnyPrefetch). Stateless: the queue is handed out in order, whoever takes them finds them there.
+                const unsigned long long pf = base + static_cast<unsigned long long>(kAnyPrefetch) * (n_warps / 4) * 32ull + static_cast<unsigned>(rank);
+                if (!busy && rank < cnt && pf < n) asm volatile("prefetch.global.L2 [%0];" ::"l"(rays + pf));
                 const uint32_t i = (!busy && rank < cnt && base + static_cast<unsigned>(rank) < n) ? static_cast<uint32_t>(base) + static_cast<uint32_t>(rank) : 0xFFFFFFFFu;
                 if (i != 0xFFFFFFFFu) {
-                    double tmax;
-                    if (GEN) {
-                        uint32_t gi, gj, gs;
-                        path_coords(gen.rp, i, gi, gj, gs);
-                        Rng grng;
-                        rng_init(grng, gen.rp.seed, gj * gen.rp.width + gi, gs, RTP_RNG_STREAM_PATH);
-                        primary_ray(gen.cam, gen.rp, gi, gj, grng, o, d);
-                        tmin = kRayEpsilon; tmax = CUDART_INF;
-                    } else {
-                        const double* rp = reinterpret_cast<const double*>(rays + i);
-                        const double2 r0 = ldg_stream2(rp), r1 = ldg_stream2(rp + 2), r2 = ldg_stream2(rp + 4), r3 = ldg_stream2(rp + 6);
-                        o = mk(r0.x, r0.y, r1.x); d = mk(r1.y, r2.x, r2.y);
-                        tmin = r3.x; tmax = r3.y;
-                    }
+                    const double* rp = reinterpret_cast<const double*>(rays + i);
+                    const double2 r0 = ldg_stream2(rp), r1 = ldg_stream2(rp + 2), r2 = ldg_stream2(rp + 4), r3 = ldg_stream2(rp + 6);
+                    o = mk(r0.x, r0.y, r1.x); d = mk(r1.y, r2.x, r2.y);
+                    tmin = r3.x;
+                    const double tmax = r3.y;
                     const D3 inv = mk(1.0 / d.x, 1.0 / d.y, 1.0 / d.z);  // utility.rs:71-77 Ray::expand
                     float s0f, s1f;
                     // eligibility: finite origin, 1e-15 <= |1/d| <= 1e15 on every axis, |o| <= 1e15 and a self-consistent slack
@@ -1662,23 +1612,21 @@ __global__ void __launch_bounds__(128, RTP_ANY_BLOCKS) trace_any_kernel(DSceneVi
         // ---- which phase: when more lanes wait for a leaf test than can walk, test leaves first (incoherent rays: a few long walks
         //      would otherwise run at a handful of lanes while most of the warp waits for its primitive tests) ---------------------
         bool leaf_first = false;
-#if RTP_ANY_PICK
         {
             const int n_walk = __popc(__ballot_sync(0xffffffffu, (leaf1 == 0u) & ((node != kNone) | (sp != sbase))));
             const int n_leaf = __popc(__ballot_sync(0xffffffffu, leaf0 != 0u));
             leaf_first = n_leaf >= tune.prim_batch && n_leaf > n_walk;
         }
-#endif
         // ---- walk: up to two steps per round ----------------------------------------------------------------------------------
         if (!leaf_first) {
 #pragma unroll
-        for (int rep = 0; rep < RTP_ANY_STEPS; ++rep) {
+        for (int rep = 0; rep < kAnySteps; ++rep) {
             if ((leaf1 == 0u) & ((node != kNone) | (sp != sbase))) {
                 // take postponed entries until one gives a node to visit: leaves go to the pending pair, entries beyond the window are
                 // dropped. (One entry per step left half of the step slots of incoherent rays without a node: RTP_LANE_STATS; an
-                // unbounded loop runs its late iterations for three or four lanes: RTP_ANY_POPLOOP bounds the pops per step.)
+                // unbounded loop runs its late iterations for three or four lanes: kAnyPopLoop bounds the pops per step.)
 #pragma unroll 1
-                for (int pops = 0; pops < RTP_ANY_POPLOOP && ((node == kNone) & (sp != sbase) & (leaf1 == 0u)); ++pops) {
+                for (int pops = 0; pops < kAnyPopLoop && ((node == kNone) & (sp != sbase) & (leaf1 == 0u)); ++pops) {
                     sp -= kAnyStride;
                     const uint2 e = lds_v2(sp);
                     const bool inside = __uint_as_float(e.y) <= T_up;  // else: the window shrank since this entry was postponed
@@ -1722,20 +1670,6 @@ __global__ void __launch_bounds__(128, RTP_ANY_BLOCKS) trace_any_kernel(DSceneVi
                     const uint32_t s1 = min(m0, m1), s2 = max(m0, m1);
 #define RTP_SEL(k) (((k) & 2u) ? (((k) & 1u) ? ch.w : ch.z) : (((k) & 1u) ? ch.y : ch.x))
                     node = kNone;
-#if RTP_ANY_BRANCHY_PUSH
-                    if (s1 != 0xFFFFFFFFu) {  // the keys are sorted: without a second child there is no third or fourth
-                        if (sp > slimit) {
-                            // no room to postpone three children: give the ray to the in-order kernel
-                            sts_u32(cold + 3u * kColdStride, __float_as_uint(-CUDART_INF_F)); sp = sbase; leaf0 = 0u; leaf1 = 0u; s0 = 0xFFFFFFFFu;
-                        } else {
-                            if (s2 != 0xFFFFFFFFu) {
-                                if (s3 != 0xFFFFFFFFu) { sts_v2(sp, RTP_SEL(s3), s3 & ~3u); sp += kAnyStride; }
-                                sts_v2(sp, RTP_SEL(s2), s2 & ~3u); sp += kAnyStride;
-                            }
-                            sts_v2(sp, RTP_SEL(s1), s1 & ~3u); sp += kAnyStride;
-                        }
-                    }
-#else
                     {
                         // the three farther children, farthest first, without branches: every lane writes its three candidate entries
                         // at consecutive positions and advances the stack top only past the ones that exist (the keys are sorted:
@@ -1752,7 +1686,6 @@ __global__ void __launch_bounds__(128, RTP_ANY_BLOCKS) trace_any_kernel(DSceneVi
                             sp = a1 + (p1 ? kAnyStride : 0u);
                         }
                     }
-#endif
                     {   // the nearest child: a node is visited next, a leaf joins the pending pair; selects only
                         const uint32_t c = RTP_SEL(s0);
                         const bool valid = s0 != 0xFFFFFFFFu, is_leaf = (c & kWideLeaf) != 0u, first = leaf0 == 0u;
@@ -1880,7 +1813,7 @@ __global__ void __launch_bounds__(256) srgb8_kernel(const double4* __restrict__ 
 // ---------------------------------------------------------------------------------------------
 
 constexpr int kPipeDepth = 3;
-constexpr size_t kAnyOrderBigScene = 262144;  // leaves from which the 4-blocks-per-SM variant is used
+constexpr size_t kAnyOrderBigScene = 262144;  // leaves from which rtp_scene_info.any_order reports 2 (the kernel is the same)
 constexpr unsigned kQueueSlots = 64;
 constexpr unsigned kLaunchSlots = 8;
 static size_t chunk_rays() {  // rays per pipeline stage: 2^18 (16 MiB of rays) unless RTP_CHUNK_LOG2 says otherwise (tuning runs)
@@ -1949,13 +1882,8 @@ struct DeviceScene {
     uint32_t wave_bounces = 0;         // stack depth the queues were sized for
     int shade_blocks = 0;              // grid of wave_shade_kernel
     uint32_t tail_threshold = 65536;   // RTP_TAIL_THRESHOLD: a launch this small is finished by one tail-mode launch (0 = never)
-    bool tail_offer = false;           // RTP_TAIL_OFFER
     size_t queue_budget_bytes = size_t(4) << 30;  // memory the integrator's per-launch buffers may take (set at upload from the free HBM)
     bool use_simple_render = false;    // RTP_RENDER_KERNEL=simple
-    bool no_fused_gen = true;          // RTP_FUSED_GEN=1: primary rays made inside the first traversal launch instead of by a generate kernel.
-                                       // Measured SLOWER (C1 2.01 vs 1.93 ms, C4 3.49 vs 3.39 ms/frame): the traversal kernel is bound by instruction
-                                       // issue, so ~250 more instructions per path (Philox, lens loop, normalise) in it and again in the shade kernel
-                                       // cost more than the 80 B/path round trip through HBM they save. Kept for A/B runs.
     bool debug_sync = false;           // RTP_DEBUG_SYNC
     double* frame = nullptr; size_t frame_elems = 0;
     uchar4* frame8 = nullptr; size_t frame8_elems = 0;  // RGBA8 output stage
@@ -2071,7 +1999,7 @@ int device_scene_upload(const FlatScene& flat, int device, DeviceScene** out) {
         if (tv && std::string(tv) == "any") want = true;
         if (tv && std::string(tv) == "inorder") want = false;
         if (const char* v = std::getenv("RTP_F32_CULLING")) if (std::atoi(v) == 0) want = false;
-        // scenes that live in HBM rather than in the caches run the spill-free 4-blocks-per-SM build of the kernel
+        // 2 marks a big scene in rtp_scene_info only: every any-order scene runs the same trace_any_kernel
         ds->any_order = (want && flat.any_ok && f32_ok) ? (flat.prim_count() >= kAnyOrderBigScene ? 2 : 1) : 0;
     }
     if (flat.dev.valid) {
@@ -2124,32 +2052,29 @@ int device_scene_upload(const FlatScene& flat, int device, DeviceScene** out) {
             if (const char* v = std::getenv("RTP_ANY_CAP")) ds->any_cap = static_cast<uint32_t>(std::max(4, std::min(48, std::atoi(v))));  // tests
             ds->any_stack_bytes = static_cast<size_t>(ds->any_cap) * 128 * sizeof(uint2) + kAnyColdBytes;  // the stacks, then the cold state
             if (ds->any_stack_bytes > 48u * 1024u) {  // deep trees: above the default limit of dynamic shared memory, every instantiation that is launched
-#define RTP_ANY_SMEM(C, O, G) if (e == cudaSuccess) e = cudaFuncSetAttribute(trace_any_kernel<C, O, G>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(ds->any_stack_bytes))
-                RTP_ANY_SMEM(false, OUT_HIT, false); RTP_ANY_SMEM(true, OUT_HIT, false); RTP_ANY_SMEM(false, OUT_FULL, false); RTP_ANY_SMEM(true, OUT_FULL, false);
-                RTP_ANY_SMEM(false, OUT_WAVE, false); RTP_ANY_SMEM(true, OUT_WAVE, false); RTP_ANY_SMEM(false, OUT_WAVE, true); RTP_ANY_SMEM(true, OUT_WAVE, true);
+#define RTP_ANY_SMEM(C, O) if (e == cudaSuccess) e = cudaFuncSetAttribute(trace_any_kernel<C, O>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(ds->any_stack_bytes))
+                RTP_ANY_SMEM(false, OUT_HIT); RTP_ANY_SMEM(true, OUT_HIT); RTP_ANY_SMEM(false, OUT_FULL); RTP_ANY_SMEM(true, OUT_FULL);
+                RTP_ANY_SMEM(false, OUT_WAVE); RTP_ANY_SMEM(true, OUT_WAVE);
 #undef RTP_ANY_SMEM
             }
-            if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&any_per_sm, trace_any_kernel<false, OUT_HIT, false>, 128, ds->any_stack_bytes);
+            if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&any_per_sm, trace_any_kernel<false, OUT_HIT>, 128, ds->any_stack_bytes);
             ds->any_blocks = prop.multiProcessorCount * std::max(any_per_sm, 1);
         }
         size_t free_b = 0, total_b = 0;
         if (e == cudaSuccess && cudaMemGetInfo(&free_b, &total_b) == cudaSuccess)
             ds->queue_budget_bytes = std::max<size_t>(size_t(1) << 30, std::min<size_t>(size_t(24) << 30, free_b / 6));
-        ds->shade_blocks = prop.multiProcessorCount * RTP_SHADE_BLOCKS;
+        ds->shade_blocks = prop.multiProcessorCount * kShadeBlocks;
         if (const char* v = std::getenv("RTP_BUILD_TIMING")) if (std::atoi(v) != 0)
             std::fprintf(stderr, "[rtp build] 4-wide tree depth %u (order-free tree: %u), %s walk (%u big primitives), %zu B of stack per block, %d traversal blocks per SM\n",
                          flat.wide_depth, flat.free_depth, ds->any_order ? "any-order" : "in-order", flat.n_big,
                          ds->any_order ? ds->any_stack_bytes : ds->stack_bytes, ds->any_order ? any_per_sm : per_sm);
         if (const char* v = std::getenv("RTP_TAIL_THRESHOLD")) ds->tail_threshold = static_cast<uint32_t>(std::max(0l, std::atol(v)));
-        if (const char* v = std::getenv("RTP_TAIL_OFFER")) ds->tail_offer = std::atoi(v) != 0;
         const char* env = std::getenv("RTP_TRACE_KERNEL");
         ds->use_simple_kernel = env && std::string(env) == "simple";
         env = std::getenv("RTP_RENDER_KERNEL");
         ds->use_simple_render = env && std::string(env) == "simple";
         env = std::getenv("RTP_DEBUG_SYNC");
         ds->debug_sync = env && std::atoi(env) != 0;
-        env = std::getenv("RTP_FUSED_GEN");
-        ds->no_fused_gen = !(env && std::atoi(env) != 0);
         if (const char* v = std::getenv("RTP_REFILL_MIN")) ds->tune.refill_min = std::max(1, std::min(32, std::atoi(v)));
         if (const char* v = std::getenv("RTP_PRIM_BATCH")) ds->tune.prim_batch = std::max(1, std::min(32, std::atoi(v)));
         if (const char* v = std::getenv("RTP_FAST_SLAB")) ds->tune.fast_slab = std::atoi(v) != 0;
@@ -2211,7 +2136,7 @@ static int debug_sync(const DeviceScene* ds, cudaStream_t st, const char* what, 
 }
 
 static int launch_trace(DeviceScene* ds, const rtp_ray* d_rays, size_t n, void* d_out, int out_mode, bool count, Counters* counters,
-                        cudaStream_t stream, const unsigned long long* n_dev = nullptr, const TailArgs* tail = nullptr, const GenArgs* gen = nullptr) {
+                        cudaStream_t stream, const unsigned long long* n_dev = nullptr, const TailArgs* tail = nullptr) {
     if (n == 0) return RTP_OK;
     const unsigned block = 128;
     ds->last_trace_launches = 1;
@@ -2262,12 +2187,10 @@ static int launch_trace(DeviceScene* ds, const rtp_ray* d_rays, size_t n, void* 
         if (pure_any) {
             const dim3 g(static_cast<unsigned>(std::min<size_t>(static_cast<size_t>(ds->any_blocks), want)));
             const DeferList defer{slot.defer_idx, slot.defer_count};
-            const GenArgs ga = gen ? *gen : GenArgs{};
-#define RTP_LAUNCH_ANY(C, O, G) trace_any_kernel<C, O, G><<<g, block, ds->any_stack_bytes, stream>>>(ds->view, d_rays, n, d_out, counters, wq, ds->tune, n_dev, defer, ga)
-            if (out_mode == OUT_FULL) { if (count) RTP_LAUNCH_ANY(true, OUT_FULL, false); else RTP_LAUNCH_ANY(false, OUT_FULL, false); }
-            else if (out_mode == OUT_WAVE && gen) { if (count) RTP_LAUNCH_ANY(true, OUT_WAVE, true); else RTP_LAUNCH_ANY(false, OUT_WAVE, true); }
-            else if (out_mode == OUT_WAVE) { if (count) RTP_LAUNCH_ANY(true, OUT_WAVE, false); else RTP_LAUNCH_ANY(false, OUT_WAVE, false); }
-            else { if (count) RTP_LAUNCH_ANY(true, OUT_HIT, false); else RTP_LAUNCH_ANY(false, OUT_HIT, false); }
+#define RTP_LAUNCH_ANY(C, O) trace_any_kernel<C, O><<<g, block, ds->any_stack_bytes, stream>>>(ds->view, d_rays, n, d_out, counters, wq, ds->tune, n_dev, defer)
+            if (out_mode == OUT_FULL) { if (count) RTP_LAUNCH_ANY(true, OUT_FULL); else RTP_LAUNCH_ANY(false, OUT_FULL); }
+            else if (out_mode == OUT_WAVE) { if (count) RTP_LAUNCH_ANY(true, OUT_WAVE); else RTP_LAUNCH_ANY(false, OUT_WAVE); }
+            else { if (count) RTP_LAUNCH_ANY(true, OUT_HIT); else RTP_LAUNCH_ANY(false, OUT_HIT); }
 #undef RTP_LAUNCH_ANY
             RTP_CUDA(cudaGetLastError());
             if (out_mode == OUT_WAVE) {
@@ -2512,43 +2435,32 @@ static int render_enqueue(DeviceScene* ds, const rtp_camera* camera, const rtp_r
         if (wave) {
             // generate -> (trace -> shade) x max_bounce; queue sizes stay on the device
             RTP_CUDA(cudaMemsetAsync(ds->wave.count, 0, 130 * sizeof(unsigned long long), st));
-            // segment 0 without a generate kernel: the pure any-order kernel makes its primary rays itself (GenArgs) and the shade
-            // kernel regenerates them; other scenes (List roots, in-order walk) and tail-mode launches read them from queue 0
-            const bool fused_gen = ds->view.root_kind == RTP_ROOT_BVH && ds->any_order && !ds->no_fused_gen &&
-                                   !(ds->tail_threshold && total <= ds->tail_threshold);
-            const GenArgs ga{cam, rp};
-            if (!fused_gen) {
-                wave_generate_kernel<<<static_cast<unsigned>((total + 255) / 256), 256, 0, st>>>(cam, rp, ds->wave, total);
-                RTP_CUDA(cudaGetLastError());
-                ++launches;
-                { int rc = debug_sync(ds, st, "wave_generate_kernel", 0); if (rc != RTP_OK) return rc; }
-            }
+            wave_generate_kernel<<<static_cast<unsigned>((total + 255) / 256), 256, 0, st>>>(cam, rp, ds->wave, total);
+            RTP_CUDA(cudaGetLastError());
+            ++launches;
+            { int rc = debug_sync(ds, st, "wave_generate_kernel", 0); if (rc != RTP_OK) return rc; }
             const unsigned shade_grid = static_cast<unsigned>(std::min<size_t>(static_cast<size_t>(ds->shade_blocks), (total + 255) / 256));
             for (uint32_t b = 0; b < p->max_bounce; ++b) {
                 int rc;
                 // a launch of at most tail_threshold paths (a 32x32 tile of main.rs:32, say) runs as generate + ONE tail-mode launch.
-                // RTP_TAIL_OFFER=1 also offers every later queue of a big launch to the tail kernel, which declines the ones above
-                // the threshold; measured on C1 it is no faster than trace/shade pairs, and neither is handing the sparse late bounces
-                // to one tail launch chosen from the previous launch's queue sizes (19 -> 12 launches per C1 frame, same 2.05 ms):
-                // a late bounce costs the latency of ONE ray segment (~30 us of dependent instructions, tools/small_batches.py),
-                // not a launch.
-                const bool tail_certain = total <= ds->tail_threshold;
+                // Offering every later queue of a big launch to the tail kernel was measured on C1 to be no faster than trace/shade
+                // pairs, and so was handing the sparse late bounces to one tail launch chosen from the previous launch's queue sizes
+                // (19 -> 12 launches per C1 frame, same 2.05 ms): a late bounce costs the latency of ONE ray segment (~30 us of
+                // dependent instructions, tools/small_batches.py), not a launch.
                 if (want_stats) next_mark(ds, st);  // even marks open a traversal span, odd marks close it
-                if (ds->tail_threshold && (tail_certain || (ds->tail_offer && b > 0))) {
-                    TailArgs ta{ds->wave, rp, ds->scratch, b, ds->tail_threshold};
+                if (ds->tail_threshold && total <= ds->tail_threshold) {
+                    TailArgs ta{ds->wave, rp, ds->scratch, b};
                     rc = launch_trace(ds, ds->wave.rays[b & 1], total, nullptr, OUT_TAIL, count, ds->counters, st, ds->wave.count + b, &ta);
                     if (rc != RTP_OK) return rc;
                     ++launches;
-                    if (tail_certain) { if (want_stats) next_mark(ds, st); break; }
+                    if (want_stats) next_mark(ds, st);
+                    break;
                 }
-                const bool gen0 = fused_gen && b == 0;
-                rc = launch_trace(ds, ds->wave.rays[b & 1], total, ds->wave.hits, OUT_WAVE, count, ds->counters, st, gen0 ? nullptr : ds->wave.count + b, nullptr,
-                                  gen0 ? &ga : nullptr);
+                rc = launch_trace(ds, ds->wave.rays[b & 1], total, ds->wave.hits, OUT_WAVE, count, ds->counters, st, ds->wave.count + b);
                 if (rc != RTP_OK) return rc;
                 if (want_stats) next_mark(ds, st);
                 if ((rc = debug_sync(ds, st, "trace kernel <OUT_WAVE>", b)) != RTP_OK) return rc;
-                if (gen0) wave_shade_kernel<true><<<shade_grid, 256, 0, st>>>(ds->view, rp, ds->wave, b, ds->scratch, cam, total);
-                else wave_shade_kernel<false><<<shade_grid, 256, 0, st>>>(ds->view, rp, ds->wave, b, ds->scratch, cam, 0);
+                wave_shade_kernel<<<shade_grid, 256, 0, st>>>(ds->view, rp, ds->wave, b, ds->scratch);
                 RTP_CUDA(cudaGetLastError());
                 if ((rc = debug_sync(ds, st, "wave_shade_kernel", b)) != RTP_OK) return rc;
                 launches += ds->last_trace_launches + 1;
@@ -2681,7 +2593,7 @@ int rtp_scene_digest(const rtp_scene* scene, uint64_t digest_out[4]) {
         }
         std::vector<DWide> wide(n_wide);
         if (n_wide) RTP_CUDA(cudaMemcpy(wide.data(), ds->wide, n_wide * sizeof(DWide), cudaMemcpyDeviceToHost));
-        // post-order over the tree from node 0: a node's hash folds its planes, its mask and, per child, the leaf word or the child's hash
+        // post-order over the tree from node 0: a node's hash folds its planes and, per child, the leaf word or the child's hash
         std::vector<uint64_t> hash(n_wide, 0);
         std::vector<uint8_t> done(n_wide, 0);
         std::vector<uint32_t> stack;
@@ -2700,7 +2612,6 @@ int rtp_scene_digest(const rtp_scene* scene, uint64_t digest_out[4]) {
             float planes[24];
             for (int k = 0; k < 24; ++k) planes[k] = (&wide[i].plane[0][0][0])[k] + 0.0f;
             uint64_t h = fnv(0xCBF29CE484222325ull, planes, sizeof planes);
-            h = fnv(h, &wide[i].big_mask, 4);
             for (int k = 0; k < 4; ++k) {
                 const uint32_t c = wide[i].child[k];
                 const uint64_t v = (c & kWideLeaf) ? static_cast<uint64_t>(c) : hash[c];

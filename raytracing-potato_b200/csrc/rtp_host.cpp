@@ -66,7 +66,6 @@ struct Builder {
     std::vector<BuildItem>& items;
     std::vector<DNode>& nodes;
     std::atomic<uint32_t> depth{0};
-    bool presorted = false;  // `items` are already in DFS-rank order (device_reference_order): build boxes only
 
     // bvh.rs:36-56 make_bvh + bvh.rs:58-67 split, writing nodes straight into pre-order position.
     // A range of n leaves occupies 2n-1 consecutive nodes starting at `base`; the left half
@@ -87,7 +86,7 @@ struct Builder {
             nd.kind = 0;  // filled by the caller once primitives are laid out
             return;
         }
-        if (!presorted) std::sort(items.begin() + lo, items.begin() + lo + n, [axis](const BuildItem& x, const BuildItem& y) {
+        std::sort(items.begin() + lo, items.begin() + lo + n, [axis](const BuildItem& x, const BuildItem& y) {
             double kx = 0.5 * (x.bmin[axis] + x.bmax[axis]);
             double ky = 0.5 * (y.bmin[axis] + y.bmax[axis]);
             if (kx != ky) return kx < ky;
@@ -352,29 +351,19 @@ static void build_wide(const std::vector<DNode>& bn, std::vector<DWide>* out_wid
     }
 }
 
-// Scene-side preparation of the any-order walk (rtp_device.cu walker_step_any, DESIGN.md §4b). Distance culling is exact only
+// Scene-side preparation of the any-order walk (rtp_device.cu trace_any_kernel, DESIGN.md §4b). Distance culling is exact only
 // with a bound on how far a primitive's computed t (hittable.rs:51-57, 85-95) can fall below the computed slab entry of its own
 // box; that bound grows with the primitive's extent (a triangle's edges, a sphere's |o - c|^2 - r^2 cancellation), so the
 // outsized primitives of a scene - the ground sphere of the bunny scenes, a floor made of two huge triangles - are taken out
-// of the culled set: up to kMaxBig "big" primitives are exempt from distance culling and tested whenever the ray enters
-// their box. A tree too deep for the shared-memory stack, or irregular boxes, and the scene keeps the in-order walk.
+// of the culled set: up to kMaxBig "big" primitives are tested when the ray starts, before its walk, and skipped when the walk
+// meets their leaves. A tree too deep for the shared-memory stack, or irregular boxes, and the scene keeps the in-order walk.
 constexpr size_t kFreeTreeLeaves = 262144;  // scenes below this size get the second, order-free culling tree
 
-// children are appended after their parents (build_wide), so one backward sweep propagates "contains a big primitive" upwards
+// the leaf words of the big primitives carry kWideBig: the walk skips them
 static void mark_big(std::vector<DWide>& wide, const std::vector<uint8_t>& is_big) {
-    std::vector<uint8_t> has_big(wide.size(), 0);
-    for (size_t i = wide.size(); i-- > 0;) {
-        DWide& w = wide[i];
-        w.big_mask = 0;
-        for (int k = 0; k < 4; ++k) {
-            const uint32_t c = w.child[k];
-            if (c == kWideEmpty) continue;
-            const bool big = (c & kWideLeaf) ? is_big[c & kWideSlotMask] != 0 : (c > i ? has_big[c] != 0 : true);
-            if (big) w.big_mask |= 1u << k;
-            if (big && (c & kWideLeaf)) w.child[k] |= kWideBig;
-        }
-        has_big[i] = w.big_mask != 0;
-    }
+    for (DWide& w : wide)
+        for (uint32_t& c : w.child)
+            if (c != kWideEmpty && (c & kWideLeaf) && is_big[c & kWideSlotMask]) c |= kWideBig;
 }
 
 static void prepare_any_order(FlatScene* out) {
@@ -768,22 +757,6 @@ int flatten_scene(const rtp_scene_desc* d, FlatScene* out, bool device_build) {
         out->nodes.assign(static_cast<size_t>(2) * n - 1, DNode{});
         lap("tables, validation, leaf boxes");
         Builder b{items, out->nodes};
-        const char* dev_env = std::getenv("RTP_DEVICE_ORDER");  // "1": only the reference ORDER on the device (round 1's first stage; tests keep it alive)
-        const bool on_device = device_build && dev_env && std::atoi(dev_env) != 0;
-        if (on_device) {
-            // bvh.rs:36-67 on the GPU: one segmented sort of all leaves per depth (rtp_build.cu), then the boxes bottom-up here
-            std::vector<double> boxes(static_cast<size_t>(n) * 6);
-            for (uint32_t i = 0; i < n; ++i)
-                for (int k = 0; k < 3; ++k) { boxes[6 * static_cast<size_t>(i) + k] = items[i].bmin[k]; boxes[6 * static_cast<size_t>(i) + 3 + k] = items[i].bmax[k]; }
-            std::vector<uint32_t> order(n);
-            int rc = device_reference_order(boxes.data(), n, order.data());
-            if (rc != RTP_OK) return rc;
-            std::vector<BuildItem> sorted(n);
-            for (uint32_t r = 0; r < n; ++r) sorted[r] = items[order[r]];
-            items.swap(sorted);
-            b.presorted = true;
-            lap("reference order on the device (segmented radix sorts)");
-        }
         b.build(0, n, 0, 0, 1, 4);  // sorts `items` into the reference's DFS-rank order
         lap("reference median-split order (Bvh::new)");
         out->depth = b.depth.load();

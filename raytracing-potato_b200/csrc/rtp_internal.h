@@ -63,8 +63,7 @@ constexpr uint32_t kWideEmpty = 0xFFFFFFFFu;
 struct alignas(128) DWide {  // 128 B = one L1/L2 line
     float plane[3][2][4];    // [axis][0 = min, 1 = max][child]
     uint32_t child[4];
-    uint32_t big_mask;       // bit k: child k is, or contains, one of the scene's "big" primitives (any-order walk: exempt from distance culling)
-    uint32_t _pad[3];
+    uint32_t _pad[4];
 };
 static_assert(sizeof(DWide) == 128, "DWide must be 128 bytes");
 
@@ -188,14 +187,14 @@ void round_out(const double* bmin, const double* bmax, float* lo, float* hi);
 void culled_set_box(const double* lo, const double* hi, float* cull);
 
 // host layer
-// device_build: compute the reference leaf order on the GPU (rtp_build.cu) when the scene is large; host-only callers pass false
+// device_build: build a large flat Bvh scene on the GPU (rtp_build.cu device_build_scene); host-only callers pass false
 int flatten_scene(const rtp_scene_desc* desc, FlatScene* out, bool device_build = false);
 
 // device layer (rtp_device.cu, rtp_build.cu)
 struct DeviceScene;
 int ensure_device();  // binds device 0 if rtp_init has not been called; RTP_ERR_CUDA without a usable sm_100 GPU
-int device_reference_order(const double* boxes /* n x {min xyz, max xyz} */, uint32_t n, uint32_t* order_out /* item index by DFS rank */);
-int device_reference_order_dev(const double* d_boxes, uint32_t n, uint32_t* d_order_out);  // the same with device pointers
+// the reference's leaf order on the device: d_boxes n x {min xyz, max xyz}, d_order_out item index by DFS rank (device pointers)
+int device_reference_order_dev(const double* d_boxes, uint32_t n, uint32_t* d_order_out);
 // The whole of flatten_scene's geometry part on the current device for a flat (un-nested) Bvh scene: leaf boxes, the reference's
 // depth-first order, the SAH culling tree over that order, primitive / attribute records, the 4-wide collapse and the any-order
 // tables. Fills out->dev and the host-side metadata. Returns RTP_OK, a negative status, or 1 = "not applicable, use the host

@@ -286,19 +286,17 @@ def test_wavefront_equals_one_thread_per_path_integrator(gpu, monkeypatch, name,
 
 
 def test_tail_mode_equals_wavefront(gpu, monkeypatch):
-    """small launches finish in ONE tail-mode launch of the traversal kernel (shading in place); with RTP_TAIL_OFFER the
-    same kernel also takes over the late, small queues of a big launch. Both must return the bits of the trace/shade pairs."""
+    """small launches finish in ONE tail-mode launch of the traversal kernel (shading in place); it must return the bits of
+    the trace/shade pairs."""
     sc = scenes.demo()
     monkeypatch.setenv("RTP_TAIL_THRESHOLD", "0")
     g0 = api.Scene(sc)
     ref, fref, sref = g0.render(200, 120, 3, max_bounce=8, seed=11)
-    for thr, offer in (("1000000", "0"), ("20000", "1"), ("3000", "1")):
-        monkeypatch.setenv("RTP_TAIL_THRESHOLD", thr)
-        monkeypatch.setenv("RTP_TAIL_OFFER", offer)
-        g = api.Scene(sc)
-        img, fg, st = g.render(200, 120, 3, max_bounce=8, seed=11)
-        assert img.tobytes() == ref.tobytes() and fg.tobytes() == fref.tobytes() and st.rays == sref.rays, (thr, offer)
-        g.close()
+    monkeypatch.setenv("RTP_TAIL_THRESHOLD", "1000000")
+    g = api.Scene(sc)
+    img, fg, st = g.render(200, 120, 3, max_bounce=8, seed=11)
+    assert img.tobytes() == ref.tobytes() and fg.tobytes() == fref.tobytes() and st.rays == sref.rays
+    g.close()
     g0.close()
 
 
