@@ -370,7 +370,8 @@ int rtp_render(rtp_scene* scene, const rtp_camera* camera, const rtp_render_para
 /* rtp_render followed by the output stage of main.rs:110-122 on the device: per pixel `to_srgb_u8` (utility.rs:212-220) of
  * the averaged colour, alpha 255 or, with RTP_RENDER_TRANSPARENT, `(255 * foreground) as u8` (main.rs:116-118). rgba_out is
  * width*height*4 bytes, pixel (i,j) at 4*(i + j*width), ready for rtp_tga_save; only the tile rectangle is written.
- * The bytes equal rtp_frame_to_srgb8 of rtp_render's frame (borderline pixels are redone with the host libm). */
+ * The bytes equal rtp_frame_to_srgb8 of rtp_render's frame (borderline pixels are redone with the host libm). A call with
+ * more than 65,536 borderline pixels among those it renders returns RTP_ERR_UNSUPPORTED (use rtp_render + rtp_frame_to_srgb8). */
 int rtp_render_srgb8(rtp_scene* scene, const rtp_camera* camera, const rtp_render_params* params, uint8_t* rgba_out,
                      rtp_stats* stats);
 /* Same with device output buffers; asynchronous on `cuda_stream` except for stats (pass NULL

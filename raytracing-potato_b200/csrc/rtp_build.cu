@@ -21,7 +21,7 @@ namespace rtp {
 #define RTP_CUDA_B(expr)                                                                             \
     do {                                                                                             \
         cudaError_t _e = (expr);                                                                     \
-        if (_e != cudaSuccess) { cleanup(); return set_error(RTP_ERR_CUDA, std::string(#expr) + ": " + cudaGetErrorString(_e)); } \
+        if (_e != cudaSuccess) { cudaGetLastError(); cleanup(); return set_error(RTP_ERR_CUDA, std::string(#expr) + ": " + cudaGetErrorString(_e)); } \
     } while (0)
 
 // keys of one depth: the item's LeafId (== its index: items arrive in LeafId order) and the sortable image of its centroid key

@@ -25,11 +25,15 @@
 
 namespace rtp {
 
+// A failed call also clears the runtime's last error, so that a refused call (an allocation that does not fit, say) does not
+// fail the next call of this thread at its first cudaGetLastError(). A sticky error stays sticky: reading it changes nothing.
 #define RTP_CUDA(expr)                                                                               \
     do {                                                                                             \
         cudaError_t _e = (expr);                                                                     \
-        if (_e != cudaSuccess)                                                                       \
+        if (_e != cudaSuccess) {                                                                     \
+            cudaGetLastError();                                                                      \
             return set_error(RTP_ERR_CUDA, std::string(#expr) + ": " + cudaGetErrorString(_e));      \
+        }                                                                                            \
     } while (0)
 
 constexpr double kRayEpsilon = 1e-3;  // utility.rs:30
@@ -1882,7 +1886,11 @@ struct DeviceScene {
     uint32_t wave_bounces = 0;         // stack depth the queues were sized for
     int shade_blocks = 0;              // grid of wave_shade_kernel
     uint32_t tail_threshold = 65536;   // RTP_TAIL_THRESHOLD: a launch this small is finished by one tail-mode launch (0 = never)
-    size_t queue_budget_bytes = size_t(4) << 30;  // memory the integrator's per-launch buffers may take (set at upload from the free HBM)
+    // memory the integrator's per-launch buffers may take (set at upload from the free HBM). A render call sizes its launches
+    // against it with its own max_bounce, and the queues it keeps afterwards hold at most max(this budget, what the call itself
+    // needs): growing them to the largest capacity seen AND the deepest stack seen would not (1080p x 16 spp at depth 1, then any
+    // frame at depth 128: a 204 GB stack), so wave_reserve then reallocates them for the call alone.
+    size_t queue_budget_bytes = size_t(4) << 30;
     bool use_simple_render = false;    // RTP_RENDER_KERNEL=simple
     bool debug_sync = false;           // RTP_DEBUG_SYNC
     double* frame = nullptr; size_t frame_elems = 0;
@@ -2328,12 +2336,22 @@ static void launch_render_paths(DeviceScene* ds, const DCamera& cam, const DRend
     else render_paths_kernel<MAXB, false><<<g, block, 0, st>>>(ds->view, cam, rp, ds->scratch, ds->counters);
 }
 
-// (re)allocates the wavefront queues for `capacity` paths per launch and a stack of `bounces` levels
+// bytes per path of one launch of the wavefront integrator: queues (2 rays, 2 states, a hit record: 176 B), the [bounce][path]
+// stack (48 B per level) and the per-path scratch (32 B)
+static size_t wave_path_bytes(uint32_t bounces) { return 176 + 48 * static_cast<size_t>(bounces) + 32; }
+
+// (re)allocates the wavefront queues for `capacity` paths per launch and a stack of `bounces` levels. The queues grow to cover
+// every shape seen so far, unless that union would cross queue_budget_bytes: then they are sized for this call alone (see
+// DeviceScene::queue_budget_bytes).
 static int wave_reserve(DeviceScene* ds, size_t capacity, uint32_t bounces) {
     WaveQueues& w = ds->wave;
     if (w.capacity >= capacity && ds->wave_bounces >= bounces) return RTP_OK;
-    capacity = std::max(capacity, w.capacity);
-    bounces = std::max(bounces, ds->wave_bounces);
+    const size_t grown_cap = std::max(capacity, w.capacity);
+    const uint32_t grown_bounces = std::max(bounces, ds->wave_bounces);
+    if (grown_cap * wave_path_bytes(grown_bounces) <= std::max(ds->queue_budget_bytes, capacity * wave_path_bytes(bounces))) {
+        capacity = grown_cap;
+        bounces = grown_bounces;
+    }
     cudaFree(w.rays[0]); cudaFree(w.rays[1]); cudaFree(w.state[0]); cudaFree(w.state[1]); cudaFree(w.hits); cudaFree(w.stack); cudaFree(w.count);
     w = WaveQueues{};
     ds->wave_bounces = 0;
@@ -2397,7 +2415,7 @@ static int render_enqueue(DeviceScene* ds, const rtp_camera* camera, const rtp_r
     // the fill and drain of ~2 x max_bounce kernels and the latency-bound sparse late bounces once (1080p x 64 spp of the C4
     // scene: 111 ms in 16 launches of 8 Mi paths, 92 ms in 4 launches of 32 Mi)
     const bool wave = !ds->use_simple_render;
-    const size_t per_path = wave ? 176 + 48 * static_cast<size_t>(p->max_bounce) + 32 : 32;
+    const size_t per_path = wave ? wave_path_bytes(p->max_bounce) : 32;
     size_t path_budget = std::max<size_t>(size_t(1) << 20, std::min<size_t>(size_t(32) << 20, ds->queue_budget_bytes / per_path));
     if (const char* v = std::getenv("RTP_PATH_BUDGET")) path_budget = std::min<size_t>(size_t(1) << 31, std::max<size_t>(1, static_cast<size_t>(std::atoll(v))));  // tests: force several launches per frame
     uint32_t per_launch = static_cast<uint32_t>(std::max<size_t>(1, std::min<size_t>(ns_total ? ns_total : 1, path_budget / npix)));
