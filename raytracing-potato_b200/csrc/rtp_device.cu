@@ -1169,6 +1169,10 @@ __global__ void __launch_bounds__(128, OUT == OUT_TAIL ? 4 : kTraceBlocksPerSM) 
         // walk, and wait here until that grid has completed and its writes are visible.
         asm volatile("griddepcontrol.wait;" ::: "memory");
         n = static_cast<size_t>(*index.count);
+        // nothing deferred (the usual case): leave before touching the queue. trace_any_kernel's last warp has rearmed it and the
+        // list is empty already, so there is nothing to reset; every warp reads the same final count, so every warp leaves. Two
+        // same-address atomics per warp of this grid (queue claim, drain count) would otherwise delay the next launch.
+        if (n == 0) return;
     }
     if (OUT == OUT_TAIL) {
         if (n == 0) return;
