@@ -503,13 +503,13 @@ void device_free_arrays(DevArrays* a) {
     *a = DevArrays{};
 }
 
-int device_build_scene(const rtp_scene_desc* d, FlatScene* out, bool timing) {
+int device_build_scene(const rtp_scene_desc* d, const Switches& sw, FlatScene* out) {
     const uint32_t n = d->n_hittables;
     if (n < 2) return 1;
     if (int rc = ensure_device()) return rc;
     auto t0 = std::chrono::steady_clock::now();
     auto lap = [&](const char* what) {
-        if (!timing) return;
+        if (!sw.build_timing) return;
         cudaDeviceSynchronize();
         auto t1 = std::chrono::steady_clock::now();
         std::fprintf(stderr, "[rtp build, device] %s: %.3f s\n", what, std::chrono::duration<double>(t1 - t0).count());

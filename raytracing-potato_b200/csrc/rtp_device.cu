@@ -443,14 +443,10 @@ struct DeferList {
     unsigned long long* count;   // entries in idx (device); reset by the in-order launch that consumes it
 };
 
-struct Tuning {
-    int refill_min;  // refill when at least this many lanes are empty
-    int prim_batch;  // run primitive tests when at least this many lanes are parked at a leaf
-    int fast_slab;   // 1: eligible rays use collide_fast
-    int f32_culling; // 1: eligible rays cull with the conservative f32 walk
-    int _reserved;   // (was: culling-tree steps per warp vote; two is compiled in, 3 and 4 measured slower)
-    int min_lanes;   // smallest number of rays a warp holds when the batch is small
-};
+// Thresholds of both persistent kernels (measured: DESIGN.md §6)
+constexpr int kRefillMin = 16;  // refill when at least this many lanes are empty
+constexpr int kPrimBatch = 4;   // run primitive tests when at least this many lanes are parked at a leaf
+constexpr int kMinLanes = 1;    // smallest number of rays a warp holds when the batch is small
 
 // Per-lane traversal state.
 //   f32-eligible lanes (m32) walk the 4-wide culling tree: `next` = node to visit, (cur, pend, c0..c3) = node whose
@@ -479,15 +475,15 @@ struct Walker {
 };
 
 // utility.rs:71-77 Ray::expand plus the derived quantities of the fast paths
-__device__ __forceinline__ void walker_start(Walker& w, const DSceneView& sc, const Tuning& tune, D3 o, D3 d, double tmin, double tmax) {
+__device__ __forceinline__ void walker_start(Walker& w, const DSceneView& sc, D3 o, D3 d, double tmin, double tmax) {
     w.o = o; w.d = d;
     w.inv = mk(1.0 / d.x, 1.0 / d.y, 1.0 / d.z);
     w.tmin = tmin;
     w.h.t = tmax; w.h.u = 0.0; w.h.v = 0.0; w.h.slot = kNoPrim; w.h.kind = 0;
-    w.fast = tune.fast_slab && finite_nonzero(w.inv.x) && finite_nonzero(w.inv.y) && finite_nonzero(w.inv.z) && finite(o.x) && finite(o.y) &&
+    w.fast = sc.fast_slab && finite_nonzero(w.inv.x) && finite_nonzero(w.inv.y) && finite_nonzero(w.inv.z) && finite(o.x) && finite(o.y) &&
              finite(o.z) && tmax >= tmin;
     w.sx = w.inv.x < 0.0; w.sy = w.inv.y < 0.0; w.sz = w.inv.z < 0.0;
-    w.m32 = w.fast && tune.f32_culling && sc.f32_culling && in_f32_range(w.inv.x) && in_f32_range(w.inv.y) && in_f32_range(w.inv.z) &&
+    w.m32 = w.fast && sc.f32_culling && in_f32_range(w.inv.x) && in_f32_range(w.inv.y) && in_f32_range(w.inv.z) &&
             fabs(o.x) <= 1e15 && fabs(o.y) <= 1e15 && fabs(o.z) <= 1e15;
     if (w.m32) {
         const double px = o.x * w.inv.x, py = o.y * w.inv.y, pz = o.z * w.inv.z;
@@ -1140,7 +1136,7 @@ __global__ void __launch_bounds__(256, kShadeBlocks) wave_shade_kernel(DSceneVie
 // The persistent traversal kernel (state and steps: Walker above). Defined here because its tail mode shades in place.
 // ---------------------------------------------------------------------------------------------
 
-// Tail mode (OUT_TAIL) of the wavefront integrator: when a launch holds at most DeviceScene::tail_threshold paths, one launch
+// Tail mode (OUT_TAIL) of the wavefront integrator: when a launch holds at most RTP_TAIL_THRESHOLD paths, one launch
 // carries every surviving path to its end. A lane whose ray is finished shades it in place (shade_vertex) and, if the
 // path scattered, restarts its walker on the scattered ray, so the remaining bounces cost one kernel instead of two
 // launches each, and the culling tree stays warm in L1 across them. Results are the same bits: per path the
@@ -1159,7 +1155,7 @@ constexpr int kTraceBlocksPerSM = 6;
 // trace_any_kernel defers (index mode).
 template <bool COUNT, int OUT, bool LIST>
 __global__ void __launch_bounds__(128, OUT == OUT_TAIL ? 4 : kTraceBlocksPerSM) trace_persistent_kernel(DSceneView sc, const rtp_ray* __restrict__ rays, size_t n, void* __restrict__ out,
-                                                                  Counters* counters, WorkQueue* wq, Tuning tune, const unsigned long long* __restrict__ n_dev,
+                                                                  Counters* counters, WorkQueue* wq, const unsigned long long* __restrict__ n_dev,
                                                                   TailArgs ta, DeferList index) {
     extern __shared__ __align__(16) uint32_t wide_stack[];  // [level][thread]
     if (n_dev) n = static_cast<size_t>(*n_dev);  // wavefront integrator: the batch size lives on the device
@@ -1197,8 +1193,10 @@ __global__ void __launch_bounds__(128, OUT == OUT_TAIL ? 4 : kTraceBlocksPerSM) 
     size_t idx = kNoRay;
     bool more = true;  // warp-uniform: the queue may still hold rays
     const size_t n_warps = static_cast<size_t>(gridDim.x) * (blockDim.x >> 5);
-    const int lane_cap = static_cast<int>(min(static_cast<size_t>(32), max(static_cast<size_t>(tune.min_lanes), (n + n_warps - 1) / n_warps)));
-    const int refill_thr = min(tune.refill_min, max(1, lane_cap / 2));
+    const int lane_cap = static_cast<int>(min(static_cast<size_t>(32), max(static_cast<size_t>(kMinLanes), (n + n_warps - 1) / n_warps)));
+    // refill at kRefillMin free lanes, or at half the cap of a warp that holds fewer rays. Written as a select: min(kRefillMin, ...)
+    // is the same value, but with the constant folded in, ptxas (CUDA 12.9) gives <false, OUT_HIT, false> 36 B more of spill stores.
+    const int refill_thr = lane_cap >= 2 * kRefillMin ? kRefillMin : max(1, lane_cap / 2);
 
     for (;;) {
         // ---- retire finished rays and refill ----------------------------------------------------------
@@ -1210,7 +1208,7 @@ __global__ void __launch_bounds__(128, OUT == OUT_TAIL ? 4 : kTraceBlocksPerSM) 
         if (OUT == OUT_TAIL) {
             // shade finished rays in place; a path that scattered keeps its lane and walks on
             const unsigned finished = __ballot_sync(0xffffffffu, fin);
-            if (finished != 0u && (__popc(finished) >= tune.prim_batch || __ballot_sync(0xffffffffu, !is_done) == 0u)) {
+            if (finished != 0u && (__popc(finished) >= kPrimBatch || __ballot_sync(0xffffffffu, !is_done) == 0u)) {
                 if (fin) {
                     uint32_t depth = pst.z & 0xFFu, nb = (pst.z >> 8) & 0xFFu, first_hit = (pst.z >> 16) & 1u;
                     const size_t p = pst.x;
@@ -1241,7 +1239,7 @@ __global__ void __launch_bounds__(128, OUT == OUT_TAIL ? 4 : kTraceBlocksPerSM) 
                     }
                     pst.z = depth | (nb << 8) | (first_hit << 16);
                     if (alive) {
-                        walker_start(w, sc, tune, o, d, kRayEpsilon, CUDART_INF);
+                        walker_start(w, sc, o, d, kRayEpsilon, CUDART_INF);
                         if (LIST) { w.m32 = false; if (sc.n_prims == 0) w.next = kEnd; }
                         lc.rays++;
                     } else {
@@ -1278,7 +1276,7 @@ __global__ void __launch_bounds__(128, OUT == OUT_TAIL ? 4 : kTraceBlocksPerSM) 
                     idx = i;
                     const double2* rp = reinterpret_cast<const double2*>(rays + i);
                     const double2 r0 = __ldg(rp), r1 = __ldg(rp + 1), r2 = __ldg(rp + 2), r3 = __ldg(rp + 3);
-                    walker_start(w, sc, tune, mk(r0.x, r0.y, r1.x), mk(r1.y, r2.x, r2.y), r3.x, r3.y);
+                    walker_start(w, sc, mk(r0.x, r0.y, r1.x), mk(r1.y, r2.x, r2.y), r3.x, r3.y);
                     if (LIST) { w.m32 = false; if (sc.n_prims == 0) w.next = kEnd; }
                     if (OUT == OUT_TAIL) pst = ta.q.state[ta.bounce & 1u][i];
                     lc.rays++;
@@ -1310,7 +1308,7 @@ __global__ void __launch_bounds__(128, OUT == OUT_TAIL ? 4 : kTraceBlocksPerSM) 
                 const unsigned walking = __ballot_sync(0xffffffffu, (w.next != kEnd) & (w.prim2 == kNoPrim) & w.m32);
                 if (walking == 0u) break;
                 const unsigned parked = __ballot_sync(0xffffffffu, w.prim != kNoPrim);
-                if (__popc(parked) >= tune.prim_batch) break;
+                if (__popc(parked) >= kPrimBatch) break;
                 if (more && min(__popc(~(walking | parked)), max(lane_cap - __popc(walking | parked), 0)) >= refill_thr) break;
             }
             // ---- lanes outside the f32 path's preconditions take one exact step per round ------------------
@@ -1437,7 +1435,7 @@ constexpr int kAnyPopLoop = 2;   // stack entries a step may take before it visi
 
 template <bool COUNT, int OUT>
 __global__ void __launch_bounds__(128, kAnyBlocks) trace_any_kernel(DSceneView sc, const rtp_ray* __restrict__ rays, size_t n, void* __restrict__ out, Counters* counters,
-                                                       WorkQueue* wq, Tuning tune, const unsigned long long* __restrict__ n_dev, DeferList defer) {
+                                                       WorkQueue* wq, const unsigned long long* __restrict__ n_dev, DeferList defer) {
     extern __shared__ __align__(16) uint32_t any_stack[];
     // the launch over the defer list (launch_trace) may be set up while this grid runs: it waits for this grid's completion itself
     asm volatile("griddepcontrol.launch_dependents;");
@@ -1464,8 +1462,8 @@ __global__ void __launch_bounds__(128, kAnyBlocks) trace_any_kernel(DSceneView s
     uint32_t leaf0 = 0u, leaf1 = 0u;  // pending leaves (raw child words, oldest first); 0 = none (child word 0 is the root, never a leaf)
     bool more = true;             // warp-uniform: the queue may still hold rays
     const size_t n_warps = static_cast<size_t>(gridDim.x) * (blockDim.x >> 5);
-    const int lane_cap = static_cast<int>(min(static_cast<size_t>(32), max(static_cast<size_t>(tune.min_lanes), (n + n_warps - 1) / n_warps)));
-    const int refill_thr = min(tune.refill_min, max(1, lane_cap / 2));
+    const int lane_cap = static_cast<int>(min(static_cast<size_t>(32), max(static_cast<size_t>(kMinLanes), (n + n_warps - 1) / n_warps)));
+    const int refill_thr = lane_cap >= 2 * kRefillMin ? kRefillMin : max(1, lane_cap / 2);
     const float4* __restrict__ tree = reinterpret_cast<const float4*>(sc.any_wide);  // a node = 8 float4: 32-bit indexing (device_scene_upload: < 2^29 nodes)
 
     // exact test of one leaf in any-order mode
@@ -1623,7 +1621,7 @@ __global__ void __launch_bounds__(128, kAnyBlocks) trace_any_kernel(DSceneView s
         {
             const int n_walk = __popc(__ballot_sync(0xffffffffu, (leaf1 == 0u) & ((node != kNone) | (sp != sbase))));
             const int n_leaf = __popc(__ballot_sync(0xffffffffu, leaf0 != 0u));
-            leaf_first = n_leaf >= tune.prim_batch && n_leaf > n_walk;
+            leaf_first = n_leaf >= kPrimBatch && n_leaf > n_walk;
         }
         // ---- walk: up to two steps per round ----------------------------------------------------------------------------------
         if (!leaf_first) {
@@ -1711,7 +1709,7 @@ __global__ void __launch_bounds__(128, kAnyBlocks) trace_any_kernel(DSceneView s
         const unsigned parked = __ballot_sync(0xffffffffu, leaf0 != 0u);
         if (parked != 0u) {
             const unsigned walking = __ballot_sync(0xffffffffu, (leaf1 == 0u) & ((node != kNone) | (sp != sbase)));
-            if (__popc(parked) >= tune.prim_batch || walking == 0u) {
+            if (__popc(parked) >= kPrimBatch || walking == 0u) {
                 if (COUNT && lane == 0 && counters) { atomicAdd(&counters->leaf_rounds, 1ull); atomicAdd(&counters->leaf_lanes, static_cast<unsigned long long>(__popc(parked))); }
                 if (leaf0 != 0u) {
                     if (!(leaf0 & kWideBig)) test_leaf(leaf0);  // big primitives were tested when the ray started
@@ -1824,14 +1822,10 @@ constexpr int kPipeDepth = 3;
 constexpr size_t kAnyOrderBigScene = 262144;  // leaves from which rtp_scene_info.any_order reports 2 (the kernel is the same)
 constexpr unsigned kQueueSlots = 64;
 constexpr unsigned kLaunchSlots = 8;
-static size_t chunk_rays() {  // rays per pipeline stage: 2^18 (16 MiB of rays) unless RTP_CHUNK_LOG2 says otherwise (tuning runs)
-    static const size_t v = [] { const char* e = std::getenv("RTP_CHUNK_LOG2"); const int l = e ? std::atoi(e) : 18; return size_t(1) << std::max(10, std::min(24, l)); }();
-    return v;
-}
-#define kChunkRays (chunk_rays())
 
 struct DeviceScene {
     int device = 0;
+    Switches sw;                       // read when the scene was created (scene_create_impl)
     DNode* nodes = nullptr;
     DWide* wide = nullptr;
     size_t n_wide = 0;
@@ -1871,8 +1865,6 @@ struct DeviceScene {
     size_t any_stack_bytes = 0;        // its dynamic shared memory: any_cap x 128 threads x 8 B of stacks + 8 KiB of cold lane state
     int any_order = 0;                 // != 0: eligible rays take the any-order walk (RTP_TRAVERSAL); 2 marks a scene of >= 262,144 leaves
     uint32_t any_cap = 0;              // any-order stack entries per lane
-    bool use_simple_kernel = false;    // RTP_TRACE_KERNEL=simple
-    Tuning tune{16, 4, 1, 1, 2, 1};           // RTP_REFILL_MIN / RTP_PRIM_BATCH / RTP_FAST_SLAB override (tuning runs only)
     cudaStream_t streams[kPipeDepth] = {nullptr, nullptr, nullptr};
     cudaEvent_t ev_begin = nullptr, ev_end = nullptr;
     cudaEvent_t render_done = nullptr; // end of the last render enqueued: the next render (any stream) waits for it before it
@@ -1889,14 +1881,11 @@ struct DeviceScene {
     WaveQueues wave{};                 // wavefront integrator queues (render_device), grown on demand
     uint32_t wave_bounces = 0;         // stack depth the queues were sized for
     int shade_blocks = 0;              // grid of wave_shade_kernel
-    uint32_t tail_threshold = 65536;   // RTP_TAIL_THRESHOLD: a launch this small is finished by one tail-mode launch (0 = never)
     // memory the integrator's per-launch buffers may take (set at upload from the free HBM). A render call sizes its launches
     // against it with its own max_bounce, and the queues it keeps afterwards hold at most max(this budget, what the call itself
     // needs): growing them to the largest capacity seen AND the deepest stack seen would not (1080p x 16 spp at depth 1, then any
     // frame at depth 128: a 204 GB stack), so wave_reserve then reallocates them for the call alone.
     size_t queue_budget_bytes = size_t(4) << 30;
-    bool use_simple_render = false;    // RTP_RENDER_KERNEL=simple
-    bool debug_sync = false;           // RTP_DEBUG_SYNC
     double* frame = nullptr; size_t frame_elems = 0;
     uchar4* frame8 = nullptr; size_t frame8_elems = 0;  // RGBA8 output stage
     SrgbFix* fixes = nullptr; unsigned int* n_fixes = nullptr;
@@ -1962,13 +1951,14 @@ static int check_device(int device) {
 
 int current_device() { return g_device; }
 
-int device_scene_upload(const FlatScene& flat, int device, DeviceScene** out) {
+int device_scene_upload(const FlatScene& flat, const Switches& sw, int device, DeviceScene** out) {
     int rc = device < 0 ? require_device() : check_device(device);
     if (rc != RTP_OK) return rc;
     if (device < 0) device = g_device;
     RTP_CUDA(cudaSetDevice(device));
     DeviceScene* ds = new DeviceScene();
     ds->device = device;
+    ds->sw = sw;
     auto bail = [&](int code) { device_scene_free(ds); return code; };
     // arrays built on a device (rtp_build.cu) are adopted there and copied peer to peer elsewhere; host-built ones are uploaded
     const bool adopt = flat.dev.valid && flat.dev.device == device && !flat.dev.adopted;  // the replica on the building device takes the arrays over
@@ -2000,20 +1990,15 @@ int device_scene_upload(const FlatScene& flat, int device, DeviceScene** out) {
         if ((rc = upload(flat.free_boxes, &ds->free_boxes, &ds->bytes)) != RTP_OK) return bail(rc);
     }
     // one stack word per tree level and thread; a tree deeper than 96 levels (degenerate geometry) does not get the f32 walk
-    // at all (view.f32_culling below), so its launches carry no stack
+    // at all (f32_culling below), so its launches carry no stack
     ds->stack_bytes = static_cast<size_t>(flat.wide_depth <= 96 ? std::max<uint32_t>(flat.wide_depth, 1u) : 1u) * 128 * sizeof(uint32_t);
-    {
-        // RTP_TRAVERSAL=any | inorder overrides the choice
-        const char* tv = std::getenv("RTP_TRAVERSAL");
-        const bool f32_ok = flat.root_kind == RTP_ROOT_BVH && flat.boxes_finite && flat.scene_mag <= 1e15 && flat.wide_depth <= 96 &&
-                            flat.wide_count() < (size_t(1) << 28) && flat.free_wide.size() < (size_t(1) << 28);  // trace_any_kernel indexes nodes as 32-bit float4 offsets
-        bool want = true;  // every eligible scene takes the any-order walk by default (measured faster from the 4,969-leaf bunny up)
-        if (tv && std::string(tv) == "any") want = true;
-        if (tv && std::string(tv) == "inorder") want = false;
-        if (const char* v = std::getenv("RTP_F32_CULLING")) if (std::atoi(v) == 0) want = false;
-        // 2 marks a big scene in rtp_scene_info only: every any-order scene runs the same trace_any_kernel
-        ds->any_order = (want && flat.any_ok && f32_ok) ? (flat.prim_count() >= kAnyOrderBigScene ? 2 : 1) : 0;
-    }
+    // the conservative f32 walk: eligible rays of this scene take it unless RTP_F32_CULLING=0
+    const bool f32_culling = sw.f32_culling && flat.root_kind == RTP_ROOT_BVH && flat.boxes_finite && flat.scene_mag <= 1e15 && flat.wide_depth <= 96;
+    // every eligible scene takes the any-order walk unless RTP_TRAVERSAL=inorder (measured faster from the 4,969-leaf bunny up); it
+    // walks in f32 and indexes nodes as 32-bit float4 offsets. 2 marks a big scene in rtp_scene_info only: every any-order scene
+    // runs the same trace_any_kernel
+    const bool any_ok = sw.any_order && flat.any_ok && f32_culling && flat.wide_count() < (size_t(1) << 28) && flat.free_wide.size() < (size_t(1) << 28);
+    ds->any_order = any_ok ? (flat.prim_count() >= kAnyOrderBigScene ? 2 : 1) : 0;
     if (flat.dev.valid) {
         if ((rc = take(&ds->prims, flat.dev.prims, flat.dev.n_prims)) != RTP_OK) return bail(rc);
         if ((rc = take(&ds->attrs, flat.dev.attrs, flat.dev.n_prims)) != RTP_OK) return bail(rc);
@@ -2061,7 +2046,7 @@ int device_scene_upload(const FlatScene& flat, int device, DeviceScene** out) {
             // overflows, is what the cap costs); a lane that would need more defers its ray to the in-order kernel
             const uint32_t any_depth = ds->free_wide ? flat.free_depth : flat.wide_depth;
             ds->any_cap = std::max<uint32_t>(4u, std::min<uint32_t>(3u * any_depth + 1u, any_depth <= 12 ? 22u : 28u));  // six blocks per SM: 22 + 8 KiB stay inside the 196 KiB carve-out, 28 + 8 KiB inside 228
-            if (const char* v = std::getenv("RTP_ANY_CAP")) ds->any_cap = static_cast<uint32_t>(std::max(4, std::min(48, std::atoi(v))));  // tests
+            if (sw.any_cap) ds->any_cap = sw.any_cap;  // tests
             ds->any_stack_bytes = static_cast<size_t>(ds->any_cap) * 128 * sizeof(uint2) + kAnyColdBytes;  // the stacks, then the cold state
             if (ds->any_stack_bytes > 48u * 1024u) {  // deep trees: above the default limit of dynamic shared memory, every instantiation that is launched
 #define RTP_ANY_SMEM(C, O) if (e == cudaSuccess) e = cudaFuncSetAttribute(trace_any_kernel<C, O>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(ds->any_stack_bytes))
@@ -2076,23 +2061,10 @@ int device_scene_upload(const FlatScene& flat, int device, DeviceScene** out) {
         if (e == cudaSuccess && cudaMemGetInfo(&free_b, &total_b) == cudaSuccess)
             ds->queue_budget_bytes = std::max<size_t>(size_t(1) << 30, std::min<size_t>(size_t(24) << 30, free_b / 6));
         ds->shade_blocks = prop.multiProcessorCount * kShadeBlocks;
-        if (const char* v = std::getenv("RTP_BUILD_TIMING")) if (std::atoi(v) != 0)
+        if (sw.build_timing)
             std::fprintf(stderr, "[rtp build] 4-wide tree depth %u (order-free tree: %u), %s walk (%u big primitives), %zu B of stack per block, %d traversal blocks per SM\n",
                          flat.wide_depth, flat.free_depth, ds->any_order ? "any-order" : "in-order", flat.n_big,
                          ds->any_order ? ds->any_stack_bytes : ds->stack_bytes, ds->any_order ? any_per_sm : per_sm);
-        if (const char* v = std::getenv("RTP_TAIL_THRESHOLD")) ds->tail_threshold = static_cast<uint32_t>(std::max(0l, std::atol(v)));
-        const char* env = std::getenv("RTP_TRACE_KERNEL");
-        ds->use_simple_kernel = env && std::string(env) == "simple";
-        env = std::getenv("RTP_RENDER_KERNEL");
-        ds->use_simple_render = env && std::string(env) == "simple";
-        env = std::getenv("RTP_DEBUG_SYNC");
-        ds->debug_sync = env && std::atoi(env) != 0;
-        if (const char* v = std::getenv("RTP_REFILL_MIN")) ds->tune.refill_min = std::max(1, std::min(32, std::atoi(v)));
-        if (const char* v = std::getenv("RTP_PRIM_BATCH")) ds->tune.prim_batch = std::max(1, std::min(32, std::atoi(v)));
-        if (const char* v = std::getenv("RTP_FAST_SLAB")) ds->tune.fast_slab = std::atoi(v) != 0;
-        if (const char* v = std::getenv("RTP_F32_CULLING")) ds->tune.f32_culling = std::atoi(v) != 0;
-        if (const char* v = std::getenv("RTP_MIN_LANES")) ds->tune.min_lanes = std::max(1, std::min(32, std::atoi(v)));
-        if (!flat.boxes_finite) ds->tune.fast_slab = 0;
     }
     for (int k = 0; k < kPipeDepth && e == cudaSuccess; ++k) e = cudaStreamCreateWithFlags(&ds->streams[k], cudaStreamNonBlocking);
     if (e == cudaSuccess) e = cudaEventCreate(&ds->ev_begin);
@@ -2104,7 +2076,7 @@ int device_scene_upload(const FlatScene& flat, int device, DeviceScene** out) {
     DSceneView& v = ds->view;
     v.nodes = ds->nodes; v.wide = ds->wide; v.wide_boxes = ds->wide_boxes; v.prims = ds->prims;
     v.any_wide = ds->free_wide ? ds->free_wide : ds->wide; v.any_boxes = ds->free_wide ? ds->free_boxes : ds->wide_boxes;
-    v.f32_culling = (flat.root_kind == RTP_ROOT_BVH && flat.boxes_finite && flat.scene_mag <= 1e15 && flat.wide_depth <= 96) ? 1u : 0u; v.attrs = ds->attrs; v.materials = ds->materials; v.textures = ds->textures;
+    v.f32_culling = f32_culling ? 1u : 0u; v.attrs = ds->attrs; v.materials = ds->materials; v.textures = ds->textures;
     v.n_nodes = flat.root_kind == RTP_ROOT_BVH ? static_cast<uint32_t>(flat.node_count()) : 0u;
     v.n_prims = static_cast<uint32_t>(flat.prim_count());
     v.root_kind = flat.root_kind;
@@ -2112,7 +2084,7 @@ int device_scene_upload(const FlatScene& flat, int device, DeviceScene** out) {
     v.any_order = ds->any_order ? 1u : 0u;
     v.any_cap = ds->any_cap;
     v.n_big = flat.n_big;
-    v._pad_any = 0;
+    v.fast_slab = flat.boxes_finite ? 1u : 0u;
     for (int k = 0; k < 8; ++k) v.big[k] = flat.big[k];
     v.any_E = flat.any_E; v.any_A = flat.any_A;
     v.any_Ef = std::nextafter(static_cast<float>(flat.any_E), std::numeric_limits<float>::infinity());  // >= any_E
@@ -2121,9 +2093,7 @@ int device_scene_upload(const FlatScene& flat, int device, DeviceScene** out) {
     v.any_Rf = flat.any_spheres ? std::nextafter(static_cast<float>(flat.any_R), std::numeric_limits<float>::infinity()) : -1.0f;
     std::memcpy(v.bg_rgb, flat.background.rgb, sizeof v.bg_rgb);
     // RTP_ANY_SETUP_CULL=0: a box that every ray enters, so every ray walks (A/B runs of the set-up cull in one process)
-    const char* cv = std::getenv("RTP_ANY_SETUP_CULL");
-    const bool setup_cull = !cv || std::atoi(cv) != 0;
-    for (int k = 0; k < 6; ++k) v.cull[k] = setup_cull ? flat.cull[k] : (k < 3 ? -1.0f : 1.0f) * std::numeric_limits<float>::infinity();
+    for (int k = 0; k < 6; ++k) v.cull[k] = sw.any_setup_cull ? flat.cull[k] : (k < 3 ? -1.0f : 1.0f) * std::numeric_limits<float>::infinity();
     *out = ds;
     return RTP_OK;
 }
@@ -2141,7 +2111,7 @@ static DCamera make_camera(const rtp_camera* c) {
 // (wavefront integrator) and `n` is only an upper bound used to size the grid.
 // RTP_DEBUG_SYNC=1: synchronise after every launch of the integrator and name the kernel that faulted
 static int debug_sync(const DeviceScene* ds, cudaStream_t st, const char* what, uint32_t bounce) {
-    if (!ds->debug_sync) return RTP_OK;
+    if (!ds->sw.debug_sync) return RTP_OK;
     cudaError_t e = cudaStreamSynchronize(st);
     if (e != cudaSuccess) return set_error(RTP_ERR_CUDA, std::string(what) + " (segment " + std::to_string(bounce) + "): " + cudaGetErrorString(e));
     return RTP_OK;
@@ -2152,7 +2122,7 @@ static int launch_trace(DeviceScene* ds, const rtp_ray* d_rays, size_t n, void* 
     if (n == 0) return RTP_OK;
     const unsigned block = 128;
     ds->last_trace_launches = 1;
-    if (ds->use_simple_kernel && !n_dev && out_mode != OUT_WAVE) {
+    if (ds->sw.simple_trace && !n_dev && out_mode != OUT_WAVE) {
         const size_t grid = (n + block - 1) / block;
         if (grid > 0x7FFFFFFFull) return set_error(RTP_ERR_INVALID, "ray batch too large for one launch");
         const dim3 g(static_cast<unsigned>(grid));
@@ -2199,7 +2169,7 @@ static int launch_trace(DeviceScene* ds, const rtp_ray* d_rays, size_t n, void* 
         if (pure_any) {
             const dim3 g(static_cast<unsigned>(std::min<size_t>(static_cast<size_t>(ds->any_blocks), want)));
             const DeferList defer{slot.defer_idx, slot.defer_count};
-#define RTP_LAUNCH_ANY(C, O) trace_any_kernel<C, O><<<g, block, ds->any_stack_bytes, stream>>>(ds->view, d_rays, n, d_out, counters, wq, ds->tune, n_dev, defer)
+#define RTP_LAUNCH_ANY(C, O) trace_any_kernel<C, O><<<g, block, ds->any_stack_bytes, stream>>>(ds->view, d_rays, n, d_out, counters, wq, n_dev, defer)
             if (out_mode == OUT_FULL) { if (count) RTP_LAUNCH_ANY(true, OUT_FULL); else RTP_LAUNCH_ANY(false, OUT_FULL); }
             else if (out_mode == OUT_WAVE) { if (count) RTP_LAUNCH_ANY(true, OUT_WAVE); else RTP_LAUNCH_ANY(false, OUT_WAVE); }
             else { if (count) RTP_LAUNCH_ANY(true, OUT_HIT); else RTP_LAUNCH_ANY(false, OUT_HIT); }
@@ -2222,7 +2192,7 @@ static int launch_trace(DeviceScene* ds, const rtp_ray* d_rays, size_t n, void* 
             cfg2.gridDim = g2; cfg2.blockDim = block; cfg2.dynamicSmemBytes = ds->inorder_stack_bytes; cfg2.stream = stream;
             cfg2.attrs = &pdl; cfg2.numAttrs = 1;
             const unsigned long long* const no_n_dev = nullptr;
-#define RTP_LAUNCH_DEFERRED(C, O) RTP_CUDA(cudaLaunchKernelEx(&cfg2, trace_persistent_kernel<C, O, false>, ds->view, d_rays, n, d_out, counters, wq, ds->tune, no_n_dev, ta, defer))
+#define RTP_LAUNCH_DEFERRED(C, O) RTP_CUDA(cudaLaunchKernelEx(&cfg2, trace_persistent_kernel<C, O, false>, ds->view, d_rays, n, d_out, counters, wq, no_n_dev, ta, defer))
             if (out_mode == OUT_FULL) { if (count) RTP_LAUNCH_DEFERRED(true, OUT_FULL); else RTP_LAUNCH_DEFERRED(false, OUT_FULL); }
             else if (out_mode == OUT_WAVE) { if (count) RTP_LAUNCH_DEFERRED(true, OUT_WAVE); else RTP_LAUNCH_DEFERRED(false, OUT_WAVE); }
             else { if (count) RTP_LAUNCH_DEFERRED(true, OUT_HIT); else RTP_LAUNCH_DEFERRED(false, OUT_HIT); }
@@ -2232,7 +2202,7 @@ static int launch_trace(DeviceScene* ds, const rtp_ray* d_rays, size_t n, void* 
             const int blocks = out_mode == OUT_TAIL ? ds->inorder_tail_blocks : ds->inorder_blocks;
             const size_t smem = ds->inorder_stack_bytes;
             const dim3 g(static_cast<unsigned>(std::min<size_t>(static_cast<size_t>(blocks), want)));
-#define RTP_LAUNCH_PERSISTENT(C, O, L) trace_persistent_kernel<C, O, L><<<g, block, smem, stream>>>(ds->view, d_rays, n, d_out, counters, wq, ds->tune, n_dev, ta, no_index)
+#define RTP_LAUNCH_PERSISTENT(C, O, L) trace_persistent_kernel<C, O, L><<<g, block, smem, stream>>>(ds->view, d_rays, n, d_out, counters, wq, n_dev, ta, no_index)
 #define RTP_LAUNCH_PERSISTENT_O(O)                                                                   \
     do {                                                                                             \
         if (list) { if (count) RTP_LAUNCH_PERSISTENT(true, O, true); else RTP_LAUNCH_PERSISTENT(false, O, true); }     \
@@ -2267,23 +2237,24 @@ static int trace_host(rtp_scene* scene, const rtp_ray* rays, size_t n, void* hit
     for (DeviceScene* ds : devs) locks.emplace_back(ds->lock);
     const size_t hit_bytes = full ? sizeof(rtp_hit_full) : sizeof(rtp_hit);
     const bool count = stats != nullptr;
-    const size_t n_chunks = (n + kChunkRays - 1) / kChunkRays;
+    const size_t chunk = size_t(1) << devs[0]->sw.chunk_log2;  // rays per pipeline stage: 2^18 (16 MiB of rays) unless RTP_CHUNK_LOG2 says otherwise
+    const size_t n_chunks = (n + chunk - 1) / chunk;
     const size_t used = std::min(N, n_chunks);  // devices that get at least one chunk
     int rc = RTP_OK;
     for (size_t d = 0; d < used && rc == RTP_OK; ++d) {
         DeviceScene* ds = devs[d];
         RTP_CUDA(cudaSetDevice(ds->device));
         for (int k = 0; k < kPipeDepth; ++k) {
-            if (!ds->stage_rays[k]) RTP_CUDA(cudaMalloc(reinterpret_cast<void**>(&ds->stage_rays[k]), kChunkRays * sizeof(rtp_ray)));
-            if (!ds->stage_hits[k]) RTP_CUDA(cudaMalloc(&ds->stage_hits[k], kChunkRays * sizeof(rtp_hit_full)));
+            if (!ds->stage_rays[k]) RTP_CUDA(cudaMalloc(reinterpret_cast<void**>(&ds->stage_rays[k]), chunk * sizeof(rtp_ray)));
+            if (!ds->stage_hits[k]) RTP_CUDA(cudaMalloc(&ds->stage_hits[k], chunk * sizeof(rtp_hit_full)));
         }
         if (count) RTP_CUDA(cudaMemsetAsync(ds->counters, 0, sizeof(Counters), ds->streams[0]));
         RTP_CUDA(cudaEventRecord(ds->ev_begin, ds->streams[0]));
         for (int k = 1; k < kPipeDepth; ++k) RTP_CUDA(cudaStreamWaitEvent(ds->streams[k], ds->ev_begin, 0));
     }
     size_t launches = 0, chunk_id = 0;
-    for (size_t off = 0; off < n && rc == RTP_OK; off += kChunkRays, ++chunk_id) {
-        const size_t m = std::min(kChunkRays, n - off);
+    for (size_t off = 0; off < n && rc == RTP_OK; off += chunk, ++chunk_id) {
+        const size_t m = std::min(chunk, n - off);
         DeviceScene* ds = devs[chunk_id % N];
         const int k = static_cast<int>((chunk_id / N) % kPipeDepth);
         cudaStream_t st = ds->streams[k];
@@ -2418,10 +2389,10 @@ static int render_enqueue(DeviceScene* ds, const rtp_camera* camera, const rtp_r
     // budget fixed when the scene was uploaded (a sixth of the free HBM, at most 24 GiB). Big launches matter: every launch pays
     // the fill and drain of ~2 x max_bounce kernels and the latency-bound sparse late bounces once (1080p x 64 spp of the C4
     // scene: 111 ms in 16 launches of 8 Mi paths, 92 ms in 4 launches of 32 Mi)
-    const bool wave = !ds->use_simple_render;
+    const bool wave = !ds->sw.simple_render;
     const size_t per_path = wave ? wave_path_bytes(p->max_bounce) : 32;
     size_t path_budget = std::max<size_t>(size_t(1) << 20, std::min<size_t>(size_t(32) << 20, ds->queue_budget_bytes / per_path));
-    if (const char* v = std::getenv("RTP_PATH_BUDGET")) path_budget = std::min<size_t>(size_t(1) << 31, std::max<size_t>(1, static_cast<size_t>(std::atoll(v))));  // tests: force several launches per frame
+    if (const size_t forced = read_path_budget()) path_budget = forced;  // tests: force several launches per frame
     uint32_t per_launch = static_cast<uint32_t>(std::max<size_t>(1, std::min<size_t>(ns_total ? ns_total : 1, path_budget / npix)));
     const size_t need = npix * per_launch;
     if (wave && ns_total) {
@@ -2470,7 +2441,7 @@ static int render_enqueue(DeviceScene* ds, const rtp_camera* camera, const rtp_r
                 // (19 -> 12 launches per C1 frame, same 2.05 ms): a late bounce costs the latency of ONE ray segment (~30 us of
                 // dependent instructions, tools/small_batches.py), not a launch.
                 if (want_stats) next_mark(ds, st);  // even marks open a traversal span, odd marks close it
-                if (ds->tail_threshold && total <= ds->tail_threshold) {
+                if (ds->sw.tail_threshold && total <= ds->sw.tail_threshold) {
                     TailArgs ta{ds->wave, rp, ds->scratch, b};
                     rc = launch_trace(ds, ds->wave.rays[b & 1], total, nullptr, OUT_TAIL, count, ds->counters, st, ds->wave.count + b, &ta);
                     if (rc != RTP_OK) return rc;
@@ -2713,7 +2684,8 @@ static int scene_create_impl(const rtp_scene_desc* desc, uint32_t device_mask, r
             if (g_device < 0) g_device = first;
             cudaSetDevice(first);  // the device part of the build (reference leaf order of big scenes) runs on the first device
         }
-        rc = flatten_scene(desc, &s->flat, /*device_build=*/true);  // validates before it touches the device
+        const Switches sw = read_switches();
+        rc = flatten_scene(desc, sw, &s->flat, /*device_build=*/true);  // validates before it touches the device
         if (rc != RTP_OK) return bail(rc);
         if (!device_mask) {
             if ((rc = require_device()) != RTP_OK) return bail(rc);
@@ -2722,7 +2694,7 @@ static int scene_create_impl(const rtp_scene_desc* desc, uint32_t device_mask, r
         for (int d = 0; d < 32 && rc == RTP_OK; ++d)
             if ((device_mask >> d) & 1u) {
                 DeviceScene* ds = nullptr;
-                rc = device_scene_upload(s->flat, d, &ds);
+                rc = device_scene_upload(s->flat, sw, d, &ds);
                 if (rc == RTP_OK) s->devs.push_back(ds);
             }
         if (rc != RTP_OK) return bail(rc);
@@ -2784,7 +2756,7 @@ int rtp_scene_get_info(const rtp_scene* scene, rtp_scene_info* info) {
 int rtp_bvh_build_order(const rtp_scene_desc* desc, uint32_t* leaf_ids_out, size_t cap, rtp_scene_info* info) {
     try {
         FlatScene flat;
-        int rc = flatten_scene(desc, &flat);
+        int rc = flatten_scene(desc, read_switches(), &flat);
         if (rc != RTP_OK) return rc;
         if (leaf_ids_out) {
             if (cap < flat.leaf_order.size()) return set_error(RTP_ERR_INVALID, "leaf_ids_out too small");
@@ -2807,7 +2779,7 @@ int rtp_bvh_culled_set(const rtp_scene_desc* desc, float box_out[6], uint32_t* f
     if (!box_out || !free_tree_leaves || !free_tree_big_leaves) return set_error(RTP_ERR_INVALID, "null argument");
     try {
         FlatScene flat;
-        int rc = flatten_scene(desc, &flat);
+        int rc = flatten_scene(desc, read_switches(), &flat);
         if (rc != RTP_OK) return rc;
         std::copy(flat.cull, flat.cull + 6, box_out);
         uint32_t leaves = 0, big = 0;
@@ -2877,7 +2849,7 @@ int rtp_trace_closest_device_counted(rtp_scene* scene, const rtp_ray* d_rays, si
     RTP_CUDA(cudaMemcpy(&c, ds->counters, sizeof c, cudaMemcpyDeviceToHost));
     float ms = 0.f;
     RTP_CUDA(cudaEventElapsedTime(&ms, ds->ev_begin, ds->ev_end));
-    if (std::getenv("RTP_LANE_STATS") && c.rounds)
+    if (ds->sw.lane_stats && c.rounds)
         std::fprintf(stderr, "[rtp lanes] %llu rounds (%.1f per ray): per round %.1f lanes can walk, %.1f hold two leaves, %.1f wait for a leaf test with nothing left to walk, %.1f hold no ray; "
                              "%llu leaf rounds at %.1f lanes\n", c.rounds, double(c.rounds) * 32.0 / double(c.rays ? c.rays : 1), double(c.lanes_walk) / c.rounds, double(c.lanes_full) / c.rounds,
                      double(c.lanes_leafwait) / c.rounds, double(c.lanes_empty) / c.rounds, c.leaf_rounds, c.leaf_rounds ? double(c.leaf_lanes) / c.leaf_rounds : 0.0);

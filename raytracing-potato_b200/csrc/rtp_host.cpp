@@ -32,6 +32,42 @@ int set_error(int code, const std::string& msg) {
     return code;
 }
 
+// The only reader of the environment (Switches, rtp_internal.h). `unset` is the value of a switch that is not set.
+static const char* env(const char* name) { return std::getenv(name); }
+static int env_flag(const char* name, int unset) {
+    const char* v = env(name);
+    return v ? (std::atoi(v) != 0 ? 1 : 0) : unset;
+}
+static long long env_number(const char* name, long long unset, long long lo, long long hi) {
+    const char* v = env(name);
+    return v ? std::min(hi, std::max(lo, std::atoll(v))) : unset;
+}
+static bool env_word(const char* name, const char* word) {
+    const char* v = env(name);
+    return v && std::strcmp(v, word) == 0;
+}
+
+Switches read_switches() {
+    Switches s;
+    s.any_order = !env_word("RTP_TRAVERSAL", "inorder");
+    s.f32_culling = env_flag("RTP_F32_CULLING", s.f32_culling);
+    s.simple_trace = env_word("RTP_TRACE_KERNEL", "simple");
+    s.simple_render = env_word("RTP_RENDER_KERNEL", "simple");
+    s.reference_tree = env_word("RTP_TREE", "reference");
+    s.free_tree = env_flag("RTP_FREE_TREE", s.free_tree);
+    s.device_build = env_flag("RTP_DEVICE_BUILD", s.device_build);
+    s.any_cap = static_cast<uint32_t>(env_number("RTP_ANY_CAP", s.any_cap, 4, 48));
+    s.any_setup_cull = env_flag("RTP_ANY_SETUP_CULL", s.any_setup_cull);
+    s.tail_threshold = static_cast<uint32_t>(env_number("RTP_TAIL_THRESHOLD", s.tail_threshold, 0, std::numeric_limits<uint32_t>::max()));
+    s.chunk_log2 = static_cast<uint32_t>(env_number("RTP_CHUNK_LOG2", s.chunk_log2, 10, 24));
+    s.build_timing = env_flag("RTP_BUILD_TIMING", s.build_timing);
+    s.debug_sync = env_flag("RTP_DEBUG_SYNC", s.debug_sync);
+    s.lane_stats = env_flag("RTP_LANE_STATS", s.lane_stats);
+    return s;
+}
+
+size_t read_path_budget() { return static_cast<size_t>(env_number("RTP_PATH_BUDGET", 0, 1, 1ll << 31)); }
+
 // f64::min / f64::max (IEEE minNum / maxNum), as used by AABB::union and the triangle box.
 static inline double min_num(double a, double b) { return std::fmin(a, b); }
 static inline double max_num(double a, double b) { return std::fmax(a, b); }
@@ -366,7 +402,7 @@ static void mark_big(std::vector<DWide>& wide, const std::vector<uint8_t>& is_bi
             if (c != kWideEmpty && (c & kWideLeaf) && is_big[c & kWideSlotMask]) c |= kWideBig;
 }
 
-static void prepare_any_order(FlatScene* out) {
+static void prepare_any_order(const Switches& sw, FlatScene* out) {
     out->any_ok = false;
     out->n_big = 0;
     const size_t n = out->prims.size();
@@ -432,8 +468,7 @@ static void prepare_any_order(FlatScene* out) {
     // 4.26 nodes per primary ray, 4 ms of build), no gain on the bunny fields (15.4 instead of 15.6 nodes, 1.5 s of build for
     // 2.5 M leaves) - so only scenes below kFreeTreeLeaves get it by default. It holds only the primitives that are not big: those
     // are tested before the walk starts, and left out the root box no longer spans the ground sphere that every ray enters.
-    const char* fv = std::getenv("RTP_FREE_TREE");
-    const bool want_free = fv ? std::atoi(fv) != 0 : n < kFreeTreeLeaves;
+    const bool want_free = sw.free_tree >= 0 ? sw.free_tree != 0 : n < kFreeTreeLeaves;
     const size_t m = n - out->n_big;
     if (!want_free || n < 2 || m == 0) return;
     double lo[3] = {1e300, 1e300, 1e300}, hi[3] = {-1e300, -1e300, -1e300};
@@ -589,7 +624,7 @@ struct NestedFlattener {
     }
 };
 
-int flatten_scene(const rtp_scene_desc* d, FlatScene* out, bool device_build) {
+int flatten_scene(const rtp_scene_desc* d, const Switches& sw, FlatScene* out, bool device_build) {
     if (!d || !out) return set_error(RTP_ERR_INVALID, "null scene description");
     if (d->abi_version != RTP_ABI_VERSION) return set_error(RTP_ERR_INVALID, "rtp_scene_desc.abi_version mismatch");
     if (d->root_kind > RTP_ROOT_LIST) return set_error(RTP_ERR_INVALID, "unknown root kind");
@@ -600,10 +635,9 @@ int flatten_scene(const rtp_scene_desc* d, FlatScene* out, bool device_build) {
         return set_error(RTP_ERR_INVALID, "Bvh::new on an empty list is unreachable!() in the reference (bvh.rs:40)");
     if (d->n_hittables >= kWideSlotMask) return set_error(RTP_ERR_INVALID, "too many hittables");
 
-    const bool timing = std::getenv("RTP_BUILD_TIMING") != nullptr;  // phase times of the host build on stderr
     auto t0 = std::chrono::steady_clock::now();
     auto lap = [&](const char* what) {
-        if (!timing) return;
+        if (!sw.build_timing) return;
         auto t1 = std::chrono::steady_clock::now();
         std::fprintf(stderr, "[rtp build] %s: %.3f s\n", what, std::chrono::duration<double>(t1 - t0).count());
         t0 = t1;
@@ -664,11 +698,10 @@ int flatten_scene(const rtp_scene_desc* d, FlatScene* out, bool device_build) {
     // Big flat Bvh scenes are built on the device from here on (rtp_build.cu device_build_scene): leaf boxes, reference order, SAH
     // culling tree, records, 4-wide collapse and the any-order tables never exist on the host. RTP_DEVICE_BUILD: "0" never,
     // "1" always (tests compare both builds), unset: scenes of >= 65,536 leaves.
-    if (device_build && !nested && d->root_kind == RTP_ROOT_BVH && n >= 2 && !(std::getenv("RTP_TREE") && std::string(std::getenv("RTP_TREE")) == "reference")) {
-        const char* dev_env = std::getenv("RTP_DEVICE_BUILD");
-        if (dev_env ? std::atoi(dev_env) != 0 : n >= 65536u) {
+    if (device_build && !nested && d->root_kind == RTP_ROOT_BVH && n >= 2 && !sw.reference_tree) {
+        if (sw.device_build >= 0 ? sw.device_build != 0 : n >= 65536u) {
             lap("tables and validation");
-            const int rc = device_build_scene(d, out, timing);
+            const int rc = device_build_scene(d, sw, out);
             if (rc == RTP_OK) { lap("device build"); return RTP_OK; }
             if (rc != 1) return rc;
             // 1: not applicable (inverted or non-finite boxes): the host path below keeps the reference topology for such scenes
@@ -770,8 +803,7 @@ int flatten_scene(const rtp_scene_desc* d, FlatScene* out, bool device_build) {
             for (int k = 0; k < 3; ++k)
                 if (!(it.bmin[k] <= it.bmax[k]) || !std::isfinite(it.bmin[k]) || !std::isfinite(it.bmax[k])) regular = false;
         if (!regular) out->boxes_finite = false;
-        const char* tree = std::getenv("RTP_TREE");  // "reference" keeps the median-split topology on the device (A/B runs, counter parity)
-        if (regular && !(tree && std::string(tree) == "reference")) {
+        if (regular && !sw.reference_tree) {  // RTP_TREE=reference keeps the median-split topology on the device (A/B runs, counter parity)
             SeqBuilder sb{items, out->nodes};
             sb.build(0, n, 0, 1, 4);
             out->device_depth = sb.depth.load();
@@ -835,7 +867,7 @@ int flatten_scene(const rtp_scene_desc* d, FlatScene* out, bool device_build) {
             if (nd.prim != kNoPrim) nd.kind = nested ? prim_h[nd.prim]->kind : d->hittables[items[nd.prim].id].kind;
         build_wide(out->nodes, &out->wide, &out->wide_boxes, &out->wide_depth);
         lap("4-wide collapse");
-        prepare_any_order(out);
+        prepare_any_order(sw, out);
         lap(out->free_wide.empty() ? "any-order walk tables" : "any-order walk tables and the order-free culling tree");
     } else {
         // a List root is traversed as a flat run of leaves without slab tests; nodes carry only the kind

@@ -116,7 +116,7 @@ struct DSceneView {  // passed by value to kernels
     uint32_t any_order;    // 1: eligible rays of this scene use it
     uint32_t any_cap;      // entries of the per-lane any-order stack
     uint32_t n_big;        // primitives exempt from distance culling (the outsized ones: extent above 16x the median), at most kMaxBig
-    uint32_t _pad_any;
+    uint32_t fast_slab;    // 1: every box is finite and ordered, so eligible rays may use the sign-selected slab test (collide_fast)
     uint32_t big[8];       // their slots | kind << 31
     double any_E;          // largest box extent of a triangle that is not big
     double any_A;          // largest |coordinate| of such a triangle
@@ -180,6 +180,29 @@ struct FlatScene {
 // error plumbing (rtp_host.cpp)
 int set_error(int code, const std::string& msg);
 
+// The library's RTP_* environment switches (INTEGRATION.md), all read by read_switches (rtp_host.cpp) and parsed one way: a 0/1
+// switch is on when it is set and atoi of its value is not 0, a number is clamped to its range, a word is compared exactly. A
+// scene reads them once when it is created and keeps them; rtp_bvh_build_order and rtp_bvh_culled_set read them when called.
+// RTP_PATH_BUDGET is the one switch read per render call (read_path_budget), so that a scene's frames may be split differently.
+struct Switches {
+    bool any_order = true;          // RTP_TRAVERSAL: "inorder" keeps every ray in the reference's visiting order
+    bool f32_culling = true;        // RTP_F32_CULLING=0: exact f64 slab tests at every node, and no any-order walk
+    bool simple_trace = false;      // RTP_TRACE_KERNEL=simple: one thread per ray
+    bool simple_render = false;     // RTP_RENDER_KERNEL=simple: one thread per path
+    bool reference_tree = false;    // RTP_TREE=reference: keep the median-split topology on the device
+    int free_tree = -1;             // RTP_FREE_TREE 0 / 1; -1 (unset): scenes below 262,144 leaves get the order-free tree
+    int device_build = -1;          // RTP_DEVICE_BUILD 0 / 1; -1 (unset): scenes of at least 65,536 leaves are built on the device
+    uint32_t any_cap = 0;           // RTP_ANY_CAP, 4..48 entries of the any-order stack; 0 (unset): from the tree's depth
+    bool any_setup_cull = true;     // RTP_ANY_SETUP_CULL=0: every any-order ray walks
+    uint32_t tail_threshold = 65536;  // RTP_TAIL_THRESHOLD: a launch of at most this many paths runs in tail mode (0 = never)
+    uint32_t chunk_log2 = 18;       // RTP_CHUNK_LOG2, 10..24: a host-buffer batch goes to the device in chunks of 2^this rays
+    bool build_timing = false;      // RTP_BUILD_TIMING: phase times of the scene build on stderr
+    bool debug_sync = false;        // RTP_DEBUG_SYNC: synchronise after every integrator launch
+    bool lane_stats = false;        // RTP_LANE_STATS: lane occupancy of counted calls on stderr
+};
+Switches read_switches();
+size_t read_path_budget();  // RTP_PATH_BUDGET, 1..2^31 paths per integrator launch; 0: unset
+
 // An exact f64 box as the f32 culling box of a DWide child: rounded outward and inflated by 2^-21 * max(|min|, |max|) per axis
 // (DESIGN.md §4; rtp_host.cpp)
 void round_out(const double* bmin, const double* bmax, float* lo, float* hi);
@@ -188,7 +211,7 @@ void culled_set_box(const double* lo, const double* hi, float* cull);
 
 // host layer
 // device_build: build a large flat Bvh scene on the GPU (rtp_build.cu device_build_scene); host-only callers pass false
-int flatten_scene(const rtp_scene_desc* desc, FlatScene* out, bool device_build = false);
+int flatten_scene(const rtp_scene_desc* desc, const Switches& sw, FlatScene* out, bool device_build = false);
 
 // device layer (rtp_device.cu, rtp_build.cu)
 struct DeviceScene;
@@ -198,10 +221,10 @@ int device_reference_order_dev(const double* d_boxes, uint32_t n, uint32_t* d_or
 // The whole of flatten_scene's geometry part on the current device for a flat (un-nested) Bvh scene: leaf boxes, the reference's
 // depth-first order, the SAH culling tree over that order, primitive / attribute records, the 4-wide collapse and the any-order
 // tables. Fills out->dev and the host-side metadata. Returns RTP_OK, a negative status, or 1 = "not applicable, use the host
-// path" (irregular boxes). `timing`: phase times on stderr.
-int device_build_scene(const rtp_scene_desc* d, FlatScene* out, bool timing);
+// path" (irregular boxes). sw.build_timing: phase times on stderr.
+int device_build_scene(const rtp_scene_desc* d, const Switches& sw, FlatScene* out);
 void device_free_arrays(DevArrays* a);
-int device_scene_upload(const FlatScene& flat, int device /* < 0: the bound device */, DeviceScene** out);
+int device_scene_upload(const FlatScene& flat, const Switches& sw, int device /* < 0: the bound device */, DeviceScene** out);
 void device_scene_free(DeviceScene* ds);
 uint64_t device_scene_bytes(const DeviceScene* ds);
 

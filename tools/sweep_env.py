@@ -1,6 +1,6 @@
 """A/B runner: times C2 (1920x1080 primary batch) and C3 (2^22 incoherent rays) on the bunny under several environment
 settings in one process (the library reads its RTP_* switches when a scene is created).
-    python tools/sweep_env.py "RTP_ANY_CAP=12" "RTP_ANY_CAP=16,RTP_REFILL_MIN=8" ...
+    python tools/sweep_env.py "RTP_ANY_CAP=12" "RTP_ANY_CAP=16,RTP_FREE_TREE=0" ...
 The first configuration is always the default (no overrides). Checks every configuration's hits against the first."""
 import os
 import sys
