@@ -350,6 +350,17 @@ int rtp_trace_closest_device(rtp_scene* scene, const rtp_ray* d_rays, size_t n, 
 int rtp_trace_closest_device_counted(rtp_scene* scene, const rtp_ray* d_rays, size_t n, rtp_hit* d_hits_out,
                                      rtp_stats* stats);
 
+/* ---------------------------------------------------------------- occlusion ------------- */
+
+/* scene.hit(ray).is_some() (hittable.rs:18-25, bvh.rs:121-124): occluded_out[i] = 1 iff ray i hits a primitive with
+ * t_min <= t <= t_max, else 0 -- bit for bit rtp_trace_closest(...).leaf != RTP_MISS. The walk stops at the first accepted leaf.
+ * Host buffers, staged and dealt out over the scene's devices like rtp_trace_closest; stats as there. */
+int rtp_trace_occluded(rtp_scene* scene, const rtp_ray* rays, size_t n, uint8_t* occluded_out, rtp_stats* stats);
+/* scene.hit(ray).is_some() for rays/results in device memory, as rtp_trace_closest_device: asynchronous on `cuda_stream`. */
+int rtp_trace_occluded_device(rtp_scene* scene, const rtp_ray* d_rays, size_t n, uint8_t* d_occluded_out, void* cuda_stream);
+/* scene.hit(ray).is_some() with the work counters of rtp_stats filled in, as rtp_trace_closest_device_counted. Synchronous. */
+int rtp_trace_occluded_device_counted(rtp_scene* scene, const rtp_ray* d_rays, size_t n, uint8_t* d_occluded_out, rtp_stats* stats);
+
 /* render.rs:32-52 `Camera::shoot` for pixel-centre samples u=(i+0.5)/W, v=(j+0.5)/H of a W×H
  * frame with lens_radius treated as 0 (no random draw): writes W*H rays, i fastest, into
  * device memory. Used to build the primary-ray batch on the device. */

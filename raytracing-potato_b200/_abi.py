@@ -198,6 +198,9 @@ PROTOTYPES = {
     "rtp_trace_closest_full": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, _P(Stats)]),
     "rtp_trace_closest_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p]),
     "rtp_trace_closest_device_counted": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, _P(Stats)]),
+    "rtp_trace_occluded": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, _P(Stats)]),
+    "rtp_trace_occluded_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p]),
+    "rtp_trace_occluded_device_counted": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, _P(Stats)]),
     "rtp_camera_rays_device": (C.c_int, [_P(Camera), C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p]),
     "rtp_camera_rays": (C.c_int, [_P(Camera), C.c_uint32, C.c_uint32, C.c_void_p]),
     "rtp_render": (C.c_int, [C.c_void_p, _P(Camera), _P(RenderParams), C.c_void_p, C.c_void_p, _P(Stats)]),

@@ -608,6 +608,25 @@ class Scene:
         _check(self._lib, self._lib.rtp_trace_closest_device_counted(self._h, d_rays, n, d_hits, C.byref(st)))
         return st
 
+    # -- scene.hit(ray).is_some() (hittable.rs:18-25, bvh.rs:121-124): does the ray hit anything in [t_min, t_max] --
+    def occluded(self, rays: np.ndarray, out: Optional[np.ndarray] = None, stats: bool = False):
+        """bool array, one entry per ray: equal to hit(rays)["leaf"] != MISS; the walk stops at the first accepted leaf"""
+        rays = _as_rays(rays)
+        occ = out if out is not None else np.empty(len(rays), dtype=np.bool_)
+        assert occ.dtype == np.bool_ and occ.flags.c_contiguous and len(occ) >= len(rays), "out must be a contiguous bool array"
+        st = A.Stats()
+        _check(self._lib, self._lib.rtp_trace_occluded(self._h, A.ptr(rays), len(rays), A.ptr(occ), C.byref(st) if stats else None))
+        return (occ, st) if stats else occ
+
+    def occluded_device(self, d_rays: int, n: int, d_out: int, stream: int = 0) -> None:
+        """d_out: n bytes of device memory, 1 = occluded, 0 = not"""
+        _check(self._lib, self._lib.rtp_trace_occluded_device(self._h, d_rays, n, d_out, stream))
+
+    def occluded_device_counted(self, d_rays: int, n: int, d_out: int) -> A.Stats:
+        st = A.Stats()
+        _check(self._lib, self._lib.rtp_trace_occluded_device_counted(self._h, d_rays, n, d_out, C.byref(st)))
+        return st
+
     # -- main.rs:61-92 --
     def render(self, width: int, height: int, num_samples: int, max_bounce: int = 8, seed: int = 1, camera: Optional[Camera] = None,
                sample_range=None, tile=None, flags: int = 0, out=None, foreground: bool = True, rows=None, device_mask: int = 0):

@@ -332,7 +332,8 @@ struct alignas(16) WaveHit {
 };
 static_assert(sizeof(WaveHit) == 32, "WaveHit must be 32 bytes");
 
-enum { OUT_HIT = 0, OUT_FULL = 1, OUT_WAVE = 2, OUT_TAIL = 3 };
+// OUT_OCCLUDED: one byte per ray, 1 iff the ray hits anything (the in-order kernel stops at the first accepted leaf, DESIGN.md §2c)
+enum { OUT_HIT = 0, OUT_FULL = 1, OUT_WAVE = 2, OUT_TAIL = 3, OUT_OCCLUDED = 4 };
 
 template <int OUT>
 __device__ __forceinline__ void write_hit(const DSceneView& sc, void* __restrict__ out, size_t i, D3 o, D3 d, const HitRec& h) {
@@ -357,6 +358,8 @@ __device__ __forceinline__ void write_hit(const DSceneView& sc, void* __restrict
         double2* w = reinterpret_cast<double2*>(static_cast<WaveHit*>(out) + i);
         w[0] = make_double2(h.t, h.u);
         w[1] = make_double2(h.v, __hiloint2double(0, static_cast<int>(h.slot == kNoPrim ? kNoPrim : (h.slot | (h.kind << 31)))));
+    } else if (OUT == OUT_OCCLUDED) {
+        static_cast<uint8_t*>(out)[i] = h.slot != kNoPrim ? 1u : 0u;
     } else {
         uint4 w;
         if (h.slot != kNoPrim) {
@@ -401,10 +404,10 @@ __device__ __forceinline__ void flush_counters(Counters* counters, const LocalCo
     }
 }
 
-// Baseline kernel: one thread per ray, no regrouping. Kept for A/B runs (RTP_TRACE_KERNEL=simple).
-template <bool COUNT, bool FULL>
-__global__ void __launch_bounds__(128) trace_closest_kernel(DSceneView sc, const rtp_ray* __restrict__ rays, size_t n, void* __restrict__ out,
-                                                            Counters* counters) {
+// Baseline kernels: one thread per ray, no regrouping. Kept for A/B runs (RTP_TRACE_KERNEL=simple).
+template <bool COUNT, int OUT>
+__device__ __forceinline__ void trace_closest_one(const DSceneView& sc, const rtp_ray* __restrict__ rays, size_t n, void* __restrict__ out,
+                                                  Counters* counters) {
     const size_t i = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
     LocalCounters lc = {0, 0, 0, 0, 0, 0, 0};
     if (i < n) {
@@ -414,9 +417,22 @@ __global__ void __launch_bounds__(128) trace_closest_kernel(DSceneView sc, const
         HitRec h;
         h.t = r3.y; h.u = 0.0; h.v = 0.0; h.kind = 0;
         closest_hit<COUNT>(sc, o, d, r3.x, h, lc);
-        write_hit<FULL ? OUT_FULL : OUT_HIT>(sc, out, i, o, d, h);
+        write_hit<OUT>(sc, out, i, o, d, h);
     }
     flush_counters<COUNT>(counters, lc);
+}
+
+template <bool COUNT, bool FULL>
+__global__ void __launch_bounds__(128) trace_closest_kernel(DSceneView sc, const rtp_ray* __restrict__ rays, size_t n, void* __restrict__ out,
+                                                            Counters* counters) {
+    trace_closest_one<COUNT, FULL ? OUT_FULL : OUT_HIT>(sc, rays, n, out, counters);
+}
+
+// occlusion: the closest hit, then `slot != kNoPrim`, which is the definition of the answer itself
+template <bool COUNT>
+__global__ void __launch_bounds__(128) trace_occluded_simple_kernel(DSceneView sc, const rtp_ray* __restrict__ rays, size_t n, void* __restrict__ out,
+                                                                    Counters* counters) {
+    trace_closest_one<COUNT, OUT_OCCLUDED>(sc, rays, n, out, counters);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1318,7 +1334,12 @@ __global__ void __launch_bounds__(128, OUT == OUT_TAIL ? 4 : kTraceBlocksPerSM) 
         }
 
         // ---- leaves: exact gate + primitive test for the parked lanes --------------------------------
-        if (w.prim != kNoPrim) walker_leaf<COUNT>(w, sc, lc);
+        if (w.prim != kNoPrim) {
+            walker_leaf<COUNT>(w, sc, lc);
+            // occlusion: T stays ray.t_max until the first accept, so that accept answers the ray (DESIGN.md §2c). The walk or
+            // List scan ends and the second pending leaf is dropped; the lane retires at the next refill.
+            if (OUT == OUT_OCCLUDED && w.h.slot != kNoPrim) { w.next = kEnd; w.prim = kNoPrim; }
+        }
     }
 
     flush_counters<COUNT>(counters, lc);
@@ -2107,7 +2128,7 @@ static DCamera make_camera(const rtp_camera* c) {
     return d;
 }
 
-// One traversal launch. out_mode: OUT_HIT / OUT_FULL / OUT_WAVE. n_dev != nullptr: the batch size is read from device memory
+// One traversal launch. out_mode: OUT_HIT / OUT_FULL / OUT_WAVE / OUT_TAIL / OUT_OCCLUDED. n_dev != nullptr: the batch size is read from device memory
 // (wavefront integrator) and `n` is only an upper bound used to size the grid.
 // RTP_DEBUG_SYNC=1: synchronise after every launch of the integrator and name the kernel that faulted
 static int debug_sync(const DeviceScene* ds, cudaStream_t st, const char* what, uint32_t bounce) {
@@ -2129,6 +2150,9 @@ static int launch_trace(DeviceScene* ds, const rtp_ray* d_rays, size_t n, void* 
         if (out_mode == OUT_FULL) {
             if (count) trace_closest_kernel<true, true><<<g, block, 0, stream>>>(ds->view, d_rays, n, d_out, counters);
             else trace_closest_kernel<false, true><<<g, block, 0, stream>>>(ds->view, d_rays, n, d_out, counters);
+        } else if (out_mode == OUT_OCCLUDED) {
+            if (count) trace_occluded_simple_kernel<true><<<g, block, 0, stream>>>(ds->view, d_rays, n, d_out, counters);
+            else trace_occluded_simple_kernel<false><<<g, block, 0, stream>>>(ds->view, d_rays, n, d_out, counters);
         } else {
             if (count) trace_closest_kernel<true, false><<<g, block, 0, stream>>>(ds->view, d_rays, n, d_out, counters);
             else trace_closest_kernel<false, false><<<g, block, 0, stream>>>(ds->view, d_rays, n, d_out, counters);
@@ -2139,8 +2163,8 @@ static int launch_trace(DeviceScene* ds, const rtp_ray* d_rays, size_t n, void* 
         const bool list = ds->view.root_kind != RTP_ROOT_BVH;
         const TailArgs ta = tail ? *tail : TailArgs{};
         // which kernel: the any-order kernel + a deferred in-order launch (eligible scenes), or the in-order kernel alone (List roots,
-        // scenes outside the preconditions, tail-mode launches)
-        const bool pure_any = !list && ds->any_order && out_mode != OUT_TAIL;
+        // scenes outside the preconditions, tail-mode launches, occlusion queries: with T fixed the walk order does not matter)
+        const bool pure_any = !list && ds->any_order && out_mode != OUT_TAIL && out_mode != OUT_OCCLUDED;
         if (n > 0xFFFFFFFEull && pure_any) return set_error(RTP_ERR_INVALID, "ray batch too large for one launch");
 
         std::lock_guard<std::mutex> guard(ds->launch_lock);
@@ -2211,6 +2235,7 @@ static int launch_trace(DeviceScene* ds, const rtp_ray* d_rays, size_t n, void* 
             if (out_mode == OUT_FULL) RTP_LAUNCH_PERSISTENT_O(OUT_FULL);
             else if (out_mode == OUT_WAVE) RTP_LAUNCH_PERSISTENT_O(OUT_WAVE);
             else if (out_mode == OUT_TAIL) RTP_LAUNCH_PERSISTENT_O(OUT_TAIL);
+            else if (out_mode == OUT_OCCLUDED) RTP_LAUNCH_PERSISTENT_O(OUT_OCCLUDED);
             else RTP_LAUNCH_PERSISTENT_O(OUT_HIT);
 #undef RTP_LAUNCH_PERSISTENT_O
 #undef RTP_LAUNCH_PERSISTENT
@@ -2229,13 +2254,14 @@ static int launch_trace(DeviceScene* ds, const rtp_ray* d_rays, size_t n, void* 
 // lives on several devices (rtp_scene_create_multi) deals its chunks out to them round-robin, so every device's host link carries
 // a share of the 80 B/ray stream. Chunks are independent: no exchange between devices.
 // `camera` != nullptr: the rays are pixel-centre camera rays generated on the device chunk by chunk (rtp_trace_camera)
-static int trace_host(rtp_scene* scene, const rtp_ray* rays, size_t n, void* hits_out, bool full, rtp_stats* stats, const DCamera* camera = nullptr,
+// out_mode: OUT_HIT (16 B rtp_hit), OUT_FULL (80 B rtp_hit_full) or OUT_OCCLUDED (1 B) records
+static int trace_host(rtp_scene* scene, const rtp_ray* rays, size_t n, void* hits_out, int out_mode, rtp_stats* stats, const DCamera* camera = nullptr,
                       uint32_t width = 0, uint32_t height = 0) {
     const std::vector<DeviceScene*>& devs = scene->devs;
     const size_t N = devs.size();
     std::vector<std::unique_lock<std::mutex>> locks;
     for (DeviceScene* ds : devs) locks.emplace_back(ds->lock);
-    const size_t hit_bytes = full ? sizeof(rtp_hit_full) : sizeof(rtp_hit);
+    const size_t hit_bytes = out_mode == OUT_FULL ? sizeof(rtp_hit_full) : out_mode == OUT_OCCLUDED ? sizeof(uint8_t) : sizeof(rtp_hit);
     const bool count = stats != nullptr;
     const size_t chunk = size_t(1) << devs[0]->sw.chunk_log2;  // rays per pipeline stage: 2^18 (16 MiB of rays) unless RTP_CHUNK_LOG2 says otherwise
     const size_t n_chunks = (n + chunk - 1) / chunk;
@@ -2269,7 +2295,7 @@ static int trace_host(rtp_scene* scene, const rtp_ray* rays, size_t n, void* hit
             }
         }
         if (e != cudaSuccess) { rc = set_error(RTP_ERR_CUDA, std::string("trace chunk: ") + cudaGetErrorString(e)); break; }
-        rc = launch_trace(ds, ds->stage_rays[k], m, ds->stage_hits[k], full ? OUT_FULL : OUT_HIT, false, count ? ds->counters : nullptr, st);
+        rc = launch_trace(ds, ds->stage_rays[k], m, ds->stage_hits[k], out_mode, false, count ? ds->counters : nullptr, st);
         if (rc != RTP_OK) break;
         launches += ds->last_trace_launches;
         e = cudaMemcpyAsync(static_cast<char*>(hits_out) + off * hit_bytes, ds->stage_hits[k], m * hit_bytes, cudaMemcpyDeviceToHost, st);
@@ -2807,14 +2833,14 @@ int rtp_trace_closest(rtp_scene* scene, const rtp_ray* rays, size_t n, rtp_hit* 
     if (!scene || (n && (!rays || !hits_out))) return set_error(RTP_ERR_INVALID, "null argument");
     if (stats) std::memset(stats, 0, sizeof *stats);
     if (n == 0) return RTP_OK;
-    return trace_host(scene, rays, n, hits_out, false, stats);
+    return trace_host(scene, rays, n, hits_out, OUT_HIT, stats);
 }
 
 int rtp_trace_closest_full(rtp_scene* scene, const rtp_ray* rays, size_t n, rtp_hit_full* hits_out, rtp_stats* stats) {
     if (!scene || (n && (!rays || !hits_out))) return set_error(RTP_ERR_INVALID, "null argument");
     if (stats) std::memset(stats, 0, sizeof *stats);
     if (n == 0) return RTP_OK;
-    return trace_host(scene, rays, n, hits_out, true, stats);
+    return trace_host(scene, rays, n, hits_out, OUT_FULL, stats);
 }
 
 int rtp_trace_camera(rtp_scene* scene, const rtp_camera* camera, uint32_t width, uint32_t height, rtp_hit* hits_out, rtp_stats* stats) {
@@ -2823,7 +2849,7 @@ int rtp_trace_camera(rtp_scene* scene, const rtp_camera* camera, uint32_t width,
     const size_t n = static_cast<size_t>(width) * height;
     if (n == 0) return RTP_OK;
     const DCamera cam = make_camera(camera);
-    return trace_host(scene, nullptr, n, hits_out, false, stats, &cam, width, height);
+    return trace_host(scene, nullptr, n, hits_out, OUT_HIT, stats, &cam, width, height);
 }
 
 int rtp_trace_closest_device(rtp_scene* scene, const rtp_ray* d_rays, size_t n, rtp_hit* d_hits_out, void* cuda_stream) {
@@ -2833,15 +2859,14 @@ int rtp_trace_closest_device(rtp_scene* scene, const rtp_ray* d_rays, size_t n, 
 }
 
 /* Counting variant used by tests and the roofline report: node visits / primitive tests for a device-resident batch. */
-int rtp_trace_closest_device_counted(rtp_scene* scene, const rtp_ray* d_rays, size_t n, rtp_hit* d_hits_out, rtp_stats* stats) {
-    if (!scene || !stats || (n && (!d_rays || !d_hits_out))) return set_error(RTP_ERR_INVALID, "null argument");
+static int trace_device_counted(rtp_scene* scene, const rtp_ray* d_rays, size_t n, void* d_out, int out_mode, rtp_stats* stats) {
     DeviceScene* ds = scene->dev;
     std::lock_guard<std::mutex> guard(ds->lock);
     RTP_CUDA(cudaSetDevice(ds->device));
     cudaStream_t st = ds->streams[0];
     RTP_CUDA(cudaMemsetAsync(ds->counters, 0, sizeof(Counters), st));
     RTP_CUDA(cudaEventRecord(ds->ev_begin, st));
-    int rc = launch_trace(ds, d_rays, n, d_hits_out, OUT_HIT, true, ds->counters, st);
+    int rc = launch_trace(ds, d_rays, n, d_out, out_mode, true, ds->counters, st);
     if (rc != RTP_OK) return rc;
     RTP_CUDA(cudaEventRecord(ds->ev_end, st));
     RTP_CUDA(cudaEventSynchronize(ds->ev_end));
@@ -2857,6 +2882,33 @@ int rtp_trace_closest_device_counted(rtp_scene* scene, const rtp_ray* d_rays, si
     stats->rays = c.rays; stats->node_visits = c.node_visits; stats->triangle_tests = c.triangle_tests; stats->sphere_tests = c.sphere_tests; stats->leaf_gates = c.leaf_gates; stats->conservative_violations = c.violations; stats->order_rewalks = c.rewalks;
     stats->device_ms = ms; stats->kernel_launches = 1;
     return RTP_OK;
+}
+
+int rtp_trace_closest_device_counted(rtp_scene* scene, const rtp_ray* d_rays, size_t n, rtp_hit* d_hits_out, rtp_stats* stats) {
+    if (!scene || !stats || (n && (!d_rays || !d_hits_out))) return set_error(RTP_ERR_INVALID, "null argument");
+    return trace_device_counted(scene, d_rays, n, d_hits_out, OUT_HIT, stats);
+}
+
+// Occlusion (DESIGN.md §2c): the in-order walk with T fixed at ray.t_max, stopped at the first accepted leaf; one byte per ray
+int rtp_trace_occluded(rtp_scene* scene, const rtp_ray* rays, size_t n, uint8_t* occluded_out, rtp_stats* stats) {
+    if (!scene || (n && (!rays || !occluded_out))) return set_error(RTP_ERR_INVALID, "null argument");
+    if (stats) std::memset(stats, 0, sizeof *stats);
+    if (n == 0) return RTP_OK;
+    return trace_host(scene, rays, n, occluded_out, OUT_OCCLUDED, stats);
+}
+
+int rtp_trace_occluded_device(rtp_scene* scene, const rtp_ray* d_rays, size_t n, uint8_t* d_occluded_out, void* cuda_stream) {
+    if (!scene || (n && (!d_rays || !d_occluded_out))) return set_error(RTP_ERR_INVALID, "null argument");
+    if (n == 0) return RTP_OK;
+    RTP_CUDA(cudaSetDevice(scene->dev->device));
+    return launch_trace(scene->dev, d_rays, n, d_occluded_out, OUT_OCCLUDED, false, nullptr, static_cast<cudaStream_t>(cuda_stream));
+}
+
+int rtp_trace_occluded_device_counted(rtp_scene* scene, const rtp_ray* d_rays, size_t n, uint8_t* d_occluded_out, rtp_stats* stats) {
+    if (!scene || !stats || (n && (!d_rays || !d_occluded_out))) return set_error(RTP_ERR_INVALID, "null argument");
+    std::memset(stats, 0, sizeof *stats);
+    if (n == 0) return RTP_OK;
+    return trace_device_counted(scene, d_rays, n, d_occluded_out, OUT_OCCLUDED, stats);
 }
 
 int rtp_camera_rays_device(const rtp_camera* camera, uint32_t width, uint32_t height, rtp_ray* d_rays_out, void* cuda_stream) {

@@ -42,6 +42,7 @@ extern "C" {
     fn rtp_scene_create_multi(desc: *const rtp_scene_desc, device_mask: u32, out: *mut *mut rtp_scene) -> c_int;
     fn rtp_scene_destroy(scene: *mut rtp_scene);
     fn rtp_trace_closest(scene: *mut rtp_scene, rays: *const rtp_ray, n: usize, hits: *mut rtp_hit, stats: *mut rtp_stats) -> c_int;
+    fn rtp_trace_occluded(scene: *mut rtp_scene, rays: *const rtp_ray, n: usize, occluded: *mut u8, stats: *mut rtp_stats) -> c_int;
     fn rtp_render(scene: *mut rtp_scene, camera: *const rtp_camera, params: *const rtp_render_params,
                   rgb: *mut f64, foreground: *mut f64, stats: *mut rtp_stats) -> c_int;
 }
@@ -114,11 +115,24 @@ impl GpuScene {
     /// Batched `Hittable::hit` on the root (bvh.rs:121-124 / hittable.rs:110-120): `hits[k].leaf` = index of the root item that holds
     /// the winner (u32::MAX on a miss), `.material` its MaterialId, `.t` = Hit::t.
     pub fn hit_batch(&self, rays: &[Ray]) -> GpuResult<Vec<rtp_hit>> {
-        let rs: Vec<rtp_ray> = rays.iter().map(|r| rtp_ray { origin: [r.origin.x, r.origin.y, r.origin.z],
-            direction: [r.direction.x, r.direction.y, r.direction.z], t_min: r.t_min, t_max: r.t_max }).collect();
+        let rs = Self::rays(rays);
         let mut hits = vec![rtp_hit { leaf: u32::MAX, material: u32::MAX, t: f64::INFINITY }; rs.len()];
         check(unsafe { rtp_trace_closest(self.0, rs.as_ptr(), rs.len(), hits.as_mut_ptr(), std::ptr::null_mut()) })?;
         Ok(hits)
+    }
+
+    /// `scene.hit(ray).is_some()` (hittable.rs:18-25, bvh.rs:121-124) for a batch: true iff the ray hits anything with
+    /// t_min <= t <= t_max, bit for bit `hit_batch(..)[k].leaf != u32::MAX`; the walk stops at the first accepted leaf.
+    pub fn occluded(&self, rays: &[Ray]) -> GpuResult<Vec<bool>> {
+        let rs = Self::rays(rays);
+        let mut occ = vec![0u8; rs.len()];
+        check(unsafe { rtp_trace_occluded(self.0, rs.as_ptr(), rs.len(), occ.as_mut_ptr(), std::ptr::null_mut()) })?;
+        Ok(occ.into_iter().map(|b| b != 0).collect())
+    }
+
+    fn rays(rays: &[Ray]) -> Vec<rtp_ray> {
+        rays.iter().map(|r| rtp_ray { origin: [r.origin.x, r.origin.y, r.origin.z],
+            direction: [r.direction.x, r.direction.y, r.direction.z], t_min: r.t_min, t_max: r.t_max }).collect()
     }
 
     fn camera(camera: &Camera) -> rtp_camera {
