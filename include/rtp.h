@@ -391,6 +391,37 @@ int rtp_render_device(rtp_scene* scene, const rtp_camera* camera, const rtp_rend
                       double* d_rgb_out, double* d_foreground_out, rtp_stats* stats,
                       void* cuda_stream);
 
+/* ---------------------------------------------------------------- adaptive render ------- */
+
+/* Stop rule of rtp_render_adaptive. */
+typedef struct rtp_adaptive_params {
+    uint32_t min_samples; /* samples of every pixel in round 1 (>= 1)                                       */
+    uint32_t max_samples; /* no pixel takes more (>= min_samples)                                           */
+    uint32_t batch;       /* samples per later round (>= 1); the last round may take fewer                   */
+    uint32_t _pad;
+    double abs_tol;       /* the standard error of a pixel's mean luminance must fall to abs_tol + rel_tol * |mean| */
+    double rel_tol;       /*   (both finite and >= 0)                                                        */
+} rtp_adaptive_params;
+
+/* rtp_render that stops each pixel once its mean has converged (DESIGN.md §6b). The tile rectangle and rows of `params` are rendered
+ * in rounds: round 1 traces samples [0, min_samples) of every pixel, each later round the next min(batch, max_samples - n) samples
+ * of every pixel still live. After every round each live pixel with n samples evaluates, in f64 without contraction, over its
+ * per-sample luminance Y_s = (0.2126 * r_s + 0.7152 * g_s) + 0.0722 * b_s summed in sample order from 0.0:
+ *     S1 = Σ Y_s, S2 = Σ Y_s * Y_s, nd = n, mean = S1 / nd, var = (S2 - S1 * mean) / (nd - 1.0), tol = abs_tol + rel_tol * fabs(mean)
+ *     stop = n >= max_samples || (n >= 2 && var / nd <= tol * tol)
+ * and a pixel that stops takes no further samples (a NaN or infinite sample keeps its pixel going to max_samples).
+ * With n_p the final count of pixel p: rgb_out / foreground_out hold Σ_{s < n_p} / n_p (the sums with RTP_RENDER_RAW_SUMS), bit for
+ * bit rtp_render(num_samples = n_p, sample range [0, n_p)) at p; samples_out[p] = n_p (may be NULL, as may foreground_out). Layout,
+ * tile, rows, seed, max_bounce and device_mask as rtp_render; only pixels of the tile rectangle and rows are written, and a frame
+ * split over several devices is bit-identical to one device. params->num_samples, sample_begin and sample_end must be 0 and flags
+ * a subset of RTP_RENDER_RAW_SUMS | RTP_RENDER_COUNTERS. stats->paths = Σ n_p; the other fields as rtp_render. Host buffers. */
+int rtp_render_adaptive(rtp_scene* scene, const rtp_camera* camera, const rtp_render_params* params, const rtp_adaptive_params* adaptive,
+                        double* rgb_out, double* foreground_out, uint32_t* samples_out, rtp_stats* stats);
+/* Same with device buffers on the scene's first device. SYNCHRONOUS: every round reads one live count back, and the call returns
+ * when its work on `cuda_stream` (NULL = the legacy default stream) is done. */
+int rtp_render_adaptive_device(rtp_scene* scene, const rtp_camera* camera, const rtp_render_params* params, const rtp_adaptive_params* adaptive,
+                               double* d_rgb_out, double* d_foreground_out, uint32_t* d_samples_out, rtp_stats* stats, void* cuda_stream);
+
 /* ---------------------------------------------------------------- random stream --------- */
 
 /* The counter-based generator that replaces `Randomizer = StdRng` (randomness.rs:5):

@@ -131,6 +131,17 @@ class RenderParams(C.Structure):
     ]
 
 
+class AdaptiveParams(C.Structure):
+    _fields_ = [
+        ("min_samples", C.c_uint32),
+        ("max_samples", C.c_uint32),
+        ("batch", C.c_uint32),
+        ("_pad", C.c_uint32),
+        ("abs_tol", C.c_double),
+        ("rel_tol", C.c_double),
+    ]
+
+
 class Stats(C.Structure):
     _fields_ = [
         ("rays", C.c_uint64),
@@ -205,6 +216,10 @@ PROTOTYPES = {
     "rtp_camera_rays": (C.c_int, [_P(Camera), C.c_uint32, C.c_uint32, C.c_void_p]),
     "rtp_render": (C.c_int, [C.c_void_p, _P(Camera), _P(RenderParams), C.c_void_p, C.c_void_p, _P(Stats)]),
     "rtp_render_device": (C.c_int, [C.c_void_p, _P(Camera), _P(RenderParams), C.c_void_p, C.c_void_p, _P(Stats), C.c_void_p]),
+    "rtp_render_adaptive": (C.c_int, [C.c_void_p, _P(Camera), _P(RenderParams), _P(AdaptiveParams), C.c_void_p, C.c_void_p, C.c_void_p, _P(Stats)]),
+    "rtp_render_adaptive_device": (
+        C.c_int, [C.c_void_p, _P(Camera), _P(RenderParams), _P(AdaptiveParams), C.c_void_p, C.c_void_p, C.c_void_p, _P(Stats), C.c_void_p]
+    ),
     "rtp_render_srgb8": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "rtp_trace_camera": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p]),
     "rtp_rng_draws": (C.c_int, [C.c_uint64, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p]),

@@ -454,6 +454,13 @@ def render_params(width, height, num_samples, max_bounce=8, seed=1, sample_begin
     return p
 
 
+def adaptive_params(min_samples, max_samples, batch, abs_tol=0.0, rel_tol=0.01) -> A.AdaptiveParams:
+    """the stop rule of rtp_render_adaptive (include/rtp.h)"""
+    a = A.AdaptiveParams()
+    a.min_samples, a.max_samples, a.batch, a.abs_tol, a.rel_tol = min_samples, max_samples, batch, abs_tol, rel_tol
+    return a
+
+
 # ------------------------------------------------------------------------------ device scene -----
 
 
@@ -656,6 +663,40 @@ class Scene:
         cc = cam.to_c()
         _check(self._lib, self._lib.rtp_render_srgb8(self._h, C.byref(cc), C.byref(p), A.ptr(rgba), C.byref(st)))
         return rgba, st
+
+    def render_adaptive(self, width: int, height: int, min_samples: int, max_samples: int, batch: int, abs_tol: float = 0.0, rel_tol: float = 0.01,
+                        max_bounce: int = 8, seed: int = 1, camera: Optional[Camera] = None, tile=None, rows=None, raw_sums: bool = False,
+                        device_mask: int = 0, out=None, counters: bool = False):
+        """render() that stops each pixel once the standard error of its mean luminance is at most abs_tol + rel_tol * |mean|
+        (rtp_render_adaptive). Returns (rgb [h, w, 3], foreground [h, w], samples [h, w] uint32, stats): every pixel equals
+        render(samples[p], sample_range=(0, samples[p])) at p. out: a triple (rgb, foreground or None, samples or None) of caller
+        buffers; pixels outside the tile and rows are left as they are."""
+        cam = camera or self.camera
+        cam = Camera(width / height, cam.fov, cam.focal_dist, cam.lens_radius, cam.transformation)  # main.rs:22 overrides the aspect
+        p = render_params(width, height, 0, max_bounce, seed, 0, 0, tile,
+                          (A.RENDER_RAW_SUMS if raw_sums else 0) | (A.RENDER_COUNTERS if counters else 0), rows, device_mask)
+        a = adaptive_params(min_samples, max_samples, batch, abs_tol, rel_tol)
+        if out is not None:
+            rgbf, fg, samples = out
+        else:
+            rgbf = np.zeros((height, width, 3), dtype=np.float64)
+            fg = np.zeros((height, width), dtype=np.float64)
+            samples = np.zeros((height, width), dtype=np.uint32)
+        st = A.Stats()
+        cc = cam.to_c()
+        _check(self._lib, self._lib.rtp_render_adaptive(self._h, C.byref(cc), C.byref(p), C.byref(a), A.ptr(rgbf),
+                                                        A.ptr(fg) if fg is not None else None, A.ptr(samples) if samples is not None else None,
+                                                        C.byref(st)))
+        return rgbf, fg, samples, st
+
+    def render_adaptive_device(self, params: A.RenderParams, adaptive: A.AdaptiveParams, camera: Camera, d_rgb: int, d_fg: int = 0,
+                               d_samples: int = 0, stream: int = 0, stats: bool = False):
+        """rtp_render_adaptive_device: device buffers on the scene's first device; returns when the frame is done"""
+        st = A.Stats()
+        cc = camera.to_c()
+        _check(self._lib, self._lib.rtp_render_adaptive_device(self._h, C.byref(cc), C.byref(params), C.byref(adaptive), d_rgb, d_fg or None,
+                                                               d_samples or None, C.byref(st) if stats else None, stream or None))
+        return st
 
     def render_device(self, params: A.RenderParams, camera: Camera, d_rgb: int, d_fg: int = 0, stream: int = 0, stats: bool = False):
         st = A.Stats()

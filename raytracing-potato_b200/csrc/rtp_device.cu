@@ -7,6 +7,7 @@
 //
 // Reference citations are file:line under /root/reference/src.
 
+#include <cub/device/device_select.cuh>
 #include <cuda_runtime.h>
 #include <math_constants.h>
 
@@ -876,13 +877,28 @@ struct DRender {
     unsigned long long seed;
 };
 
-// path p of a launch = (tile pixel p / n_samples, sample p % n_samples): the samples of one pixel sit in adjacent lanes,
+// Which tile pixel the k-th pixel slot of a launch is, as a compile-time policy of the integrator kernels. A launch has
+// map.count(rp) slots; the tile pixel index is row-major over the rows of this launch (rp.tile_w wide).
+struct DenseTile {  // rtp_render: every pixel of the tile rectangle, slot k = tile pixel k
+    __device__ __forceinline__ size_t count(const DRender& rp) const { return static_cast<size_t>(rp.tile_w) * rp.tile_h; }
+    __device__ __forceinline__ uint32_t pixel(uint32_t k) const { return k; }
+};
+struct LiveList {   // rtp_render_adaptive: the pixels still sampling in this round, slot k = tile pixel live[k]
+    const uint32_t* live;
+    uint32_t n;
+    __device__ __forceinline__ size_t count(const DRender&) const { return n; }
+    __device__ __forceinline__ uint32_t pixel(uint32_t k) const { return __ldg(live + k); }
+};
+
+// path p of a launch = (pixel slot p / n_samples, sample p % n_samples): the samples of one pixel sit in adjacent lanes,
 // so a warp's primary rays are as coherent as they can be
-__device__ __forceinline__ void path_coords(const DRender& rp, size_t p, uint32_t& i, uint32_t& j, uint32_t& smp) {
+template <class Map>
+__device__ __forceinline__ void path_coords(const DRender& rp, const Map& map, size_t p, uint32_t& i, uint32_t& j, uint32_t& smp) {
     // a launch holds at most 32 Mi paths (render_enqueue): 32-bit divisions (the 64-bit ones were 3.6 % of the shade kernel)
     const uint32_t p32 = static_cast<uint32_t>(p);
-    const uint32_t pix = p32 / rp.n_samples;
-    smp = rp.sample_begin + (p32 - pix * rp.n_samples);
+    const uint32_t k = p32 / rp.n_samples;
+    smp = rp.sample_begin + (p32 - k * rp.n_samples);
+    const uint32_t pix = map.pixel(k);
     const uint32_t row = pix / rp.tile_w;
     i = rp.tile_x + (pix - row * rp.tile_w);
     j = rp.tile_y + rp.row_offset + row * rp.row_stride;
@@ -970,16 +986,16 @@ __device__ __forceinline__ bool shade_vertex(const DSceneView& sc, D3& o, D3& d,
 
 // Baseline integrator: one thread per camera path, whole bounce loop in one thread, exact f64 stack-free walk.
 // Kept for A/B runs (RTP_RENDER_KERNEL=simple) and as the second implementation the wavefront path is tested against.
-template <int MAXB, bool COUNT>
+template <int MAXB, bool COUNT, class Map>
 __global__ void __launch_bounds__(128) render_paths_kernel(DSceneView sc, DCamera cam, DRender rp, double4* __restrict__ scratch,
-                                                            Counters* counters) {
-    const size_t npix = static_cast<size_t>(rp.tile_w) * rp.tile_h;
+                                                            Counters* counters, Map map) {
+    const size_t npix = map.count(rp);
     const size_t total = npix * rp.n_samples;
     const size_t p = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
     LocalCounters lc = {0, 0, 0, 0, 0, 0, 0};
     if (p < total) {
         uint32_t i, j, smp;
-        path_coords(rp, p, i, j, smp);
+        path_coords(rp, map, p, i, j, smp);
         Rng rng;
         rng_init(rng, rp.seed, j * rp.width + i, smp, RTP_RNG_STREAM_PATH);
         D3 o, d;
@@ -1036,12 +1052,13 @@ struct WaveQueues {
     size_t capacity;             // paths per launch the buffers were sized for (stride of `stack`)
 };
 
-__global__ void __launch_bounds__(256) wave_generate_kernel(DCamera cam, DRender rp, WaveQueues wq, size_t total) {
+template <class Map>
+__global__ void __launch_bounds__(256) wave_generate_kernel(DCamera cam, DRender rp, WaveQueues wq, size_t total, Map map) {
     const size_t p = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
     if (p == 0) wq.count[0] = total;
     if (p >= total) return;
     uint32_t i, j, smp;
-    path_coords(rp, p, i, j, smp);
+    path_coords(rp, map, p, i, j, smp);
     Rng rng;
     rng_init(rng, rp.seed, j * rp.width + i, smp, RTP_RNG_STREAM_PATH);
     D3 o, d;
@@ -1065,7 +1082,9 @@ __device__ __noinline__ void trace_deferred(const DSceneView& sc, D3 o, D3 d, Hi
 }
 
 constexpr int kShadeBlocks = 3;  // resident blocks per SM wave_shade_kernel is built for, and its grid
-__global__ void __launch_bounds__(256, kShadeBlocks) wave_shade_kernel(DSceneView sc, DRender rp, WaveQueues wq, uint32_t bounce, double4* __restrict__ scratch) {
+template <class Map>
+__global__ void __launch_bounds__(256, kShadeBlocks) wave_shade_kernel(DSceneView sc, DRender rp, WaveQueues wq, uint32_t bounce, double4* __restrict__ scratch,
+                                                                       Map map) {
     const size_t n = static_cast<size_t>(wq.count[bounce]);
     const int cur = bounce & 1, nxt = cur ^ 1;
     const unsigned lane = threadIdx.x & 31u;
@@ -1098,7 +1117,7 @@ __global__ void __launch_bounds__(256, kShadeBlocks) wave_shade_kernel(DSceneVie
             } else {
                 if (bounce == 0) first_hit = 1u;
                 uint32_t i, j, smp;
-                path_coords(rp, p, i, j, smp);
+                path_coords(rp, map, p, i, j, smp);
                 Rng rng;
                 rng_init(rng, rp.seed, j * rp.width + i, smp, RTP_RNG_STREAM_PATH);
                 rng.k = st.y;
@@ -1235,7 +1254,7 @@ __global__ void __launch_bounds__(128, OUT == OUT_TAIL ? 4 : kTraceBlocksPerSM) 
                     } else {
                         if (depth == ta.rp.max_bounce) first_hit = 1u;  // the path's first segment (render.rs:102-122)
                         uint32_t pi, pj, smp;
-                        path_coords(ta.rp, p, pi, pj, smp);
+                        path_coords(ta.rp, DenseTile{}, p, pi, pj, smp);  // tail mode serves rtp_render only
                         Rng rng;
                         rng_init(rng, ta.rp.seed, pj * ta.rp.width + pi, smp, RTP_RNG_STREAM_PATH);
                         rng.k = pst.y;
@@ -1794,6 +1813,77 @@ __global__ void __launch_bounds__(256) write_frame_kernel(const double4* __restr
     if (fg) fg[px] = a.w;
 }
 
+// ---------------------------------------------------------------------------------------------
+// rtp_render_adaptive (DESIGN.md §6b). Per tile pixel: acc (the colour / foreground sums of resolve_kernel), the luminance
+// moments (Σ Y, Σ Y²) and the sample count; per live slot a keep flag. Every sum starts at 0.0 and runs in sample order, so a
+// pixel that stops after n samples holds the bits rtp_render's resolve_kernel holds for the sample range [0, n).
+// ---------------------------------------------------------------------------------------------
+
+struct StopRule {
+    double abs_tol, rel_tol;
+    uint32_t max_samples, _pad;
+};
+
+__global__ void __launch_bounds__(256) adaptive_init_kernel(double4* __restrict__ acc, double2* __restrict__ moments, uint32_t* __restrict__ count,
+                                                            uint32_t* __restrict__ live, size_t npix) {
+    const size_t pix = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+    if (pix >= npix) return;
+    acc[pix] = make_double4(0.0, 0.0, 0.0, 0.0);
+    moments[pix] = make_double2(0.0, 0.0);
+    count[pix] = 0u;
+    live[pix] = static_cast<uint32_t>(pix);
+}
+
+// One launch of a round: for live slot k, the launch's samples of tile pixel live[k] (scratch[k * n_samples + s], path_coords)
+// are folded into its sums in sample order. On the round's last launch the stop rule decides keep[k].
+__global__ void __launch_bounds__(256) adaptive_resolve_kernel(const double4* __restrict__ scratch, const uint32_t* __restrict__ live, uint32_t n_live,
+                                                               uint32_t n_samples, double4* __restrict__ acc, double2* __restrict__ moments,
+                                                               uint32_t* __restrict__ count, uint8_t* __restrict__ keep, int last_launch, StopRule rule) {
+    const size_t k = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+    if (k >= n_live) return;
+    const uint32_t pix = live[k];
+    double4 a = acc[pix];
+    double2 m = moments[pix];
+    for (uint32_t s = 0; s < n_samples; ++s) {
+        const double4 c = scratch[k * n_samples + s];
+        a.x += c.x; a.y += c.y; a.z += c.z; a.w += c.w;
+        const double y = (0.2126 * c.x + 0.7152 * c.y) + 0.0722 * c.z;
+        m.x += y; m.y += y * y;
+    }
+    acc[pix] = a;
+    moments[pix] = m;
+    const uint32_t n = count[pix] + n_samples;
+    count[pix] = n;
+    if (last_launch) {
+        const double nd = static_cast<double>(n);
+        const double mean = m.x / nd;
+        const double var = (m.y - m.x * mean) / (nd - 1.0);
+        const double tol = rule.abs_tol + rule.rel_tol * fabs(mean);
+        const bool stop = n >= rule.max_samples || (n >= 2u && var / nd <= tol * tol);  // NaN / inf: false, the pixel goes on
+        keep[k] = stop ? 0 : 1;
+    }
+}
+
+// write_frame_kernel with each pixel's own divisor: its sample count (no division with RTP_RENDER_RAW_SUMS)
+__global__ void __launch_bounds__(256) adaptive_write_kernel(const double4* __restrict__ acc, const uint32_t* __restrict__ count, DRender rp, int raw_sums,
+                                                             double* __restrict__ rgb, double* __restrict__ fg, uint32_t* __restrict__ samples) {
+    const size_t npix = static_cast<size_t>(rp.tile_w) * rp.tile_h;
+    const size_t pix = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+    if (pix >= npix) return;
+    const uint32_t i = rp.tile_x + static_cast<uint32_t>(pix % rp.tile_w);
+    const uint32_t j = rp.tile_y + rp.row_offset + static_cast<uint32_t>(pix / rp.tile_w) * rp.row_stride;
+    const size_t px = static_cast<size_t>(i) + static_cast<size_t>(j) * rp.width;
+    double4 a = acc[pix];
+    const uint32_t n = count[pix];
+    if (!raw_sums) {
+        const double divisor = static_cast<double>(n);
+        a.x = a.x / divisor; a.y = a.y / divisor; a.z = a.z / divisor; a.w = a.w / divisor;
+    }
+    rgb[3 * px + 0] = a.x; rgb[3 * px + 1] = a.y; rgb[3 * px + 2] = a.z;
+    if (fg) fg[px] = a.w;
+    if (samples) samples[px] = n;
+}
+
 // Output stage (main.rs:110-122 + utility.rs:212-220 to_srgb_u8): colour = sum / divisor, clamp, gamma 1/2.2, `as u8`;
 // alpha = 255, or (255 * foreground) as u8 with RTP_RENDER_TRANSPARENT. CUDA's pow and the host libm's powf may differ in
 // the last ulps, which matters only when 255 * x^(1/2.2) lands within 1e-9 of an integer: those pixels (a handful per
@@ -1899,7 +1989,13 @@ struct DeviceScene {
     void* stage_hits[kPipeDepth] = {nullptr, nullptr, nullptr};
     double4* scratch = nullptr; size_t scratch_elems = 0;
     double4* acc = nullptr; size_t acc_elems = 0;
-    WaveQueues wave{};                 // wavefront integrator queues (render_device), grown on demand
+    // rtp_render_adaptive, per tile pixel and grown like acc: luminance moments (16 B), sample count (4 B), keep flag (1 B), two live-list entries (8 B): 29 B beside acc's 32.
+    // The live count of a round goes through n_live to a pinned word that the host reads.
+    double2* moments = nullptr; uint32_t* counts = nullptr; uint8_t* keep = nullptr; uint32_t* live[2] = {nullptr, nullptr};
+    size_t adaptive_elems = 0;
+    void* select_tmp = nullptr; size_t select_tmp_bytes = 0;  // cub::DeviceSelect::Flagged
+    uint32_t* n_live = nullptr; uint32_t* n_live_host = nullptr;
+    WaveQueues wave{};                // wavefront integrator queues (render_device), grown on demand
     uint32_t wave_bounces = 0;         // stack depth the queues were sized for
     int shade_blocks = 0;              // grid of wave_shade_kernel
     // memory the integrator's per-launch buffers may take (set at upload from the free HBM). A render call sizes its launches
@@ -1908,6 +2004,7 @@ struct DeviceScene {
     // frame at depth 128: a 204 GB stack), so wave_reserve then reallocates them for the call alone.
     size_t queue_budget_bytes = size_t(4) << 30;
     double* frame = nullptr; size_t frame_elems = 0;
+    uint32_t* frame_samples = nullptr; size_t frame_samples_elems = 0;  // rtp_render_adaptive's samples_out
     uchar4* frame8 = nullptr; size_t frame8_elems = 0;  // RGBA8 output stage
     SrgbFix* fixes = nullptr; unsigned int* n_fixes = nullptr;
     unsigned int n_fix_host = 0;       // n_fixes of the last rtp_render_srgb8, copied back with the frame
@@ -1940,6 +2037,9 @@ void device_scene_free(DeviceScene* ds) {
     if (ds->ev_end) cudaEventDestroy(ds->ev_end);
     for (cudaEvent_t ev : ds->ev_pool) cudaEventDestroy(ev);
     if (ds->render_done) cudaEventDestroy(ds->render_done);
+    cudaFree(ds->moments); cudaFree(ds->counts); cudaFree(ds->keep); cudaFree(ds->live[0]); cudaFree(ds->live[1]);
+    cudaFree(ds->select_tmp); cudaFree(ds->n_live); cudaFree(ds->frame_samples);
+    if (ds->n_live_host) cudaFreeHost(ds->n_live_host);
     cudaFree(ds->scratch); cudaFree(ds->acc); cudaFree(ds->frame); cudaFree(ds->frame8); cudaFree(ds->fixes); cudaFree(ds->n_fixes);
     cudaFree(ds->wave.rays[0]); cudaFree(ds->wave.rays[1]); cudaFree(ds->wave.state[0]); cudaFree(ds->wave.state[1]);
     cudaFree(ds->wave.hits); cudaFree(ds->wave.stack); cudaFree(ds->wave.count);
@@ -2329,12 +2429,12 @@ static int trace_host(rtp_scene* scene, const rtp_ray* rays, size_t n, void* hit
     return rc;
 }
 
-template <int MAXB>
-static void launch_render_paths(DeviceScene* ds, const DCamera& cam, const DRender& rp, size_t total, bool count, cudaStream_t st) {
+template <int MAXB, class Map>
+static void launch_render_paths(DeviceScene* ds, const DCamera& cam, const DRender& rp, const Map& map, size_t total, bool count, cudaStream_t st) {
     const unsigned block = 128;
     const dim3 g(static_cast<unsigned>((total + block - 1) / block));
-    if (count) render_paths_kernel<MAXB, true><<<g, block, 0, st>>>(ds->view, cam, rp, ds->scratch, ds->counters);
-    else render_paths_kernel<MAXB, false><<<g, block, 0, st>>>(ds->view, cam, rp, ds->scratch, ds->counters);
+    if (count) render_paths_kernel<MAXB, true><<<g, block, 0, st>>>(ds->view, cam, rp, ds->scratch, ds->counters, map);
+    else render_paths_kernel<MAXB, false><<<g, block, 0, st>>>(ds->view, cam, rp, ds->scratch, ds->counters, map);
 }
 
 // bytes per path of one launch of the wavefront integrator: queues (2 rays, 2 states, a hit record: 176 B), the [bounce][path]
@@ -2384,11 +2484,14 @@ static cudaEvent_t next_mark(DeviceScene* ds, cudaStream_t st) {
     return ev;
 }
 
-static int render_enqueue(DeviceScene* ds, const rtp_camera* camera, const rtp_render_params* p, double* d_rgb, double* d_fg, bool want_stats,
-                          cudaStream_t st, uchar4* d_rgba8 = nullptr) {
+// The pixels a render call covers: checks the frame, tile and row parameters shared by rtp_render and rtp_render_adaptive and
+// returns the DRender of the call (tile_h = rows of the tile rectangle this call renders; sample range still unset).
+// fixed_spp: rtp_render's sample range is checked too (rtp_render_adaptive checks its own).
+static int render_rect(const rtp_render_params* p, bool fixed_spp, DRender* rp) {
     if (p->max_bounce < 1) return set_error(RTP_ERR_INVALID, "assert!(depth >= 1) (render.rs:97)");
     if (p->max_bounce > 128) return set_error(RTP_ERR_UNSUPPORTED, "max_bounce > 128");
-    if (p->width == 0 || p->height == 0 || p->sample_end < p->sample_begin || p->num_samples == 0) return set_error(RTP_ERR_INVALID, "bad frame parameters");
+    if (p->width == 0 || p->height == 0 || (fixed_spp && (p->sample_end < p->sample_begin || p->num_samples == 0)))
+        return set_error(RTP_ERR_INVALID, "bad frame parameters");
     if (static_cast<uint64_t>(p->width) * p->height > 0xFFFFFFFFull) return set_error(RTP_ERR_INVALID, "frame too large");
     const uint32_t tx = p->tile_x, ty = p->tile_y;
     if (tx >= p->width || ty >= p->height) return set_error(RTP_ERR_INVALID, "tile outside frame");
@@ -2397,6 +2500,92 @@ static int render_enqueue(DeviceScene* ds, const rtp_camera* camera, const rtp_r
     const uint32_t rs = p->row_stride ? p->row_stride : 1u, ro = p->row_offset;
     if (ro >= rs) return set_error(RTP_ERR_INVALID, "row_offset must be below row_stride");
     const uint32_t th = ro < th_full ? (th_full - ro + rs - 1u) / rs : 0u;  // rows of the tile rectangle this call renders
+    rp->width = p->width; rp->height = p->height; rp->max_bounce = p->max_bounce;
+    rp->tile_x = tx; rp->tile_y = ty; rp->tile_w = tw; rp->tile_h = th;
+    rp->row_offset = ro; rp->row_stride = rs;
+    rp->sample_begin = 0; rp->n_samples = 0;
+    rp->_pad = 0; rp->seed = p->seed;
+    return RTP_OK;
+}
+
+// Paths per launch of the integrator for a call with max_bounce `bounces`: up to 32 Mi paths (wavefront queues 176 B + 48 B x
+// max_bounce per path, scratch 32 B), within the memory budget fixed when the scene was uploaded (a sixth of the free HBM, at most
+// 24 GiB). Big launches matter: every launch pays the fill and drain of ~2 x max_bounce kernels and the latency-bound sparse late
+// bounces once (1080p x 64 spp of the C4 scene: 111 ms in 16 launches of 8 Mi paths, 92 ms in 4 launches of 32 Mi)
+static size_t path_budget(const DeviceScene* ds, uint32_t bounces) {
+    const size_t per_path = ds->sw.simple_render ? 32 : wave_path_bytes(bounces);
+    size_t budget = std::max<size_t>(size_t(1) << 20, std::min<size_t>(size_t(32) << 20, ds->queue_budget_bytes / per_path));
+    if (const size_t forced = read_path_budget()) budget = forced;  // tests: force several launches per frame
+    return budget;
+}
+
+// the integrator's per-launch buffers for launches of up to `need` paths
+static int reserve_paths(DeviceScene* ds, size_t need, uint32_t bounces) {
+    if (!ds->sw.simple_render) {
+        int rc = wave_reserve(ds, need, bounces);
+        if (rc != RTP_OK) return rc;
+    }
+    if (ds->scratch_elems < need) {
+        cudaFree(ds->scratch); ds->scratch = nullptr; ds->scratch_elems = 0;
+        RTP_CUDA(cudaMalloc(reinterpret_cast<void**>(&ds->scratch), need * sizeof(double4)));
+        ds->scratch_elems = need;
+    }
+    return RTP_OK;
+}
+
+// One launch of the integrator: the `total` paths of rp's sample range over the pixel slots of `map`, traced to their end; path p's
+// colour and foreground land in ds->scratch[p]. Adds the kernels it queued to *launches.
+template <class Map>
+static int launch_paths(DeviceScene* ds, const DCamera& cam, const DRender& rp, const Map& map, size_t total, bool count, bool want_stats,
+                        cudaStream_t st, size_t* launches) {
+    if (ds->sw.simple_render) {
+        if (rp.max_bounce <= 8) launch_render_paths<8>(ds, cam, rp, map, total, count, st);
+        else if (rp.max_bounce <= 32) launch_render_paths<32>(ds, cam, rp, map, total, count, st);
+        else launch_render_paths<128>(ds, cam, rp, map, total, count, st);
+        RTP_CUDA(cudaGetLastError());
+        ++*launches;
+        return RTP_OK;
+    }
+    // generate -> (trace -> shade) x max_bounce; queue sizes stay on the device
+    RTP_CUDA(cudaMemsetAsync(ds->wave.count, 0, 130 * sizeof(unsigned long long), st));
+    wave_generate_kernel<<<static_cast<unsigned>((total + 255) / 256), 256, 0, st>>>(cam, rp, ds->wave, total, map);
+    RTP_CUDA(cudaGetLastError());
+    ++*launches;
+    { int rc = debug_sync(ds, st, "wave_generate_kernel", 0); if (rc != RTP_OK) return rc; }
+    const unsigned shade_grid = static_cast<unsigned>(std::min<size_t>(static_cast<size_t>(ds->shade_blocks), (total + 255) / 256));
+    for (uint32_t b = 0; b < rp.max_bounce; ++b) {
+        int rc;
+        // a launch of at most tail_threshold paths (a 32x32 tile of main.rs:32, say) runs as generate + ONE tail-mode launch.
+        // Offering every later queue of a big launch to the tail kernel was measured on C1 to be no faster than trace/shade
+        // pairs, and so was handing the sparse late bounces to one tail launch chosen from the previous launch's queue sizes
+        // (19 -> 12 launches per C1 frame, same 2.05 ms): a late bounce costs the latency of ONE ray segment (~30 us of
+        // dependent instructions, tools/small_batches.py), not a launch. Tail mode maps paths to pixels densely: rtp_render only.
+        if (want_stats) next_mark(ds, st);  // even marks open a traversal span, odd marks close it
+        if (std::is_same<Map, DenseTile>::value && ds->sw.tail_threshold && total <= ds->sw.tail_threshold) {
+            TailArgs ta{ds->wave, rp, ds->scratch, b};
+            rc = launch_trace(ds, ds->wave.rays[b & 1], total, nullptr, OUT_TAIL, count, ds->counters, st, ds->wave.count + b, &ta);
+            if (rc != RTP_OK) return rc;
+            ++*launches;
+            if (want_stats) next_mark(ds, st);
+            break;
+        }
+        rc = launch_trace(ds, ds->wave.rays[b & 1], total, ds->wave.hits, OUT_WAVE, count, ds->counters, st, ds->wave.count + b);
+        if (rc != RTP_OK) return rc;
+        if (want_stats) next_mark(ds, st);
+        if ((rc = debug_sync(ds, st, "trace kernel <OUT_WAVE>", b)) != RTP_OK) return rc;
+        wave_shade_kernel<<<shade_grid, 256, 0, st>>>(ds->view, rp, ds->wave, b, ds->scratch, map);
+        RTP_CUDA(cudaGetLastError());
+        if ((rc = debug_sync(ds, st, "wave_shade_kernel", b)) != RTP_OK) return rc;
+        *launches += ds->last_trace_launches + 1;
+    }
+    return RTP_OK;
+}
+
+static int render_enqueue(DeviceScene* ds, const rtp_camera* camera, const rtp_render_params* p, double* d_rgb, double* d_fg, bool want_stats,
+                          cudaStream_t st, uchar4* d_rgba8 = nullptr) {
+    DRender rp;
+    if (int rc = render_rect(p, true, &rp)) return rc;
+    const uint32_t tw = rp.tile_w, th = rp.tile_h;
 
     // the scratch below is shared by every render on this scene: a render queued on another stream must be over first
     if (ds->render_pending) RTP_CUDA(cudaStreamWaitEvent(st, ds->render_done, 0));
@@ -2411,24 +2600,10 @@ static int render_enqueue(DeviceScene* ds, const rtp_camera* camera, const rtp_r
     }
     if (npix == 0) return RTP_OK;  // no row of the rectangle falls to this call
     const uint32_t ns_total = p->sample_end - p->sample_begin;
-    // samples per launch: up to 32 Mi paths (wavefront queues 176 B + 48 B x max_bounce per path, scratch 32 B), within the memory
-    // budget fixed when the scene was uploaded (a sixth of the free HBM, at most 24 GiB). Big launches matter: every launch pays
-    // the fill and drain of ~2 x max_bounce kernels and the latency-bound sparse late bounces once (1080p x 64 spp of the C4
-    // scene: 111 ms in 16 launches of 8 Mi paths, 92 ms in 4 launches of 32 Mi)
-    const bool wave = !ds->sw.simple_render;
-    const size_t per_path = wave ? wave_path_bytes(p->max_bounce) : 32;
-    size_t path_budget = std::max<size_t>(size_t(1) << 20, std::min<size_t>(size_t(32) << 20, ds->queue_budget_bytes / per_path));
-    if (const size_t forced = read_path_budget()) path_budget = forced;  // tests: force several launches per frame
-    uint32_t per_launch = static_cast<uint32_t>(std::max<size_t>(1, std::min<size_t>(ns_total ? ns_total : 1, path_budget / npix)));
-    const size_t need = npix * per_launch;
-    if (wave && ns_total) {
-        int rc = wave_reserve(ds, need, p->max_bounce);
+    const uint32_t per_launch = static_cast<uint32_t>(std::max<size_t>(1, std::min<size_t>(ns_total ? ns_total : 1, path_budget(ds, p->max_bounce) / npix)));
+    if (ns_total) {
+        int rc = reserve_paths(ds, npix * per_launch, p->max_bounce);
         if (rc != RTP_OK) return rc;
-    }
-    if (ds->scratch_elems < need) {
-        cudaFree(ds->scratch); ds->scratch = nullptr; ds->scratch_elems = 0;
-        RTP_CUDA(cudaMalloc(reinterpret_cast<void**>(&ds->scratch), need * sizeof(double4)));
-        ds->scratch_elems = need;
     }
     if (ds->acc_elems < npix) {
         cudaFree(ds->acc); ds->acc = nullptr; ds->acc_elems = 0;
@@ -2437,11 +2612,6 @@ static int render_enqueue(DeviceScene* ds, const rtp_camera* camera, const rtp_r
     }
     const bool count = (p->flags & RTP_RENDER_COUNTERS) != 0;
     const DCamera cam = make_camera(camera);
-    DRender rp;
-    rp.width = p->width; rp.height = p->height; rp.max_bounce = p->max_bounce;
-    rp.tile_x = tx; rp.tile_y = ty; rp.tile_w = tw; rp.tile_h = th;
-    rp.row_offset = ro; rp.row_stride = rs;
-    rp._pad = 0; rp.seed = p->seed;
 
     if (!want_stats) RTP_CUDA(cudaMemsetAsync(ds->counters, 0, sizeof(Counters), st));
     size_t launches = 0;
@@ -2450,47 +2620,8 @@ static int render_enqueue(DeviceScene* ds, const rtp_camera* camera, const rtp_r
     for (uint32_t s0 = 0; s0 < ns_total; s0 += per_launch) {
         rp.sample_begin = p->sample_begin + s0;
         rp.n_samples = std::min(per_launch, ns_total - s0);
-        const size_t total = npix * rp.n_samples;
-        if (wave) {
-            // generate -> (trace -> shade) x max_bounce; queue sizes stay on the device
-            RTP_CUDA(cudaMemsetAsync(ds->wave.count, 0, 130 * sizeof(unsigned long long), st));
-            wave_generate_kernel<<<static_cast<unsigned>((total + 255) / 256), 256, 0, st>>>(cam, rp, ds->wave, total);
-            RTP_CUDA(cudaGetLastError());
-            ++launches;
-            { int rc = debug_sync(ds, st, "wave_generate_kernel", 0); if (rc != RTP_OK) return rc; }
-            const unsigned shade_grid = static_cast<unsigned>(std::min<size_t>(static_cast<size_t>(ds->shade_blocks), (total + 255) / 256));
-            for (uint32_t b = 0; b < p->max_bounce; ++b) {
-                int rc;
-                // a launch of at most tail_threshold paths (a 32x32 tile of main.rs:32, say) runs as generate + ONE tail-mode launch.
-                // Offering every later queue of a big launch to the tail kernel was measured on C1 to be no faster than trace/shade
-                // pairs, and so was handing the sparse late bounces to one tail launch chosen from the previous launch's queue sizes
-                // (19 -> 12 launches per C1 frame, same 2.05 ms): a late bounce costs the latency of ONE ray segment (~30 us of
-                // dependent instructions, tools/small_batches.py), not a launch.
-                if (want_stats) next_mark(ds, st);  // even marks open a traversal span, odd marks close it
-                if (ds->sw.tail_threshold && total <= ds->sw.tail_threshold) {
-                    TailArgs ta{ds->wave, rp, ds->scratch, b};
-                    rc = launch_trace(ds, ds->wave.rays[b & 1], total, nullptr, OUT_TAIL, count, ds->counters, st, ds->wave.count + b, &ta);
-                    if (rc != RTP_OK) return rc;
-                    ++launches;
-                    if (want_stats) next_mark(ds, st);
-                    break;
-                }
-                rc = launch_trace(ds, ds->wave.rays[b & 1], total, ds->wave.hits, OUT_WAVE, count, ds->counters, st, ds->wave.count + b);
-                if (rc != RTP_OK) return rc;
-                if (want_stats) next_mark(ds, st);
-                if ((rc = debug_sync(ds, st, "trace kernel <OUT_WAVE>", b)) != RTP_OK) return rc;
-                wave_shade_kernel<<<shade_grid, 256, 0, st>>>(ds->view, rp, ds->wave, b, ds->scratch);
-                RTP_CUDA(cudaGetLastError());
-                if ((rc = debug_sync(ds, st, "wave_shade_kernel", b)) != RTP_OK) return rc;
-                launches += ds->last_trace_launches + 1;
-            }
-        } else {
-            if (p->max_bounce <= 8) launch_render_paths<8>(ds, cam, rp, total, count, st);
-            else if (p->max_bounce <= 32) launch_render_paths<32>(ds, cam, rp, total, count, st);
-            else launch_render_paths<128>(ds, cam, rp, total, count, st);
-            RTP_CUDA(cudaGetLastError());
-            ++launches;
-        }
+        int rc = launch_paths(ds, cam, rp, DenseTile{}, npix * rp.n_samples, count, want_stats, st, &launches);
+        if (rc != RTP_OK) return rc;
         resolve_kernel<<<static_cast<unsigned>((npix + 255) / 256), 256, 0, st>>>(ds->scratch, ds->acc, npix, rp.n_samples, first ? 1 : 0);
         RTP_CUDA(cudaGetLastError());
         ++launches;
@@ -2540,6 +2671,199 @@ static int render_device(rtp_scene* scene, const rtp_camera* camera, const rtp_r
     int rc = render_enqueue(ds, camera, p, d_rgb, d_fg, stats != nullptr, st, d_rgba8);
     if (rc != RTP_OK) return rc;
     return stats ? render_finish(ds, stats) : RTP_OK;
+}
+
+static void add_stats(rtp_stats* total, const rtp_stats& one) {
+    total->rays += one.rays; total->paths += one.paths; total->node_visits += one.node_visits; total->triangle_tests += one.triangle_tests;
+    total->sphere_tests += one.sphere_tests; total->leaf_gates += one.leaf_gates; total->conservative_violations += one.conservative_violations;
+    total->order_rewalks += one.order_rewalks; total->kernel_launches += one.kernel_launches;
+    total->device_ms = std::max(total->device_ms, one.device_ms);  // the devices run side by side
+    total->trace_ms = std::max(total->trace_ms, one.trace_ms); total->shade_ms = std::max(total->shade_ms, one.shade_ms);
+}
+
+// ---------------------------------------------------------------------------------------------
+// rtp_render_adaptive (DESIGN.md §6b): rounds of samples over the pixels that are still live. Round 1 traces samples
+// [0, min_samples) of every pixel, each later round the next min(batch, max_samples - n) samples of the live pixels. A round is
+// split into launches by the path budget like rtp_render's sample range, each launch followed by adaptive_resolve_kernel; the last
+// one decides the keep flags, a stable select builds the next live list and its length is read back. Tail mode is not used: it
+// maps paths to pixels densely.
+// ---------------------------------------------------------------------------------------------
+
+static int check_adaptive(const rtp_render_params* p, const rtp_adaptive_params* a) {
+    if (a->min_samples == 0 || a->min_samples > a->max_samples || a->batch == 0)
+        return set_error(RTP_ERR_INVALID, "adaptive: need 0 < min_samples <= max_samples and batch > 0");
+    if (!(a->abs_tol >= 0.0) || !(a->rel_tol >= 0.0) || std::isinf(a->abs_tol) || std::isinf(a->rel_tol))
+        return set_error(RTP_ERR_INVALID, "adaptive: abs_tol and rel_tol must be finite and >= 0");
+    if (p->num_samples || p->sample_begin || p->sample_end)
+        return set_error(RTP_ERR_INVALID, "adaptive: the call owns the sample range; num_samples, sample_begin and sample_end must be 0");
+    if (p->flags & ~(RTP_RENDER_RAW_SUMS | RTP_RENDER_COUNTERS))
+        return set_error(RTP_ERR_INVALID, "adaptive: flags other than RTP_RENDER_RAW_SUMS | RTP_RENDER_COUNTERS");
+    return RTP_OK;
+}
+
+// one device's share of an adaptive frame
+struct AdaptiveDev {
+    DeviceScene* ds = nullptr;
+    cudaStream_t st = nullptr;
+    rtp_render_params p{};  // this device's rows
+    double* d_rgb = nullptr; double* d_fg = nullptr; uint32_t* d_samples = nullptr;
+    DRender rp{};
+    size_t npix = 0;
+    uint32_t n_live = 0;    // length of live list `cur`
+    int cur = 0;
+    size_t launches = 0;
+    uint64_t paths = 0;
+    bool begun = false;     // holds the scene's scratch: render_done must be recorded
+};
+
+template <class T>
+static int grow(T** buf, size_t n) {
+    cudaFree(*buf); *buf = nullptr;
+    RTP_CUDA(cudaMalloc(reinterpret_cast<void**>(buf), std::max<size_t>(n, 1) * sizeof(T)));
+    return RTP_OK;
+}
+
+static int adaptive_begin(AdaptiveDev& d, bool want_stats) {
+    DeviceScene* ds = d.ds;
+    if (int rc = render_rect(&d.p, false, &d.rp)) return rc;
+    if (ds->render_pending) RTP_CUDA(cudaStreamWaitEvent(d.st, ds->render_done, 0));
+    d.begun = true;
+    ds->ev_used = 0;
+    RTP_CUDA(cudaMemsetAsync(ds->counters, 0, sizeof(Counters), d.st));
+    if (want_stats) {
+        RTP_CUDA(cudaEventRecord(ds->ev_begin, d.st));
+        RTP_CUDA(cudaEventRecord(ds->ev_end, d.st));
+    }
+    d.npix = static_cast<size_t>(d.rp.tile_w) * d.rp.tile_h;
+    if (d.npix == 0) return RTP_OK;  // no row of the rectangle falls to this device
+    if (d.npix > static_cast<size_t>(std::numeric_limits<int>::max()))  // cub::DeviceSelect counts items in int
+        return set_error(RTP_ERR_UNSUPPORTED, "adaptive: more than 2^31 - 1 pixels on one device");
+    if (ds->acc_elems < d.npix) {
+        if (int rc = grow(&ds->acc, d.npix)) return rc;
+        ds->acc_elems = d.npix;
+    }
+    if (ds->adaptive_elems < d.npix) {
+        ds->adaptive_elems = 0;
+        int rc = grow(&ds->moments, d.npix);
+        if (rc == RTP_OK) rc = grow(&ds->counts, d.npix);
+        if (rc == RTP_OK) rc = grow(&ds->keep, d.npix);
+        if (rc == RTP_OK) rc = grow(&ds->live[0], d.npix);
+        if (rc == RTP_OK) rc = grow(&ds->live[1], d.npix);
+        if (rc != RTP_OK) return rc;
+        ds->adaptive_elems = d.npix;
+    }
+    size_t tmp = 0;
+    RTP_CUDA(cub::DeviceSelect::Flagged(nullptr, tmp, static_cast<const uint32_t*>(ds->live[0]), ds->keep, ds->live[1], ds->n_live, static_cast<int>(d.npix), d.st));
+    if (ds->select_tmp_bytes < tmp) {
+        ds->select_tmp_bytes = 0;
+        if (int rc = grow(reinterpret_cast<uint8_t**>(&ds->select_tmp), tmp)) return rc;
+        ds->select_tmp_bytes = tmp;
+    }
+    if (!ds->n_live) {
+        if (int rc = grow(&ds->n_live, 1)) return rc;
+        RTP_CUDA(cudaHostAlloc(reinterpret_cast<void**>(&ds->n_live_host), sizeof(uint32_t), cudaHostAllocPortable));
+    }
+    adaptive_init_kernel<<<static_cast<unsigned>((d.npix + 255) / 256), 256, 0, d.st>>>(ds->acc, ds->moments, ds->counts, ds->live[0], d.npix);
+    RTP_CUDA(cudaGetLastError());
+    ++d.launches;
+    d.n_live = static_cast<uint32_t>(d.npix);
+    d.cur = 0;
+    return RTP_OK;
+}
+
+// queues samples [s0, s0 + B) of every live pixel, the stop rule and the selection of the next live list; its length is copied
+// to ds->n_live_host
+static int adaptive_round(AdaptiveDev& d, const DCamera& cam, uint32_t s0, uint32_t B, const StopRule& rule, bool count, bool want_stats) {
+    DeviceScene* ds = d.ds;
+    const uint32_t per_launch = static_cast<uint32_t>(std::max<size_t>(1, std::min<size_t>(B, path_budget(ds, d.p.max_bounce) / d.n_live)));
+    if (int rc = reserve_paths(ds, static_cast<size_t>(d.n_live) * per_launch, d.p.max_bounce)) return rc;
+    const LiveList map{ds->live[d.cur], d.n_live};
+    const unsigned grid = (d.n_live + 255u) / 256u;
+    for (uint32_t l0 = 0; l0 < B; l0 += per_launch) {
+        d.rp.sample_begin = s0 + l0;
+        d.rp.n_samples = std::min(per_launch, B - l0);
+        int rc = launch_paths(ds, cam, d.rp, map, static_cast<size_t>(d.n_live) * d.rp.n_samples, count, want_stats, d.st, &d.launches);
+        if (rc != RTP_OK) return rc;
+        adaptive_resolve_kernel<<<grid, 256, 0, d.st>>>(ds->scratch, map.live, d.n_live, d.rp.n_samples, ds->acc, ds->moments, ds->counts, ds->keep,
+                                                        l0 + per_launch >= B ? 1 : 0, rule);
+        RTP_CUDA(cudaGetLastError());
+        ++d.launches;
+    }
+    d.paths += static_cast<uint64_t>(d.n_live) * B;
+    size_t tmp = ds->select_tmp_bytes;
+    RTP_CUDA(cub::DeviceSelect::Flagged(ds->select_tmp, tmp, map.live, ds->keep, ds->live[d.cur ^ 1], ds->n_live, static_cast<int>(d.n_live), d.st));
+    d.launches += 2;  // the selection's scan-state initialisation and the select kernel
+    RTP_CUDA(cudaMemcpyAsync(ds->n_live_host, ds->n_live, sizeof(uint32_t), cudaMemcpyDeviceToHost, d.st));
+    d.cur ^= 1;
+    return RTP_OK;
+}
+
+// Renders every device's share round by round: a round is queued on each device that still has live pixels, then every live count
+// is read back. On return (also after an error) every device's work is queued and its output written or abandoned; the caller
+// synchronises the streams.
+static int render_adaptive(std::vector<AdaptiveDev>& devs, const rtp_camera* camera, const rtp_adaptive_params* a, bool want_stats) {
+    const DCamera cam = make_camera(camera);
+    const StopRule rule{a->abs_tol, a->rel_tol, a->max_samples, 0u};
+    const bool count = (devs[0].p.flags & RTP_RENDER_COUNTERS) != 0;
+    int rc = RTP_OK;
+    for (AdaptiveDev& d : devs) {
+        if (rc == RTP_OK) rc = cudaSetDevice(d.ds->device) == cudaSuccess ? adaptive_begin(d, want_stats) : set_error(RTP_ERR_CUDA, "cudaSetDevice");
+    }
+    uint32_t n = 0, B = a->min_samples;
+    while (rc == RTP_OK) {
+        bool queued = false;
+        for (AdaptiveDev& d : devs) {
+            if (rc != RTP_OK || d.n_live == 0) continue;
+            cudaSetDevice(d.ds->device);
+            rc = adaptive_round(d, cam, n, B, rule, count, want_stats);
+            queued = true;
+        }
+        if (!queued) break;
+        for (AdaptiveDev& d : devs) {
+            if (d.n_live == 0) continue;
+            cudaSetDevice(d.ds->device);
+            const cudaError_t e = cudaStreamSynchronize(d.st);
+            if (e != cudaSuccess && rc == RTP_OK) rc = set_error(RTP_ERR_CUDA, std::string("adaptive round: ") + cudaGetErrorString(e));
+            d.n_live = rc == RTP_OK ? *d.ds->n_live_host : 0u;
+        }
+        n += B;
+        if (n >= a->max_samples) break;  // the stop rule has stopped every pixel
+        B = std::min(a->batch, a->max_samples - n);
+    }
+    const int raw = (devs[0].p.flags & RTP_RENDER_RAW_SUMS) ? 1 : 0;
+    for (AdaptiveDev& d : devs) {
+        if (!d.begun) continue;
+        DeviceScene* ds = d.ds;
+        cudaSetDevice(ds->device);
+        if (rc == RTP_OK && d.npix) {
+            adaptive_write_kernel<<<static_cast<unsigned>((d.npix + 255) / 256), 256, 0, d.st>>>(ds->acc, ds->counts, d.rp, raw, d.d_rgb, d.d_fg, d.d_samples);
+            if (cudaGetLastError() != cudaSuccess) rc = set_error(RTP_ERR_CUDA, "adaptive_write_kernel launch");
+            ++d.launches;
+        }
+        ds->pending_launches = d.launches;
+        ds->pending_paths = d.paths;
+        if (want_stats) cudaEventRecord(ds->ev_end, d.st);
+        cudaEventRecord(ds->render_done, d.st);
+        ds->render_pending = true;
+    }
+    return rc;
+}
+
+// waits for every device's stream and, if asked, sums their stats
+static int adaptive_finish(std::vector<AdaptiveDev>& devs, int rc, rtp_stats* stats) {
+    rtp_stats total;
+    std::memset(&total, 0, sizeof total);
+    for (AdaptiveDev& d : devs) {
+        cudaSetDevice(d.ds->device);
+        const cudaError_t e = cudaStreamSynchronize(d.st);
+        if (e != cudaSuccess && rc == RTP_OK) rc = set_error(RTP_ERR_CUDA, std::string("adaptive render: ") + cudaGetErrorString(e));
+        if (rc != RTP_OK || !stats) continue;
+        rtp_stats one;
+        rc = render_finish(d.ds, &one);
+        add_stats(&total, one);
+    }
+    if (stats && rc == RTP_OK) *stats = total;
+    return rc;
 }
 
 }  // namespace rtp
@@ -3032,11 +3356,7 @@ static int render_host(rtp_scene* scene, const rtp_camera* camera, const rtp_ren
             rtp_stats one;
             int r2 = render_finish(ds, &one);
             if (r2 != RTP_OK) { rc = r2; continue; }
-            total.rays += one.rays; total.paths += one.paths; total.node_visits += one.node_visits; total.triangle_tests += one.triangle_tests;
-            total.sphere_tests += one.sphere_tests; total.leaf_gates += one.leaf_gates; total.conservative_violations += one.conservative_violations;
-            total.order_rewalks += one.order_rewalks; total.kernel_launches += one.kernel_launches;
-            total.device_ms = std::max(total.device_ms, one.device_ms);  // the devices run side by side
-            total.trace_ms = std::max(total.trace_ms, one.trace_ms); total.shade_ms = std::max(total.shade_ms, one.shade_ms);
+            add_stats(&total, one);
         }
     }
     cudaSetDevice(scene->dev->device);
@@ -3054,6 +3374,82 @@ int rtp_render(rtp_scene* scene, const rtp_camera* camera, const rtp_render_para
                rtp_stats* stats) {
     if (!scene || !camera || !params || !rgb_out) return set_error(RTP_ERR_INVALID, "null argument");
     return render_host(scene, camera, params, rgb_out, foreground_out, nullptr, stats);
+}
+
+// The rows of the tile rectangle are dealt out to the devices as in render_host; each device runs its own live list through the same
+// rounds, and only its rows travel back.
+int rtp_render_adaptive(rtp_scene* scene, const rtp_camera* camera, const rtp_render_params* params, const rtp_adaptive_params* adaptive,
+                        double* rgb_out, double* foreground_out, uint32_t* samples_out, rtp_stats* stats) {
+    if (!scene || !camera || !params || !adaptive || !rgb_out) return set_error(RTP_ERR_INVALID, "null argument");
+    if (int rc = check_adaptive(params, adaptive)) return rc;
+    const size_t npx = static_cast<size_t>(params->width) * params->height;
+    if (npx == 0) return set_error(RTP_ERR_INVALID, "bad frame parameters");
+    std::vector<AdaptiveDev> devs;
+    for (DeviceScene* ds : scene->devs)
+        if (params->device_mask == 0 || ((params->device_mask >> ds->device) & 1u)) { devs.emplace_back(); devs.back().ds = ds; devs.back().st = ds->streams[0]; }
+    if (devs.empty()) return set_error(RTP_ERR_INVALID, "device_mask names no device of this scene");
+    const uint32_t N = static_cast<uint32_t>(devs.size());
+    const uint32_t rs0 = params->row_stride ? params->row_stride : 1u, ro0 = params->row_offset;
+    const uint32_t W = params->width, tx = params->tile_x, ty = params->tile_y;
+    const uint32_t tw = params->tile_w ? params->tile_w : W - tx, th_full = params->tile_h ? params->tile_h : params->height - ty;
+    std::vector<std::unique_lock<std::mutex>> locks;
+    for (AdaptiveDev& d : devs) locks.emplace_back(d.ds->lock);
+    int rc = RTP_OK;
+    for (uint32_t k = 0; k < N && rc == RTP_OK; ++k) {
+        AdaptiveDev& d = devs[k];
+        DeviceScene* ds = d.ds;
+        RTP_CUDA(cudaSetDevice(ds->device));
+        d.p = *params;
+        d.p.row_offset = ro0 + k * rs0;  // rows ro0 + m * rs0 of the caller's split; device k takes m = k, k + N, ...
+        d.p.row_stride = rs0 * N;
+        if (ds->frame_elems < npx * 4) {
+            ds->frame_elems = 0;
+            if ((rc = grow(&ds->frame, npx * 4)) != RTP_OK) break;
+            ds->frame_elems = npx * 4;
+        }
+        if (samples_out && ds->frame_samples_elems < npx) {
+            ds->frame_samples_elems = 0;
+            if ((rc = grow(&ds->frame_samples, npx)) != RTP_OK) break;
+            ds->frame_samples_elems = npx;
+        }
+        d.d_rgb = ds->frame;
+        d.d_fg = foreground_out ? ds->frame + npx * 3 : nullptr;
+        d.d_samples = samples_out ? ds->frame_samples : nullptr;
+    }
+    if (rc == RTP_OK) rc = render_adaptive(devs, camera, adaptive, stats != nullptr);
+    for (uint32_t k = 0; k < N && rc == RTP_OK; ++k) {  // only the rows this device rendered travel back
+        AdaptiveDev& d = devs[k];
+        if (d.p.row_offset >= th_full || tx >= W) continue;
+        cudaSetDevice(d.ds->device);
+        const uint32_t rows = (th_full - d.p.row_offset + d.p.row_stride - 1u) / d.p.row_stride;
+        const size_t first = static_cast<size_t>(tx) + static_cast<size_t>(ty + d.p.row_offset) * W;
+        const size_t row_px = static_cast<size_t>(W) * d.p.row_stride;
+        cudaError_t e = cudaMemcpy2DAsync(rgb_out + 3 * first, row_px * 24, d.d_rgb + 3 * first, row_px * 24, static_cast<size_t>(tw) * 24, rows, cudaMemcpyDeviceToHost, d.st);
+        if (e == cudaSuccess && foreground_out)
+            e = cudaMemcpy2DAsync(foreground_out + first, row_px * 8, d.d_fg + first, row_px * 8, static_cast<size_t>(tw) * 8, rows, cudaMemcpyDeviceToHost, d.st);
+        if (e == cudaSuccess && samples_out)
+            e = cudaMemcpy2DAsync(samples_out + first, row_px * 4, d.d_samples + first, row_px * 4, static_cast<size_t>(tw) * 4, rows, cudaMemcpyDeviceToHost, d.st);
+        if (e != cudaSuccess) rc = set_error(RTP_ERR_CUDA, std::string("adaptive frame copy: ") + cudaGetErrorString(e));
+    }
+    rc = adaptive_finish(devs, rc, stats);
+    cudaSetDevice(scene->dev->device);
+    return rc;
+}
+
+int rtp_render_adaptive_device(rtp_scene* scene, const rtp_camera* camera, const rtp_render_params* params, const rtp_adaptive_params* adaptive,
+                               double* d_rgb_out, double* d_foreground_out, uint32_t* d_samples_out, rtp_stats* stats, void* cuda_stream) {
+    if (!scene || !camera || !params || !adaptive || !d_rgb_out) return set_error(RTP_ERR_INVALID, "null argument");
+    if (int rc = check_adaptive(params, adaptive)) return rc;
+    std::vector<AdaptiveDev> devs(1);
+    AdaptiveDev& d = devs[0];
+    d.ds = scene->dev;
+    std::lock_guard<std::mutex> guard(d.ds->lock);
+    RTP_CUDA(cudaSetDevice(d.ds->device));
+    d.st = static_cast<cudaStream_t>(cuda_stream);
+    d.p = *params;
+    d.d_rgb = d_rgb_out; d.d_fg = d_foreground_out; d.d_samples = d_samples_out;
+    const int rc = render_adaptive(devs, camera, adaptive, stats != nullptr);
+    return adaptive_finish(devs, rc, stats);
 }
 
 }  // extern "C"

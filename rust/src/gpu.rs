@@ -31,6 +31,8 @@ use std::os::raw::{c_char, c_int};
     pub device_mask: u32, pub row_offset: u32, pub row_stride: u32 }
 #[repr(C)] #[derive(Default, Debug)] pub struct rtp_stats { pub rays: u64, pub paths: u64, pub node_visits: u64, pub triangle_tests: u64, pub sphere_tests: u64,
     pub leaf_gates: u64, pub conservative_violations: u64, pub device_ms: f64, pub kernel_launches: u64, pub order_rewalks: u64, pub trace_ms: f64, pub shade_ms: f64 }
+#[repr(C)] #[derive(Default, Clone, Copy)] pub struct rtp_adaptive_params { pub min_samples: u32, pub max_samples: u32, pub batch: u32, pub _pad: u32,
+    pub abs_tol: f64, pub rel_tol: f64 }
 pub enum rtp_scene {}
 
 #[link(name = "rtp_b200")]
@@ -45,6 +47,8 @@ extern "C" {
     fn rtp_trace_occluded(scene: *mut rtp_scene, rays: *const rtp_ray, n: usize, occluded: *mut u8, stats: *mut rtp_stats) -> c_int;
     fn rtp_render(scene: *mut rtp_scene, camera: *const rtp_camera, params: *const rtp_render_params,
                   rgb: *mut f64, foreground: *mut f64, stats: *mut rtp_stats) -> c_int;
+    fn rtp_render_adaptive(scene: *mut rtp_scene, camera: *const rtp_camera, params: *const rtp_render_params, adaptive: *const rtp_adaptive_params,
+                           rgb: *mut f64, foreground: *mut f64, samples: *mut u32, stats: *mut rtp_stats) -> c_int;
 }
 
 type GpuResult<T> = Result<T, Box<dyn std::error::Error>>; // the crate's loaders return Result<_, Box<dyn Error>> (mesh.rs:145)
