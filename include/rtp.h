@@ -391,6 +391,27 @@ int rtp_render_device(rtp_scene* scene, const rtp_camera* camera, const rtp_rend
                       double* d_rgb_out, double* d_foreground_out, rtp_stats* stats,
                       void* cuda_stream);
 
+/* ---------------------------------------------------------------- render AOVs ----------- */
+
+/* rtp_render plus two guide buffers for a denoiser (DESIGN.md §6c). rgb_out and foreground_out hold exactly what rtp_render writes
+ * for the same params. For sample s of a pixel, take the closest hit of the path's first segment (render.rs:102):
+ *     A_s = the material's Absorb::evaluate at that hit (material.rs:74-81: Blackbody 0, Whitebody 1, Albedo rgb, AlbedoMap sampled
+ *           at the hit's position and uv), whether or not the material scatters;
+ *     N_s = Hit::normal in world space, not flipped toward the ray (a sphere's normalize(p - c), hittable.rs:60; a triangle's
+ *           interpolated vertex normal, not renormalised, hittable.rs:105);
+ *     both (0, 0, 0) on a miss.
+ * albedo_out[3p + c] = Σ_s A_s[c] / num_samples and normal_out likewise: f64 sums from 0.0 in sample order, no contraction, the
+ * colour's divisor (none with RTP_RENDER_RAW_SUMS); an averaged normal is not renormalised. Layout as rgb_out; foreground_out,
+ * albedo_out and normal_out may each be NULL. Tile rectangle, rows, sample range, seed, max_bounce and device_mask as rtp_render;
+ * only pixels of the tile rectangle and rows are written, and a frame split over several devices is bit-identical to one device.
+ * flags must be a subset of RTP_RENDER_RAW_SUMS | RTP_RENDER_COUNTERS. stats as rtp_render. Host buffers. */
+int rtp_render_aov(rtp_scene* scene, const rtp_camera* camera, const rtp_render_params* params,
+                   double* rgb_out, double* foreground_out, double* albedo_out, double* normal_out, rtp_stats* stats);
+/* Same with device buffers on the scene's first device; asynchronous on `cuda_stream` except for stats, as rtp_render_device. */
+int rtp_render_aov_device(rtp_scene* scene, const rtp_camera* camera, const rtp_render_params* params,
+                          double* d_rgb_out, double* d_foreground_out, double* d_albedo_out, double* d_normal_out,
+                          rtp_stats* stats, void* cuda_stream);
+
 /* ---------------------------------------------------------------- adaptive render ------- */
 
 /* Stop rule of rtp_render_adaptive. */

@@ -216,6 +216,10 @@ PROTOTYPES = {
     "rtp_camera_rays": (C.c_int, [_P(Camera), C.c_uint32, C.c_uint32, C.c_void_p]),
     "rtp_render": (C.c_int, [C.c_void_p, _P(Camera), _P(RenderParams), C.c_void_p, C.c_void_p, _P(Stats)]),
     "rtp_render_device": (C.c_int, [C.c_void_p, _P(Camera), _P(RenderParams), C.c_void_p, C.c_void_p, _P(Stats), C.c_void_p]),
+    "rtp_render_aov": (C.c_int, [C.c_void_p, _P(Camera), _P(RenderParams), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, _P(Stats)]),
+    "rtp_render_aov_device": (
+        C.c_int, [C.c_void_p, _P(Camera), _P(RenderParams), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, _P(Stats), C.c_void_p]
+    ),
     "rtp_render_adaptive": (C.c_int, [C.c_void_p, _P(Camera), _P(RenderParams), _P(AdaptiveParams), C.c_void_p, C.c_void_p, C.c_void_p, _P(Stats)]),
     "rtp_render_adaptive_device": (
         C.c_int, [C.c_void_p, _P(Camera), _P(RenderParams), _P(AdaptiveParams), C.c_void_p, C.c_void_p, C.c_void_p, _P(Stats), C.c_void_p]

@@ -652,6 +652,37 @@ class Scene:
         _check(self._lib, self._lib.rtp_render(self._h, C.byref(cc), C.byref(p), A.ptr(rgbf), A.ptr(fg) if fg is not None else None, C.byref(st)))
         return rgbf, fg, st
 
+    def render_aov(self, width: int, height: int, num_samples: int, max_bounce: int = 8, seed: int = 1, camera: Optional[Camera] = None,
+                   sample_range=None, tile=None, flags: int = 0, out=None, foreground: bool = True, rows=None, device_mask: int = 0):
+        """render() plus each pixel's mean first-vertex albedo and normal, the guide buffers of a denoiser (rtp_render_aov). Returns
+        (rgb [h, w, 3], foreground [h, w], albedo [h, w, 3], normal [h, w, 3], stats); rgb and foreground are render()'s bits.
+        out: a 4-tuple (rgb, foreground, albedo, normal) of caller buffers, any but rgb may be None"""
+        cam = camera or self.camera
+        cam = Camera(width / height, cam.fov, cam.focal_dist, cam.lens_radius, cam.transformation)  # main.rs:22 overrides the aspect
+        p = render_params(width, height, num_samples, max_bounce, seed,
+                          sample_range[0] if sample_range else 0, sample_range[1] if sample_range else None, tile, flags, rows, device_mask)
+        if out is not None:
+            rgbf, fg, albedo, normal = out
+        else:
+            rgbf = np.zeros((height, width, 3), dtype=np.float64)
+            fg = np.zeros((height, width), dtype=np.float64) if foreground else None
+            albedo = np.zeros((height, width, 3), dtype=np.float64)
+            normal = np.zeros((height, width, 3), dtype=np.float64)
+        st = A.Stats()
+        cc = cam.to_c()
+        opt = lambda a: A.ptr(a) if a is not None else None  # noqa: E731
+        _check(self._lib, self._lib.rtp_render_aov(self._h, C.byref(cc), C.byref(p), A.ptr(rgbf), opt(fg), opt(albedo), opt(normal), C.byref(st)))
+        return rgbf, fg, albedo, normal, st
+
+    def render_aov_device(self, params: A.RenderParams, camera: Camera, d_rgb: int, d_fg: int = 0, d_albedo: int = 0, d_normal: int = 0,
+                          stream: int = 0, stats: bool = False):
+        """rtp_render_aov_device: device buffers on the scene's first device; asynchronous on `stream` unless stats"""
+        st = A.Stats()
+        cc = camera.to_c()
+        _check(self._lib, self._lib.rtp_render_aov_device(self._h, C.byref(cc), C.byref(params), d_rgb, d_fg or None, d_albedo or None,
+                                                          d_normal or None, C.byref(st) if stats else None, stream or None))
+        return st
+
     def render_srgb8(self, width: int, height: int, num_samples: int, max_bounce: int = 8, seed: int = 1, camera: Optional[Camera] = None,
                      tile=None, transparent_background: bool = False, out: Optional[np.ndarray] = None, rows=None, device_mask: int = 0):
         """main.rs:61-122: render + tile merge + to_srgb_u8 with the output stage on the device; [height, width, 4] uint8, ready for tga.save"""

@@ -890,6 +890,28 @@ struct LiveList {   // rtp_render_adaptive: the pixels still sampling in this ro
     __device__ __forceinline__ uint32_t pixel(uint32_t k) const { return __ldg(live + k); }
 };
 
+// What a path's first vertex leaves for rtp_render_aov (DESIGN.md §6c): the material's absorb there and Hit::normal; (0, 0, 0) on a miss
+struct FirstVertex {
+    D3 albedo, normal;
+};
+
+// Whether the integrator kernels capture each path's FirstVertex, as a compile-time policy. A launch with AovRecords writes one
+// 48-byte record per path p: (albedo.x, albedo.y) (albedo.z, normal.x) (normal.y, normal.z) at rec + 3 p.
+struct NoAov {  // rtp_render, rtp_render_srgb8, rtp_render_adaptive
+    static constexpr bool kOn = false;
+    __device__ __forceinline__ void record(size_t, const FirstVertex&) const {}
+};
+struct AovRecords {  // rtp_render_aov
+    static constexpr bool kOn = true;
+    double2* rec;
+    __device__ __forceinline__ void record(size_t p, const FirstVertex& f) const {
+        double2* r = rec + 3 * p;
+        r[0] = make_double2(f.albedo.x, f.albedo.y);
+        r[1] = make_double2(f.albedo.z, f.normal.x);
+        r[2] = make_double2(f.normal.y, f.normal.z);
+    }
+};
+
 // path p of a launch = (pixel slot p / n_samples, sample p % n_samples): the samples of one pixel sit in adjacent lanes,
 // so a warp's primary rays are as coherent as they can be
 template <class Map>
@@ -920,7 +942,9 @@ __device__ __forceinline__ D3 shade_miss(const DSceneView& sc, D3 d) {
 }
 
 // render.rs:105-115 for a hit: returns true when the material scattered (then o, d hold the scattered ray, render.rs:111-114).
-__device__ __forceinline__ bool shade_vertex(const DSceneView& sc, D3& o, D3& d, const HitRec& h, Rng& rng, D3& emit, D3& absorb) {
+// fv != nullptr: the vertex's absorb and Hit::normal are stored there too (rtp_render_aov's first vertex).
+__device__ __forceinline__ bool shade_vertex(const DSceneView& sc, D3& o, D3& d, const HitRec& h, Rng& rng, D3& emit, D3& absorb,
+                                             FirstVertex* fv = nullptr) {
     Surface s;
 #ifdef RTP_DEVICE_CHECKS
     if (h.slot >= sc.n_prims) printf("shade_vertex: slot %u of %u kind %u t %g\n", h.slot, sc.n_prims, h.kind, h.t);
@@ -980,15 +1004,16 @@ __device__ __forceinline__ bool shade_vertex(const DSceneView& sc, D3& o, D3& d,
         default: absorb = mk(0.0, 0.0, 0.0); break;
     }
     emit = emit_evaluate(sc, __ldg(&m->emit_kind), __ldg(&m->emit_texture), m->emit_rgb, d, s.position, s.normal, s.u, s.v);
+    if (fv) { fv->albedo = absorb; fv->normal = s.normal; }
     o = s.position; d = sd;
     return scattered;
 }
 
 // Baseline integrator: one thread per camera path, whole bounce loop in one thread, exact f64 stack-free walk.
 // Kept for A/B runs (RTP_RENDER_KERNEL=simple) and as the second implementation the wavefront path is tested against.
-template <int MAXB, bool COUNT, class Map>
+template <int MAXB, bool COUNT, class Map, class Aov>
 __global__ void __launch_bounds__(128) render_paths_kernel(DSceneView sc, DCamera cam, DRender rp, double4* __restrict__ scratch,
-                                                            Counters* counters, Map map) {
+                                                            Counters* counters, Map map, Aov aov) {
     const size_t npix = map.count(rp);
     const size_t total = npix * rp.n_samples;
     const size_t p = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
@@ -1006,6 +1031,7 @@ __global__ void __launch_bounds__(128) render_paths_kernel(DSceneView sc, DCamer
         D3 L = mk(0.0, 0.0, 0.0);
         uint32_t depth = rp.max_bounce;
         bool first = true, first_hit = false;
+        FirstVertex fv = {mk(0.0, 0.0, 0.0), mk(0.0, 0.0, 0.0)};
         for (;;) {
             if (!first && depth == 0) { L = mk(0.0, 0.0, 0.0); break; }  // render.rs:128-131
             HitRec h;
@@ -1014,7 +1040,7 @@ __global__ void __launch_bounds__(128) render_paths_kernel(DSceneView sc, DCamer
             if (h.slot == kNoPrim) { L = shade_miss(sc, d); break; }
             if (first) first_hit = true;
             D3 emit, absorb;
-            if (!shade_vertex(sc, o, d, h, rng, emit, absorb)) {  // render.rs:108-110: emit + rgb(0,0,0)
+            if (!shade_vertex(sc, o, d, h, rng, emit, absorb, Aov::kOn && first ? &fv : nullptr)) {  // render.rs:108-110: emit + rgb(0,0,0)
                 L = emit + mk(0.0, 0.0, 0.0);
                 break;
             }
@@ -1029,6 +1055,7 @@ __global__ void __launch_bounds__(128) render_paths_kernel(DSceneView sc, DCamer
             L = mk(emit_stack[b][0], emit_stack[b][1], emit_stack[b][2]) + cmul(mk(absorb_stack[b][0], absorb_stack[b][1], absorb_stack[b][2]), L);
         }
         scratch[p] = make_double4(L.x, L.y, L.z, first_hit ? 1.0 : 0.0);
+        aov.record(p, fv);
     }
     flush_counters<COUNT>(counters, lc);
 }
@@ -1082,9 +1109,10 @@ __device__ __noinline__ void trace_deferred(const DSceneView& sc, D3 o, D3 d, Hi
 }
 
 constexpr int kShadeBlocks = 3;  // resident blocks per SM wave_shade_kernel is built for, and its grid
-template <class Map>
+// With Aov::kOn the bounce-0 launch records every path's FirstVertex (its queue holds every path of the launch, hit or miss).
+template <class Map, class Aov>
 __global__ void __launch_bounds__(256, kShadeBlocks) wave_shade_kernel(DSceneView sc, DRender rp, WaveQueues wq, uint32_t bounce, double4* __restrict__ scratch,
-                                                                       Map map) {
+                                                                       Map map, Aov aov) {
     const size_t n = static_cast<size_t>(wq.count[bounce]);
     const int cur = bounce & 1, nxt = cur ^ 1;
     const unsigned lane = threadIdx.x & 31u;
@@ -1106,6 +1134,7 @@ __global__ void __launch_bounds__(256, kShadeBlocks) wave_shade_kernel(DSceneVie
             uint32_t depth = st.z & 0xFFu, nb = (st.z >> 8) & 0xFFu, first_hit = (st.z >> 16) & 1u;
             const size_t p = st.x;
             D3 L = mk(0.0, 0.0, 0.0);
+            FirstVertex fv = {mk(0.0, 0.0, 0.0), mk(0.0, 0.0, 0.0)};
             HitRec h;
             h.t = h0.x; h.u = h0.y; h.v = h1.x; h.slot = slotkind & 0x7FFFFFFFu; h.kind = slotkind >> 31;
             if (slotkind == kDeferredHit) {
@@ -1122,7 +1151,7 @@ __global__ void __launch_bounds__(256, kShadeBlocks) wave_shade_kernel(DSceneVie
                 rng_init(rng, rp.seed, j * rp.width + i, smp, RTP_RNG_STREAM_PATH);
                 rng.k = st.y;
                 D3 emit, absorb;
-                if (!shade_vertex(sc, o, d, h, rng, emit, absorb)) {  // render.rs:108-110: emit + rgb(0,0,0)
+                if (!shade_vertex(sc, o, d, h, rng, emit, absorb, Aov::kOn && bounce == 0 ? &fv : nullptr)) {  // render.rs:108-110: emit + rgb(0,0,0)
                     L = emit + mk(0.0, 0.0, 0.0);
                 } else {
                     double2* sp = wq.stack + (static_cast<size_t>(nb) * wq.capacity + p) * 3;
@@ -1145,6 +1174,7 @@ __global__ void __launch_bounds__(256, kShadeBlocks) wave_shade_kernel(DSceneVie
                 }
                 scratch[p] = make_double4(L.x, L.y, L.z, first_hit ? 1.0 : 0.0);
             }
+            if (Aov::kOn && bounce == 0) aov.record(p, fv);
             st.z = depth | (nb << 8) | (first_hit << 16);
         }
         // compaction: survivors of this warp take consecutive slots of the next queue
@@ -1813,6 +1843,39 @@ __global__ void __launch_bounds__(256) write_frame_kernel(const double4* __restr
     if (fg) fg[px] = a.w;
 }
 
+// rtp_render_aov (DESIGN.md §6c): resolve_kernel for the launch's AovRecords. acc is 3 double2 per tile pixel, (albedo, normal)
+// summed from 0.0 in sample order like the colour.
+__global__ void __launch_bounds__(256) aov_resolve_kernel(const double2* __restrict__ rec, double2* __restrict__ acc, size_t npix, uint32_t n_samples,
+                                                           int first_launch) {
+    const size_t pix = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+    if (pix >= npix) return;
+    double2 a0 = make_double2(0.0, 0.0), a1 = a0, a2 = a0;
+    if (!first_launch) { a0 = acc[3 * pix]; a1 = acc[3 * pix + 1]; a2 = acc[3 * pix + 2]; }
+    for (uint32_t s = 0; s < n_samples; ++s) {
+        const double2* r = rec + 3 * (pix * n_samples + s);  // path_coords: the samples of a pixel are adjacent
+        const double2 r0 = r[0], r1 = r[1], r2 = r[2];
+        a0.x += r0.x; a0.y += r0.y; a1.x += r1.x; a1.y += r1.y; a2.x += r2.x; a2.y += r2.y;
+    }
+    acc[3 * pix] = a0; acc[3 * pix + 1] = a1; acc[3 * pix + 2] = a2;
+}
+
+// write_frame_kernel for the AOV sums; albedo / normal may each be null
+__global__ void __launch_bounds__(256) aov_write_kernel(const double2* __restrict__ acc, DRender rp, double divisor, double* __restrict__ albedo,
+                                                         double* __restrict__ normal) {
+    const size_t npix = static_cast<size_t>(rp.tile_w) * rp.tile_h;
+    const size_t pix = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+    if (pix >= npix) return;
+    const uint32_t i = rp.tile_x + static_cast<uint32_t>(pix % rp.tile_w);
+    const uint32_t j = rp.tile_y + rp.row_offset + static_cast<uint32_t>(pix / rp.tile_w) * rp.row_stride;
+    const size_t px = static_cast<size_t>(i) + static_cast<size_t>(j) * rp.width;
+    const double2 a0 = acc[3 * pix], a1 = acc[3 * pix + 1], a2 = acc[3 * pix + 2];
+    double v[6] = {a0.x, a0.y, a1.x, a1.y, a2.x, a2.y};
+    if (divisor != 0.0)
+        for (int k = 0; k < 6; ++k) v[k] = v[k] / divisor;
+    if (albedo) { albedo[3 * px + 0] = v[0]; albedo[3 * px + 1] = v[1]; albedo[3 * px + 2] = v[2]; }
+    if (normal) { normal[3 * px + 0] = v[3]; normal[3 * px + 1] = v[4]; normal[3 * px + 2] = v[5]; }
+}
+
 // ---------------------------------------------------------------------------------------------
 // rtp_render_adaptive (DESIGN.md §6b). Per tile pixel: acc (the colour / foreground sums of resolve_kernel), the luminance
 // moments (Σ Y, Σ Y²) and the sample count; per live slot a keep flag. Every sum starts at 0.0 and runs in sample order, so a
@@ -1995,6 +2058,9 @@ struct DeviceScene {
     size_t adaptive_elems = 0;
     void* select_tmp = nullptr; size_t select_tmp_bytes = 0;  // cub::DeviceSelect::Flagged
     uint32_t* n_live = nullptr; uint32_t* n_live_host = nullptr;
+    // rtp_render_aov: the AovRecords of a launch (3 double2 per path, grown like scratch) and their sums (3 double2 per tile pixel)
+    double2* aov_rec = nullptr; size_t aov_rec_elems = 0;
+    double2* aov_acc = nullptr; size_t aov_acc_elems = 0;
     WaveQueues wave{};                // wavefront integrator queues (render_device), grown on demand
     uint32_t wave_bounces = 0;         // stack depth the queues were sized for
     int shade_blocks = 0;              // grid of wave_shade_kernel
@@ -2040,6 +2106,7 @@ void device_scene_free(DeviceScene* ds) {
     cudaFree(ds->moments); cudaFree(ds->counts); cudaFree(ds->keep); cudaFree(ds->live[0]); cudaFree(ds->live[1]);
     cudaFree(ds->select_tmp); cudaFree(ds->n_live); cudaFree(ds->frame_samples);
     if (ds->n_live_host) cudaFreeHost(ds->n_live_host);
+    cudaFree(ds->aov_rec); cudaFree(ds->aov_acc);
     cudaFree(ds->scratch); cudaFree(ds->acc); cudaFree(ds->frame); cudaFree(ds->frame8); cudaFree(ds->fixes); cudaFree(ds->n_fixes);
     cudaFree(ds->wave.rays[0]); cudaFree(ds->wave.rays[1]); cudaFree(ds->wave.state[0]); cudaFree(ds->wave.state[1]);
     cudaFree(ds->wave.hits); cudaFree(ds->wave.stack); cudaFree(ds->wave.count);
@@ -2429,12 +2496,13 @@ static int trace_host(rtp_scene* scene, const rtp_ray* rays, size_t n, void* hit
     return rc;
 }
 
-template <int MAXB, class Map>
-static void launch_render_paths(DeviceScene* ds, const DCamera& cam, const DRender& rp, const Map& map, size_t total, bool count, cudaStream_t st) {
+template <int MAXB, class Map, class Aov>
+static void launch_render_paths(DeviceScene* ds, const DCamera& cam, const DRender& rp, const Map& map, const Aov& aov, size_t total, bool count,
+                                cudaStream_t st) {
     const unsigned block = 128;
     const dim3 g(static_cast<unsigned>((total + block - 1) / block));
-    if (count) render_paths_kernel<MAXB, true><<<g, block, 0, st>>>(ds->view, cam, rp, ds->scratch, ds->counters, map);
-    else render_paths_kernel<MAXB, false><<<g, block, 0, st>>>(ds->view, cam, rp, ds->scratch, ds->counters, map);
+    if (count) render_paths_kernel<MAXB, true><<<g, block, 0, st>>>(ds->view, cam, rp, ds->scratch, ds->counters, map, aov);
+    else render_paths_kernel<MAXB, false><<<g, block, 0, st>>>(ds->view, cam, rp, ds->scratch, ds->counters, map, aov);
 }
 
 // bytes per path of one launch of the wavefront integrator: queues (2 rays, 2 states, a hit record: 176 B), the [bounce][path]
@@ -2511,16 +2579,17 @@ static int render_rect(const rtp_render_params* p, bool fixed_spp, DRender* rp) 
 // Paths per launch of the integrator for a call with max_bounce `bounces`: up to 32 Mi paths (wavefront queues 176 B + 48 B x
 // max_bounce per path, scratch 32 B), within the memory budget fixed when the scene was uploaded (a sixth of the free HBM, at most
 // 24 GiB). Big launches matter: every launch pays the fill and drain of ~2 x max_bounce kernels and the latency-bound sparse late
-// bounces once (1080p x 64 spp of the C4 scene: 111 ms in 16 launches of 8 Mi paths, 92 ms in 4 launches of 32 Mi)
-static size_t path_budget(const DeviceScene* ds, uint32_t bounces) {
-    const size_t per_path = ds->sw.simple_render ? 32 : wave_path_bytes(bounces);
+// bounces once (1080p x 64 spp of the C4 scene: 111 ms in 16 launches of 8 Mi paths, 92 ms in 4 launches of 32 Mi). An AOV call
+// (rtp_render_aov) adds its 48-byte AovRecords per path.
+static size_t path_budget(const DeviceScene* ds, uint32_t bounces, bool aov = false) {
+    const size_t per_path = (ds->sw.simple_render ? 32 : wave_path_bytes(bounces)) + (aov ? 3 * sizeof(double2) : 0);
     size_t budget = std::max<size_t>(size_t(1) << 20, std::min<size_t>(size_t(32) << 20, ds->queue_budget_bytes / per_path));
     if (const size_t forced = read_path_budget()) budget = forced;  // tests: force several launches per frame
     return budget;
 }
 
-// the integrator's per-launch buffers for launches of up to `need` paths
-static int reserve_paths(DeviceScene* ds, size_t need, uint32_t bounces) {
+// the integrator's per-launch buffers for launches of up to `need` paths (aov: with their AovRecords)
+static int reserve_paths(DeviceScene* ds, size_t need, uint32_t bounces, bool aov = false) {
     if (!ds->sw.simple_render) {
         int rc = wave_reserve(ds, need, bounces);
         if (rc != RTP_OK) return rc;
@@ -2530,18 +2599,24 @@ static int reserve_paths(DeviceScene* ds, size_t need, uint32_t bounces) {
         RTP_CUDA(cudaMalloc(reinterpret_cast<void**>(&ds->scratch), need * sizeof(double4)));
         ds->scratch_elems = need;
     }
+    if (aov && ds->aov_rec_elems < need) {
+        cudaFree(ds->aov_rec); ds->aov_rec = nullptr; ds->aov_rec_elems = 0;
+        RTP_CUDA(cudaMalloc(reinterpret_cast<void**>(&ds->aov_rec), need * 3 * sizeof(double2)));
+        ds->aov_rec_elems = need;
+    }
     return RTP_OK;
 }
 
 // One launch of the integrator: the `total` paths of rp's sample range over the pixel slots of `map`, traced to their end; path p's
-// colour and foreground land in ds->scratch[p]. Adds the kernels it queued to *launches.
-template <class Map>
-static int launch_paths(DeviceScene* ds, const DCamera& cam, const DRender& rp, const Map& map, size_t total, bool count, bool want_stats,
-                        cudaStream_t st, size_t* launches) {
+// colour and foreground land in ds->scratch[p], and with AovRecords its first vertex in aov.rec[3 p ...]. Adds the kernels it queued
+// to *launches.
+template <class Map, class Aov>
+static int launch_paths(DeviceScene* ds, const DCamera& cam, const DRender& rp, const Map& map, const Aov& aov, size_t total, bool count,
+                        bool want_stats, cudaStream_t st, size_t* launches) {
     if (ds->sw.simple_render) {
-        if (rp.max_bounce <= 8) launch_render_paths<8>(ds, cam, rp, map, total, count, st);
-        else if (rp.max_bounce <= 32) launch_render_paths<32>(ds, cam, rp, map, total, count, st);
-        else launch_render_paths<128>(ds, cam, rp, map, total, count, st);
+        if (rp.max_bounce <= 8) launch_render_paths<8>(ds, cam, rp, map, aov, total, count, st);
+        else if (rp.max_bounce <= 32) launch_render_paths<32>(ds, cam, rp, map, aov, total, count, st);
+        else launch_render_paths<128>(ds, cam, rp, map, aov, total, count, st);
         RTP_CUDA(cudaGetLastError());
         ++*launches;
         return RTP_OK;
@@ -2559,9 +2634,10 @@ static int launch_paths(DeviceScene* ds, const DCamera& cam, const DRender& rp, 
         // Offering every later queue of a big launch to the tail kernel was measured on C1 to be no faster than trace/shade
         // pairs, and so was handing the sparse late bounces to one tail launch chosen from the previous launch's queue sizes
         // (19 -> 12 launches per C1 frame, same 2.05 ms): a late bounce costs the latency of ONE ray segment (~30 us of
-        // dependent instructions, tools/small_batches.py), not a launch. Tail mode maps paths to pixels densely: rtp_render only.
+        // dependent instructions, tools/small_batches.py), not a launch. Tail mode maps paths to pixels densely and records no
+        // first vertex: rtp_render only.
         if (want_stats) next_mark(ds, st);  // even marks open a traversal span, odd marks close it
-        if (std::is_same<Map, DenseTile>::value && ds->sw.tail_threshold && total <= ds->sw.tail_threshold) {
+        if (std::is_same<Map, DenseTile>::value && !Aov::kOn && ds->sw.tail_threshold && total <= ds->sw.tail_threshold) {
             TailArgs ta{ds->wave, rp, ds->scratch, b};
             rc = launch_trace(ds, ds->wave.rays[b & 1], total, nullptr, OUT_TAIL, count, ds->counters, st, ds->wave.count + b, &ta);
             if (rc != RTP_OK) return rc;
@@ -2573,7 +2649,7 @@ static int launch_paths(DeviceScene* ds, const DCamera& cam, const DRender& rp, 
         if (rc != RTP_OK) return rc;
         if (want_stats) next_mark(ds, st);
         if ((rc = debug_sync(ds, st, "trace kernel <OUT_WAVE>", b)) != RTP_OK) return rc;
-        wave_shade_kernel<<<shade_grid, 256, 0, st>>>(ds->view, rp, ds->wave, b, ds->scratch, map);
+        wave_shade_kernel<<<shade_grid, 256, 0, st>>>(ds->view, rp, ds->wave, b, ds->scratch, map, aov);
         RTP_CUDA(cudaGetLastError());
         if ((rc = debug_sync(ds, st, "wave_shade_kernel", b)) != RTP_OK) return rc;
         *launches += ds->last_trace_launches + 1;
@@ -2581,8 +2657,16 @@ static int launch_paths(DeviceScene* ds, const DCamera& cam, const DRender& rp, 
     return RTP_OK;
 }
 
+// The AOV buffers of an rtp_render_aov call (device pointers, either may be null)
+struct AovFrame {
+    double* albedo;
+    double* normal;
+};
+
+// aov != nullptr: an rtp_render_aov call. Its launches record every path's first vertex and never take tail mode; the records are
+// folded into ds->aov_acc beside the colour and written to aov's buffers with the colour's divisor.
 static int render_enqueue(DeviceScene* ds, const rtp_camera* camera, const rtp_render_params* p, double* d_rgb, double* d_fg, bool want_stats,
-                          cudaStream_t st, uchar4* d_rgba8 = nullptr) {
+                          cudaStream_t st, uchar4* d_rgba8 = nullptr, const AovFrame* aov = nullptr) {
     DRender rp;
     if (int rc = render_rect(p, true, &rp)) return rc;
     const uint32_t tw = rp.tile_w, th = rp.tile_h;
@@ -2600,15 +2684,20 @@ static int render_enqueue(DeviceScene* ds, const rtp_camera* camera, const rtp_r
     }
     if (npix == 0) return RTP_OK;  // no row of the rectangle falls to this call
     const uint32_t ns_total = p->sample_end - p->sample_begin;
-    const uint32_t per_launch = static_cast<uint32_t>(std::max<size_t>(1, std::min<size_t>(ns_total ? ns_total : 1, path_budget(ds, p->max_bounce) / npix)));
+    const uint32_t per_launch = static_cast<uint32_t>(std::max<size_t>(1, std::min<size_t>(ns_total ? ns_total : 1, path_budget(ds, p->max_bounce, aov != nullptr) / npix)));
     if (ns_total) {
-        int rc = reserve_paths(ds, npix * per_launch, p->max_bounce);
+        int rc = reserve_paths(ds, npix * per_launch, p->max_bounce, aov != nullptr);
         if (rc != RTP_OK) return rc;
     }
     if (ds->acc_elems < npix) {
         cudaFree(ds->acc); ds->acc = nullptr; ds->acc_elems = 0;
         RTP_CUDA(cudaMalloc(reinterpret_cast<void**>(&ds->acc), npix * sizeof(double4)));
         ds->acc_elems = npix;
+    }
+    if (aov && ds->aov_acc_elems < npix) {
+        cudaFree(ds->aov_acc); ds->aov_acc = nullptr; ds->aov_acc_elems = 0;
+        RTP_CUDA(cudaMalloc(reinterpret_cast<void**>(&ds->aov_acc), npix * 3 * sizeof(double2)));
+        ds->aov_acc_elems = npix;
     }
     const bool count = (p->flags & RTP_RENDER_COUNTERS) != 0;
     const DCamera cam = make_camera(camera);
@@ -2617,14 +2706,21 @@ static int render_enqueue(DeviceScene* ds, const rtp_camera* camera, const rtp_r
     size_t launches = 0;
     bool first = true;
     if (ns_total == 0) RTP_CUDA(cudaMemsetAsync(ds->acc, 0, npix * sizeof(double4), st));
+    if (ns_total == 0 && aov) RTP_CUDA(cudaMemsetAsync(ds->aov_acc, 0, npix * 3 * sizeof(double2), st));
     for (uint32_t s0 = 0; s0 < ns_total; s0 += per_launch) {
         rp.sample_begin = p->sample_begin + s0;
         rp.n_samples = std::min(per_launch, ns_total - s0);
-        int rc = launch_paths(ds, cam, rp, DenseTile{}, npix * rp.n_samples, count, want_stats, st, &launches);
+        int rc = aov ? launch_paths(ds, cam, rp, DenseTile{}, AovRecords{ds->aov_rec}, npix * rp.n_samples, count, want_stats, st, &launches)
+                     : launch_paths(ds, cam, rp, DenseTile{}, NoAov{}, npix * rp.n_samples, count, want_stats, st, &launches);
         if (rc != RTP_OK) return rc;
         resolve_kernel<<<static_cast<unsigned>((npix + 255) / 256), 256, 0, st>>>(ds->scratch, ds->acc, npix, rp.n_samples, first ? 1 : 0);
         RTP_CUDA(cudaGetLastError());
         ++launches;
+        if (aov) {
+            aov_resolve_kernel<<<static_cast<unsigned>((npix + 255) / 256), 256, 0, st>>>(ds->aov_rec, ds->aov_acc, npix, rp.n_samples, first ? 1 : 0);
+            RTP_CUDA(cudaGetLastError());
+            ++launches;
+        }
         first = false;
     }
     const double divisor = (p->flags & RTP_RENDER_RAW_SUMS) ? 0.0 : static_cast<double>(p->num_samples);
@@ -2637,6 +2733,11 @@ static int render_enqueue(DeviceScene* ds, const rtp_camera* camera, const rtp_r
     }
     RTP_CUDA(cudaGetLastError());
     ++launches;
+    if (aov) {
+        aov_write_kernel<<<static_cast<unsigned>((npix + 255) / 256), 256, 0, st>>>(ds->aov_acc, rp, divisor, aov->albedo, aov->normal);
+        RTP_CUDA(cudaGetLastError());
+        ++launches;
+    }
     ds->pending_launches = launches;
     ds->pending_paths = static_cast<uint64_t>(npix) * ns_total;
     if (want_stats) RTP_CUDA(cudaEventRecord(ds->ev_end, st));
@@ -2666,9 +2767,9 @@ static int render_finish(DeviceScene* ds, rtp_stats* stats) {
 }
 
 static int render_device(rtp_scene* scene, const rtp_camera* camera, const rtp_render_params* p, double* d_rgb, double* d_fg, rtp_stats* stats,
-                         cudaStream_t st, uchar4* d_rgba8 = nullptr) {
+                         cudaStream_t st, uchar4* d_rgba8 = nullptr, const AovFrame* aov = nullptr) {
     DeviceScene* ds = scene->dev;
-    int rc = render_enqueue(ds, camera, p, d_rgb, d_fg, stats != nullptr, st, d_rgba8);
+    int rc = render_enqueue(ds, camera, p, d_rgb, d_fg, stats != nullptr, st, d_rgba8, aov);
     if (rc != RTP_OK) return rc;
     return stats ? render_finish(ds, stats) : RTP_OK;
 }
@@ -2782,7 +2883,7 @@ static int adaptive_round(AdaptiveDev& d, const DCamera& cam, uint32_t s0, uint3
     for (uint32_t l0 = 0; l0 < B; l0 += per_launch) {
         d.rp.sample_begin = s0 + l0;
         d.rp.n_samples = std::min(per_launch, B - l0);
-        int rc = launch_paths(ds, cam, d.rp, map, static_cast<size_t>(d.n_live) * d.rp.n_samples, count, want_stats, d.st, &d.launches);
+        int rc = launch_paths(ds, cam, d.rp, map, NoAov{}, static_cast<size_t>(d.n_live) * d.rp.n_samples, count, want_stats, d.st, &d.launches);
         if (rc != RTP_OK) return rc;
         adaptive_resolve_kernel<<<grid, 256, 0, d.st>>>(ds->scratch, map.live, d.n_live, d.rp.n_samples, ds->acc, ds->moments, ds->counts, ds->keep,
                                                         l0 + per_launch >= B ? 1 : 0, rule);
@@ -3276,8 +3377,9 @@ int rtp_render_device(rtp_scene* scene, const rtp_camera* camera, const rtp_rend
 // the devices taking part (params->device_mask), every device renders ALL samples of its rows and copies them straight into the
 // caller's frame: no exchange between devices, and since a pixel's value depends only on (seed, pixel, sample) the frame is
 // bit-identical to a one-device render. All devices are driven from this one host thread: render_enqueue never synchronises.
+// aov != nullptr (host pointers, either may be null): an rtp_render_aov call, whose staging frame holds 6 more doubles per pixel.
 static int render_host(rtp_scene* scene, const rtp_camera* camera, const rtp_render_params* params, double* rgb_out, double* foreground_out,
-                       uint8_t* rgba_out, rtp_stats* stats) {
+                       uint8_t* rgba_out, rtp_stats* stats, const AovFrame* aov = nullptr) {
     const size_t npx = static_cast<size_t>(params->width) * params->height;
     if (npx == 0) return set_error(RTP_ERR_INVALID, "bad frame parameters");
     std::vector<DeviceScene*> devs;
@@ -3308,13 +3410,14 @@ static int render_host(rtp_scene* scene, const rtp_camera* camera, const rtp_ren
                 RTP_CUDA(cudaMalloc(reinterpret_cast<void**>(&ds->fixes), kSrgbFixCap * sizeof(SrgbFix)));
                 RTP_CUDA(cudaMalloc(reinterpret_cast<void**>(&ds->n_fixes), sizeof(unsigned int)));
             }
-        } else if (ds->frame_elems < npx * 4) {
+        } else if (ds->frame_elems < npx * (aov ? 10 : 4)) {  // rgb, foreground [, albedo, normal]
             cudaFree(ds->frame); ds->frame = nullptr; ds->frame_elems = 0;
-            RTP_CUDA(cudaMalloc(reinterpret_cast<void**>(&ds->frame), npx * 4 * sizeof(double)));
-            ds->frame_elems = npx * 4;
+            RTP_CUDA(cudaMalloc(reinterpret_cast<void**>(&ds->frame), npx * (aov ? 10 : 4) * sizeof(double)));
+            ds->frame_elems = npx * (aov ? 10 : 4);
         }
+        const AovFrame d_aov = {aov && aov->albedo ? ds->frame + npx * 4 : nullptr, aov && aov->normal ? ds->frame + npx * 7 : nullptr};
         rc = render_enqueue(ds, camera, &p, rgba_out ? nullptr : ds->frame, (!rgba_out && foreground_out) ? ds->frame + npx * 3 : nullptr, stats != nullptr, st,
-                            rgba_out ? ds->frame8 : nullptr);
+                            rgba_out ? ds->frame8 : nullptr, aov ? &d_aov : nullptr);
         if (rc != RTP_OK) break;
         // only the rows this device rendered travel back (main.rs:86-87 writes per tile)
         if (p.row_offset >= th_full || tx >= W) continue;
@@ -3328,6 +3431,10 @@ static int render_host(rtp_scene* scene, const rtp_camera* camera, const rtp_ren
             RTP_CUDA(cudaMemcpy2DAsync(rgb_out + 3 * first, row_px * 24, ds->frame + 3 * first, row_px * 24, static_cast<size_t>(tw) * 24, rows, cudaMemcpyDeviceToHost, st));
             if (foreground_out)
                 RTP_CUDA(cudaMemcpy2DAsync(foreground_out + first, row_px * 8, ds->frame + npx * 3 + first, row_px * 8, static_cast<size_t>(tw) * 8, rows, cudaMemcpyDeviceToHost, st));
+            if (d_aov.albedo)
+                RTP_CUDA(cudaMemcpy2DAsync(aov->albedo + 3 * first, row_px * 24, d_aov.albedo + 3 * first, row_px * 24, static_cast<size_t>(tw) * 24, rows, cudaMemcpyDeviceToHost, st));
+            if (d_aov.normal)
+                RTP_CUDA(cudaMemcpy2DAsync(aov->normal + 3 * first, row_px * 24, d_aov.normal + 3 * first, row_px * 24, static_cast<size_t>(tw) * 24, rows, cudaMemcpyDeviceToHost, st));
         }
     }
     // wait for every device that was given work, even after an error on a later one
@@ -3374,6 +3481,31 @@ int rtp_render(rtp_scene* scene, const rtp_camera* camera, const rtp_render_para
                rtp_stats* stats) {
     if (!scene || !camera || !params || !rgb_out) return set_error(RTP_ERR_INVALID, "null argument");
     return render_host(scene, camera, params, rgb_out, foreground_out, nullptr, stats);
+}
+
+// rtp_render plus each pixel's mean first-vertex albedo and normal (DESIGN.md §6c)
+static int check_aov(const rtp_scene* scene, const rtp_camera* camera, const rtp_render_params* params, const double* rgb_out) {
+    if (!scene || !camera || !params || !rgb_out) return set_error(RTP_ERR_INVALID, "null argument");
+    if (params->flags & ~(RTP_RENDER_RAW_SUMS | RTP_RENDER_COUNTERS))
+        return set_error(RTP_ERR_INVALID, "aov: flags other than RTP_RENDER_RAW_SUMS | RTP_RENDER_COUNTERS");
+    return RTP_OK;
+}
+
+int rtp_render_aov(rtp_scene* scene, const rtp_camera* camera, const rtp_render_params* params, double* rgb_out, double* foreground_out,
+                   double* albedo_out, double* normal_out, rtp_stats* stats) {
+    if (int rc = check_aov(scene, camera, params, rgb_out)) return rc;
+    const AovFrame aov = {albedo_out, normal_out};
+    return render_host(scene, camera, params, rgb_out, foreground_out, nullptr, stats, &aov);
+}
+
+int rtp_render_aov_device(rtp_scene* scene, const rtp_camera* camera, const rtp_render_params* params, double* d_rgb_out, double* d_foreground_out,
+                          double* d_albedo_out, double* d_normal_out, rtp_stats* stats, void* cuda_stream) {
+    if (int rc = check_aov(scene, camera, params, d_rgb_out)) return rc;
+    DeviceScene* ds = scene->dev;
+    std::lock_guard<std::mutex> guard(ds->lock);
+    RTP_CUDA(cudaSetDevice(ds->device));
+    const AovFrame aov = {d_albedo_out, d_normal_out};
+    return render_device(scene, camera, params, d_rgb_out, d_foreground_out, stats, static_cast<cudaStream_t>(cuda_stream), nullptr, &aov);
 }
 
 // The rows of the tile rectangle are dealt out to the devices as in render_host; each device runs its own live list through the same

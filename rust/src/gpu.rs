@@ -49,6 +49,8 @@ extern "C" {
                   rgb: *mut f64, foreground: *mut f64, stats: *mut rtp_stats) -> c_int;
     fn rtp_render_adaptive(scene: *mut rtp_scene, camera: *const rtp_camera, params: *const rtp_render_params, adaptive: *const rtp_adaptive_params,
                            rgb: *mut f64, foreground: *mut f64, samples: *mut u32, stats: *mut rtp_stats) -> c_int;
+    fn rtp_render_aov(scene: *mut rtp_scene, camera: *const rtp_camera, params: *const rtp_render_params,
+                      rgb: *mut f64, foreground: *mut f64, albedo: *mut f64, normal: *mut f64, stats: *mut rtp_stats) -> c_int;
 }
 
 type GpuResult<T> = Result<T, Box<dyn std::error::Error>>; // the crate's loaders return Result<_, Box<dyn Error>> (mesh.rs:145)
@@ -167,6 +169,21 @@ impl GpuScene {
         let mut stats = rtp_stats::default();
         check(unsafe { rtp_render(self.0, &Self::camera(camera), &p, rgb.as_mut_ptr(), fg.as_mut_ptr(), &mut stats) })?;
         Ok((rgb, fg, stats))
+    }
+
+    /// render_frame plus the guide buffers of a denoiser: per pixel the mean over its samples of the first vertex's
+    /// `Absorb::evaluate` (material.rs:74-81) and `Hit::normal` (not flipped, not renormalised; (0, 0, 0) for a miss).
+    /// Returns (rgb, foreground, albedo, normal, stats); rgb and foreground are render_frame's bits.
+    pub fn render_frame_aov(&self, camera: &Camera, sampler: &Multisampler, max_bounce: u32, seed: u64)
+                            -> GpuResult<(Vec<f64>, Vec<f64>, Vec<f64>, Vec<f64>, rtp_stats)> {
+        let npx = (sampler.width * sampler.height) as usize;
+        let (mut rgb, mut fg, mut albedo, mut normal) = (vec![0.0; 3 * npx], vec![0.0; npx], vec![0.0; 3 * npx], vec![0.0; 3 * npx]);
+        let p = rtp_render_params { width: sampler.width, height: sampler.height, num_samples: sampler.num_samples, max_bounce, seed,
+            sample_begin: 0, sample_end: sampler.num_samples, ..Default::default() };
+        let mut stats = rtp_stats::default();
+        check(unsafe { rtp_render_aov(self.0, &Self::camera(camera), &p, rgb.as_mut_ptr(), fg.as_mut_ptr(), albedo.as_mut_ptr(),
+                                      normal.as_mut_ptr(), &mut stats) })?;
+        Ok((rgb, fg, albedo, normal, stats))
     }
 }
 
