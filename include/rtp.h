@@ -458,10 +458,24 @@ int rtp_rng_draws(uint64_t seed, uint32_t index_lo, uint32_t index_hi, uint32_t 
 /* ---------------------------------------------------------------- diagnostics ----------- */
 
 /* Structural digests of a scene's device-resident build, read back from its first device: [0] the exact binary culling tree
- * (pre-order boxes, skip pointers, leaf slots), [1] primitive and attribute records in rank order, [2] the 4-wide culling tree,
- * hashed from the root down so that the numbering of its nodes does not matter, [3] number of 4-wide nodes | levels << 32.
+ * (pre-order boxes, skip pointers, leaf slots), [1] primitive and attribute records in rank order, [2] the 4-wide culling tree
+ * with its culled-set box, then the order-free culling tree if there is one, each hashed from the root down so that the numbering
+ * of its nodes does not matter, [3] number of 4-wide nodes | levels << 32.
  * Two builds of the same description (host build, device build: RTP_DEVICE_BUILD) must agree in all four. Tests only. */
 int rtp_scene_digest(const rtp_scene* scene, uint64_t digest_out[4]);
+
+/* The any-order walk's scene tables as the scene holds them (DESIGN.md §4b); all zero except the empty culled-set box when the
+ * scene does not take that walk. Tests only. */
+typedef struct rtp_any_tables {
+    uint32_t n_big;        /* outsized primitives tested before the walk, at most 8                                  */
+    uint32_t big[8];       /* their slots (DFS ranks) | kind << 31, largest extent first, ties by slot; 0 past n_big  */
+    uint32_t any_spheres;  /* 1: some sphere is not big                                                             */
+    double any_E, any_A;   /* triangles that are not big: largest extent, largest |coordinate|, each x (1 + 1e-12)   */
+    double any_C, any_R;   /* spheres that are not big: largest |box coordinate|, largest radius, each x (1 + 1e-12) */
+    double scene_mag;      /* largest |coordinate| of any leaf box                                                  */
+    float cull[6];         /* culled-set box: min xyz, max xyz rounded out to f32; (+inf, -inf) if empty            */
+} rtp_any_tables;
+int rtp_scene_any_tables(const rtp_scene* scene, rtp_any_tables* out);
 
 /* Measured f64 instruction throughput of the bound device, in 1e9 unfused f64 operations (DMUL or DADD, the
  * only kind the path executes: the reference never contracts a*b+c) per second: the denominator of the

@@ -176,6 +176,20 @@ class SceneInfo(C.Structure):
     ]
 
 
+class AnyTables(C.Structure):
+    _fields_ = [
+        ("n_big", C.c_uint32),
+        ("big", C.c_uint32 * 8),
+        ("any_spheres", C.c_uint32),
+        ("any_E", C.c_double),
+        ("any_A", C.c_double),
+        ("any_C", C.c_double),
+        ("any_R", C.c_double),
+        ("scene_mag", C.c_double),
+        ("cull", C.c_float * 6),
+    ]
+
+
 class Image(C.Structure):
     _fields_ = [("rgba", C.c_void_p), ("width", C.c_uint32), ("height", C.c_uint32)]
 
@@ -229,6 +243,7 @@ PROTOTYPES = {
     "rtp_rng_draws": (C.c_int, [C.c_uint64, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p]),
     "rtp_probe_fp64": (C.c_int, [C.POINTER(C.c_double)]),
     "rtp_scene_digest": (C.c_int, [C.c_void_p, C.POINTER(C.c_uint64)]),
+    "rtp_scene_any_tables": (C.c_int, [C.c_void_p, _P(AnyTables)]),
 }
 
 # RTP_B200_LIB: another build of the same library (kernel A/B runs from tools/); it is still this product's CUDA library

@@ -568,6 +568,12 @@ class Scene:
         _check(self._lib, self._lib.rtp_scene_digest(self._h, out))
         return tuple(int(x) for x in out)
 
+    def any_tables(self) -> A.AnyTables:
+        """the any-order walk's scene tables (rtp_scene_any_tables): big primitives, slack constants, scene magnitude, culled-set box"""
+        t = A.AnyTables()
+        _check(self._lib, self._lib.rtp_scene_any_tables(self._h, C.byref(t)))
+        return t
+
     def devices(self) -> int:
         """bit d set = the scene holds a replica on CUDA device d"""
         m = C.c_uint32(0)

@@ -130,6 +130,7 @@ int device_reference_order_dev(const double* d_boxes, uint32_t n, uint32_t* d_or
 //   records                DPrim / DAttr in rank order (flatten_scene)
 //   4-wide collapse        WideBuilder: expand the internal child of largest area until four children
 //   any-order tables       prepare_any_order: big primitives (extent > 16 x median, the eight largest), E / A / C / R, scene magnitude
+//   order-free tree        prepare_any_order's build_free_tree itself, on the host, over the leaf boxes read back
 // The SAH build is level-synchronous: all ranges of one depth are processed by a handful of whole-array passes — a forward and a
 // backward segmented scan of box unions (cub::DeviceScan::InclusiveScanByKey: library code for this once-per-scene stage), a cost
 // pass with a per-range atomic minimum, and a split pass that writes the nodes of that depth straight into their pre-order slots.
@@ -171,10 +172,11 @@ struct MeshRef {  // one rtp_mesh on the device: where its vertices / indices st
 };
 
 // ---- leaf boxes + validation (flatten_scene "leaf boxes") ----------------------------------------------------------------------------
-// status[0]: smallest failing hittable index + 1 (0 = none), status[1]: its error class, status[2]: 1 = some box is inverted or non-finite
+// status[0]: index << 3 | error class of the smallest failing hittable (all ones: none; one atomic word, so that the class belongs
+// to the index), status[1]: 1 = some box is inverted or non-finite
 __global__ void __launch_bounds__(256) leaf_boxes_kernel(const rtp_hittable* __restrict__ hs, uint32_t n, const MeshRef* __restrict__ meshes, uint32_t n_meshes,
                                                           uint32_t n_materials, const rtp_vertex* __restrict__ verts, const uint32_t* __restrict__ idx,
-                                                          Box6* __restrict__ boxes, unsigned int* __restrict__ status) {
+                                                          Box6* __restrict__ boxes, unsigned long long* __restrict__ status) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     const rtp_hittable h = hs[i];
@@ -203,14 +205,11 @@ __global__ void __launch_bounds__(256) leaf_boxes_kernel(const rtp_hittable* __r
             const double key = 0.5 * (b.lo[k] + b.hi[k]);
             if (key != key) err = 4;  // partial_cmp().unwrap() panics on NaN (bvh.rs:63)
         }
-    if (err) {
-        const unsigned int prev = atomicMin(&status[0], i + 1u);
-        if (i + 1u <= prev) status[1] = err;  // racy among equal-index writers only (there are none)
-    }
+    if (err) atomicMin(&status[0], static_cast<unsigned long long>(i) << 3 | err);
     bool regular = true;
     for (int k = 0; k < 3; ++k)
         if (!(b.lo[k] <= b.hi[k]) || !(fabs(b.lo[k]) <= 1.7976931348623157e308) || !(fabs(b.hi[k]) <= 1.7976931348623157e308)) regular = false;
-    if (!regular) status[2] = 1u;
+    if (!regular) status[1] = 1ull;
     boxes[i] = b;
 }
 
@@ -543,29 +542,29 @@ int device_build_scene(const rtp_scene_desc* d, const Switches& sw, FlatScene* o
     // ---- leaf boxes + validation -----------------------------------------------------------------------------------------------------------
     const unsigned grid = (n + 255) / 256;
     Box6 *d_boxes = nullptr, *d_ranked = nullptr;
-    unsigned int* d_status = nullptr;
+    unsigned long long* d_status = nullptr;
     RTP_DALLOC(d_boxes, static_cast<size_t>(n) * sizeof(Box6));
     RTP_DALLOC(d_ranked, static_cast<size_t>(n) * sizeof(Box6));
-    RTP_DALLOC(d_status, 4 * sizeof(unsigned int));
+    RTP_DALLOC(d_status, 2 * sizeof(unsigned long long));
     {
-        const unsigned int init[4] = {0xFFFFFFFFu, 0u, 0u, 0u};
+        const unsigned long long init[2] = {~0ull, 0ull};
         RTP_CUDA_B(cudaMemcpy(d_status, init, sizeof init, cudaMemcpyHostToDevice));
     }
     leaf_boxes_kernel<<<grid, 256>>>(d_hs, n, d_refs, d->n_meshes, d->n_materials, d_verts, d_idx, d_boxes, d_status);
     RTP_CUDA_B(cudaGetLastError());
-    unsigned int status[4];
+    unsigned long long status[2];
     RTP_CUDA_B(cudaMemcpy(status, d_status, sizeof status, cudaMemcpyDeviceToHost));
-    if (status[0] != 0xFFFFFFFFu) {
+    if (status[0] != ~0ull) {
         cleanup();
-        const uint32_t bad = status[0] - 1u;
-        switch (status[1]) {
+        const uint64_t bad = status[0] >> 3;
+        switch (status[0] & 7u) {
             case 1: return set_error(RTP_ERR_INVALID, "sphere material out of range");
             case 2: return set_error(RTP_ERR_INVALID, "triangle id out of range");
             case 4: return set_error(RTP_ERR_INVALID, "NaN bounding-box centroid in hittable " + std::to_string(bad));
             default: return set_error(RTP_ERR_INVALID, "unknown hittable kind");
         }
     }
-    if (status[2]) { cleanup(); return 1; }  // inverted / non-finite boxes keep the reference topology: host path (DESIGN.md §2)
+    if (status[1]) { cleanup(); return 1; }  // inverted / non-finite boxes keep the reference topology: host path (DESIGN.md §2)
     lap("leaf boxes and validation");
 
     // ---- reference order (bvh.rs:36-67), boxes stay on the device ----------------------------------------------------------------------------
@@ -719,6 +718,8 @@ int device_build_scene(const rtp_scene_desc* d, const Switches& sw, FlatScene* o
     size_t n_wide = 0;
     for (int pass = 0; pass < 2; ++pass) {
         if (pass == 1) {
+            // as prepare_any_order: a tree too deep for the any-order walk's stack gets no any-order tables, so no leaf is marked big
+            if (level_size.size() > 48) { n_big = 0; std::fill(h_big, h_big + 8, 0u); }
             for (uint32_t m : level_size) n_wide += m;
             RTP_DALLOC(d_wide, n_wide * sizeof(DWide));
             RTP_DALLOC(d_wboxes, n_wide * 24 * sizeof(double));
@@ -752,6 +753,19 @@ int device_build_scene(const rtp_scene_desc* d, const Switches& sw, FlatScene* o
     }
     lap("4-wide collapse (breadth first)");
 
+    // ---- order-free culling tree: the host's builder over the leaf boxes, read back ----------------------------------------------------------
+    const bool any_ok = level_size.size() <= 48;
+    out->n_big = n_big;
+    if (any_ok && n > n_big && want_free_tree(sw, n)) {
+        std::vector<Box6> boxes(n);
+        RTP_CUDA_B(cudaMemcpy(boxes.data(), d_ranked, static_cast<size_t>(n) * sizeof(Box6), cudaMemcpyDeviceToHost));
+        std::vector<uint8_t> kind(n), is_big(n, 0);
+        for (uint32_t s = 0; s < n; ++s) kind[s] = static_cast<uint8_t>(d->hittables[out->leaf_order[s]].kind);
+        for (uint32_t k = 0; k < n_big; ++k) is_big[h_big[k] & 0x7FFFFFFFu] = 1;
+        build_free_tree(boxes[0].lo, boxes[0].hi, sizeof(Box6) / sizeof(double), kind, is_big, out);
+        lap("order-free culling tree (host)");
+    }
+
     // ---- hand over -------------------------------------------------------------------------------------------------------------------------------
     RTP_CUDA_B(cudaDeviceSynchronize());
     auto keep = [&](void* p) { scratch.erase(std::remove(scratch.begin(), scratch.end(), p), scratch.end()); };
@@ -772,21 +786,19 @@ int device_build_scene(const rtp_scene_desc* d, const Switches& sw, FlatScene* o
     }
     out->boxes_finite = true;
     out->scene_mag = as_double(hc.mag);
-    out->n_big = n_big;
-    for (int k = 0; k < 8; ++k) out->big[k] = h_big[k];
-    out->any_E = as_double(hc.E) * (1.0 + 1e-12);
-    out->any_A = as_double(hc.A) * (1.0 + 1e-12);
-    out->any_C = as_double(hc.C) * (1.0 + 1e-12);
-    out->any_R = as_double(hc.R) * (1.0 + 1e-12);
-    out->any_spheres = hc.spheres != 0u;
-    {
+    out->any_ok = any_ok;
+    if (any_ok) {
+        for (int k = 0; k < 8; ++k) out->big[k] = h_big[k];
+        out->any_E = as_double(hc.E) * (1.0 + 1e-12);
+        out->any_A = as_double(hc.A) * (1.0 + 1e-12);
+        out->any_C = as_double(hc.C) * (1.0 + 1e-12);
+        out->any_R = as_double(hc.R) * (1.0 + 1e-12);
+        out->any_spheres = hc.spheres != 0u;
         double lo[3], hi[3];
         for (int k = 0; k < 3; ++k) { lo[k] = from_order_key(~hc.lo[k]); hi[k] = from_order_key(hc.hi[k]); }
         if (hc.hi[0] == 0ull) lo[0] = 1.0, hi[0] = 0.0;  // every primitive is big: the empty box
         culled_set_box(lo, hi, out->cull);
     }
-    out->any_ok = out->wide_depth <= 48;
-    out->free_depth = 0;
     return RTP_OK;
 #undef RTP_DALLOC
 }

@@ -2005,6 +2005,7 @@ struct DeviceScene {
     size_t n_wide = 0;
     double* wide_boxes = nullptr;
     DWide* free_wide = nullptr;        // order-free culling tree of a big scene (any-order lanes), or nullptr
+    size_t n_free_wide = 0;
     double* free_boxes = nullptr;
     size_t stack_bytes = 0;            // dynamic shared memory of the persistent kernels: wide_depth x 128 threads x 4 B
     DPrim* prims = nullptr;
@@ -2176,6 +2177,7 @@ int device_scene_upload(const FlatScene& flat, const Switches& sw, int device, D
     if (!flat.free_wide.empty()) {
         if ((rc = upload(flat.free_wide, &ds->free_wide, &ds->bytes)) != RTP_OK) return bail(rc);
         if ((rc = upload(flat.free_boxes, &ds->free_boxes, &ds->bytes)) != RTP_OK) return bail(rc);
+        ds->n_free_wide = flat.free_wide.size();
     }
     // one stack word per tree level and thread; a tree deeper than 96 levels (degenerate geometry) does not get the f32 walk
     // at all (f32_culling below), so its launches carry no stack
@@ -3035,44 +3037,68 @@ int rtp_scene_digest(const rtp_scene* scene, uint64_t digest_out[4]) {
             if (n_prims) RTP_CUDA(cudaMemcpy(attrs.data(), ds->attrs, n_prims * sizeof(DAttr), cudaMemcpyDeviceToHost));
             h1 = fnv(h1, attrs.data(), n_prims * sizeof(DAttr));
         }
-        std::vector<DWide> wide(n_wide);
-        if (n_wide) RTP_CUDA(cudaMemcpy(wide.data(), ds->wide, n_wide * sizeof(DWide), cudaMemcpyDeviceToHost));
-        // post-order over the tree from node 0: a node's hash folds its planes and, per child, the leaf word or the child's hash
-        std::vector<uint64_t> hash(n_wide, 0);
-        std::vector<uint8_t> done(n_wide, 0);
-        std::vector<uint32_t> stack;
-        uint32_t levels = 0;
-        std::vector<uint32_t> depth_of(n_wide, 0);
-        if (n_wide) { stack.push_back(0); depth_of[0] = 1; }
-        while (!stack.empty()) {
-            const uint32_t i = stack.back();
-            bool ready = true;
-            for (int k = 0; k < 4; ++k) {
-                const uint32_t c = wide[i].child[k];
-                if (!(c & kWideLeaf) && !done[c]) { if (c >= n_wide) return set_error(RTP_ERR_INVALID, "4-wide tree: child index out of range"); depth_of[c] = depth_of[i] + 1; stack.push_back(c); ready = false; }
+        // a 4-wide tree hashed from its root down: a node's hash folds its planes and, per child, the leaf word or the child's hash
+        // (post-order from node 0), so that the numbering of the nodes does not matter. Returns 0 and sets *bad on a dangling child.
+        auto tree_hash = [&](const DWide* d_wide, size_t n, uint32_t* levels, bool* bad) -> uint64_t {
+            std::vector<DWide> wide(n);
+            if (n && cudaMemcpy(wide.data(), d_wide, n * sizeof(DWide), cudaMemcpyDeviceToHost) != cudaSuccess) { *bad = true; return 0; }
+            std::vector<uint64_t> hash(n, 0);
+            std::vector<uint8_t> done(n, 0);
+            std::vector<uint32_t> stack, depth_of(n, 0);
+            *levels = 0;
+            if (n) { stack.push_back(0); depth_of[0] = 1; }
+            while (!stack.empty()) {
+                const uint32_t i = stack.back();
+                bool ready = true;
+                for (int k = 0; k < 4; ++k) {
+                    const uint32_t c = wide[i].child[k];
+                    if (!(c & kWideLeaf) && !done[c]) { if (c >= n) { *bad = true; return 0; } depth_of[c] = depth_of[i] + 1; stack.push_back(c); ready = false; }
+                }
+                if (!ready) continue;
+                stack.pop_back();
+                float planes[24];
+                for (int k = 0; k < 24; ++k) planes[k] = (&wide[i].plane[0][0][0])[k] + 0.0f;
+                uint64_t h = fnv(0xCBF29CE484222325ull, planes, sizeof planes);
+                for (int k = 0; k < 4; ++k) {
+                    const uint32_t c = wide[i].child[k];
+                    const uint64_t v = (c & kWideLeaf) ? static_cast<uint64_t>(c) : hash[c];
+                    h = fnv(h, &v, 8);
+                }
+                hash[i] = h; done[i] = 1;
+                *levels = std::max(*levels, depth_of[i]);
             }
-            if (!ready) continue;
-            stack.pop_back();
-            float planes[24];
-            for (int k = 0; k < 24; ++k) planes[k] = (&wide[i].plane[0][0][0])[k] + 0.0f;
-            uint64_t h = fnv(0xCBF29CE484222325ull, planes, sizeof planes);
-            for (int k = 0; k < 4; ++k) {
-                const uint32_t c = wide[i].child[k];
-                const uint64_t v = (c & kWideLeaf) ? static_cast<uint64_t>(c) : hash[c];
-                h = fnv(h, &v, 8);
-            }
-            hash[i] = h; done[i] = 1;
-            levels = std::max(levels, depth_of[i]);
-        }
+            return n ? hash[0] : 0;
+        };
+        uint32_t levels = 0, free_levels = 0;
+        bool bad = false;
+        uint64_t h2 = tree_hash(ds->wide, n_wide, &levels, &bad);
         if (n_wide) {  // the culled-set box belongs to the culling tree
             float cull[6];
             for (int k = 0; k < 6; ++k) cull[k] = ds->view.cull[k] + 0.0f;
-            hash[0] = fnv(hash[0], cull, sizeof cull);
+            h2 = fnv(h2, cull, sizeof cull);
         }
-        digest_out[0] = h0; digest_out[1] = h1; digest_out[2] = n_wide ? hash[0] : 0; digest_out[3] = static_cast<uint64_t>(n_wide) | (static_cast<uint64_t>(levels) << 32);
+        if (ds->free_wide) {  // and so does the order-free tree of the any-order lanes
+            const uint64_t hf = tree_hash(ds->free_wide, ds->n_free_wide, &free_levels, &bad);
+            h2 = fnv(h2, &hf, 8);
+        }
+        if (bad) return set_error(RTP_ERR_INVALID, "4-wide tree: child index out of range or unreadable");
+        digest_out[0] = h0; digest_out[1] = h1; digest_out[2] = h2; digest_out[3] = static_cast<uint64_t>(n_wide) | (static_cast<uint64_t>(levels) << 32);
     } catch (const std::exception& e) {
         return set_error(RTP_ERR_NOMEM, e.what());
     }
+    return RTP_OK;
+}
+
+int rtp_scene_any_tables(const rtp_scene* scene, rtp_any_tables* out) {
+    if (!scene || !out) return set_error(RTP_ERR_INVALID, "null argument");
+    const FlatScene& f = scene->flat;
+    std::memset(out, 0, sizeof *out);
+    out->n_big = f.n_big;
+    for (int k = 0; k < 8; ++k) out->big[k] = f.big[k];
+    out->any_spheres = f.any_spheres ? 1u : 0u;
+    out->any_E = f.any_E; out->any_A = f.any_A; out->any_C = f.any_C; out->any_R = f.any_R;
+    out->scene_mag = f.scene_mag;
+    for (int k = 0; k < 6; ++k) out->cull[k] = f.cull[k];
     return RTP_OK;
 }
 

@@ -393,7 +393,6 @@ static void build_wide(const std::vector<DNode>& bn, std::vector<DWide>* out_wid
 // outsized primitives of a scene - the ground sphere of the bunny scenes, a floor made of two huge triangles - are taken out
 // of the culled set: up to kMaxBig "big" primitives are tested when the ray starts, before its walk, and skipped when the walk
 // meets their leaves. A tree too deep for the shared-memory stack, or irregular boxes, and the scene keeps the in-order walk.
-constexpr size_t kFreeTreeLeaves = 262144;  // scenes below this size get the second, order-free culling tree
 
 // the leaf words of the big primitives carry kWideBig: the walk skips them
 static void mark_big(std::vector<DWide>& wide, const std::vector<uint8_t>& is_big) {
@@ -462,20 +461,24 @@ static void prepare_any_order(const Switches& sw, FlatScene* out) {
     mark_big(out->wide, is_big);
     out->any_ok = true;
 
-    // Free tree. The any-order walk does not need its leaves in the reference's depth-first order (only the re-walk does), so
-    // its lanes may walk a second culling tree built over the MORTON order of the leaf centroids with the same SAH-over-a-sequence
-    // builder and the same 4-wide collapse; its leaves carry the same slots. Measured: 4-6 % faster on the bunny (4.06 instead of
-    // 4.26 nodes per primary ray, 4 ms of build), no gain on the bunny fields (15.4 instead of 15.6 nodes, 1.5 s of build for
-    // 2.5 M leaves) - so only scenes below kFreeTreeLeaves get it by default. It holds only the primitives that are not big: those
-    // are tested before the walk starts, and left out the root box no longer spans the ground sphere that every ray enters.
-    const bool want_free = sw.free_tree >= 0 ? sw.free_tree != 0 : n < kFreeTreeLeaves;
-    const size_t m = n - out->n_big;
-    if (!want_free || n < 2 || m == 0) return;
+    if (n >= 2 && n > out->n_big && want_free_tree(sw, n)) build_free_tree(out->prims[0].bmin, out->prims[0].bmax, sizeof(DPrim) / sizeof(double), kind, is_big, out);
+}
+
+// Free tree. The any-order walk does not need its leaves in the reference's depth-first order (only the re-walk does), so
+// its lanes may walk a second culling tree built over the MORTON order of the leaf centroids with the same SAH-over-a-sequence
+// builder and the same 4-wide collapse; its leaves carry the same slots. Measured: 4-6 % faster on the bunny (4.06 instead of
+// 4.26 nodes per primary ray, 4 ms of build), no gain on the bunny fields (15.4 instead of 15.6 nodes, 1.5 s of build for
+// 2.5 M leaves) - so only scenes below kFreeTreeLeaves get it by default. It holds only the primitives that are not big: those
+// are tested before the walk starts, and left out the root box no longer spans the ground sphere that every ray enters.
+void build_free_tree(const double* bmin, const double* bmax, size_t stride, const std::vector<uint8_t>& kind, const std::vector<uint8_t>& is_big,
+                     FlatScene* out) {
+    const size_t n = kind.size(), m = n - out->n_big;
+    auto lo_of = [&](size_t s) { return bmin + s * stride; };
+    auto hi_of = [&](size_t s) { return bmax + s * stride; };
     double lo[3] = {1e300, 1e300, 1e300}, hi[3] = {-1e300, -1e300, -1e300};
     for (size_t s = 0; s < n; ++s) {
         if (is_big[s]) continue;
-        const DPrim& p = out->prims[s];
-        for (int k = 0; k < 3; ++k) { const double c = 0.5 * (p.bmin[k] + p.bmax[k]); lo[k] = std::fmin(lo[k], c); hi[k] = std::fmax(hi[k], c); }
+        for (int k = 0; k < 3; ++k) { const double c = 0.5 * (lo_of(s)[k] + hi_of(s)[k]); lo[k] = std::fmin(lo[k], c); hi[k] = std::fmax(hi[k], c); }
     }
     auto spread = [](uint64_t x) {  // 21 bits -> every third bit
         x &= 0x1FFFFFull;
@@ -488,10 +491,9 @@ static void prepare_any_order(const Switches& sw, FlatScene* out) {
         for (size_t s = a; s < b; ++s) {
             uint64_t key = 0;  // big primitives sort first and are dropped below
             if (!is_big[s]) {
-                const DPrim& p = out->prims[s];
                 uint64_t q[3];
                 for (int k = 0; k < 3; ++k) {
-                    const double c = 0.5 * (p.bmin[k] + p.bmax[k]), ext = hi[k] - lo[k];
+                    const double c = 0.5 * (lo_of(s)[k] + hi_of(s)[k]), ext = hi[k] - lo[k];
                     const double f = ext > 0.0 ? (c - lo[k]) / ext : 0.0;
                     q[k] = static_cast<uint64_t>(std::fmin(std::fmax(f, 0.0), 1.0) * 2097151.0);
                 }
@@ -503,10 +505,10 @@ static void prepare_any_order(const Switches& sw, FlatScene* out) {
     std::sort(keyed.begin(), keyed.end());
     std::vector<BuildItem> seq(m);
     for (size_t i = 0; i < m; ++i) {
-        const DPrim& p = out->prims[keyed[out->n_big + i].second];
-        seq[i].id = keyed[out->n_big + i].second;
-        std::memcpy(seq[i].bmin, p.bmin, sizeof p.bmin);
-        std::memcpy(seq[i].bmax, p.bmax, sizeof p.bmax);
+        const uint32_t s = keyed[out->n_big + i].second;
+        seq[i].id = s;
+        std::memcpy(seq[i].bmin, lo_of(s), sizeof seq[i].bmin);
+        std::memcpy(seq[i].bmax, hi_of(s), sizeof seq[i].bmax);
     }
     std::vector<DNode> nodes(2 * m - 1);
     SeqBuilder sb{seq, nodes};
@@ -727,27 +729,30 @@ int flatten_scene(const rtp_scene_desc* d, const Switches& sw, FlatScene* out, b
         }
     } else {
     items.resize(n);
-    std::atomic<int> first_bad{0};
+    // the error of the smallest failing index, whichever chunk finds it first (the device build reports the same one): a chunk
+    // stops at its first failure, or once a smaller failing index is known
+    std::atomic<uint32_t> first_bad{std::numeric_limits<uint32_t>::max()};
+    int bad_code = RTP_OK;
     std::string bad_msg;
     std::mutex bad_lock;
-    auto fail = [&](int code, const std::string& msg) {
+    auto fail = [&](uint32_t i, int code, const std::string& msg) {
         std::lock_guard<std::mutex> g(bad_lock);
-        if (!first_bad.load()) { first_bad.store(code); bad_msg = msg; }
+        if (i < first_bad.load()) { first_bad.store(i); bad_code = code; bad_msg = msg; }
     };
     parallel_chunks(n, [&](size_t lo_i, size_t hi_i) {
-      for (uint32_t i = static_cast<uint32_t>(lo_i); i < hi_i && !first_bad.load(std::memory_order_relaxed); ++i) {
+      for (uint32_t i = static_cast<uint32_t>(lo_i); i < hi_i && i < first_bad.load(std::memory_order_relaxed); ++i) {
         const rtp_hittable& h = d->hittables[i];
         BuildItem& it = items[i];
         it.id = i;
         if (h.kind == RTP_HITTABLE_SPHERE) {
-            if (h.material >= d->n_materials) { fail(RTP_ERR_INVALID, "sphere material out of range"); return; }
+            if (h.material >= d->n_materials) { fail(i, RTP_ERR_INVALID, "sphere material out of range"); return; }
             for (int k = 0; k < 3; ++k) {
                 it.bmin[k] = h.center[k] - h.radius;
                 it.bmax[k] = h.center[k] + h.radius;
             }
         } else if (h.kind == RTP_HITTABLE_TRIANGLE) {
             if (h.mesh >= d->n_meshes || static_cast<uint64_t>(h.triangle) + 3 > d->meshes[h.mesh].n_indices)
-                { fail(RTP_ERR_INVALID, "triangle id out of range"); return; }
+                { fail(i, RTP_ERR_INVALID, "triangle id out of range"); return; }
             const rtp_mesh& m = d->meshes[h.mesh];
             const double* a = m.vertices[m.indices[h.triangle + 0]].position;
             const double* b = m.vertices[m.indices[h.triangle + 1]].position;
@@ -757,17 +762,17 @@ int flatten_scene(const rtp_scene_desc* d, const Switches& sw, FlatScene* out, b
                 it.bmax[k] = max_num(max_num(a[k], b[k]), c[k]);
             }
         } else {
-            { fail(RTP_ERR_INVALID, "unknown hittable kind"); return; }
+            { fail(i, RTP_ERR_INVALID, "unknown hittable kind"); return; }
         }
         if (d->root_kind == RTP_ROOT_BVH)
             for (int k = 0; k < 3; ++k) {
                 double key = 0.5 * (it.bmin[k] + it.bmax[k]);
                 if (key != key)  // partial_cmp().unwrap() panics on NaN (bvh.rs:63)
-                    { fail(RTP_ERR_INVALID, "NaN bounding-box centroid in hittable " + std::to_string(i)); return; }
+                    { fail(i, RTP_ERR_INVALID, "NaN bounding-box centroid in hittable " + std::to_string(i)); return; }
             }
       }
     });
-    if (first_bad.load()) return set_error(first_bad.load(), bad_msg);
+    if (bad_code != RTP_OK) return set_error(bad_code, bad_msg);
     }
 
     // ---- tree ---------------------------------------------------------------------------------

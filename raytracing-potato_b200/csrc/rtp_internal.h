@@ -209,6 +209,15 @@ void round_out(const double* bmin, const double* bmax, float* lo, float* hi);
 // DSceneView::cull of the union [lo, hi] of the leaf boxes that are not big; lo > hi: there are none
 void culled_set_box(const double* lo, const double* hi, float* cull);
 
+// The any-order walk's second, order-free culling tree (prepare_any_order, rtp_host.cpp): RTP_FREE_TREE, or by default every scene
+// below kFreeTreeLeaves leaves, gets one
+constexpr size_t kFreeTreeLeaves = 262144;
+inline bool want_free_tree(const Switches& sw, size_t n_leaves) { return sw.free_tree >= 0 ? sw.free_tree != 0 : n_leaves < kFreeTreeLeaves; }
+// Builds that tree over the primitives that are not big into out->free_wide / free_boxes / free_depth; out->n_big is set. Slot s has
+// the leaf box bmin[s * stride + k], bmax[s * stride + k] (k = 0..2), kind[s] and is_big[s]. Both scene builds call it.
+void build_free_tree(const double* bmin, const double* bmax, size_t stride, const std::vector<uint8_t>& kind, const std::vector<uint8_t>& is_big,
+                     FlatScene* out);
+
 // host layer
 // device_build: build a large flat Bvh scene on the GPU (rtp_build.cu device_build_scene); host-only callers pass false
 int flatten_scene(const rtp_scene_desc* desc, const Switches& sw, FlatScene* out, bool device_build = false);
@@ -220,7 +229,7 @@ int ensure_device();  // binds device 0 if rtp_init has not been called; RTP_ERR
 int device_reference_order_dev(const double* d_boxes, uint32_t n, uint32_t* d_order_out);
 // The whole of flatten_scene's geometry part on the current device for a flat (un-nested) Bvh scene: leaf boxes, the reference's
 // depth-first order, the SAH culling tree over that order, primitive / attribute records, the 4-wide collapse and the any-order
-// tables. Fills out->dev and the host-side metadata. Returns RTP_OK, a negative status, or 1 = "not applicable, use the host
+// tables; then the host's order-free tree when want_free_tree asks for it. Fills out->dev and the host-side metadata. Returns RTP_OK, a negative status, or 1 = "not applicable, use the host
 // path" (irregular boxes). sw.build_timing: phase times on stderr.
 int device_build_scene(const rtp_scene_desc* d, const Switches& sw, FlatScene* out);
 void device_free_arrays(DevArrays* a);

@@ -42,6 +42,7 @@ def test_struct_layouts_match_the_header(tmp_path):
         "rtp_emit": C.sizeof(A.Emit), "rtp_material": C.sizeof(A.Material), "rtp_texture": C.sizeof(A.Texture),
         "rtp_scene_desc": C.sizeof(A.SceneDesc), "rtp_camera": C.sizeof(A.Camera), "rtp_render_params": C.sizeof(A.RenderParams),
         "rtp_stats": C.sizeof(A.Stats), "rtp_scene_info": C.sizeof(A.SceneInfo), "rtp_image": C.sizeof(A.Image),
+        "rtp_any_tables": C.sizeof(A.AnyTables),
     }
     offsets = {
         ("rtp_material", "emit"): A.Material.emit.offset, ("rtp_texture", "rgba"): A.Texture.rgba.offset,
@@ -51,6 +52,7 @@ def test_struct_layouts_match_the_header(tmp_path):
         ("rtp_scene_desc", "nested"): A.SceneDesc.nested.offset, ("rtp_scene_desc", "n_nested"): A.SceneDesc.n_nested.offset,
         ("rtp_stats", "device_ms"): A.Stats.device_ms.offset, ("rtp_stats", "trace_ms"): A.Stats.trace_ms.offset, ("rtp_hit_full", "uv"): A.HIT_FULL_DTYPE.fields["uv"][1],
         ("rtp_hittable", "center"): A.HITTABLE_DTYPE.fields["center"][1],
+        ("rtp_any_tables", "any_E"): A.AnyTables.any_E.offset, ("rtp_any_tables", "cull"): A.AnyTables.cull.offset,
     }
     src = ['#include <stdio.h>', '#include <stddef.h>', f'#include "{HEADER}"', "int main(void){"]
     for s in structs:
