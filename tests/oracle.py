@@ -57,6 +57,9 @@ def lib():
             "orc_trace_one": (C.c_int, [C.c_void_p, P(A.Camera), P(A.RenderParams), C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p, P(C.c_int), P(C.c_uint32)]),
             "orc_texture_sample": (C.c_int, [C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p]),
             "orc_noise_integer": (C.c_int64, [C.c_int64, C.c_int64, C.c_int64, C.c_int64]),
+            "orc_scene_set_libm": (C.c_int, [C.c_void_p, C.c_int]),
+            "orc_device_atan2_n": (None, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+            "orc_device_asin_n": (None, [C.c_void_p, C.c_size_t, C.c_void_p]),
         }
         for name, (res, args) in sigs.items():
             fn = getattr(L, name)
@@ -148,6 +151,22 @@ def aabb_collide(bmin, bmax, ray) -> bool:
     return bool(lib().orc_aabb_collide(A.ptr(bmin), A.ptr(bmax), A.ptr(r)))
 
 
+def device_atan2(y, x) -> np.ndarray:
+    """CUDA's double atan2 (the oracle's transcription of libdevice), elementwise over broadcast arrays."""
+    y, x = (np.array(a, dtype=np.float64) for a in np.broadcast_arrays(y, x))
+    out = np.empty(y.shape, dtype=np.float64)
+    lib().orc_device_atan2_n(A.ptr(y), A.ptr(x), y.size, A.ptr(out))
+    return out
+
+
+def device_asin(x) -> np.ndarray:
+    """CUDA's double asin (the oracle's transcription of libdevice), elementwise."""
+    x = np.array(x, dtype=np.float64)
+    out = np.empty(x.shape, dtype=np.float64)
+    lib().orc_device_asin_n(A.ptr(x), x.size, A.ptr(out))
+    return out
+
+
 def camera_rays(camera: api.Camera, width, height) -> np.ndarray:
     out = np.empty(width * height, dtype=A.RAY_DTYPE)
     cc = camera.to_c()
@@ -156,14 +175,18 @@ def camera_rays(camera: api.Camera, width, height) -> np.ndarray:
 
 
 class Scene:
-    """Oracle twin of rtp_b200.api.Scene."""
+    """Oracle twin of rtp_b200.api.Scene.
 
-    def __init__(self, scene: api.ExampleScene):
+    libm picks the atan2 / asin of sphere and sky uv: "host" is the C library's (the reference's), "device" is CUDA's,
+    with which the device's images are equal to the oracle's bit for bit."""
+
+    def __init__(self, scene: api.ExampleScene, libm="host"):
         desc, keep = api.build_desc(scene)
         h = C.c_void_p()
         _check(lib().orc_scene_create(C.byref(desc), C.byref(h)))
         self._h = h
         self.camera = scene.camera
+        _check(lib().orc_scene_set_libm(h, {"host": 0, "device": 1}[libm]))
 
     def close(self):
         if self._h:

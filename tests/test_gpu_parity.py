@@ -1,7 +1,9 @@
 """GPU parity proper: the CUDA path, called through the C ABI, against the CPU oracle on the same inputs.
 
 Bar (BASELINE.json north_star): closest-hit ids bit-exact; triangle t within 4 ULP (we assert 0 ULP, since the
-kernels keep the reference's operation order unfused); images per pixel within the stated tolerance.
+kernels keep the reference's operation order unfused). Images, foregrounds and ray counts equal the oracle's bit for bit when the
+oracle's uv uses CUDA's atan2 / asin (oracle.Scene(sc, libm="device")); tests/test_device_libm.py measures on the CPU what the
+host libm moves instead (texture lookups only).
 """
 import math
 
@@ -37,7 +39,7 @@ def assert_hits_equal(g, o, what=""):
 @pytest.fixture(scope="module")
 def bunny_pair(gpu):
     sc = scenes.bunny_lambert()
-    return sc, api.Scene(sc), oracle.Scene(sc)
+    return sc, api.Scene(sc), oracle.Scene(sc, libm="device")
 
 
 def primary(sc, w, h):
@@ -99,10 +101,8 @@ def test_full_hit_record(bunny_pair):
     for f in ("t", "position", "normal", "uv"):
         assert hg[f][tri].tobytes() == ho[f][tri].tobytes(), f
     sph = ho["leaf"] == 4968
-    for f in ("t", "position", "normal"):
+    for f in ("t", "position", "normal", "uv"):  # sphere uv: the oracle runs CUDA's atan2 / asin
         assert hg[f][sph].tobytes() == ho[f][sph].tobytes(), f
-    # sphere uv goes through atan2/asin: CUDA and glibc may differ by an ulp or two
-    assert np.allclose(hg["uv"][sph], ho["uv"][sph], rtol=0, atol=1e-14)
 
 
 def test_counters_match_oracle(bunny_pair, monkeypatch):
@@ -232,41 +232,48 @@ def image_report(a, b):
     return dict(max=float(d.max()), rmse=float(np.sqrt((d * d).mean())), differing=int((a != b).any(axis=-1).sum()), pixels=a.shape[0] * a.shape[1])
 
 
-# Tolerance for image parity. The integrator reproduces the oracle's arithmetic order, RNG stream and sample
-# summation order, so pixels are expected bit-identical; the only operations not bit-pinned are atan2/asin
-# (CUDA libm vs glibc, <= 2 ulp), which can move a texture lookup across a texel boundary. We therefore require
-# RMSE <= 1e-6 and at most 0.1% of pixels differing at all.
-IMG_RMSE = 1e-6
-IMG_FRAC = 1e-3
+def assert_images_equal(got, want, what=""):
+    """bit-for-bit equality of two frames (or any f64 arrays), NaN-aware: a NaN must be NaN on both sides (its payload is the
+    hardware's), every other value must have the same bits. The integrator reproduces the oracle's arithmetic order, RNG stream and
+    sample summation order, and the oracle's uv runs CUDA's atan2 / asin, so nothing is left to a tolerance."""
+    got, want = np.ascontiguousarray(got, dtype=np.float64), np.ascontiguousarray(want, dtype=np.float64)
+    assert got.shape == want.shape, (what, got.shape, want.shape)
+    gn, wn = np.isnan(got), np.isnan(want)
+    same = np.where(gn | wn, gn & wn, got.view(np.uint64) == want.view(np.uint64))
+    if not same.all():
+        bad = np.argwhere(~same)
+        raise AssertionError(f"{what}: {len(bad)} values differ, first at {tuple(bad[0])}: {got[tuple(bad[0])]!r} vs {want[tuple(bad[0])]!r}; "
+                             f"{image_report(np.nan_to_num(got), np.nan_to_num(want)) if got.ndim == 3 else ''}")
 
 
-@pytest.mark.parametrize("name,w,h,spp", [
+RENDER_CASES = [  # (example scene, width, height, spp) of test_render_matches_oracle, max_bounce 8, seed 1
     ("bunny_lambert", 320, 180, 4), ("bunny", 160, 90, 2), ("glass_bunny", 160, 90, 4), ("demo", 192, 108, 4),
     ("three_balls", 128, 128, 8), ("two_balls", 128, 128, 4), ("earth", 128, 128, 4), ("one_triangle", 128, 128, 2),
     ("more_balls_optimized", 160, 160, 2), ("more_balls", 48, 48, 1),
-])
+]
+
+
+@pytest.mark.parametrize("name,w,h,spp", RENDER_CASES)
 def test_render_matches_oracle(gpu, name, w, h, spp):
     sc = getattr(scenes, name)()
-    g, o = api.Scene(sc), oracle.Scene(sc)
+    g, o = api.Scene(sc), oracle.Scene(sc, libm="device")
     ig, fg, sg = g.render(w, h, spp, max_bounce=8, seed=1)
     io, fo, so = o.render(w, h, spp, max_bounce=8, seed=1)
-    rep = image_report(ig, io)
-    assert rep["rmse"] <= IMG_RMSE and rep["differing"] <= max(1, IMG_FRAC * rep["pixels"]), rep
+    assert_images_equal(ig, io, name)
     assert (fg == fo).all()
     assert sg.paths == so.paths == w * h * spp
-    assert abs(int(sg.rays) - int(so.rays)) <= 8 * max(1, rep["differing"]) * spp, (sg.rays, so.rays)
+    assert sg.rays == so.rays, (sg.rays, so.rays)
     g.close(); o.close()
 
 
 def test_c1_config_reduced_spp(gpu):
     """BASELINE config C1 geometry and resolution (640x360, depth 8) at 2 spp so the oracle finishes in seconds"""
     sc = scenes.bunny_lambert()
-    g, o = api.Scene(sc), oracle.Scene(sc)
+    g, o = api.Scene(sc), oracle.Scene(sc, libm="device")
     ig, fg, sg = g.render(640, 360, 2, seed=1)
     io, fo, so = o.render(640, 360, 2, seed=1)
-    rep = image_report(ig, io)
-    assert rep["rmse"] <= IMG_RMSE and rep["differing"] <= IMG_FRAC * rep["pixels"], rep
-    assert sg.rays == so.rays or rep["differing"] > 0
+    assert_images_equal(ig, io, "C1")
+    assert (fg == fo).all() and sg.rays == so.rays, (sg.rays, so.rays)
 
 
 @pytest.mark.parametrize("name,depth", [("demo", 8), ("glass_bunny", 1), ("glass_bunny", 2), ("glass_bunny", 12), ("bunny_lambert", 40), ("three_balls", 3)])
@@ -375,7 +382,7 @@ def test_c4_full_resolution_frame_properties(gpu):
     tiles stitched through the tail-mode path equal the whole-frame wavefront render bit for bit; a sample-range split
     reproduces the frame up to f64 re-association; and the oracle agrees on a 96x54 crop rendered as its own tile."""
     sc = scenes.demo()
-    g, o = api.Scene(sc), oracle.Scene(sc)
+    g, o = api.Scene(sc), oracle.Scene(sc, libm="device")
     w, h = 1920, 1080
     full, ffg, st = g.render(w, h, 2, seed=5)
     assert st.paths == w * h * 2 and st.rays >= st.paths
@@ -388,10 +395,10 @@ def test_c4_full_resolution_frame_properties(gpu):
     assert np.allclose((a + b) / 2, full, rtol=1e-14, atol=1e-15)
     tile = (900, 500, 96, 54)
     ref = np.zeros_like(full)
-    o_img, _, _ = o.render(w, h, 2, seed=5, tile=tile)
+    o_img, o_fg, _ = o.render(w, h, 2, seed=5, tile=tile)
     crop = (slice(tile[1], tile[1] + tile[3]), slice(tile[0], tile[0] + tile[2]))
-    rep = image_report(full[crop], o_img[crop])
-    assert rep["rmse"] <= IMG_RMSE and rep["differing"] <= max(1, IMG_FRAC * rep["pixels"]), rep
+    assert_images_equal(full[crop], o_img[crop], "C4 crop")
+    assert (ffg[crop] == o_fg[crop]).all()
     g.close(); o.close()
 
 
@@ -399,7 +406,7 @@ def test_c5_reduced_bunny_field_matches_oracle(gpu):
     """BASELINE config C5 scene generator at 8x4 copies (158,977 leaves): closest hits and a small render vs the oracle. The full
     64x32 field (10.2 M triangles, 5 GiB) is exercised by tools/c5_run.py, which checks the f32-culled walk against the exact walk."""
     sc = scenes.bunny_field(8, 4)
-    g, o = api.Scene(sc), oracle.Scene(sc)
+    g, o = api.Scene(sc), oracle.Scene(sc, libm="device")
     assert g.info().n_leaves == o.info().n_leaves == 8 * 4 * 4968 + 1
     assert (g.leaf_order() == o.leaf_order()).all()
     cam = api.Camera(16 / 9, sc.camera.fov, sc.camera.focal_dist, 0.0, sc.camera.transformation)
@@ -411,8 +418,8 @@ def test_c5_reduced_bunny_field_matches_oracle(gpu):
     assert_hits_equal_bits(g.hit(both), o.hit(both))
     ig, fg, sg = g.render(160, 90, 2, seed=2)
     io, fo, so = o.render(160, 90, 2, seed=2)
-    rep = image_report(ig, io)
-    assert rep["rmse"] <= IMG_RMSE and rep["differing"] <= max(1, IMG_FRAC * rep["pixels"]), rep
+    assert_images_equal(ig, io, "C5")
+    assert (fg == fo).all() and sg.rays == so.rays, (sg.rays, so.rays)
     g.close(); o.close()
 
 
@@ -424,14 +431,14 @@ def test_nan_uv_samples_texel_row_zero_like_rust(gpu):
 
     sc = scenes.bunny_lambert()
     sc.camera = Camera(1.0, sc.camera.fov, 1.0, 0.0, Transformation.lookat([0.0, 0.3, 2.0], [0.0, 2.5, 0.0], [0.0, 3.0, 0.0]))
-    g, o = api.Scene(sc), oracle.Scene(sc)
+    g, o = api.Scene(sc), oracle.Scene(sc, libm="device")
     cam = api.Camera(1.0, sc.camera.fov, 1.0, 0.0, sc.camera.transformation)
     rays = oracle.camera_rays(cam, 64, 64)
     assert (np.abs(rays["direction"][:, 1]) > 1.0).any()  # the premise: asin gets arguments outside [-1, 1]
-    ig, fg, _ = g.render(64, 64, 2, seed=4)
-    io, fo, _ = o.render(64, 64, 2, seed=4)
-    rep = image_report(ig, io)
-    assert rep["rmse"] <= IMG_RMSE and rep["differing"] <= max(1, IMG_FRAC * rep["pixels"]), rep
+    ig, fg, sg = g.render(64, 64, 2, seed=4)
+    io, fo, so = o.render(64, 64, 2, seed=4)
+    assert_images_equal(ig, io, "NaN uv")
+    assert (fg == fo).all() and sg.rays == so.rays, (sg.rays, so.rays)
     g.close(); o.close()
 
 
@@ -441,16 +448,15 @@ def test_output_stage_on_device(gpu, name):
     against this library's own f64 frame and against the oracle's (where the oracle's frame is bit-identical); the transparent
     background variant writes alpha = (255 * foreground) as u8; tiles stitch."""
     sc = getattr(scenes, name)()
-    g, o = api.Scene(sc), oracle.Scene(sc)
+    g, o = api.Scene(sc), oracle.Scene(sc, libm="device")
     w, h, spp = 240, 135, 3
     frame, fg, _ = g.render(w, h, spp, seed=6)
     rgba, st = g.render_srgb8(w, h, spp, seed=6)
     assert rgba.tobytes() == api.to_srgb_u8(frame).tobytes()
     assert st.paths == w * h * spp
     io, fo, _ = o.render(w, h, spp, seed=6)
-    same = (io == frame).all(axis=-1)
-    assert same.mean() > 0.999
-    assert (rgba[same] == oracle.to_srgb_u8(io)[same]).all()
+    assert_images_equal(frame, io, name)
+    assert rgba.tobytes() == oracle.to_srgb_u8(io).tobytes()
     ta, _ = g.render_srgb8(w, h, spp, seed=6, transparent_background=True)
     assert (ta[..., :3] == rgba[..., :3]).all()
     assert (ta[..., 3] == np.minimum(255.0 * fg, 255.0).astype(np.uint8)).all()
@@ -511,12 +517,11 @@ def test_thin_lens_camera(gpu):
     sc = scenes.demo()
     c = sc.camera
     sc.camera = Camera(c.aspect_ratio, c.fov, 3.2, 0.08, c.transformation)
-    g, o = api.Scene(sc), oracle.Scene(sc)
+    g, o = api.Scene(sc), oracle.Scene(sc, libm="device")
     ig, fg, sg = g.render(192, 108, 4, seed=8)
     io, fo, so = o.render(192, 108, 4, seed=8)
-    rep = image_report(ig, io)
-    assert rep["rmse"] <= IMG_RMSE and rep["differing"] <= max(1, IMG_FRAC * rep["pixels"]), rep
-    assert (fg == fo).all() and sg.paths == so.paths
+    assert_images_equal(ig, io, "thin lens")
+    assert (fg == fo).all() and sg.paths == so.paths and sg.rays == so.rays
     sharp, _, _ = g.render(192, 108, 4, seed=8, camera=Camera(c.aspect_ratio, c.fov, 3.2, 0.0, c.transformation))
     assert not np.array_equal(sharp, ig)  # the lens does something
     g.close(); o.close()
@@ -585,14 +590,13 @@ def test_degenerate_scene_sizes(gpu, kind):
     else:
         sc.root_kind, sc.hittables = "list", api.Hittable.Sphere([0.0, 0.0, 0.0], 0.7, 1)
     sc.hittables = np.atleast_1d(sc.hittables)
-    g, o = api.Scene(sc), oracle.Scene(sc)
+    g, o = api.Scene(sc), oracle.Scene(sc, libm="device")
     cam = api.Camera(1.0, sc.camera.fov, sc.camera.focal_dist, 0.0, sc.camera.transformation)
     rays = oracle.camera_rays(cam, 64, 64)
     assert_hits_equal_bits(g.hit(rays), o.hit(rays))
     ig, fg, sg = g.render(48, 48, 3, seed=2)
     io, fo, so = o.render(48, 48, 3, seed=2)
-    rep = image_report(ig, io)
-    assert rep["rmse"] <= IMG_RMSE and rep["differing"] <= max(1, IMG_FRAC * rep["pixels"]), rep
+    assert_images_equal(ig, io, kind)
     assert (fg == fo).all() and sg.rays == so.rays
     g.close(); o.close()
 
@@ -656,12 +660,12 @@ def test_exact_ties_and_degenerate_primitives(gpu):
     gi.close(); oi.close()
 
 
-def test_material_and_texture_zoo(gpu):
-    """every Scatter / Absorb / Emit / Texture variant at unusual parameters in one scene, rendered against the oracle: metal with
-    fuzz 5 (most reflections end below the surface and are absorbed, material.rs:141-150), dielectrics of index 0.5, 1.0 and 2.4
-    (total internal reflection both ways, utility.rs:110-119), WhiteBody / BlackBody, emissive DebugNormals / Color / SkySphere
-    used as a SURFACE emit, Missing / DebugUVs / Solid / Image / Noise / Perlin textures and a checker of checkers; a triangle
-    mesh with per-vertex uvs carries an AlbedoMap."""
+def material_zoo_scene():
+    """every Scatter / Absorb / Emit / Texture variant at unusual parameters in one scene: metal with fuzz 5 (most reflections end
+    below the surface and are absorbed, material.rs:141-150), dielectrics of index 0.5, 1.0 and 2.4 (total internal reflection both
+    ways, utility.rs:110-119), WhiteBody / BlackBody, emissive DebugNormals / Color / SkySphere used as a SURFACE emit, Missing /
+    DebugUVs / Solid / Image / Noise / Perlin textures and a checker of checkers; a triangle mesh with per-vertex uvs carries an
+    AlbedoMap."""
     from rtp_b200.api import Absorb, Camera, Emit, Hittable, Material, Mesh, SceneData, Scatter, Texture, Transformation, ExampleScene
 
     textures = [Texture.Image(assets.earthmap()), Texture.Missing, Texture.DebugUVs, Texture.Solid(rgb(0.9, 0.2, 0.1)), Texture.Noise(7), Texture.Perlin(-3),
@@ -688,14 +692,17 @@ def test_material_and_texture_zoo(gpu):
         parts.append(Hittable.Sphere([2.2 * math.cos(ang), 0.5, 2.2 * math.sin(ang)], 0.5, k if k < 5 else k + 1))
     parts.append(Hittable.Sphere([0.0, 0.8, 0.0], 0.8, 3))
     cam = Camera(1.0, 1.0, 1.0, 0.0, Transformation.lookat([0.0, 4.0, 6.0], [0.0, 0.3, 0.0], [0.0, 1.0, 0.0]))
-    sc = ExampleScene(cam, SceneData(materials, textures, [quad]), "bvh", Hittable.concat(parts), Emit.SkyGradient)
-    g, o = api.Scene(sc), oracle.Scene(sc)
+    return ExampleScene(cam, SceneData(materials, textures, [quad]), "bvh", Hittable.concat(parts), Emit.SkyGradient)
+
+
+def test_material_and_texture_zoo(gpu):
+    """material_zoo_scene rendered against the oracle"""
+    sc = material_zoo_scene()
+    g, o = api.Scene(sc), oracle.Scene(sc, libm="device")
     ig, fg, sg = g.render(200, 200, 6, max_bounce=12, seed=21)
     io, fo, so = o.render(200, 200, 6, max_bounce=12, seed=21)
-    rep = image_report(ig, io)
-    # the DebugUVs texture turns the sphere uv — atan2 / asin, the two operations CUDA and glibc do not share bit for bit — into a
-    # COLOUR, so here the ulp shows up in pixel values instead of (rarely) moving a texel: bound the size, not the count
-    assert rep["rmse"] <= 1e-12 and rep["max"] <= 1e-12, rep
+    # the DebugUVs texture turns the sphere uv (atan2 / asin) into a COLOUR: every last bit of the uv shows in the frame
+    assert_images_equal(ig, io, "zoo")
     assert (fg == fo).all() and sg.rays == so.rays
     assert sg.rays / sg.paths > 1.5  # the zoo really bounces
     g.close(); o.close()
@@ -819,7 +826,7 @@ def test_any_order_walk_axis_aligned_geometry_and_exact_ties(gpu, monkeypatch, f
     rays["origin"][k:2 * k] = [0.25, 0.5, 4.0]
     vert = np.stack([rng.integers(-4, 5, k), rng.integers(-4, 5, k), np.zeros(k)], axis=1).astype(np.float64)
     rays["direction"][k:2 * k] = vert - rays["origin"][k:2 * k]
-    o = oracle.Scene(sc)
+    o = oracle.Scene(sc, libm="device")
     want = o.hit(rays)
     import torch
 
@@ -837,8 +844,8 @@ def test_any_order_walk_axis_aligned_geometry_and_exact_ties(gpu, monkeypatch, f
     # the same through the integrator (wavefront and tail-mode launches walk with the same lanes)
     ig, fg, sg = g.render(96, 64, 2, seed=4)
     io, fo, so = o.render(96, 64, 2, seed=4)
-    rep = image_report(ig, io)
-    assert rep["rmse"] <= IMG_RMSE and rep["differing"] <= max(1, IMG_FRAC * rep["pixels"]), rep
+    assert_images_equal(ig, io, "axis-aligned")
+    assert (fg == fo).all() and sg.rays == so.rays, (sg.rays, so.rays)
     g.close(); o.close()
 
 
@@ -846,12 +853,11 @@ def test_any_order_walk_axis_aligned_geometry_and_exact_ties(gpu, monkeypatch, f
 def test_any_order_walk_renders_match_oracle(gpu, monkeypatch, name, w, h, spp):
     monkeypatch.setenv("RTP_TRAVERSAL", "any")
     sc = getattr(scenes, name)()
-    g, o = api.Scene(sc), oracle.Scene(sc)
+    g, o = api.Scene(sc), oracle.Scene(sc, libm="device")
     ig, fg, sg = g.render(w, h, spp, seed=3)
     io, fo, so = o.render(w, h, spp, seed=3)
-    rep = image_report(ig, io)
-    assert rep["rmse"] <= IMG_RMSE and rep["differing"] <= max(1, IMG_FRAC * rep["pixels"]), rep
-    assert sg.rays == so.rays or rep["differing"] > 0
+    assert_images_equal(ig, io, name)
+    assert (fg == fo).all() and sg.rays == so.rays, (sg.rays, so.rays)
     ig2, _, _ = g.render(w, h, spp, seed=3, tile=(32, 16, 32, 32))  # a 32x32 tile runs as one tail-mode launch
     assert np.array_equal(ig2[16:48, 32:64], ig[16:48, 32:64])
     g.close(); o.close()
@@ -866,7 +872,7 @@ def test_any_order_stack_overflow_hands_the_ray_to_the_in_order_walk(gpu, monkey
     monkeypatch.setenv("RTP_TRAVERSAL", "any")
     sc = scenes.bunny_lambert()
     rays = _mixed_rays(sc)
-    o = oracle.Scene(sc)
+    o = oracle.Scene(sc, libm="device")
     want = o.hit(rays)
     d_rays = torch.from_numpy(rays.view(np.float64).reshape(-1, 8)).cuda()
     d_hits = torch.empty((len(rays), 2), dtype=torch.float64, device="cuda")
@@ -883,8 +889,8 @@ def test_any_order_stack_overflow_hands_the_ray_to_the_in_order_walk(gpu, monkey
             assert st.order_rewalks <= len(rays) // 1000, st.order_rewalks
         ig, fg, sg = g.render(64, 48, 2, seed=8)
         io, fo, so = o.render(64, 48, 2, seed=8)
-        rep = image_report(ig, io)
-        assert rep["rmse"] <= IMG_RMSE and rep["differing"] <= max(1, IMG_FRAC * rep["pixels"]), rep
+        assert_images_equal(ig, io, f"cap {cap}")
+        assert (fg == fo).all() and sg.rays == so.rays, (cap, sg.rays, so.rays)
         g.close()
     o.close()
 
@@ -983,7 +989,7 @@ def test_any_order_walk_on_sphere_scenes(gpu, monkeypatch, name):
     rays["origin"], rays["direction"] = o, d / np.linalg.norm(d, axis=1, keepdims=True)
     rays["t_min"], rays["t_max"] = 1e-3, np.inf
     rays = np.concatenate([oracle.camera_rays(cam, 160, 160), rays])
-    orc = oracle.Scene(sc)
+    orc = oracle.Scene(sc, libm="device")
     want = orc.hit(rays)
     d_rays = torch.from_numpy(rays.view(np.float64).reshape(-1, 8)).cuda()
     d_hits = torch.empty((len(rays), 2), dtype=torch.float64, device="cuda")
@@ -1000,8 +1006,8 @@ def test_any_order_walk_on_sphere_scenes(gpu, monkeypatch, name):
         if order == "any":
             ig, fg, sg = g.render(96, 96, 2, seed=6)
             io, fo, so = orc.render(96, 96, 2, seed=6)
-            rep = image_report(ig, io)
-            assert rep["rmse"] <= IMG_RMSE and rep["differing"] <= max(1, IMG_FRAC * rep["pixels"]), rep
+            assert_images_equal(ig, io, name)
+            assert (fg == fo).all() and sg.rays == so.rays, (sg.rays, so.rays)
         g.close()
     if name in ("more_balls_optimized", "sphere_soup"):
         assert visits["any"] < visits["inorder"], visits
@@ -1019,7 +1025,7 @@ def test_c5_full_field_sampled_rays_equal_oracle(gpu):
     g = api.Scene(sc)
     info = g.info()
     assert info.n_leaves == 10_174_465 and info.n_nodes == 2 * 10_174_465 - 1 and info.any_order != 0
-    o = oracle.Scene(sc)
+    o = oracle.Scene(sc, libm="device")
     assert o.info().depth == info.depth
     W, H = 3840, 2160
     cam = api.Camera(W / H, sc.camera.fov, sc.camera.focal_dist, 0.0, sc.camera.transformation)
@@ -1050,7 +1056,8 @@ def test_c5_full_field_sampled_rays_equal_oracle(gpu):
     ig, fg, _ = g.render(W, H, 2, max_bounce=8, seed=1, tile=tile)
     io, fo, _ = o.render(W, H, 2, max_bounce=8, seed=1, tile=tile)
     sl = (slice(tile[1], tile[1] + tile[3]), slice(tile[0], tile[0] + tile[2]))
-    assert np.sqrt(((ig[sl] - io[sl]) ** 2).mean()) <= IMG_RMSE and (fg[sl] == fo[sl]).all()
+    assert_images_equal(ig[sl], io[sl], "C5 tile")
+    assert (fg[sl] == fo[sl]).all()
     g.close(); o.close()
 
 

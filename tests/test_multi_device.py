@@ -9,6 +9,7 @@ import pytest
 import oracle
 from rtp_b200 import _abi as A
 from rtp_b200 import api, scenes
+from test_gpu_parity import assert_images_equal
 
 pytestmark = pytest.mark.gpu
 
@@ -52,10 +53,11 @@ def test_row_split_covers_the_frame_bit_for_bit(gpu):
 def test_row_split_equals_oracle(gpu):
     sc = scenes.bunny_lambert()
     with api.Scene(sc) as g:
-        o = oracle.Scene(sc)
-        ig, fg, _ = g.render(64, 36, 2, max_bounce=8, seed=2, rows=(1, 3))
-        io, fo, _ = o.render(64, 36, 2, max_bounce=8, seed=2, rows=(1, 3))
-        assert np.sqrt(((ig - io) ** 2).mean()) <= 1e-6 and (fg == fo).all()
+        o = oracle.Scene(sc, libm="device")
+        ig, fg, sg = g.render(64, 36, 2, max_bounce=8, seed=2, rows=(1, 3))
+        io, fo, so = o.render(64, 36, 2, max_bounce=8, seed=2, rows=(1, 3))
+        assert_images_equal(ig, io, "rows (1, 3)")
+        assert (fg == fo).all() and sg.rays == so.rays, (sg.rays, so.rays)
         assert (ig[0::3] == 0).all() and (ig[2::3] == 0).all()  # other rows untouched
         o.close()
 
@@ -97,7 +99,8 @@ def test_one_call_two_devices(gpu, monkeypatch):
         r1, _ = one.render_srgb8(w, h, spp, seed=7)
         r2, _ = two.render_srgb8(w, h, spp, seed=7)
         assert r1.tobytes() == r2.tobytes()
-        o = oracle.Scene(sc)
-        io, fo, _ = o.render(w, h, spp, max_bounce=8, seed=7)
-        assert np.sqrt(((i2 - io) ** 2).mean()) <= 1e-6
+        o = oracle.Scene(sc, libm="device")
+        io, fo, so = o.render(w, h, spp, max_bounce=8, seed=7)
+        assert_images_equal(i2, io, "two devices")
+        assert (f2 == fo).all() and s2.rays == so.rays, (s2.rays, so.rays)
         o.close()

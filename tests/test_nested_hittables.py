@@ -13,6 +13,7 @@ import oracle
 from rtp_b200 import _abi as A
 from rtp_b200 import api
 from test_bvh_restatement import MISS, Box, LiteralBvh, div, soup_rays, soup_scene
+from test_gpu_parity import assert_images_equal
 
 
 class Node:
@@ -247,7 +248,7 @@ def test_nesting_errors_are_the_reference_panics():
 def test_gpu_nested_scene_equals_oracle_and_literal(seed, root_kind, monkeypatch):
     sc, tree = nested_scene(seed, root_kind)
     lit = LiteralNested(sc, root_kind, tree)
-    o = oracle.Scene(sc)
+    o = oracle.Scene(sc, libm="device")
     rays = soup_rays(seed + 20, 6000)
     want = o.hit_full(rays)
     for env in ({}, {"RTP_TRAVERSAL": "inorder"}, {"RTP_TRACE_KERNEL": "simple"}, {"RTP_F32_CULLING": "0"}):
@@ -258,13 +259,15 @@ def test_gpu_nested_scene_equals_oracle_and_literal(seed, root_kind, monkeypatch
             assert (got["leaf"] == want["leaf"]).all() and (got["material"] == want["material"]).all(), env
             assert got["t"].tobytes() == want["t"].tobytes(), env
             assert got["position"].tobytes() == want["position"].tobytes() and got["normal"].tobytes() == want["normal"].tobytes(), env
+            assert got["uv"].tobytes() == want["uv"].tobytes(), env
             if not env:
                 check_against_literal(got[:400], lit, rays[:400])
         for k in env:
             monkeypatch.delenv(k)
     # and through the integrator
     with api.Scene(sc) as g:
-        ig, fg, _ = g.render(48, 32, 2, max_bounce=4, seed=3)
-        io, fo, _ = o.render(48, 32, 2, max_bounce=4, seed=3)
-        assert np.sqrt(((ig - io) ** 2).mean()) <= 1e-6 and (fg == fo).all()
+        ig, fg, sg = g.render(48, 32, 2, max_bounce=4, seed=3)
+        io, fo, so = o.render(48, 32, 2, max_bounce=4, seed=3)
+        assert_images_equal(ig, io, f"nested {seed} {root_kind}")
+        assert (fg == fo).all() and sg.rays == so.rays, (sg.rays, so.rays)
     o.close()

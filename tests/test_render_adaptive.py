@@ -2,9 +2,8 @@
 
 The reference for the stop decisions is `stop_counts` below, a numpy model of the stop rule that works on per-sample colours in the
 rule's own operation order. On the CPU it is checked on oracle colours; on the GPU the library's decisions must equal the model
-applied to the GPU's own per-sample colours (rtp_render of one-sample ranges with RTP_RENDER_RAW_SUMS: the GPU's atan2 / asin may
-differ from the host libm by an ulp, so the oracle's colours are not the input for that check). The pixels themselves are checked
-bit for bit against rtp_render at each pixel's own sample count.
+applied to the GPU's own per-sample colours (rtp_render of one-sample ranges with RTP_RENDER_RAW_SUMS). The pixels themselves are
+checked bit for bit against rtp_render at each pixel's own sample count, and against the oracle run with CUDA's atan2 / asin.
 """
 import ctypes as C
 import os
@@ -16,7 +15,7 @@ import pytest
 import oracle
 from rtp_b200 import _abi as A
 from rtp_b200 import api, scenes
-from test_gpu_parity import IMG_FRAC, IMG_RMSE, image_report
+from test_gpu_parity import assert_images_equal
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 HEADER = os.path.join(ROOT, "include", "rtp.h")
@@ -332,12 +331,11 @@ def test_invalid_arguments(cases, case, entry):
 def test_groups_match_the_oracle(cases):
     c = cases("demo")
     img, fg, n, _ = c.render()
-    o = oracle.Scene(c.sc)
+    o = oracle.Scene(c.sc, libm="device")
     for k in np.unique(n):
         io, fo, _ = o.render(W, H, int(k), max_bounce=DEPTH, seed=SEED, sample_range=(0, int(k)))
         sel = n == k
-        rep = image_report(img[sel][None], io[sel][None])
-        assert rep["rmse"] <= IMG_RMSE and rep["differing"] <= max(1, IMG_FRAC * rep["pixels"]), (k, rep)
+        assert_images_equal(img[sel], io[sel], f"{k} samples")
         assert (fg[sel] == fo[sel]).all()
     o.close()
 
