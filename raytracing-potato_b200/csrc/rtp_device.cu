@@ -1829,14 +1829,19 @@ __global__ void __launch_bounds__(256) resolve_kernel(const double4* __restrict_
     acc[pix] = a;
 }
 
+// the frame pixel of tile pixel `pix` of a launch (row-major over the launch's rows, rp.tile_w wide): the output kernels' mapping
+__device__ __forceinline__ size_t frame_pixel(const DRender& rp, size_t pix) {
+    const uint32_t i = rp.tile_x + static_cast<uint32_t>(pix % rp.tile_w);
+    const uint32_t j = rp.tile_y + rp.row_offset + static_cast<uint32_t>(pix / rp.tile_w) * rp.row_stride;
+    return static_cast<size_t>(i) + static_cast<size_t>(j) * rp.width;
+}
+
 __global__ void __launch_bounds__(256) write_frame_kernel(const double4* __restrict__ acc, DRender rp, double divisor, double* __restrict__ rgb,
                                                            double* __restrict__ fg) {
     const size_t npix = static_cast<size_t>(rp.tile_w) * rp.tile_h;
     const size_t pix = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
     if (pix >= npix) return;
-    const uint32_t i = rp.tile_x + static_cast<uint32_t>(pix % rp.tile_w);
-    const uint32_t j = rp.tile_y + rp.row_offset + static_cast<uint32_t>(pix / rp.tile_w) * rp.row_stride;
-    const size_t px = static_cast<size_t>(i) + static_cast<size_t>(j) * rp.width;
+    const size_t px = frame_pixel(rp, pix);
     double4 a = acc[pix];
     if (divisor != 0.0) { a.x = a.x / divisor; a.y = a.y / divisor; a.z = a.z / divisor; a.w = a.w / divisor; }
     rgb[3 * px + 0] = a.x; rgb[3 * px + 1] = a.y; rgb[3 * px + 2] = a.z;
@@ -1865,9 +1870,7 @@ __global__ void __launch_bounds__(256) aov_write_kernel(const double2* __restric
     const size_t npix = static_cast<size_t>(rp.tile_w) * rp.tile_h;
     const size_t pix = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
     if (pix >= npix) return;
-    const uint32_t i = rp.tile_x + static_cast<uint32_t>(pix % rp.tile_w);
-    const uint32_t j = rp.tile_y + rp.row_offset + static_cast<uint32_t>(pix / rp.tile_w) * rp.row_stride;
-    const size_t px = static_cast<size_t>(i) + static_cast<size_t>(j) * rp.width;
+    const size_t px = frame_pixel(rp, pix);
     const double2 a0 = acc[3 * pix], a1 = acc[3 * pix + 1], a2 = acc[3 * pix + 2];
     double v[6] = {a0.x, a0.y, a1.x, a1.y, a2.x, a2.y};
     if (divisor != 0.0)
@@ -1933,9 +1936,7 @@ __global__ void __launch_bounds__(256) adaptive_write_kernel(const double4* __re
     const size_t npix = static_cast<size_t>(rp.tile_w) * rp.tile_h;
     const size_t pix = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
     if (pix >= npix) return;
-    const uint32_t i = rp.tile_x + static_cast<uint32_t>(pix % rp.tile_w);
-    const uint32_t j = rp.tile_y + rp.row_offset + static_cast<uint32_t>(pix / rp.tile_w) * rp.row_stride;
-    const size_t px = static_cast<size_t>(i) + static_cast<size_t>(j) * rp.width;
+    const size_t px = frame_pixel(rp, pix);
     double4 a = acc[pix];
     const uint32_t n = count[pix];
     if (!raw_sums) {
@@ -1964,9 +1965,7 @@ __global__ void __launch_bounds__(256) srgb8_kernel(const double4* __restrict__ 
     const size_t npix = static_cast<size_t>(rp.tile_w) * rp.tile_h;
     const size_t pix = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
     if (pix >= npix) return;
-    const uint32_t i = rp.tile_x + static_cast<uint32_t>(pix % rp.tile_w);
-    const uint32_t j = rp.tile_y + rp.row_offset + static_cast<uint32_t>(pix / rp.tile_w) * rp.row_stride;
-    const size_t px = static_cast<size_t>(i) + static_cast<size_t>(j) * rp.width;
+    const size_t px = frame_pixel(rp, pix);
     double4 a = acc[pix];
     if (divisor != 0.0) { a.x = a.x / divisor; a.y = a.y / divisor; a.z = a.z / divisor; a.w = a.w / divisor; }
     const double c[3] = {a.x, a.y, a.z};
@@ -1996,6 +1995,27 @@ constexpr int kPipeDepth = 3;
 constexpr size_t kAnyOrderBigScene = 262144;  // leaves from which rtp_scene_info.any_order reports 2 (the kernel is the same)
 constexpr unsigned kQueueSlots = 64;
 constexpr unsigned kLaunchSlots = 8;
+
+// A per-scene device buffer that grows to the largest size a call has asked of it. It frees its memory when destroyed, on the
+// device current then: a DeviceScene is deleted with its own device current (device_scene_free).
+template <class T>
+struct DevBuf {
+    T* ptr = nullptr;
+    size_t n = 0;  // elements allocated
+    DevBuf() = default;
+    DevBuf(const DevBuf&) = delete;
+    DevBuf& operator=(const DevBuf&) = delete;
+    ~DevBuf() { cudaFree(ptr); }
+    // room for `want` elements; the contents do not survive a reallocation, and a failed one leaves the buffer empty
+    int reserve(size_t want) {
+        if (n >= want) return RTP_OK;
+        cudaFree(ptr); ptr = nullptr; n = 0;
+        const size_t m = std::max<size_t>(want, 1);
+        RTP_CUDA(cudaMalloc(reinterpret_cast<void**>(&ptr), m * sizeof(T)));
+        n = m;
+        return RTP_OK;
+    }
+};
 
 struct DeviceScene {
     int device = 0;
@@ -2047,21 +2067,18 @@ struct DeviceScene {
     std::vector<cudaEvent_t> ev_pool;  // render calls with stats: marks around the traversal launches (trace_ms / shade_ms)
     size_t ev_used = 0;
     size_t last_trace_launches = 1;    // kernels the last launch_trace call queued (2 with the deferred in-order launch)
-    size_t pending_launches = 0;       // of the render enqueued last (render_enqueue -> render_finish)
+    size_t pending_launches = 0;       // of the render enqueued last (render_end -> render_finish)
     uint64_t pending_paths = 0;
-    rtp_ray* stage_rays[kPipeDepth] = {nullptr, nullptr, nullptr};
-    void* stage_hits[kPipeDepth] = {nullptr, nullptr, nullptr};
-    double4* scratch = nullptr; size_t scratch_elems = 0;
-    double4* acc = nullptr; size_t acc_elems = 0;
+    DevBuf<rtp_ray> stage_rays[kPipeDepth];  // trace_host's pipeline stages
+    DevBuf<rtp_hit_full> stage_hits[kPipeDepth];
+    DevBuf<double4> scratch, acc;
     // rtp_render_adaptive, per tile pixel and grown like acc: luminance moments (16 B), sample count (4 B), keep flag (1 B), two live-list entries (8 B): 29 B beside acc's 32.
     // The live count of a round goes through n_live to a pinned word that the host reads.
-    double2* moments = nullptr; uint32_t* counts = nullptr; uint8_t* keep = nullptr; uint32_t* live[2] = {nullptr, nullptr};
-    size_t adaptive_elems = 0;
-    void* select_tmp = nullptr; size_t select_tmp_bytes = 0;  // cub::DeviceSelect::Flagged
-    uint32_t* n_live = nullptr; uint32_t* n_live_host = nullptr;
+    DevBuf<double2> moments; DevBuf<uint32_t> counts; DevBuf<uint8_t> keep; DevBuf<uint32_t> live[2];
+    DevBuf<uint8_t> select_tmp;  // cub::DeviceSelect::Flagged
+    DevBuf<uint32_t> n_live; uint32_t* n_live_host = nullptr;
     // rtp_render_aov: the AovRecords of a launch (3 double2 per path, grown like scratch) and their sums (3 double2 per tile pixel)
-    double2* aov_rec = nullptr; size_t aov_rec_elems = 0;
-    double2* aov_acc = nullptr; size_t aov_acc_elems = 0;
+    DevBuf<double2> aov_rec, aov_acc;
     WaveQueues wave{};                // wavefront integrator queues (render_device), grown on demand
     uint32_t wave_bounces = 0;         // stack depth the queues were sized for
     int shade_blocks = 0;              // grid of wave_shade_kernel
@@ -2070,10 +2087,10 @@ struct DeviceScene {
     // needs): growing them to the largest capacity seen AND the deepest stack seen would not (1080p x 16 spp at depth 1, then any
     // frame at depth 128: a 204 GB stack), so wave_reserve then reallocates them for the call alone.
     size_t queue_budget_bytes = size_t(4) << 30;
-    double* frame = nullptr; size_t frame_elems = 0;
-    uint32_t* frame_samples = nullptr; size_t frame_samples_elems = 0;  // rtp_render_adaptive's samples_out
-    uchar4* frame8 = nullptr; size_t frame8_elems = 0;  // RGBA8 output stage
-    SrgbFix* fixes = nullptr; unsigned int* n_fixes = nullptr;
+    DevBuf<double> frame;               // staging planes of the host-buffer render calls (render_host, rtp_render_adaptive)
+    DevBuf<uint32_t> frame_samples;     // rtp_render_adaptive's samples_out
+    DevBuf<uchar4> frame8;              // RGBA8 output stage
+    DevBuf<SrgbFix> fixes; DevBuf<unsigned int> n_fixes;
     unsigned int n_fix_host = 0;       // n_fixes of the last rtp_render_srgb8, copied back with the frame
 };
 
@@ -2096,19 +2113,13 @@ void device_scene_free(DeviceScene* ds) {
         cudaFree(sl.defer_idx);
         if (sl.last_use) cudaEventDestroy(sl.last_use);
     }
-    for (int k = 0; k < kPipeDepth; ++k) {
+    for (int k = 0; k < kPipeDepth; ++k)
         if (ds->streams[k]) cudaStreamDestroy(ds->streams[k]);
-        cudaFree(ds->stage_rays[k]); cudaFree(ds->stage_hits[k]);
-    }
     if (ds->ev_begin) cudaEventDestroy(ds->ev_begin);
     if (ds->ev_end) cudaEventDestroy(ds->ev_end);
     for (cudaEvent_t ev : ds->ev_pool) cudaEventDestroy(ev);
     if (ds->render_done) cudaEventDestroy(ds->render_done);
-    cudaFree(ds->moments); cudaFree(ds->counts); cudaFree(ds->keep); cudaFree(ds->live[0]); cudaFree(ds->live[1]);
-    cudaFree(ds->select_tmp); cudaFree(ds->n_live); cudaFree(ds->frame_samples);
     if (ds->n_live_host) cudaFreeHost(ds->n_live_host);
-    cudaFree(ds->aov_rec); cudaFree(ds->aov_acc);
-    cudaFree(ds->scratch); cudaFree(ds->acc); cudaFree(ds->frame); cudaFree(ds->frame8); cudaFree(ds->fixes); cudaFree(ds->n_fixes);
     cudaFree(ds->wave.rays[0]); cudaFree(ds->wave.rays[1]); cudaFree(ds->wave.state[0]); cudaFree(ds->wave.state[1]);
     cudaFree(ds->wave.hits); cudaFree(ds->wave.stack); cudaFree(ds->wave.count);
     delete ds;
@@ -2419,6 +2430,29 @@ static int launch_trace(DeviceScene* ds, const rtp_ray* d_rays, size_t n, void* 
     return RTP_OK;
 }
 
+// The scene's counters and the ev_begin -> ev_end time of the finished call that used them last, as the rtp_stats fields they give
+// (every other field 0). c != nullptr: the raw counters too.
+static int read_stats(const DeviceScene* ds, rtp_stats* stats, Counters* c = nullptr) {
+    Counters local;
+    if (!c) c = &local;
+    RTP_CUDA(cudaMemcpy(c, ds->counters, sizeof *c, cudaMemcpyDeviceToHost));
+    float ms = 0.f;
+    RTP_CUDA(cudaEventElapsedTime(&ms, ds->ev_begin, ds->ev_end));
+    std::memset(stats, 0, sizeof *stats);
+    stats->rays = c->rays; stats->node_visits = c->node_visits; stats->triangle_tests = c->triangle_tests; stats->sphere_tests = c->sphere_tests;
+    stats->leaf_gates = c->leaf_gates; stats->conservative_violations = c->violations; stats->order_rewalks = c->rewalks;
+    stats->device_ms = ms;
+    return RTP_OK;
+}
+
+static void add_stats(rtp_stats* total, const rtp_stats& one) {
+    total->rays += one.rays; total->paths += one.paths; total->node_visits += one.node_visits; total->triangle_tests += one.triangle_tests;
+    total->sphere_tests += one.sphere_tests; total->leaf_gates += one.leaf_gates; total->conservative_violations += one.conservative_violations;
+    total->order_rewalks += one.order_rewalks; total->kernel_launches += one.kernel_launches;
+    total->device_ms = std::max(total->device_ms, one.device_ms);  // the devices run side by side
+    total->trace_ms = std::max(total->trace_ms, one.trace_ms); total->shade_ms = std::max(total->shade_ms, one.shade_ms);
+}
+
 // Host-buffer batch: chunks flow H2D → kernel → D2H on kPipeDepth streams per device so copies overlap traversal; a scene that
 // lives on several devices (rtp_scene_create_multi) deals its chunks out to them round-robin, so every device's host link carries
 // a share of the 80 B/ray stream. Chunks are independent: no exchange between devices.
@@ -2440,8 +2474,8 @@ static int trace_host(rtp_scene* scene, const rtp_ray* rays, size_t n, void* hit
         DeviceScene* ds = devs[d];
         RTP_CUDA(cudaSetDevice(ds->device));
         for (int k = 0; k < kPipeDepth; ++k) {
-            if (!ds->stage_rays[k]) RTP_CUDA(cudaMalloc(reinterpret_cast<void**>(&ds->stage_rays[k]), chunk * sizeof(rtp_ray)));
-            if (!ds->stage_hits[k]) RTP_CUDA(cudaMalloc(&ds->stage_hits[k], chunk * sizeof(rtp_hit_full)));
+            if ((rc = ds->stage_rays[k].reserve(chunk)) != RTP_OK) return rc;
+            if ((rc = ds->stage_hits[k].reserve(chunk)) != RTP_OK) return rc;
         }
         if (count) RTP_CUDA(cudaMemsetAsync(ds->counters, 0, sizeof(Counters), ds->streams[0]));
         RTP_CUDA(cudaEventRecord(ds->ev_begin, ds->streams[0]));
@@ -2456,18 +2490,18 @@ static int trace_host(rtp_scene* scene, const rtp_ray* rays, size_t n, void* hit
         cudaError_t e = N > 1 ? cudaSetDevice(ds->device) : cudaSuccess;
         if (e == cudaSuccess) {
             if (camera) {
-                camera_rays_kernel<<<static_cast<unsigned>((m + 255) / 256), 256, 0, st>>>(*camera, width, height, ds->stage_rays[k], off, m);
+                camera_rays_kernel<<<static_cast<unsigned>((m + 255) / 256), 256, 0, st>>>(*camera, width, height, ds->stage_rays[k].ptr, off, m);
                 e = cudaGetLastError();
                 ++launches;
             } else {
-                e = cudaMemcpyAsync(ds->stage_rays[k], rays + off, m * sizeof(rtp_ray), cudaMemcpyHostToDevice, st);
+                e = cudaMemcpyAsync(ds->stage_rays[k].ptr, rays + off, m * sizeof(rtp_ray), cudaMemcpyHostToDevice, st);
             }
         }
         if (e != cudaSuccess) { rc = set_error(RTP_ERR_CUDA, std::string("trace chunk: ") + cudaGetErrorString(e)); break; }
-        rc = launch_trace(ds, ds->stage_rays[k], m, ds->stage_hits[k], out_mode, false, count ? ds->counters : nullptr, st);
+        rc = launch_trace(ds, ds->stage_rays[k].ptr, m, ds->stage_hits[k].ptr, out_mode, false, count ? ds->counters : nullptr, st);
         if (rc != RTP_OK) break;
         launches += ds->last_trace_launches;
-        e = cudaMemcpyAsync(static_cast<char*>(hits_out) + off * hit_bytes, ds->stage_hits[k], m * hit_bytes, cudaMemcpyDeviceToHost, st);
+        e = cudaMemcpyAsync(static_cast<char*>(hits_out) + off * hit_bytes, ds->stage_hits[k].ptr, m * hit_bytes, cudaMemcpyDeviceToHost, st);
         if (e != cudaSuccess) rc = set_error(RTP_ERR_CUDA, std::string("trace chunk: ") + cudaGetErrorString(e));
     }
     // drain every device that was given work (also after an error: nothing may stay in flight on the staging buffers)
@@ -2483,14 +2517,8 @@ static int trace_host(rtp_scene* scene, const rtp_ray* rays, size_t n, void* hit
         else cudaStreamSynchronize(ds->streams[0]);
         if (e != cudaSuccess && rc == RTP_OK) rc = set_error(RTP_ERR_CUDA, std::string("trace: ") + cudaGetErrorString(e));
         if (stats && rc == RTP_OK) {
-            Counters c;
-            float ms = 0.f;
-            e = cudaMemcpy(&c, ds->counters, sizeof c, cudaMemcpyDeviceToHost);
-            if (e == cudaSuccess) e = cudaEventElapsedTime(&ms, ds->ev_begin, ds->ev_end);
-            if (e != cudaSuccess) { rc = set_error(RTP_ERR_CUDA, std::string("trace stats: ") + cudaGetErrorString(e)); continue; }
-            total.rays += c.rays; total.node_visits += c.node_visits; total.triangle_tests += c.triangle_tests; total.sphere_tests += c.sphere_tests;
-            total.leaf_gates += c.leaf_gates; total.conservative_violations += c.violations; total.order_rewalks += c.rewalks;
-            total.device_ms = std::max(total.device_ms, static_cast<double>(ms));
+            rtp_stats one;
+            if ((rc = read_stats(ds, &one)) == RTP_OK) add_stats(&total, one);
         }
     }
     if (N > 1) cudaSetDevice(scene->dev->device);
@@ -2503,8 +2531,8 @@ static void launch_render_paths(DeviceScene* ds, const DCamera& cam, const DRend
                                 cudaStream_t st) {
     const unsigned block = 128;
     const dim3 g(static_cast<unsigned>((total + block - 1) / block));
-    if (count) render_paths_kernel<MAXB, true><<<g, block, 0, st>>>(ds->view, cam, rp, ds->scratch, ds->counters, map, aov);
-    else render_paths_kernel<MAXB, false><<<g, block, 0, st>>>(ds->view, cam, rp, ds->scratch, ds->counters, map, aov);
+    if (count) render_paths_kernel<MAXB, true><<<g, block, 0, st>>>(ds->view, cam, rp, ds->scratch.ptr, ds->counters, map, aov);
+    else render_paths_kernel<MAXB, false><<<g, block, 0, st>>>(ds->view, cam, rp, ds->scratch.ptr, ds->counters, map, aov);
 }
 
 // bytes per path of one launch of the wavefront integrator: queues (2 rays, 2 states, a hit record: 176 B), the [bounce][path]
@@ -2578,6 +2606,32 @@ static int render_rect(const rtp_render_params* p, bool fixed_spp, DRender* rp) 
     return RTP_OK;
 }
 
+// Takes the scene's render scratch (integrator queues, accumulators, counters, time marks) for a call on `st`: checks the call's
+// pixels (render_rect), orders `st` after the render queued last on any stream, zeroes the counters and opens the timed span.
+// On RTP_OK the call holds the scratch until render_end, which it runs after an error too.
+static int render_begin(DeviceScene* ds, const rtp_render_params* p, bool fixed_spp, bool want_stats, cudaStream_t st, DRender* rp) {
+    if (int rc = render_rect(p, fixed_spp, rp)) return rc;
+    if (ds->render_pending) RTP_CUDA(cudaStreamWaitEvent(st, ds->render_done, 0));
+    ds->ev_used = 0;
+    RTP_CUDA(cudaMemsetAsync(ds->counters, 0, sizeof(Counters), st));
+    if (want_stats) {
+        RTP_CUDA(cudaEventRecord(ds->ev_begin, st));
+        RTP_CUDA(cudaEventRecord(ds->ev_end, st));
+    }
+    return RTP_OK;
+}
+
+// Releases the scratch after the call's last launch on `st`: keeps its kernel and path counts for render_finish, closes the timed
+// span and records render_done, which the next render waits for before it touches the scratch, also when this call failed part way.
+static int render_end(DeviceScene* ds, cudaStream_t st, bool want_stats, size_t launches, uint64_t paths) {
+    ds->pending_launches = launches;
+    ds->pending_paths = paths;
+    if (want_stats) RTP_CUDA(cudaEventRecord(ds->ev_end, st));
+    RTP_CUDA(cudaEventRecord(ds->render_done, st));
+    ds->render_pending = true;
+    return RTP_OK;
+}
+
 // Paths per launch of the integrator for a call with max_bounce `bounces`: up to 32 Mi paths (wavefront queues 176 B + 48 B x
 // max_bounce per path, scratch 32 B), within the memory budget fixed when the scene was uploaded (a sixth of the free HBM, at most
 // 24 GiB). Big launches matter: every launch pays the fill and drain of ~2 x max_bounce kernels and the latency-bound sparse late
@@ -2596,17 +2650,8 @@ static int reserve_paths(DeviceScene* ds, size_t need, uint32_t bounces, bool ao
         int rc = wave_reserve(ds, need, bounces);
         if (rc != RTP_OK) return rc;
     }
-    if (ds->scratch_elems < need) {
-        cudaFree(ds->scratch); ds->scratch = nullptr; ds->scratch_elems = 0;
-        RTP_CUDA(cudaMalloc(reinterpret_cast<void**>(&ds->scratch), need * sizeof(double4)));
-        ds->scratch_elems = need;
-    }
-    if (aov && ds->aov_rec_elems < need) {
-        cudaFree(ds->aov_rec); ds->aov_rec = nullptr; ds->aov_rec_elems = 0;
-        RTP_CUDA(cudaMalloc(reinterpret_cast<void**>(&ds->aov_rec), need * 3 * sizeof(double2)));
-        ds->aov_rec_elems = need;
-    }
-    return RTP_OK;
+    if (int rc = ds->scratch.reserve(need)) return rc;
+    return aov ? ds->aov_rec.reserve(need * 3) : RTP_OK;
 }
 
 // One launch of the integrator: the `total` paths of rp's sample range over the pixel slots of `map`, traced to their end; path p's
@@ -2640,7 +2685,7 @@ static int launch_paths(DeviceScene* ds, const DCamera& cam, const DRender& rp, 
         // first vertex: rtp_render only.
         if (want_stats) next_mark(ds, st);  // even marks open a traversal span, odd marks close it
         if (std::is_same<Map, DenseTile>::value && !Aov::kOn && ds->sw.tail_threshold && total <= ds->sw.tail_threshold) {
-            TailArgs ta{ds->wave, rp, ds->scratch, b};
+            TailArgs ta{ds->wave, rp, ds->scratch.ptr, b};
             rc = launch_trace(ds, ds->wave.rays[b & 1], total, nullptr, OUT_TAIL, count, ds->counters, st, ds->wave.count + b, &ta);
             if (rc != RTP_OK) return rc;
             ++*launches;
@@ -2651,7 +2696,7 @@ static int launch_paths(DeviceScene* ds, const DCamera& cam, const DRender& rp, 
         if (rc != RTP_OK) return rc;
         if (want_stats) next_mark(ds, st);
         if ((rc = debug_sync(ds, st, "trace kernel <OUT_WAVE>", b)) != RTP_OK) return rc;
-        wave_shade_kernel<<<shade_grid, 256, 0, st>>>(ds->view, rp, ds->wave, b, ds->scratch, map, aov);
+        wave_shade_kernel<<<shade_grid, 256, 0, st>>>(ds->view, rp, ds->wave, b, ds->scratch.ptr, map, aov);
         RTP_CUDA(cudaGetLastError());
         if ((rc = debug_sync(ds, st, "wave_shade_kernel", b)) != RTP_OK) return rc;
         *launches += ds->last_trace_launches + 1;
@@ -2670,101 +2715,76 @@ struct AovFrame {
 static int render_enqueue(DeviceScene* ds, const rtp_camera* camera, const rtp_render_params* p, double* d_rgb, double* d_fg, bool want_stats,
                           cudaStream_t st, uchar4* d_rgba8 = nullptr, const AovFrame* aov = nullptr) {
     DRender rp;
-    if (int rc = render_rect(p, true, &rp)) return rc;
-    const uint32_t tw = rp.tile_w, th = rp.tile_h;
-
-    // the scratch below is shared by every render on this scene: a render queued on another stream must be over first
-    if (ds->render_pending) RTP_CUDA(cudaStreamWaitEvent(st, ds->render_done, 0));
-    ds->ev_used = 0;
-    ds->pending_launches = 0;
-    ds->pending_paths = 0;
-    const size_t npix = static_cast<size_t>(tw) * th;
-    if (want_stats) {
-        RTP_CUDA(cudaMemsetAsync(ds->counters, 0, sizeof(Counters), st));
-        RTP_CUDA(cudaEventRecord(ds->ev_begin, st));
-        RTP_CUDA(cudaEventRecord(ds->ev_end, st));
-    }
-    if (npix == 0) return RTP_OK;  // no row of the rectangle falls to this call
+    if (int rc = render_begin(ds, p, true, want_stats, st, &rp)) return rc;
+    const size_t npix = static_cast<size_t>(rp.tile_w) * rp.tile_h;
     const uint32_t ns_total = p->sample_end - p->sample_begin;
-    const uint32_t per_launch = static_cast<uint32_t>(std::max<size_t>(1, std::min<size_t>(ns_total ? ns_total : 1, path_budget(ds, p->max_bounce, aov != nullptr) / npix)));
-    if (ns_total) {
-        int rc = reserve_paths(ds, npix * per_launch, p->max_bounce, aov != nullptr);
-        if (rc != RTP_OK) return rc;
-    }
-    if (ds->acc_elems < npix) {
-        cudaFree(ds->acc); ds->acc = nullptr; ds->acc_elems = 0;
-        RTP_CUDA(cudaMalloc(reinterpret_cast<void**>(&ds->acc), npix * sizeof(double4)));
-        ds->acc_elems = npix;
-    }
-    if (aov && ds->aov_acc_elems < npix) {
-        cudaFree(ds->aov_acc); ds->aov_acc = nullptr; ds->aov_acc_elems = 0;
-        RTP_CUDA(cudaMalloc(reinterpret_cast<void**>(&ds->aov_acc), npix * 3 * sizeof(double2)));
-        ds->aov_acc_elems = npix;
-    }
-    const bool count = (p->flags & RTP_RENDER_COUNTERS) != 0;
-    const DCamera cam = make_camera(camera);
-
-    if (!want_stats) RTP_CUDA(cudaMemsetAsync(ds->counters, 0, sizeof(Counters), st));
     size_t launches = 0;
-    bool first = true;
-    if (ns_total == 0) RTP_CUDA(cudaMemsetAsync(ds->acc, 0, npix * sizeof(double4), st));
-    if (ns_total == 0 && aov) RTP_CUDA(cudaMemsetAsync(ds->aov_acc, 0, npix * 3 * sizeof(double2), st));
-    for (uint32_t s0 = 0; s0 < ns_total; s0 += per_launch) {
-        rp.sample_begin = p->sample_begin + s0;
-        rp.n_samples = std::min(per_launch, ns_total - s0);
-        int rc = aov ? launch_paths(ds, cam, rp, DenseTile{}, AovRecords{ds->aov_rec}, npix * rp.n_samples, count, want_stats, st, &launches)
-                     : launch_paths(ds, cam, rp, DenseTile{}, NoAov{}, npix * rp.n_samples, count, want_stats, st, &launches);
-        if (rc != RTP_OK) return rc;
-        resolve_kernel<<<static_cast<unsigned>((npix + 255) / 256), 256, 0, st>>>(ds->scratch, ds->acc, npix, rp.n_samples, first ? 1 : 0);
+    auto enqueue = [&]() -> int {
+        if (npix == 0) return RTP_OK;  // no row of the rectangle falls to this call
+        const uint32_t per_launch = static_cast<uint32_t>(std::max<size_t>(1, std::min<size_t>(ns_total ? ns_total : 1, path_budget(ds, p->max_bounce, aov != nullptr) / npix)));
+        if (ns_total) {
+            int rc = reserve_paths(ds, npix * per_launch, p->max_bounce, aov != nullptr);
+            if (rc != RTP_OK) return rc;
+        }
+        if (int rc = ds->acc.reserve(npix)) return rc;
+        if (aov) {
+            if (int rc = ds->aov_acc.reserve(npix * 3)) return rc;
+        }
+        const bool count = (p->flags & RTP_RENDER_COUNTERS) != 0;
+        const DCamera cam = make_camera(camera);
+
+        bool first = true;
+        if (ns_total == 0) RTP_CUDA(cudaMemsetAsync(ds->acc.ptr, 0, npix * sizeof(double4), st));
+        if (ns_total == 0 && aov) RTP_CUDA(cudaMemsetAsync(ds->aov_acc.ptr, 0, npix * 3 * sizeof(double2), st));
+        for (uint32_t s0 = 0; s0 < ns_total; s0 += per_launch) {
+            rp.sample_begin = p->sample_begin + s0;
+            rp.n_samples = std::min(per_launch, ns_total - s0);
+            int rc = aov ? launch_paths(ds, cam, rp, DenseTile{}, AovRecords{ds->aov_rec.ptr}, npix * rp.n_samples, count, want_stats, st, &launches)
+                         : launch_paths(ds, cam, rp, DenseTile{}, NoAov{}, npix * rp.n_samples, count, want_stats, st, &launches);
+            if (rc != RTP_OK) return rc;
+            resolve_kernel<<<static_cast<unsigned>((npix + 255) / 256), 256, 0, st>>>(ds->scratch.ptr, ds->acc.ptr, npix, rp.n_samples, first ? 1 : 0);
+            RTP_CUDA(cudaGetLastError());
+            ++launches;
+            if (aov) {
+                aov_resolve_kernel<<<static_cast<unsigned>((npix + 255) / 256), 256, 0, st>>>(ds->aov_rec.ptr, ds->aov_acc.ptr, npix, rp.n_samples, first ? 1 : 0);
+                RTP_CUDA(cudaGetLastError());
+                ++launches;
+            }
+            first = false;
+        }
+        const double divisor = (p->flags & RTP_RENDER_RAW_SUMS) ? 0.0 : static_cast<double>(p->num_samples);
+        if (d_rgba8) {
+            RTP_CUDA(cudaMemsetAsync(ds->n_fixes.ptr, 0, sizeof(unsigned int), st));
+            srgb8_kernel<<<static_cast<unsigned>((npix + 255) / 256), 256, 0, st>>>(ds->acc.ptr, rp, divisor, (p->flags & RTP_RENDER_TRANSPARENT) ? 1 : 0, d_rgba8,
+                                                                                    ds->fixes.ptr, ds->n_fixes.ptr, kSrgbFixCap);
+        } else {
+            write_frame_kernel<<<static_cast<unsigned>((npix + 255) / 256), 256, 0, st>>>(ds->acc.ptr, rp, divisor, d_rgb, d_fg);
+        }
         RTP_CUDA(cudaGetLastError());
         ++launches;
         if (aov) {
-            aov_resolve_kernel<<<static_cast<unsigned>((npix + 255) / 256), 256, 0, st>>>(ds->aov_rec, ds->aov_acc, npix, rp.n_samples, first ? 1 : 0);
+            aov_write_kernel<<<static_cast<unsigned>((npix + 255) / 256), 256, 0, st>>>(ds->aov_acc.ptr, rp, divisor, aov->albedo, aov->normal);
             RTP_CUDA(cudaGetLastError());
             ++launches;
         }
-        first = false;
-    }
-    const double divisor = (p->flags & RTP_RENDER_RAW_SUMS) ? 0.0 : static_cast<double>(p->num_samples);
-    if (d_rgba8) {
-        RTP_CUDA(cudaMemsetAsync(ds->n_fixes, 0, sizeof(unsigned int), st));
-        srgb8_kernel<<<static_cast<unsigned>((npix + 255) / 256), 256, 0, st>>>(ds->acc, rp, divisor, (p->flags & RTP_RENDER_TRANSPARENT) ? 1 : 0, d_rgba8,
-                                                                                ds->fixes, ds->n_fixes, kSrgbFixCap);
-    } else {
-        write_frame_kernel<<<static_cast<unsigned>((npix + 255) / 256), 256, 0, st>>>(ds->acc, rp, divisor, d_rgb, d_fg);
-    }
-    RTP_CUDA(cudaGetLastError());
-    ++launches;
-    if (aov) {
-        aov_write_kernel<<<static_cast<unsigned>((npix + 255) / 256), 256, 0, st>>>(ds->aov_acc, rp, divisor, aov->albedo, aov->normal);
-        RTP_CUDA(cudaGetLastError());
-        ++launches;
-    }
-    ds->pending_launches = launches;
-    ds->pending_paths = static_cast<uint64_t>(npix) * ns_total;
-    if (want_stats) RTP_CUDA(cudaEventRecord(ds->ev_end, st));
-    RTP_CUDA(cudaEventRecord(ds->render_done, st));
-    ds->render_pending = true;
-    return RTP_OK;
+        return RTP_OK;
+    };
+    const int rc = enqueue();
+    const int rc_end = render_end(ds, st, want_stats, launches, static_cast<uint64_t>(npix) * ns_total);
+    return rc != RTP_OK ? rc : rc_end;
 }
 
 // waits for the frame enqueued last on this device and fills `stats` (all fields)
 static int render_finish(DeviceScene* ds, rtp_stats* stats) {
     RTP_CUDA(cudaEventSynchronize(ds->ev_end));
-    Counters c;
-    RTP_CUDA(cudaMemcpy(&c, ds->counters, sizeof c, cudaMemcpyDeviceToHost));
-    float ms = 0.f;
-    RTP_CUDA(cudaEventElapsedTime(&ms, ds->ev_begin, ds->ev_end));
+    if (int rc = read_stats(ds, stats)) return rc;
     double trace_ms = 0.0;
     for (size_t k = 0; k + 1 < ds->ev_used; k += 2) {
         float span = 0.f;
         if (cudaEventElapsedTime(&span, ds->ev_pool[k], ds->ev_pool[k + 1]) == cudaSuccess) trace_ms += span;
     }
-    std::memset(stats, 0, sizeof *stats);
-    stats->rays = c.rays; stats->paths = ds->pending_paths;
-    stats->node_visits = c.node_visits; stats->triangle_tests = c.triangle_tests; stats->sphere_tests = c.sphere_tests; stats->leaf_gates = c.leaf_gates; stats->conservative_violations = c.violations; stats->order_rewalks = c.rewalks;
-    stats->device_ms = ms; stats->kernel_launches = ds->pending_launches;
-    stats->trace_ms = trace_ms; stats->shade_ms = std::max(0.0, static_cast<double>(ms) - trace_ms);
+    stats->paths = ds->pending_paths; stats->kernel_launches = ds->pending_launches;
+    stats->trace_ms = trace_ms; stats->shade_ms = std::max(0.0, stats->device_ms - trace_ms);
     return RTP_OK;
 }
 
@@ -2774,14 +2794,6 @@ static int render_device(rtp_scene* scene, const rtp_camera* camera, const rtp_r
     int rc = render_enqueue(ds, camera, p, d_rgb, d_fg, stats != nullptr, st, d_rgba8, aov);
     if (rc != RTP_OK) return rc;
     return stats ? render_finish(ds, stats) : RTP_OK;
-}
-
-static void add_stats(rtp_stats* total, const rtp_stats& one) {
-    total->rays += one.rays; total->paths += one.paths; total->node_visits += one.node_visits; total->triangle_tests += one.triangle_tests;
-    total->sphere_tests += one.sphere_tests; total->leaf_gates += one.leaf_gates; total->conservative_violations += one.conservative_violations;
-    total->order_rewalks += one.order_rewalks; total->kernel_launches += one.kernel_launches;
-    total->device_ms = std::max(total->device_ms, one.device_ms);  // the devices run side by side
-    total->trace_ms = std::max(total->trace_ms, one.trace_ms); total->shade_ms = std::max(total->shade_ms, one.shade_ms);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -2808,7 +2820,7 @@ static int check_adaptive(const rtp_render_params* p, const rtp_adaptive_params*
 struct AdaptiveDev {
     DeviceScene* ds = nullptr;
     cudaStream_t st = nullptr;
-    rtp_render_params p{};  // this device's rows
+    const rtp_render_params* p = nullptr;  // this device's rows
     double* d_rgb = nullptr; double* d_fg = nullptr; uint32_t* d_samples = nullptr;
     DRender rp{};
     size_t npix = 0;
@@ -2816,57 +2828,28 @@ struct AdaptiveDev {
     int cur = 0;
     size_t launches = 0;
     uint64_t paths = 0;
-    bool begun = false;     // holds the scene's scratch: render_done must be recorded
 };
 
-template <class T>
-static int grow(T** buf, size_t n) {
-    cudaFree(*buf); *buf = nullptr;
-    RTP_CUDA(cudaMalloc(reinterpret_cast<void**>(buf), std::max<size_t>(n, 1) * sizeof(T)));
-    return RTP_OK;
-}
-
-static int adaptive_begin(AdaptiveDev& d, bool want_stats) {
+// sizes the adaptive buffers for d's pixels and queues their initialisation: every pixel live, no sample yet
+static int adaptive_init(AdaptiveDev& d) {
     DeviceScene* ds = d.ds;
-    if (int rc = render_rect(&d.p, false, &d.rp)) return rc;
-    if (ds->render_pending) RTP_CUDA(cudaStreamWaitEvent(d.st, ds->render_done, 0));
-    d.begun = true;
-    ds->ev_used = 0;
-    RTP_CUDA(cudaMemsetAsync(ds->counters, 0, sizeof(Counters), d.st));
-    if (want_stats) {
-        RTP_CUDA(cudaEventRecord(ds->ev_begin, d.st));
-        RTP_CUDA(cudaEventRecord(ds->ev_end, d.st));
-    }
     d.npix = static_cast<size_t>(d.rp.tile_w) * d.rp.tile_h;
     if (d.npix == 0) return RTP_OK;  // no row of the rectangle falls to this device
     if (d.npix > static_cast<size_t>(std::numeric_limits<int>::max()))  // cub::DeviceSelect counts items in int
         return set_error(RTP_ERR_UNSUPPORTED, "adaptive: more than 2^31 - 1 pixels on one device");
-    if (ds->acc_elems < d.npix) {
-        if (int rc = grow(&ds->acc, d.npix)) return rc;
-        ds->acc_elems = d.npix;
-    }
-    if (ds->adaptive_elems < d.npix) {
-        ds->adaptive_elems = 0;
-        int rc = grow(&ds->moments, d.npix);
-        if (rc == RTP_OK) rc = grow(&ds->counts, d.npix);
-        if (rc == RTP_OK) rc = grow(&ds->keep, d.npix);
-        if (rc == RTP_OK) rc = grow(&ds->live[0], d.npix);
-        if (rc == RTP_OK) rc = grow(&ds->live[1], d.npix);
-        if (rc != RTP_OK) return rc;
-        ds->adaptive_elems = d.npix;
-    }
+    int rc = ds->acc.reserve(d.npix);
+    if (rc == RTP_OK) rc = ds->moments.reserve(d.npix);
+    if (rc == RTP_OK) rc = ds->counts.reserve(d.npix);
+    if (rc == RTP_OK) rc = ds->keep.reserve(d.npix);
+    if (rc == RTP_OK) rc = ds->live[0].reserve(d.npix);
+    if (rc == RTP_OK) rc = ds->live[1].reserve(d.npix);
+    if (rc == RTP_OK) rc = ds->n_live.reserve(1);
+    if (rc != RTP_OK) return rc;
     size_t tmp = 0;
-    RTP_CUDA(cub::DeviceSelect::Flagged(nullptr, tmp, static_cast<const uint32_t*>(ds->live[0]), ds->keep, ds->live[1], ds->n_live, static_cast<int>(d.npix), d.st));
-    if (ds->select_tmp_bytes < tmp) {
-        ds->select_tmp_bytes = 0;
-        if (int rc = grow(reinterpret_cast<uint8_t**>(&ds->select_tmp), tmp)) return rc;
-        ds->select_tmp_bytes = tmp;
-    }
-    if (!ds->n_live) {
-        if (int rc = grow(&ds->n_live, 1)) return rc;
-        RTP_CUDA(cudaHostAlloc(reinterpret_cast<void**>(&ds->n_live_host), sizeof(uint32_t), cudaHostAllocPortable));
-    }
-    adaptive_init_kernel<<<static_cast<unsigned>((d.npix + 255) / 256), 256, 0, d.st>>>(ds->acc, ds->moments, ds->counts, ds->live[0], d.npix);
+    RTP_CUDA(cub::DeviceSelect::Flagged(nullptr, tmp, static_cast<const uint32_t*>(ds->live[0].ptr), ds->keep.ptr, ds->live[1].ptr, ds->n_live.ptr, static_cast<int>(d.npix), d.st));
+    if ((rc = ds->select_tmp.reserve(tmp)) != RTP_OK) return rc;
+    if (!ds->n_live_host) RTP_CUDA(cudaHostAlloc(reinterpret_cast<void**>(&ds->n_live_host), sizeof(uint32_t), cudaHostAllocPortable));
+    adaptive_init_kernel<<<static_cast<unsigned>((d.npix + 255) / 256), 256, 0, d.st>>>(ds->acc.ptr, ds->moments.ptr, ds->counts.ptr, ds->live[0].ptr, d.npix);
     RTP_CUDA(cudaGetLastError());
     ++d.launches;
     d.n_live = static_cast<uint32_t>(d.npix);
@@ -2878,25 +2861,25 @@ static int adaptive_begin(AdaptiveDev& d, bool want_stats) {
 // to ds->n_live_host
 static int adaptive_round(AdaptiveDev& d, const DCamera& cam, uint32_t s0, uint32_t B, const StopRule& rule, bool count, bool want_stats) {
     DeviceScene* ds = d.ds;
-    const uint32_t per_launch = static_cast<uint32_t>(std::max<size_t>(1, std::min<size_t>(B, path_budget(ds, d.p.max_bounce) / d.n_live)));
-    if (int rc = reserve_paths(ds, static_cast<size_t>(d.n_live) * per_launch, d.p.max_bounce)) return rc;
-    const LiveList map{ds->live[d.cur], d.n_live};
+    const uint32_t per_launch = static_cast<uint32_t>(std::max<size_t>(1, std::min<size_t>(B, path_budget(ds, d.rp.max_bounce) / d.n_live)));
+    if (int rc = reserve_paths(ds, static_cast<size_t>(d.n_live) * per_launch, d.rp.max_bounce)) return rc;
+    const LiveList map{ds->live[d.cur].ptr, d.n_live};
     const unsigned grid = (d.n_live + 255u) / 256u;
     for (uint32_t l0 = 0; l0 < B; l0 += per_launch) {
         d.rp.sample_begin = s0 + l0;
         d.rp.n_samples = std::min(per_launch, B - l0);
         int rc = launch_paths(ds, cam, d.rp, map, NoAov{}, static_cast<size_t>(d.n_live) * d.rp.n_samples, count, want_stats, d.st, &d.launches);
         if (rc != RTP_OK) return rc;
-        adaptive_resolve_kernel<<<grid, 256, 0, d.st>>>(ds->scratch, map.live, d.n_live, d.rp.n_samples, ds->acc, ds->moments, ds->counts, ds->keep,
+        adaptive_resolve_kernel<<<grid, 256, 0, d.st>>>(ds->scratch.ptr, map.live, d.n_live, d.rp.n_samples, ds->acc.ptr, ds->moments.ptr, ds->counts.ptr, ds->keep.ptr,
                                                         l0 + per_launch >= B ? 1 : 0, rule);
         RTP_CUDA(cudaGetLastError());
         ++d.launches;
     }
     d.paths += static_cast<uint64_t>(d.n_live) * B;
-    size_t tmp = ds->select_tmp_bytes;
-    RTP_CUDA(cub::DeviceSelect::Flagged(ds->select_tmp, tmp, map.live, ds->keep, ds->live[d.cur ^ 1], ds->n_live, static_cast<int>(d.n_live), d.st));
+    size_t tmp = ds->select_tmp.n;
+    RTP_CUDA(cub::DeviceSelect::Flagged(ds->select_tmp.ptr, tmp, map.live, ds->keep.ptr, ds->live[d.cur ^ 1].ptr, ds->n_live.ptr, static_cast<int>(d.n_live), d.st));
     d.launches += 2;  // the selection's scan-state initialisation and the select kernel
-    RTP_CUDA(cudaMemcpyAsync(ds->n_live_host, ds->n_live, sizeof(uint32_t), cudaMemcpyDeviceToHost, d.st));
+    RTP_CUDA(cudaMemcpyAsync(ds->n_live_host, ds->n_live.ptr, sizeof(uint32_t), cudaMemcpyDeviceToHost, d.st));
     d.cur ^= 1;
     return RTP_OK;
 }
@@ -2907,10 +2890,14 @@ static int adaptive_round(AdaptiveDev& d, const DCamera& cam, uint32_t s0, uint3
 static int render_adaptive(std::vector<AdaptiveDev>& devs, const rtp_camera* camera, const rtp_adaptive_params* a, bool want_stats) {
     const DCamera cam = make_camera(camera);
     const StopRule rule{a->abs_tol, a->rel_tol, a->max_samples, 0u};
-    const bool count = (devs[0].p.flags & RTP_RENDER_COUNTERS) != 0;
+    const bool count = (devs[0].p->flags & RTP_RENDER_COUNTERS) != 0;
     int rc = RTP_OK;
+    size_t begun = 0;  // devs[0, begun) hold their scene's render scratch
     for (AdaptiveDev& d : devs) {
-        if (rc == RTP_OK) rc = cudaSetDevice(d.ds->device) == cudaSuccess ? adaptive_begin(d, want_stats) : set_error(RTP_ERR_CUDA, "cudaSetDevice");
+        if (cudaSetDevice(d.ds->device) != cudaSuccess) { rc = set_error(RTP_ERR_CUDA, "cudaSetDevice"); break; }
+        if ((rc = render_begin(d.ds, d.p, false, want_stats, d.st, &d.rp)) != RTP_OK) break;
+        ++begun;
+        if ((rc = adaptive_init(d)) != RTP_OK) break;
     }
     uint32_t n = 0, B = a->min_samples;
     while (rc == RTP_OK) {
@@ -2933,38 +2920,108 @@ static int render_adaptive(std::vector<AdaptiveDev>& devs, const rtp_camera* cam
         if (n >= a->max_samples) break;  // the stop rule has stopped every pixel
         B = std::min(a->batch, a->max_samples - n);
     }
-    const int raw = (devs[0].p.flags & RTP_RENDER_RAW_SUMS) ? 1 : 0;
-    for (AdaptiveDev& d : devs) {
-        if (!d.begun) continue;
+    const int raw = (devs[0].p->flags & RTP_RENDER_RAW_SUMS) ? 1 : 0;
+    for (size_t k = 0; k < begun; ++k) {
+        AdaptiveDev& d = devs[k];
         DeviceScene* ds = d.ds;
         cudaSetDevice(ds->device);
         if (rc == RTP_OK && d.npix) {
-            adaptive_write_kernel<<<static_cast<unsigned>((d.npix + 255) / 256), 256, 0, d.st>>>(ds->acc, ds->counts, d.rp, raw, d.d_rgb, d.d_fg, d.d_samples);
+            adaptive_write_kernel<<<static_cast<unsigned>((d.npix + 255) / 256), 256, 0, d.st>>>(ds->acc.ptr, ds->counts.ptr, d.rp, raw, d.d_rgb, d.d_fg, d.d_samples);
             if (cudaGetLastError() != cudaSuccess) rc = set_error(RTP_ERR_CUDA, "adaptive_write_kernel launch");
             ++d.launches;
         }
-        ds->pending_launches = d.launches;
-        ds->pending_paths = d.paths;
-        if (want_stats) cudaEventRecord(ds->ev_end, d.st);
-        cudaEventRecord(ds->render_done, d.st);
-        ds->render_pending = true;
+        const int rc_end = render_end(ds, d.st, want_stats, d.launches, d.paths);
+        if (rc == RTP_OK) rc = rc_end;
     }
     return rc;
 }
 
-// waits for every device's stream and, if asked, sums their stats
-static int adaptive_finish(std::vector<AdaptiveDev>& devs, int rc, rtp_stats* stats) {
+// ---------------------------------------------------------------------------------------------
+// The host-buffer render calls (rtp_render, rtp_render_srgb8, rtp_render_aov, rtp_render_adaptive) on one or several devices. The
+// rows of the tile rectangle are dealt out round-robin to the devices taking part (params->device_mask); every device renders ALL
+// samples of its rows into a frame-sized staging buffer, and only its rows travel back into the caller's frame: no exchange between
+// devices, and since a pixel's value depends only on (seed, pixel, sample) the frame is bit-identical to a one-device render. All
+// devices are driven from the calling thread: nothing is synchronised until every device's work is queued.
+// ---------------------------------------------------------------------------------------------
+
+// one device's share of a host-buffer render call
+struct FrameDev {
+    DeviceScene* ds;
+    rtp_render_params p;  // the call's parameters with this device's rows
+    std::unique_lock<std::mutex> lock;
+};
+
+// selects and locks the devices of params->device_mask (0: every device of the scene) and deals the rows out to them
+static int deal_rows(rtp_scene* scene, const rtp_render_params* params, std::vector<FrameDev>* devs) {
+    for (DeviceScene* ds : scene->devs)
+        if (params->device_mask == 0 || ((params->device_mask >> ds->device) & 1u)) devs->push_back({ds, *params, std::unique_lock<std::mutex>(ds->lock)});
+    if (devs->empty()) return set_error(RTP_ERR_INVALID, "device_mask names no device of this scene");
+    const uint32_t N = static_cast<uint32_t>(devs->size());
+    const uint32_t rs0 = params->row_stride ? params->row_stride : 1u;
+    for (uint32_t k = 0; k < N; ++k) {
+        rtp_render_params& p = (*devs)[k].p;
+        p.row_offset = params->row_offset + k * rs0;  // rows ro0 + m * rs0 of the caller's split; device k takes m = k, k + N, ...
+        p.row_stride = rs0 * N;
+    }
+    return RTP_OK;
+}
+
+// one plane of a frame: the caller's buffer (nullptr: not asked for), the device's frame-sized staging buffer, bytes per pixel
+struct Plane {
+    void* host;
+    const void* dev;
+    size_t px_bytes;
+};
+
+// queues on `st` the copy of the rows `p` covers (main.rs:86-87 writes per tile) from the device's planes into the caller's
+static int copy_rows(const rtp_render_params& p, cudaStream_t st, std::initializer_list<Plane> planes) {
+    DRender rp;
+    if (int rc = render_rect(&p, false, &rp)) return rc;
+    if (rp.tile_h == 0) return RTP_OK;  // no row of the rectangle fell to this device
+    const size_t first = rp.tile_x + static_cast<size_t>(rp.tile_y + rp.row_offset) * rp.width;
+    const size_t row_px = static_cast<size_t>(rp.width) * rp.row_stride;
+    for (const Plane& pl : planes) {
+        if (!pl.host) continue;
+        const size_t b = pl.px_bytes;
+        const cudaError_t e = cudaMemcpy2DAsync(static_cast<char*>(pl.host) + first * b, row_px * b, static_cast<const char*>(pl.dev) + first * b, row_px * b,
+                                                rp.tile_w * b, rp.tile_h, cudaMemcpyDeviceToHost, st);
+        if (e != cudaSuccess) return set_error(RTP_ERR_CUDA, std::string("frame copy: ") + cudaGetErrorString(e));
+    }
+    return RTP_OK;
+}
+
+// rtp_render_srgb8 on a finished device: redoes its borderline pixels with the host libm (utility.rs:213 powf as the reference's
+// target evaluates it)
+static int srgb_fixup(const DeviceScene* ds, uint8_t* rgba_out) {
+    const unsigned int n_fix = ds->n_fix_host;
+    if (n_fix > kSrgbFixCap) return set_error(RTP_ERR_UNSUPPORTED, "more than 65536 pixels need the host libm fix-up; use rtp_render + rtp_frame_to_srgb8");
+    if (n_fix == 0) return RTP_OK;
+    std::vector<SrgbFix> fixes(n_fix);
+    if (cudaMemcpy(fixes.data(), ds->fixes.ptr, n_fix * sizeof(SrgbFix), cudaMemcpyDeviceToHost) != cudaSuccess) return set_error(RTP_ERR_CUDA, "fix-up list copy");
+    for (const SrgbFix& f : fixes) {
+        uint8_t px[4];
+        rtp_frame_to_srgb8(f.rgb, 1, 1, px);
+        std::memcpy(rgba_out + 4 * static_cast<size_t>(f.pixel), px, 3);
+    }
+    return RTP_OK;
+}
+
+// Waits for every device of the call, also after an error on another one (nothing may stay in flight on a scene's scratch), then
+// applies the sRGB fix-up (rgba_out != nullptr) and sums the devices' stats. Leaves the scene's first device current.
+static int finish_frame(rtp_scene* scene, std::vector<FrameDev>& devs, int rc, rtp_stats* stats, uint8_t* rgba_out) {
     rtp_stats total;
     std::memset(&total, 0, sizeof total);
-    for (AdaptiveDev& d : devs) {
-        cudaSetDevice(d.ds->device);
-        const cudaError_t e = cudaStreamSynchronize(d.st);
-        if (e != cudaSuccess && rc == RTP_OK) rc = set_error(RTP_ERR_CUDA, std::string("adaptive render: ") + cudaGetErrorString(e));
+    for (FrameDev& d : devs) {
+        DeviceScene* ds = d.ds;
+        cudaSetDevice(ds->device);
+        const cudaError_t e = cudaStreamSynchronize(ds->streams[0]);
+        if (e != cudaSuccess && rc == RTP_OK) rc = set_error(RTP_ERR_CUDA, std::string("render: ") + cudaGetErrorString(e));
+        if (rc == RTP_OK && rgba_out && ds->pending_launches) rc = srgb_fixup(ds, rgba_out);
         if (rc != RTP_OK || !stats) continue;
         rtp_stats one;
-        rc = render_finish(d.ds, &one);
-        add_stats(&total, one);
+        if ((rc = render_finish(ds, &one)) == RTP_OK) add_stats(&total, one);
     }
+    cudaSetDevice(scene->dev->device);
     if (stats && rc == RTP_OK) *stats = total;
     return rc;
 }
@@ -3322,16 +3379,12 @@ static int trace_device_counted(rtp_scene* scene, const rtp_ray* d_rays, size_t 
     RTP_CUDA(cudaEventRecord(ds->ev_end, st));
     RTP_CUDA(cudaEventSynchronize(ds->ev_end));
     Counters c;
-    RTP_CUDA(cudaMemcpy(&c, ds->counters, sizeof c, cudaMemcpyDeviceToHost));
-    float ms = 0.f;
-    RTP_CUDA(cudaEventElapsedTime(&ms, ds->ev_begin, ds->ev_end));
+    if ((rc = read_stats(ds, stats, &c)) != RTP_OK) return rc;
+    stats->kernel_launches = 1;
     if (ds->sw.lane_stats && c.rounds)
         std::fprintf(stderr, "[rtp lanes] %llu rounds (%.1f per ray): per round %.1f lanes can walk, %.1f hold two leaves, %.1f wait for a leaf test with nothing left to walk, %.1f hold no ray; "
                              "%llu leaf rounds at %.1f lanes\n", c.rounds, double(c.rounds) * 32.0 / double(c.rays ? c.rays : 1), double(c.lanes_walk) / c.rounds, double(c.lanes_full) / c.rounds,
                      double(c.lanes_leafwait) / c.rounds, double(c.lanes_empty) / c.rounds, c.leaf_rounds, c.leaf_rounds ? double(c.leaf_lanes) / c.leaf_rounds : 0.0);
-    std::memset(stats, 0, sizeof *stats);
-    stats->rays = c.rays; stats->node_visits = c.node_visits; stats->triangle_tests = c.triangle_tests; stats->sphere_tests = c.sphere_tests; stats->leaf_gates = c.leaf_gates; stats->conservative_violations = c.violations; stats->order_rewalks = c.rewalks;
-    stats->device_ms = ms; stats->kernel_launches = 1;
     return RTP_OK;
 }
 
@@ -3399,102 +3452,41 @@ int rtp_render_device(rtp_scene* scene, const rtp_camera* camera, const rtp_rend
     return render_device(scene, camera, params, d_rgb_out, d_foreground_out, stats, static_cast<cudaStream_t>(cuda_stream));
 }
 
-// rtp_render / rtp_render_srgb8: host buffers, one or several devices. The rows of the tile rectangle are dealt out round-robin to
-// the devices taking part (params->device_mask), every device renders ALL samples of its rows and copies them straight into the
-// caller's frame: no exchange between devices, and since a pixel's value depends only on (seed, pixel, sample) the frame is
-// bit-identical to a one-device render. All devices are driven from this one host thread: render_enqueue never synchronises.
+// rtp_render / rtp_render_srgb8 / rtp_render_aov with host buffers, on the devices of params->device_mask (see deal_rows).
 // aov != nullptr (host pointers, either may be null): an rtp_render_aov call, whose staging frame holds 6 more doubles per pixel.
 static int render_host(rtp_scene* scene, const rtp_camera* camera, const rtp_render_params* params, double* rgb_out, double* foreground_out,
                        uint8_t* rgba_out, rtp_stats* stats, const AovFrame* aov = nullptr) {
     const size_t npx = static_cast<size_t>(params->width) * params->height;
     if (npx == 0) return set_error(RTP_ERR_INVALID, "bad frame parameters");
-    std::vector<DeviceScene*> devs;
-    for (DeviceScene* ds : scene->devs)
-        if (params->device_mask == 0 || ((params->device_mask >> ds->device) & 1u)) devs.push_back(ds);
-    if (devs.empty()) return set_error(RTP_ERR_INVALID, "device_mask names no device of this scene");
-    const uint32_t N = static_cast<uint32_t>(devs.size());
-    const uint32_t rs0 = params->row_stride ? params->row_stride : 1u, ro0 = params->row_offset;
-    const uint32_t W = params->width, tx = params->tile_x, ty = params->tile_y;
-    const uint32_t tw = params->tile_w ? params->tile_w : W - tx, th_full = params->tile_h ? params->tile_h : params->height - ty;
-    std::vector<std::unique_lock<std::mutex>> locks;
-    for (DeviceScene* ds : devs) locks.emplace_back(ds->lock);
+    std::vector<FrameDev> devs;
+    if (int rc = deal_rows(scene, params, &devs)) return rc;
     int rc = RTP_OK;
-    for (uint32_t k = 0; k < N && rc == RTP_OK; ++k) {
-        DeviceScene* ds = devs[k];
-        RTP_CUDA(cudaSetDevice(ds->device));
+    for (FrameDev& d : devs) {
+        DeviceScene* ds = d.ds;
         cudaStream_t st = ds->streams[0];
-        rtp_render_params p = *params;
-        p.row_offset = ro0 + k * rs0;  // rows ro0 + m * rs0 of the caller's split; device k takes m = k, k + N, ...
-        p.row_stride = rs0 * N;
+        if (cudaSetDevice(ds->device) != cudaSuccess) { rc = set_error(RTP_ERR_CUDA, "cudaSetDevice"); break; }
         if (rgba_out) {
-            if (ds->frame8_elems < npx) {
-                cudaFree(ds->frame8); ds->frame8 = nullptr; ds->frame8_elems = 0;
-                RTP_CUDA(cudaMalloc(reinterpret_cast<void**>(&ds->frame8), npx * sizeof(uchar4)));
-                ds->frame8_elems = npx;
+            rc = ds->frame8.reserve(npx);
+            if (rc == RTP_OK) rc = ds->fixes.reserve(kSrgbFixCap);
+            if (rc == RTP_OK) rc = ds->n_fixes.reserve(1);
+            if (rc == RTP_OK) rc = render_enqueue(ds, camera, &d.p, nullptr, nullptr, stats != nullptr, st, ds->frame8.ptr);
+            if (rc == RTP_OK) rc = copy_rows(d.p, st, {{rgba_out, ds->frame8.ptr, 4}});
+            if (rc == RTP_OK && ds->pending_launches) {
+                const cudaError_t e = cudaMemcpyAsync(&ds->n_fix_host, ds->n_fixes.ptr, sizeof(unsigned int), cudaMemcpyDeviceToHost, st);
+                if (e != cudaSuccess) rc = set_error(RTP_ERR_CUDA, std::string("fix-up count copy: ") + cudaGetErrorString(e));
             }
-            if (!ds->fixes) {
-                RTP_CUDA(cudaMalloc(reinterpret_cast<void**>(&ds->fixes), kSrgbFixCap * sizeof(SrgbFix)));
-                RTP_CUDA(cudaMalloc(reinterpret_cast<void**>(&ds->n_fixes), sizeof(unsigned int)));
-            }
-        } else if (ds->frame_elems < npx * (aov ? 10 : 4)) {  // rgb, foreground [, albedo, normal]
-            cudaFree(ds->frame); ds->frame = nullptr; ds->frame_elems = 0;
-            RTP_CUDA(cudaMalloc(reinterpret_cast<void**>(&ds->frame), npx * (aov ? 10 : 4) * sizeof(double)));
-            ds->frame_elems = npx * (aov ? 10 : 4);
-        }
-        const AovFrame d_aov = {aov && aov->albedo ? ds->frame + npx * 4 : nullptr, aov && aov->normal ? ds->frame + npx * 7 : nullptr};
-        rc = render_enqueue(ds, camera, &p, rgba_out ? nullptr : ds->frame, (!rgba_out && foreground_out) ? ds->frame + npx * 3 : nullptr, stats != nullptr, st,
-                            rgba_out ? ds->frame8 : nullptr, aov ? &d_aov : nullptr);
-        if (rc != RTP_OK) break;
-        // only the rows this device rendered travel back (main.rs:86-87 writes per tile)
-        if (p.row_offset >= th_full || tx >= W) continue;
-        const uint32_t rows = (th_full - p.row_offset + p.row_stride - 1u) / p.row_stride;
-        const size_t first = static_cast<size_t>(tx) + static_cast<size_t>(ty + p.row_offset) * W;
-        const size_t row_px = static_cast<size_t>(W) * p.row_stride;
-        if (rgba_out) {
-            RTP_CUDA(cudaMemcpy2DAsync(rgba_out + 4 * first, row_px * 4, ds->frame8 + first, row_px * 4, static_cast<size_t>(tw) * 4, rows, cudaMemcpyDeviceToHost, st));
-            RTP_CUDA(cudaMemcpyAsync(&ds->n_fix_host, ds->n_fixes, sizeof(unsigned int), cudaMemcpyDeviceToHost, st));
         } else {
-            RTP_CUDA(cudaMemcpy2DAsync(rgb_out + 3 * first, row_px * 24, ds->frame + 3 * first, row_px * 24, static_cast<size_t>(tw) * 24, rows, cudaMemcpyDeviceToHost, st));
-            if (foreground_out)
-                RTP_CUDA(cudaMemcpy2DAsync(foreground_out + first, row_px * 8, ds->frame + npx * 3 + first, row_px * 8, static_cast<size_t>(tw) * 8, rows, cudaMemcpyDeviceToHost, st));
-            if (d_aov.albedo)
-                RTP_CUDA(cudaMemcpy2DAsync(aov->albedo + 3 * first, row_px * 24, d_aov.albedo + 3 * first, row_px * 24, static_cast<size_t>(tw) * 24, rows, cudaMemcpyDeviceToHost, st));
-            if (d_aov.normal)
-                RTP_CUDA(cudaMemcpy2DAsync(aov->normal + 3 * first, row_px * 24, d_aov.normal + 3 * first, row_px * 24, static_cast<size_t>(tw) * 24, rows, cudaMemcpyDeviceToHost, st));
+            if ((rc = ds->frame.reserve(npx * (aov ? 10 : 4))) != RTP_OK) break;  // rgb, foreground [, albedo, normal]
+            double* f = ds->frame.ptr;
+            const AovFrame d_aov = {aov && aov->albedo ? f + npx * 4 : nullptr, aov && aov->normal ? f + npx * 7 : nullptr};
+            rc = render_enqueue(ds, camera, &d.p, f, foreground_out ? f + npx * 3 : nullptr, stats != nullptr, st, nullptr, aov ? &d_aov : nullptr);
+            if (rc == RTP_OK)
+                rc = copy_rows(d.p, st, {{rgb_out, f, 24}, {foreground_out, f + npx * 3, 8}, {d_aov.albedo ? aov->albedo : nullptr, d_aov.albedo, 24},
+                                         {d_aov.normal ? aov->normal : nullptr, d_aov.normal, 24}});
         }
+        if (rc != RTP_OK) break;
     }
-    // wait for every device that was given work, even after an error on a later one
-    rtp_stats total;
-    std::memset(&total, 0, sizeof total);
-    for (uint32_t k = 0; k < N; ++k) {
-        DeviceScene* ds = devs[k];
-        cudaSetDevice(ds->device);
-        cudaError_t e = cudaStreamSynchronize(ds->streams[0]);
-        if (e != cudaSuccess && rc == RTP_OK) rc = set_error(RTP_ERR_CUDA, std::string("render: ") + cudaGetErrorString(e));
-        if (rc != RTP_OK) continue;
-        if (rgba_out && ds->pending_launches) {
-            const unsigned int n_fix = ds->n_fix_host;
-            if (n_fix > kSrgbFixCap) { rc = set_error(RTP_ERR_UNSUPPORTED, "more than 65536 pixels need the host libm fix-up; use rtp_render + rtp_frame_to_srgb8"); continue; }
-            if (n_fix) {  // redo the borderline pixels with the host libm (utility.rs:213 powf as the reference's target evaluates it)
-                std::vector<SrgbFix> fixes(n_fix);
-                if (cudaMemcpy(fixes.data(), ds->fixes, n_fix * sizeof(SrgbFix), cudaMemcpyDeviceToHost) != cudaSuccess) { rc = set_error(RTP_ERR_CUDA, "fix-up list copy"); continue; }
-                for (const SrgbFix& f : fixes) {
-                    uint8_t px[4];
-                    rtp_frame_to_srgb8(f.rgb, 1, 1, px);
-                    std::memcpy(rgba_out + 4 * static_cast<size_t>(f.pixel), px, 3);
-                }
-            }
-        }
-        if (stats) {
-            rtp_stats one;
-            int r2 = render_finish(ds, &one);
-            if (r2 != RTP_OK) { rc = r2; continue; }
-            add_stats(&total, one);
-        }
-    }
-    cudaSetDevice(scene->dev->device);
-    if (stats && rc == RTP_OK) *stats = total;
-    return rc;
+    return finish_frame(scene, devs, rc, stats, rgba_out);
 }
 
 int rtp_render_srgb8(rtp_scene* scene, const rtp_camera* camera, const rtp_render_params* params, uint8_t* rgba_out, rtp_stats* stats) {
@@ -3542,56 +3534,28 @@ int rtp_render_adaptive(rtp_scene* scene, const rtp_camera* camera, const rtp_re
     if (int rc = check_adaptive(params, adaptive)) return rc;
     const size_t npx = static_cast<size_t>(params->width) * params->height;
     if (npx == 0) return set_error(RTP_ERR_INVALID, "bad frame parameters");
-    std::vector<AdaptiveDev> devs;
-    for (DeviceScene* ds : scene->devs)
-        if (params->device_mask == 0 || ((params->device_mask >> ds->device) & 1u)) { devs.emplace_back(); devs.back().ds = ds; devs.back().st = ds->streams[0]; }
-    if (devs.empty()) return set_error(RTP_ERR_INVALID, "device_mask names no device of this scene");
-    const uint32_t N = static_cast<uint32_t>(devs.size());
-    const uint32_t rs0 = params->row_stride ? params->row_stride : 1u, ro0 = params->row_offset;
-    const uint32_t W = params->width, tx = params->tile_x, ty = params->tile_y;
-    const uint32_t tw = params->tile_w ? params->tile_w : W - tx, th_full = params->tile_h ? params->tile_h : params->height - ty;
-    std::vector<std::unique_lock<std::mutex>> locks;
-    for (AdaptiveDev& d : devs) locks.emplace_back(d.ds->lock);
+    std::vector<FrameDev> frame;
+    if (int rc = deal_rows(scene, params, &frame)) return rc;
+    std::vector<AdaptiveDev> devs(frame.size());
     int rc = RTP_OK;
-    for (uint32_t k = 0; k < N && rc == RTP_OK; ++k) {
+    for (size_t k = 0; k < frame.size() && rc == RTP_OK; ++k) {
         AdaptiveDev& d = devs[k];
-        DeviceScene* ds = d.ds;
-        RTP_CUDA(cudaSetDevice(ds->device));
-        d.p = *params;
-        d.p.row_offset = ro0 + k * rs0;  // rows ro0 + m * rs0 of the caller's split; device k takes m = k, k + N, ...
-        d.p.row_stride = rs0 * N;
-        if (ds->frame_elems < npx * 4) {
-            ds->frame_elems = 0;
-            if ((rc = grow(&ds->frame, npx * 4)) != RTP_OK) break;
-            ds->frame_elems = npx * 4;
-        }
-        if (samples_out && ds->frame_samples_elems < npx) {
-            ds->frame_samples_elems = 0;
-            if ((rc = grow(&ds->frame_samples, npx)) != RTP_OK) break;
-            ds->frame_samples_elems = npx;
-        }
-        d.d_rgb = ds->frame;
-        d.d_fg = foreground_out ? ds->frame + npx * 3 : nullptr;
-        d.d_samples = samples_out ? ds->frame_samples : nullptr;
+        DeviceScene* ds = frame[k].ds;
+        if (cudaSetDevice(ds->device) != cudaSuccess) { rc = set_error(RTP_ERR_CUDA, "cudaSetDevice"); break; }
+        rc = ds->frame.reserve(npx * 4);
+        if (rc == RTP_OK && samples_out) rc = ds->frame_samples.reserve(npx);
+        d.ds = ds; d.st = ds->streams[0]; d.p = &frame[k].p;
+        d.d_rgb = ds->frame.ptr;
+        d.d_fg = foreground_out ? ds->frame.ptr + npx * 3 : nullptr;
+        d.d_samples = samples_out ? ds->frame_samples.ptr : nullptr;
     }
     if (rc == RTP_OK) rc = render_adaptive(devs, camera, adaptive, stats != nullptr);
-    for (uint32_t k = 0; k < N && rc == RTP_OK; ++k) {  // only the rows this device rendered travel back
-        AdaptiveDev& d = devs[k];
-        if (d.p.row_offset >= th_full || tx >= W) continue;
+    for (size_t k = 0; k < devs.size() && rc == RTP_OK; ++k) {
+        const AdaptiveDev& d = devs[k];
         cudaSetDevice(d.ds->device);
-        const uint32_t rows = (th_full - d.p.row_offset + d.p.row_stride - 1u) / d.p.row_stride;
-        const size_t first = static_cast<size_t>(tx) + static_cast<size_t>(ty + d.p.row_offset) * W;
-        const size_t row_px = static_cast<size_t>(W) * d.p.row_stride;
-        cudaError_t e = cudaMemcpy2DAsync(rgb_out + 3 * first, row_px * 24, d.d_rgb + 3 * first, row_px * 24, static_cast<size_t>(tw) * 24, rows, cudaMemcpyDeviceToHost, d.st);
-        if (e == cudaSuccess && foreground_out)
-            e = cudaMemcpy2DAsync(foreground_out + first, row_px * 8, d.d_fg + first, row_px * 8, static_cast<size_t>(tw) * 8, rows, cudaMemcpyDeviceToHost, d.st);
-        if (e == cudaSuccess && samples_out)
-            e = cudaMemcpy2DAsync(samples_out + first, row_px * 4, d.d_samples + first, row_px * 4, static_cast<size_t>(tw) * 4, rows, cudaMemcpyDeviceToHost, d.st);
-        if (e != cudaSuccess) rc = set_error(RTP_ERR_CUDA, std::string("adaptive frame copy: ") + cudaGetErrorString(e));
+        rc = copy_rows(*d.p, d.st, {{rgb_out, d.d_rgb, 24}, {foreground_out, d.d_fg, 8}, {samples_out, d.d_samples, 4}});
     }
-    rc = adaptive_finish(devs, rc, stats);
-    cudaSetDevice(scene->dev->device);
-    return rc;
+    return finish_frame(scene, frame, rc, stats, nullptr);
 }
 
 int rtp_render_adaptive_device(rtp_scene* scene, const rtp_camera* camera, const rtp_render_params* params, const rtp_adaptive_params* adaptive,
@@ -3604,10 +3568,13 @@ int rtp_render_adaptive_device(rtp_scene* scene, const rtp_camera* camera, const
     std::lock_guard<std::mutex> guard(d.ds->lock);
     RTP_CUDA(cudaSetDevice(d.ds->device));
     d.st = static_cast<cudaStream_t>(cuda_stream);
-    d.p = *params;
+    d.p = params;
     d.d_rgb = d_rgb_out; d.d_fg = d_foreground_out; d.d_samples = d_samples_out;
-    const int rc = render_adaptive(devs, camera, adaptive, stats != nullptr);
-    return adaptive_finish(devs, rc, stats);
+    int rc = render_adaptive(devs, camera, adaptive, stats != nullptr);
+    const cudaError_t e = cudaStreamSynchronize(d.st);
+    if (e != cudaSuccess && rc == RTP_OK) rc = set_error(RTP_ERR_CUDA, std::string("adaptive render: ") + cudaGetErrorString(e));
+    if (rc == RTP_OK && stats) rc = render_finish(d.ds, stats);
+    return rc;
 }
 
 }  // extern "C"
