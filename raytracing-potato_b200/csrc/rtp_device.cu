@@ -663,6 +663,15 @@ __device__ __forceinline__ void camera_shoot(const DCamera& cam, double u, doubl
            ((m[2] * origin.x + m[5] * origin.y) + m[8] * origin.z) + cam.pos[2]);
 }
 
+// a ray from o along d with the reference's interval [kRayEpsilon, inf) (render.rs:104)
+__device__ __forceinline__ void store_ray(rtp_ray* r, D3 o, D3 d) {
+    double2* out = reinterpret_cast<double2*>(r);
+    out[0] = make_double2(o.x, o.y);
+    out[1] = make_double2(o.z, d.x);
+    out[2] = make_double2(d.y, d.z);
+    out[3] = make_double2(kRayEpsilon, CUDART_INF);
+}
+
 // writes the rays of pixels [first, first + count) (i fastest) to rays[0 .. count)
 __global__ void __launch_bounds__(256) camera_rays_kernel(DCamera cam, uint32_t width, uint32_t height, rtp_ray* __restrict__ rays_out, size_t first, size_t count) {
     const size_t q = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
@@ -674,11 +683,7 @@ __global__ void __launch_bounds__(256) camera_rays_kernel(DCamera cam, uint32_t 
     const double v = (static_cast<double>(j) + 0.5) / static_cast<double>(height);
     D3 o, d;
     camera_shoot(cam, u, v, 0.0, 0.0, o, d);
-    double2* out = reinterpret_cast<double2*>(rays + p);
-    out[0] = make_double2(o.x, o.y);
-    out[1] = make_double2(o.z, d.x);
-    out[2] = make_double2(d.y, d.z);
-    out[3] = make_double2(kRayEpsilon, CUDART_INF);
+    store_ray(rays + p, o, d);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -913,17 +918,21 @@ struct AovRecords {  // rtp_render_aov
 };
 
 // path p of a launch = (pixel slot p / n_samples, sample p % n_samples): the samples of one pixel sit in adjacent lanes,
-// so a warp's primary rays are as coherent as they can be
+// so a warp's primary rays are as coherent as they can be. Returns the path's random stream at its first draw; (i, j) is its
+// frame pixel.
 template <class Map>
-__device__ __forceinline__ void path_coords(const DRender& rp, const Map& map, size_t p, uint32_t& i, uint32_t& j, uint32_t& smp) {
+__device__ __forceinline__ Rng path_rng(const DRender& rp, const Map& map, size_t p, uint32_t& i, uint32_t& j) {
     // a launch holds at most 32 Mi paths (render_enqueue): 32-bit divisions (the 64-bit ones were 3.6 % of the shade kernel)
     const uint32_t p32 = static_cast<uint32_t>(p);
     const uint32_t k = p32 / rp.n_samples;
-    smp = rp.sample_begin + (p32 - k * rp.n_samples);
+    const uint32_t smp = rp.sample_begin + (p32 - k * rp.n_samples);
     const uint32_t pix = map.pixel(k);
     const uint32_t row = pix / rp.tile_w;
     i = rp.tile_x + (pix - row * rp.tile_w);
     j = rp.tile_y + rp.row_offset + row * rp.row_stride;
+    Rng rng;
+    rng_init(rng, rp.seed, j * rp.width + i, smp, RTP_RNG_STREAM_PATH);
+    return rng;
 }
 
 // main.rs:70-76: jittered uv (render.rs:76-81), lens sample (render.rs:36, drawn even when lens_radius == 0), Camera::shoot
@@ -1019,10 +1028,8 @@ __global__ void __launch_bounds__(128) render_paths_kernel(DSceneView sc, DCamer
     const size_t p = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
     LocalCounters lc = {0, 0, 0, 0, 0, 0, 0};
     if (p < total) {
-        uint32_t i, j, smp;
-        path_coords(rp, map, p, i, j, smp);
-        Rng rng;
-        rng_init(rng, rp.seed, j * rp.width + i, smp, RTP_RNG_STREAM_PATH);
+        uint32_t i, j;
+        Rng rng = path_rng(rp, map, p, i, j);
         D3 o, d;
         primary_ray(cam, rp, i, j, rng, o, d);
 
@@ -1070,13 +1077,27 @@ __global__ void __launch_bounds__(128) render_paths_kernel(DSceneView sc, DCamer
 // in a [bounce][path] stack, read back once when the path ends.
 // ---------------------------------------------------------------------------------------------
 
+constexpr uint32_t kMaxBounce = 128;  // deepest max_bounce a render call takes
+
 struct WaveQueues {
+    static constexpr size_t kLevel = 3;  // double2 per path and level of `stack`
     rtp_ray* rays[2];
-    uint4* state[2];             // x = path index, y = next RNG draw, z = depth_left | nb << 8 | first_hit << 16
+    uint4* state[2];             // PathState::pack()
     WaveHit* hits;
     double2* stack;              // [bounce][path][3] double2: (emit.x, emit.y) (emit.z, absorb.x) (absorb.y, absorb.z)
     unsigned long long* count;   // [max_bounce + 1]
     size_t capacity;             // paths per launch the buffers were sized for (stride of `stack`)
+    // path p's entry at level b of `stack`
+    __device__ __forceinline__ double2* level(size_t b, size_t p) const { return stack + (b * capacity + p) * kLevel; }
+};
+
+// A path between two vertices, as its 16-byte queue record holds it: x = path index, y = next RNG draw,
+// z = depth left | stack height << 8 | first-hit flag << 16
+struct PathState {
+    size_t p;  // 64-bit: held as 32 bits, it costs tail mode 48 B more of spill stores (ptxas, CUDA 12.9)
+    uint32_t k, depth, nb, first_hit;
+    __device__ __forceinline__ static PathState unpack(uint4 s) { return {s.x, s.y, s.z & 0xFFu, (s.z >> 8) & 0xFFu, (s.z >> 16) & 1u}; }
+    __device__ __forceinline__ uint4 pack() const { return make_uint4(static_cast<uint32_t>(p), k, depth | (nb << 8) | (first_hit << 16), 0u); }
 };
 
 template <class Map>
@@ -1084,18 +1105,54 @@ __global__ void __launch_bounds__(256) wave_generate_kernel(DCamera cam, DRender
     const size_t p = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
     if (p == 0) wq.count[0] = total;
     if (p >= total) return;
-    uint32_t i, j, smp;
-    path_coords(rp, map, p, i, j, smp);
-    Rng rng;
-    rng_init(rng, rp.seed, j * rp.width + i, smp, RTP_RNG_STREAM_PATH);
+    uint32_t i, j;
+    Rng rng = path_rng(rp, map, p, i, j);
     D3 o, d;
     primary_ray(cam, rp, i, j, rng, o, d);
-    double2* out = reinterpret_cast<double2*>(wq.rays[0] + p);
-    out[0] = make_double2(o.x, o.y);
-    out[1] = make_double2(o.z, d.x);
-    out[2] = make_double2(d.y, d.z);
-    out[3] = make_double2(kRayEpsilon, CUDART_INF);
-    wq.state[0][p] = make_uint4(static_cast<uint32_t>(p), rng.k, rp.max_bounce, 0u);
+    store_ray(wq.rays[0] + p, o, d);
+    wq.state[0][p] = PathState{p, rng.k, rp.max_bounce, 0u, 0u}.pack();
+}
+
+// One vertex of a wavefront path (render.rs:102-131): the path's segment (o, d) missed (`miss`) or ended at h. `first`: the
+// path's first segment, whose hit sets the foreground flag and, with fv != nullptr, records the vertex in *fv. A miss or a vertex
+// that does not scatter ends the path with radiance L. A scattering vertex pushes (emit, absorb) onto the stack, leaves the
+// scattered ray in (o, d) and spends one level of depth; at depth 0 the continuation returns black without tracing
+// (render.rs:128-131), so L, black on entry, stays black. Returns whether the path lives on.
+template <class Map>
+__device__ __forceinline__ bool path_vertex(const DSceneView& sc, const DRender& rp, const Map& map, const WaveQueues& wq, PathState& s, bool first,
+                                            bool miss, const HitRec& h, D3& o, D3& d, D3& L, FirstVertex* fv) {
+    if (miss) {
+        L = shade_miss(sc, d);
+        return false;
+    }
+    if (first) s.first_hit = 1u;
+    uint32_t i, j;
+    Rng rng = path_rng(rp, map, s.p, i, j);
+    rng.k = s.k;
+    D3 emit, absorb;
+    if (!shade_vertex(sc, o, d, h, rng, emit, absorb, first ? fv : nullptr)) {  // render.rs:108-110: emit + rgb(0,0,0)
+        L = emit + mk(0.0, 0.0, 0.0);
+        return false;
+    }
+    double2* sp = wq.level(s.nb, s.p);
+    sp[0] = make_double2(emit.x, emit.y);
+    sp[1] = make_double2(emit.z, absorb.x);
+    sp[2] = make_double2(absorb.y, absorb.z);
+    ++s.nb;
+    s.depth -= 1;
+    s.k = rng.k;
+    return s.depth != 0;
+}
+
+// The end of a wavefront path whose last vertex left radiance L: render.rs:108-115 / 135-142, emit + absorb ⊙ (inner) folded
+// inside-out like the recursion, into scratch[p] with the foreground flag
+__device__ __forceinline__ void path_end(const WaveQueues& wq, const PathState& s, D3 L, double4* scratch) {
+    for (int b = static_cast<int>(s.nb) - 1; b >= 0; --b) {
+        const double2* sp = wq.level(b, s.p);
+        const double2 s0 = sp[0], s1 = sp[1], s2 = sp[2];
+        L = mk(s0.x, s0.y, s1.x) + cmul(mk(s1.y, s2.x, s2.y), L);
+    }
+    scratch[s.p] = make_double4(L.x, L.y, L.z, s.first_hit ? 1.0 : 0.0);
 }
 
 // A ray trace_any_kernel did not answer inside the wavefront integrator (not eligible for the f32 walk, stack overflow, abnormal leaf in
@@ -1115,6 +1172,7 @@ __global__ void __launch_bounds__(256, kShadeBlocks) wave_shade_kernel(DSceneVie
                                                                        Map map, Aov aov) {
     const size_t n = static_cast<size_t>(wq.count[bounce]);
     const int cur = bounce & 1, nxt = cur ^ 1;
+    const bool first = bounce == 0;
     const unsigned lane = threadIdx.x & 31u;
     const size_t stride = static_cast<size_t>(gridDim.x) * blockDim.x;
     // warp-uniform trip count: every lane of a warp takes part in the compaction ballot
@@ -1127,12 +1185,10 @@ __global__ void __launch_bounds__(256, kShadeBlocks) wave_shade_kernel(DSceneVie
             const double2* rp2 = reinterpret_cast<const double2*>(wq.rays[cur] + q);
             const double2 r0 = rp2[0], r1 = rp2[1], r2 = rp2[2];
             o = mk(r0.x, r0.y, r1.x); d = mk(r1.y, r2.x, r2.y);
-            st = wq.state[cur][q];
+            PathState s = PathState::unpack(wq.state[cur][q]);
             const double2* hp = reinterpret_cast<const double2*>(wq.hits + q);
             const double2 h0 = hp[0], h1 = hp[1];
             uint32_t slotkind = static_cast<uint32_t>(__double2loint(h1.y));
-            uint32_t depth = st.z & 0xFFu, nb = (st.z >> 8) & 0xFFu, first_hit = (st.z >> 16) & 1u;
-            const size_t p = st.x;
             D3 L = mk(0.0, 0.0, 0.0);
             FirstVertex fv = {mk(0.0, 0.0, 0.0), mk(0.0, 0.0, 0.0)};
             HitRec h;
@@ -1141,41 +1197,10 @@ __global__ void __launch_bounds__(256, kShadeBlocks) wave_shade_kernel(DSceneVie
                 trace_deferred(sc, o, d, h);
                 slotkind = h.slot == kNoPrim ? kNoPrim : 0u;
             }
-            if (slotkind == kNoPrim) {
-                L = shade_miss(sc, d);
-            } else {
-                if (bounce == 0) first_hit = 1u;
-                uint32_t i, j, smp;
-                path_coords(rp, map, p, i, j, smp);
-                Rng rng;
-                rng_init(rng, rp.seed, j * rp.width + i, smp, RTP_RNG_STREAM_PATH);
-                rng.k = st.y;
-                D3 emit, absorb;
-                if (!shade_vertex(sc, o, d, h, rng, emit, absorb, Aov::kOn && bounce == 0 ? &fv : nullptr)) {  // render.rs:108-110: emit + rgb(0,0,0)
-                    L = emit + mk(0.0, 0.0, 0.0);
-                } else {
-                    double2* sp = wq.stack + (static_cast<size_t>(nb) * wq.capacity + p) * 3;
-                    sp[0] = make_double2(emit.x, emit.y);
-                    sp[1] = make_double2(emit.z, absorb.x);
-                    sp[2] = make_double2(absorb.y, absorb.z);
-                    ++nb;
-                    depth -= 1;
-                    st.y = rng.k;
-                    if (depth == 0) L = mk(0.0, 0.0, 0.0);  // render.rs:128-131: the continuation returns black without tracing
-                    else alive = true;
-                }
-            }
-            if (!alive) {
-                // render.rs:108-115 / 135-142: emit + absorb ⊙ (inner), folded inside-out like the recursion
-                for (int b = static_cast<int>(nb) - 1; b >= 0; --b) {
-                    const double2* sp = wq.stack + (static_cast<size_t>(b) * wq.capacity + p) * 3;
-                    const double2 s0 = sp[0], s1 = sp[1], s2 = sp[2];
-                    L = mk(s0.x, s0.y, s1.x) + cmul(mk(s1.y, s2.x, s2.y), L);
-                }
-                scratch[p] = make_double4(L.x, L.y, L.z, first_hit ? 1.0 : 0.0);
-            }
-            if (Aov::kOn && bounce == 0) aov.record(p, fv);
-            st.z = depth | (nb << 8) | (first_hit << 16);
+            alive = path_vertex(sc, rp, map, wq, s, first, slotkind == kNoPrim, h, o, d, L, Aov::kOn ? &fv : nullptr);
+            if (!alive) path_end(wq, s, L, scratch);
+            if (Aov::kOn && first) aov.record(s.p, fv);
+            st = s.pack();
         }
         // compaction: survivors of this warp take consecutive slots of the next queue
         const unsigned live = __ballot_sync(0xffffffffu, alive);
@@ -1186,11 +1211,7 @@ __global__ void __launch_bounds__(256, kShadeBlocks) wave_shade_kernel(DSceneVie
             base = __shfl_sync(0xffffffffu, base, leader);
             if (alive) {
                 const size_t dst = static_cast<size_t>(base) + __popc(live & ((1u << lane) - 1u));
-                double2* out = reinterpret_cast<double2*>(wq.rays[nxt] + dst);
-                out[0] = make_double2(o.x, o.y);
-                out[1] = make_double2(o.z, d.x);
-                out[2] = make_double2(d.y, d.z);
-                out[3] = make_double2(kRayEpsilon, CUDART_INF);
+                store_ray(wq.rays[nxt] + dst, o, d);
                 wq.state[nxt][dst] = st;
             }
         }
@@ -1202,15 +1223,14 @@ __global__ void __launch_bounds__(256, kShadeBlocks) wave_shade_kernel(DSceneVie
 // ---------------------------------------------------------------------------------------------
 
 // Tail mode (OUT_TAIL) of the wavefront integrator: when a launch holds at most RTP_TAIL_THRESHOLD paths, one launch
-// carries every surviving path to its end. A lane whose ray is finished shades it in place (shade_vertex) and, if the
-// path scattered, restarts its walker on the scattered ray, so the remaining bounces cost one kernel instead of two
+// after generate carries every path of queue 0 to its end. A lane whose ray is finished shades it in place (path_vertex)
+// and, if the path scattered, restarts its walker on the scattered ray, so the bounces cost one kernel instead of two
 // launches each, and the culling tree stays warm in L1 across them. Results are the same bits: per path the
-// sequence ray -> closest hit -> shade_vertex is the one the trace/shade kernels perform.
+// sequence ray -> closest hit -> path_vertex is the one the trace/shade kernels perform.
 struct TailArgs {
     WaveQueues q;
     DRender rp;
     double4* scratch;
-    uint32_t bounce;
 };
 
 constexpr int kTraceBlocksPerSM = 6;
@@ -1234,10 +1254,6 @@ __global__ void __launch_bounds__(128, OUT == OUT_TAIL ? 4 : kTraceBlocksPerSM) 
         // list is empty already, so there is nothing to reset; every warp reads the same final count, so every warp leaves. Two
         // same-address atomics per warp of this grid (queue claim, drain count) would otherwise delay the next launch.
         if (n == 0) return;
-    }
-    if (OUT == OUT_TAIL) {
-        if (n == 0) return;
-        rays = ta.q.rays[ta.bounce & 1u];
     }
     uint4 pst = make_uint4(0, 0, 0, 0);  // tail mode: the path state of the lane's ray (WaveQueues::state)
     const unsigned lane = threadIdx.x & 31u;
@@ -1275,45 +1291,17 @@ __global__ void __launch_bounds__(128, OUT == OUT_TAIL ? 4 : kTraceBlocksPerSM) 
             const unsigned finished = __ballot_sync(0xffffffffu, fin);
             if (finished != 0u && (__popc(finished) >= kPrimBatch || __ballot_sync(0xffffffffu, !is_done) == 0u)) {
                 if (fin) {
-                    uint32_t depth = pst.z & 0xFFu, nb = (pst.z >> 8) & 0xFFu, first_hit = (pst.z >> 16) & 1u;
-                    const size_t p = pst.x;
-                    bool alive = false;
+                    PathState s = PathState::unpack(pst);
                     D3 L = mk(0.0, 0.0, 0.0), o = w.o, d = w.d;
-                    if (w.h.slot == kNoPrim) {
-                        L = shade_miss(sc, d);
-                    } else {
-                        if (depth == ta.rp.max_bounce) first_hit = 1u;  // the path's first segment (render.rs:102-122)
-                        uint32_t pi, pj, smp;
-                        path_coords(ta.rp, DenseTile{}, p, pi, pj, smp);  // tail mode serves rtp_render only
-                        Rng rng;
-                        rng_init(rng, ta.rp.seed, pj * ta.rp.width + pi, smp, RTP_RNG_STREAM_PATH);
-                        rng.k = pst.y;
-                        D3 emit, absorb;
-                        if (!shade_vertex(sc, o, d, w.h, rng, emit, absorb)) {
-                            L = emit + mk(0.0, 0.0, 0.0);
-                        } else {
-                            double2* sp = ta.q.stack + (static_cast<size_t>(nb) * ta.q.capacity + p) * 3;
-                            sp[0] = make_double2(emit.x, emit.y);
-                            sp[1] = make_double2(emit.z, absorb.x);
-                            sp[2] = make_double2(absorb.y, absorb.z);
-                            ++nb;
-                            depth -= 1;
-                            pst.y = rng.k;
-                            if (depth != 0) alive = true;  // render.rs:128-131 otherwise
-                        }
-                    }
-                    pst.z = depth | (nb << 8) | (first_hit << 16);
+                    // a path at full depth is on its first segment; tail mode serves rtp_render only: dense slots, no first vertex
+                    const bool alive = path_vertex(sc, ta.rp, DenseTile{}, ta.q, s, s.depth == ta.rp.max_bounce, w.h.slot == kNoPrim, w.h, o, d, L, nullptr);
+                    pst = s.pack();
                     if (alive) {
                         walker_start(w, sc, o, d, kRayEpsilon, CUDART_INF);
                         if (LIST) { w.m32 = false; if (sc.n_prims == 0) w.next = kEnd; }
                         lc.rays++;
                     } else {
-                        for (int b = static_cast<int>(nb) - 1; b >= 0; --b) {
-                            const double2* sp = ta.q.stack + (static_cast<size_t>(b) * ta.q.capacity + p) * 3;
-                            const double2 s0 = sp[0], s1 = sp[1], s2 = sp[2];
-                            L = mk(s0.x, s0.y, s1.x) + cmul(mk(s1.y, s2.x, s2.y), L);
-                        }
-                        ta.scratch[p] = make_double4(L.x, L.y, L.z, first_hit ? 1.0 : 0.0);
+                        path_end(ta.q, s, L, ta.scratch);
                         idx = kNoRay;
                     }
                 }
@@ -1343,7 +1331,7 @@ __global__ void __launch_bounds__(128, OUT == OUT_TAIL ? 4 : kTraceBlocksPerSM) 
                     const double2 r0 = __ldg(rp), r1 = __ldg(rp + 1), r2 = __ldg(rp + 2), r3 = __ldg(rp + 3);
                     walker_start(w, sc, mk(r0.x, r0.y, r1.x), mk(r1.y, r2.x, r2.y), r3.x, r3.y);
                     if (LIST) { w.m32 = false; if (sc.n_prims == 0) w.next = kEnd; }
-                    if (OUT == OUT_TAIL) pst = ta.q.state[ta.bounce & 1u][i];
+                    if (OUT == OUT_TAIL) pst = ta.q.state[0][i];
                     lc.rays++;
                 }
             }
@@ -1399,8 +1387,7 @@ __global__ void __launch_bounds__(128, OUT == OUT_TAIL ? 4 : kTraceBlocksPerSM) 
         if (atomicAdd(&wq->done_blocks, 1u) == static_cast<unsigned>(n_warps) - 1u) {
             wq->next = 0ull;
             wq->done_blocks = 0u;
-            if (OUT == OUT_TAIL) ta.q.count[ta.bounce] = 0ull;  // every path is finished: the launches that follow find empty queues
-            if (index.idx) *index.count = 0ull;                 // the deferred rays are done: rearm the list for the next launch
+            if (index.idx) *index.count = 0ull;  // the deferred rays are done: rearm the list for the next launch
             __threadfence();
         }
     }
@@ -1823,7 +1810,7 @@ __global__ void __launch_bounds__(256) resolve_kernel(const double4* __restrict_
     if (pix >= npix) return;
     double4 a = first_launch ? make_double4(0.0, 0.0, 0.0, 0.0) : acc[pix];
     for (uint32_t s = 0; s < n_samples; ++s) {
-        const double4 c = scratch[pix * n_samples + s];  // path_coords: the samples of a pixel are adjacent
+        const double4 c = scratch[pix * n_samples + s];  // path_rng: the samples of a pixel are adjacent
         a.x += c.x; a.y += c.y; a.z += c.z; a.w += c.w;
     }
     acc[pix] = a;
@@ -1857,7 +1844,7 @@ __global__ void __launch_bounds__(256) aov_resolve_kernel(const double2* __restr
     double2 a0 = make_double2(0.0, 0.0), a1 = a0, a2 = a0;
     if (!first_launch) { a0 = acc[3 * pix]; a1 = acc[3 * pix + 1]; a2 = acc[3 * pix + 2]; }
     for (uint32_t s = 0; s < n_samples; ++s) {
-        const double2* r = rec + 3 * (pix * n_samples + s);  // path_coords: the samples of a pixel are adjacent
+        const double2* r = rec + 3 * (pix * n_samples + s);  // path_rng: the samples of a pixel are adjacent
         const double2 r0 = r[0], r1 = r[1], r2 = r[2];
         a0.x += r0.x; a0.y += r0.y; a1.x += r1.x; a1.y += r1.y; a2.x += r2.x; a2.y += r2.y;
     }
@@ -1900,7 +1887,7 @@ __global__ void __launch_bounds__(256) adaptive_init_kernel(double4* __restrict_
     live[pix] = static_cast<uint32_t>(pix);
 }
 
-// One launch of a round: for live slot k, the launch's samples of tile pixel live[k] (scratch[k * n_samples + s], path_coords)
+// One launch of a round: for live slot k, the launch's samples of tile pixel live[k] (scratch[k * n_samples + s], path_rng)
 // are folded into its sums in sample order. On the round's last launch the stop rule decides keep[k].
 __global__ void __launch_bounds__(256) adaptive_resolve_kernel(const double4* __restrict__ scratch, const uint32_t* __restrict__ live, uint32_t n_live,
                                                                uint32_t n_samples, double4* __restrict__ acc, double2* __restrict__ moments,
@@ -2006,10 +1993,11 @@ struct DevBuf {
     DevBuf(const DevBuf&) = delete;
     DevBuf& operator=(const DevBuf&) = delete;
     ~DevBuf() { cudaFree(ptr); }
+    void release() { cudaFree(ptr); ptr = nullptr; n = 0; }
     // room for `want` elements; the contents do not survive a reallocation, and a failed one leaves the buffer empty
     int reserve(size_t want) {
         if (n >= want) return RTP_OK;
-        cudaFree(ptr); ptr = nullptr; n = 0;
+        release();
         const size_t m = std::max<size_t>(want, 1);
         RTP_CUDA(cudaMalloc(reinterpret_cast<void**>(&ptr), m * sizeof(T)));
         n = m;
@@ -2044,8 +2032,7 @@ struct DeviceScene {
     struct LaunchSlot {
         WorkQueue* wq = nullptr;
         unsigned long long* defer_count = nullptr;
-        uint32_t* defer_idx = nullptr;
-        size_t defer_cap = 0;
+        DevBuf<uint32_t> defer_idx;
         cudaEvent_t last_use = nullptr;
         cudaStream_t stream = nullptr;  // stream of the last launch that used the slot
         bool used = false;
@@ -2079,8 +2066,15 @@ struct DeviceScene {
     DevBuf<uint32_t> n_live; uint32_t* n_live_host = nullptr;
     // rtp_render_aov: the AovRecords of a launch (3 double2 per path, grown like scratch) and their sums (3 double2 per tile pixel)
     DevBuf<double2> aov_rec, aov_acc;
-    WaveQueues wave{};                // wavefront integrator queues (render_device), grown on demand
-    uint32_t wave_bounces = 0;         // stack depth the queues were sized for
+    // wavefront integrator queues (WaveQueues), grown on demand by wave_reserve for wave_capacity paths per launch and a stack of
+    // wave_bounces levels
+    DevBuf<rtp_ray> wave_rays[2];
+    DevBuf<uint4> wave_state[2];
+    DevBuf<WaveHit> wave_hits;
+    DevBuf<double2> wave_stack;
+    DevBuf<unsigned long long> wave_count;
+    size_t wave_capacity = 0;
+    uint32_t wave_bounces = 0;
     int shade_blocks = 0;              // grid of wave_shade_kernel
     // memory the integrator's per-launch buffers may take (set at upload from the free HBM). A render call sizes its launches
     // against it with its own max_bounce, and the queues it keeps afterwards hold at most max(this budget, what the call itself
@@ -2109,10 +2103,8 @@ void device_scene_free(DeviceScene* ds) {
     for (uint8_t* p : ds->images) cudaFree(p);
     cudaFree(ds->counters);
     cudaFree(ds->queues);
-    for (DeviceScene::LaunchSlot& sl : ds->slots) {
-        cudaFree(sl.defer_idx);
+    for (DeviceScene::LaunchSlot& sl : ds->slots)
         if (sl.last_use) cudaEventDestroy(sl.last_use);
-    }
     for (int k = 0; k < kPipeDepth; ++k)
         if (ds->streams[k]) cudaStreamDestroy(ds->streams[k]);
     if (ds->ev_begin) cudaEventDestroy(ds->ev_begin);
@@ -2120,8 +2112,6 @@ void device_scene_free(DeviceScene* ds) {
     for (cudaEvent_t ev : ds->ev_pool) cudaEventDestroy(ev);
     if (ds->render_done) cudaEventDestroy(ds->render_done);
     if (ds->n_live_host) cudaFreeHost(ds->n_live_host);
-    cudaFree(ds->wave.rays[0]); cudaFree(ds->wave.rays[1]); cudaFree(ds->wave.state[0]); cudaFree(ds->wave.state[1]);
-    cudaFree(ds->wave.hits); cudaFree(ds->wave.stack); cudaFree(ds->wave.count);
     delete ds;
 }
 
@@ -2361,18 +2351,15 @@ static int launch_trace(DeviceScene* ds, const rtp_ray* d_rays, size_t n, void* 
             RTP_CUDA(cudaStreamWaitEvent(stream, pick->last_use, 0));  // its previous launch, on another stream, must be over
         }
         DeviceScene::LaunchSlot& slot = *pick;
-        if (pure_any && slot.defer_cap < n) {
-            if (slot.used) RTP_CUDA(cudaEventSynchronize(slot.last_use));
-            cudaFree(slot.defer_idx); slot.defer_idx = nullptr; slot.defer_cap = 0;
-            const size_t cap = std::max<size_t>(n, 65536);
-            RTP_CUDA(cudaMalloc(reinterpret_cast<void**>(&slot.defer_idx), cap * sizeof(uint32_t)));
-            slot.defer_cap = cap;
+        if (pure_any && slot.defer_idx.n < n) {
+            if (slot.used) RTP_CUDA(cudaEventSynchronize(slot.last_use));  // its last launch may still read the list
+            if (int rc = slot.defer_idx.reserve(std::max<size_t>(n, 65536))) return rc;
         }
         WorkQueue* wq = slot.wq;
         const DeferList no_index{nullptr, nullptr};
         if (pure_any) {
             const dim3 g(static_cast<unsigned>(std::min<size_t>(static_cast<size_t>(ds->any_blocks), want)));
-            const DeferList defer{slot.defer_idx, slot.defer_count};
+            const DeferList defer{slot.defer_idx.ptr, slot.defer_count};
 #define RTP_LAUNCH_ANY(C, O) trace_any_kernel<C, O><<<g, block, ds->any_stack_bytes, stream>>>(ds->view, d_rays, n, d_out, counters, wq, n_dev, defer)
             if (out_mode == OUT_FULL) { if (count) RTP_LAUNCH_ANY(true, OUT_FULL); else RTP_LAUNCH_ANY(false, OUT_FULL); }
             else if (out_mode == OUT_WAVE) { if (count) RTP_LAUNCH_ANY(true, OUT_WAVE); else RTP_LAUNCH_ANY(false, OUT_WAVE); }
@@ -2535,35 +2522,46 @@ static void launch_render_paths(DeviceScene* ds, const DCamera& cam, const DRend
     else render_paths_kernel<MAXB, false><<<g, block, 0, st>>>(ds->view, cam, rp, ds->scratch.ptr, ds->counters, map, aov);
 }
 
-// bytes per path of one launch of the wavefront integrator: queues (2 rays, 2 states, a hit record: 176 B), the [bounce][path]
-// stack (48 B per level) and the per-path scratch (32 B)
-static size_t wave_path_bytes(uint32_t bounces) { return 176 + 48 * static_cast<size_t>(bounces) + 32; }
+// bytes per path of one launch of the wavefront integrator: what wave_reserve allocates per path (two queue rays and states, a hit
+// record, `bounces` levels of the [bounce][path] stack: 192 B + 48 B per level) and the path's scratch entry (32 B)
+static size_t wave_path_bytes(uint32_t bounces) {
+    return 2 * (sizeof(rtp_ray) + sizeof(uint4)) + sizeof(WaveHit) + WaveQueues::kLevel * sizeof(double2) * bounces + sizeof(double4);
+}
 
-// (re)allocates the wavefront queues for `capacity` paths per launch and a stack of `bounces` levels. The queues grow to cover
-// every shape seen so far, unless that union would cross queue_budget_bytes: then they are sized for this call alone (see
-// DeviceScene::queue_budget_bytes).
+constexpr size_t kWaveCounts = kMaxBounce + 2;  // count[b] for b <= kMaxBounce, and one spare
+
+// Sizes the wavefront queues for `capacity` paths per launch and a stack of `bounces` levels. The queues grow to cover every
+// shape seen so far, unless that union would cross queue_budget_bytes: then they are sized for this call alone (see
+// DeviceScene::queue_budget_bytes), and the larger ones are let go first.
 static int wave_reserve(DeviceScene* ds, size_t capacity, uint32_t bounces) {
-    WaveQueues& w = ds->wave;
-    if (w.capacity >= capacity && ds->wave_bounces >= bounces) return RTP_OK;
-    const size_t grown_cap = std::max(capacity, w.capacity);
+    if (ds->wave_capacity >= capacity && ds->wave_bounces >= bounces) return RTP_OK;
+    const size_t grown_cap = std::max(capacity, ds->wave_capacity);
     const uint32_t grown_bounces = std::max(bounces, ds->wave_bounces);
     if (grown_cap * wave_path_bytes(grown_bounces) <= std::max(ds->queue_budget_bytes, capacity * wave_path_bytes(bounces))) {
         capacity = grown_cap;
         bounces = grown_bounces;
+    } else {
+        for (int k = 0; k < 2; ++k) { ds->wave_rays[k].release(); ds->wave_state[k].release(); }
+        ds->wave_hits.release(); ds->wave_stack.release();
     }
-    cudaFree(w.rays[0]); cudaFree(w.rays[1]); cudaFree(w.state[0]); cudaFree(w.state[1]); cudaFree(w.hits); cudaFree(w.stack); cudaFree(w.count);
-    w = WaveQueues{};
+    ds->wave_capacity = 0;
     ds->wave_bounces = 0;
     for (int k = 0; k < 2; ++k) {
-        RTP_CUDA(cudaMalloc(reinterpret_cast<void**>(&w.rays[k]), capacity * sizeof(rtp_ray)));
-        RTP_CUDA(cudaMalloc(reinterpret_cast<void**>(&w.state[k]), capacity * sizeof(uint4)));
+        if (int rc = ds->wave_rays[k].reserve(capacity)) return rc;
+        if (int rc = ds->wave_state[k].reserve(capacity)) return rc;
     }
-    RTP_CUDA(cudaMalloc(reinterpret_cast<void**>(&w.hits), capacity * sizeof(WaveHit)));
-    RTP_CUDA(cudaMalloc(reinterpret_cast<void**>(&w.stack), capacity * bounces * 3 * sizeof(double2)));
-    RTP_CUDA(cudaMalloc(reinterpret_cast<void**>(&w.count), 130 * sizeof(unsigned long long)));
-    w.capacity = capacity;
+    if (int rc = ds->wave_hits.reserve(capacity)) return rc;
+    if (int rc = ds->wave_stack.reserve(capacity * bounces * WaveQueues::kLevel)) return rc;
+    if (int rc = ds->wave_count.reserve(kWaveCounts)) return rc;
+    ds->wave_capacity = capacity;
     ds->wave_bounces = bounces;
     return RTP_OK;
+}
+
+// the queues as the integrator kernels take them
+static WaveQueues wave_queues(const DeviceScene* ds) {
+    return WaveQueues{{ds->wave_rays[0].ptr, ds->wave_rays[1].ptr}, {ds->wave_state[0].ptr, ds->wave_state[1].ptr}, ds->wave_hits.ptr,
+                      ds->wave_stack.ptr, ds->wave_count.ptr, ds->wave_capacity};
 }
 
 constexpr unsigned int kSrgbFixCap = 1u << 16;
@@ -2587,7 +2585,7 @@ static cudaEvent_t next_mark(DeviceScene* ds, cudaStream_t st) {
 // fixed_spp: rtp_render's sample range is checked too (rtp_render_adaptive checks its own).
 static int render_rect(const rtp_render_params* p, bool fixed_spp, DRender* rp) {
     if (p->max_bounce < 1) return set_error(RTP_ERR_INVALID, "assert!(depth >= 1) (render.rs:97)");
-    if (p->max_bounce > 128) return set_error(RTP_ERR_UNSUPPORTED, "max_bounce > 128");
+    if (p->max_bounce > kMaxBounce) return set_error(RTP_ERR_UNSUPPORTED, "max_bounce > 128");
     if (p->width == 0 || p->height == 0 || (fixed_spp && (p->sample_end < p->sample_begin || p->num_samples == 0)))
         return set_error(RTP_ERR_INVALID, "bad frame parameters");
     if (static_cast<uint64_t>(p->width) * p->height > 0xFFFFFFFFull) return set_error(RTP_ERR_INVALID, "frame too large");
@@ -2632,11 +2630,11 @@ static int render_end(DeviceScene* ds, cudaStream_t st, bool want_stats, size_t 
     return RTP_OK;
 }
 
-// Paths per launch of the integrator for a call with max_bounce `bounces`: up to 32 Mi paths (wavefront queues 176 B + 48 B x
-// max_bounce per path, scratch 32 B), within the memory budget fixed when the scene was uploaded (a sixth of the free HBM, at most
-// 24 GiB). Big launches matter: every launch pays the fill and drain of ~2 x max_bounce kernels and the latency-bound sparse late
-// bounces once (1080p x 64 spp of the C4 scene: 111 ms in 16 launches of 8 Mi paths, 92 ms in 4 launches of 32 Mi). An AOV call
-// (rtp_render_aov) adds its 48-byte AovRecords per path.
+// Paths per launch of the integrator for a call with max_bounce `bounces`: up to 32 Mi paths (wave_path_bytes per path), within
+// the memory budget fixed when the scene was uploaded (a sixth of the free HBM, at most 24 GiB). Big launches matter: every launch
+// pays the fill and drain of ~2 x max_bounce kernels and the latency-bound sparse late bounces once (1080p x 64 spp of the C4
+// scene: 111 ms in 16 launches of 8 Mi paths, 92 ms in 4 launches of 32 Mi). An AOV call (rtp_render_aov) adds its 48-byte
+// AovRecords per path.
 static size_t path_budget(const DeviceScene* ds, uint32_t bounces, bool aov = false) {
     const size_t per_path = (ds->sw.simple_render ? 32 : wave_path_bytes(bounces)) + (aov ? 3 * sizeof(double2) : 0);
     size_t budget = std::max<size_t>(size_t(1) << 20, std::min<size_t>(size_t(32) << 20, ds->queue_budget_bytes / per_path));
@@ -2663,40 +2661,40 @@ static int launch_paths(DeviceScene* ds, const DCamera& cam, const DRender& rp, 
     if (ds->sw.simple_render) {
         if (rp.max_bounce <= 8) launch_render_paths<8>(ds, cam, rp, map, aov, total, count, st);
         else if (rp.max_bounce <= 32) launch_render_paths<32>(ds, cam, rp, map, aov, total, count, st);
-        else launch_render_paths<128>(ds, cam, rp, map, aov, total, count, st);
+        else launch_render_paths<kMaxBounce>(ds, cam, rp, map, aov, total, count, st);
         RTP_CUDA(cudaGetLastError());
         ++*launches;
         return RTP_OK;
     }
     // generate -> (trace -> shade) x max_bounce; queue sizes stay on the device
-    RTP_CUDA(cudaMemsetAsync(ds->wave.count, 0, 130 * sizeof(unsigned long long), st));
-    wave_generate_kernel<<<static_cast<unsigned>((total + 255) / 256), 256, 0, st>>>(cam, rp, ds->wave, total, map);
+    const WaveQueues wq = wave_queues(ds);
+    RTP_CUDA(cudaMemsetAsync(wq.count, 0, kWaveCounts * sizeof(unsigned long long), st));
+    wave_generate_kernel<<<static_cast<unsigned>((total + 255) / 256), 256, 0, st>>>(cam, rp, wq, total, map);
     RTP_CUDA(cudaGetLastError());
     ++*launches;
     { int rc = debug_sync(ds, st, "wave_generate_kernel", 0); if (rc != RTP_OK) return rc; }
+    // a launch of at most tail_threshold paths (a 32x32 tile of main.rs:32, say) runs as generate + ONE tail-mode launch.
+    // Offering every later queue of a big launch to the tail kernel was measured on C1 to be no faster than trace/shade
+    // pairs, and so was handing the sparse late bounces to one tail launch chosen from the previous launch's queue sizes
+    // (19 -> 12 launches per C1 frame, same 2.05 ms): a late bounce costs the latency of ONE ray segment (~30 us of
+    // dependent instructions, tools/small_batches.py), not a launch. Tail mode maps paths to pixels densely and records no
+    // first vertex: rtp_render only.
+    if (std::is_same<Map, DenseTile>::value && !Aov::kOn && ds->sw.tail_threshold && total <= ds->sw.tail_threshold) {
+        if (want_stats) next_mark(ds, st);  // even marks open a traversal span, odd marks close it
+        const TailArgs ta{wq, rp, ds->scratch.ptr};
+        if (int rc = launch_trace(ds, wq.rays[0], total, nullptr, OUT_TAIL, count, ds->counters, st, wq.count, &ta)) return rc;
+        ++*launches;
+        if (want_stats) next_mark(ds, st);
+        return RTP_OK;
+    }
     const unsigned shade_grid = static_cast<unsigned>(std::min<size_t>(static_cast<size_t>(ds->shade_blocks), (total + 255) / 256));
     for (uint32_t b = 0; b < rp.max_bounce; ++b) {
-        int rc;
-        // a launch of at most tail_threshold paths (a 32x32 tile of main.rs:32, say) runs as generate + ONE tail-mode launch.
-        // Offering every later queue of a big launch to the tail kernel was measured on C1 to be no faster than trace/shade
-        // pairs, and so was handing the sparse late bounces to one tail launch chosen from the previous launch's queue sizes
-        // (19 -> 12 launches per C1 frame, same 2.05 ms): a late bounce costs the latency of ONE ray segment (~30 us of
-        // dependent instructions, tools/small_batches.py), not a launch. Tail mode maps paths to pixels densely and records no
-        // first vertex: rtp_render only.
-        if (want_stats) next_mark(ds, st);  // even marks open a traversal span, odd marks close it
-        if (std::is_same<Map, DenseTile>::value && !Aov::kOn && ds->sw.tail_threshold && total <= ds->sw.tail_threshold) {
-            TailArgs ta{ds->wave, rp, ds->scratch.ptr, b};
-            rc = launch_trace(ds, ds->wave.rays[b & 1], total, nullptr, OUT_TAIL, count, ds->counters, st, ds->wave.count + b, &ta);
-            if (rc != RTP_OK) return rc;
-            ++*launches;
-            if (want_stats) next_mark(ds, st);
-            break;
-        }
-        rc = launch_trace(ds, ds->wave.rays[b & 1], total, ds->wave.hits, OUT_WAVE, count, ds->counters, st, ds->wave.count + b);
+        if (want_stats) next_mark(ds, st);
+        int rc = launch_trace(ds, wq.rays[b & 1], total, wq.hits, OUT_WAVE, count, ds->counters, st, wq.count + b);
         if (rc != RTP_OK) return rc;
         if (want_stats) next_mark(ds, st);
         if ((rc = debug_sync(ds, st, "trace kernel <OUT_WAVE>", b)) != RTP_OK) return rc;
-        wave_shade_kernel<<<shade_grid, 256, 0, st>>>(ds->view, rp, ds->wave, b, ds->scratch.ptr, map, aov);
+        wave_shade_kernel<<<shade_grid, 256, 0, st>>>(ds->view, rp, wq, b, ds->scratch.ptr, map, aov);
         RTP_CUDA(cudaGetLastError());
         if ((rc = debug_sync(ds, st, "wave_shade_kernel", b)) != RTP_OK) return rc;
         *launches += ds->last_trace_launches + 1;
